@@ -2,7 +2,7 @@
 """bench.py — trees/sec of Argmax inference on 50-taxa x 1024-site alignments (BASELINE.json metric, configs[1]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch 512] [--scaling strong|weak] [--impl ours|reference]
-                    [--precision bf16x3|fp32] [--workload config2|config4|config1]
+                    [--precision bf16x3|fp32] [--workload config2|config4|config1] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (encode + 49 learned-NJ steps) over a batch of synthetic MSAs
 (config 2: iid tokens over A,C,G,T,gap, seed 1234; weights torch.manual_seed(0) default init — the shipped
@@ -77,6 +77,33 @@ def algorithmic_flops(R, Cc, layers=6):
         "node_derive": R * 3 * 2 * Cc * D * D,
     }
     return fl
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirpath, arrays, world=1, rank=0):
+    """--dump-outputs: the arrays one timed step returned to its caller (first axis = alignment; under several ranks gathered in
+    rank order, i.e. the batch order) as dirpath/<name>.npy in float32 - merge indices are small integers, exact in float32.
+    Above DUMP_LIMIT_BYTES in all, the same rows of every array are kept: a sorted sample drawn with seed 0, so that two builds
+    run with the same arguments write the same alignments."""
+    import numpy as np
+    host = {k: v.cpu().numpy().astype(np.float32) for k, v in arrays.items()}
+    if world > 1:
+        import torch.distributed as dist
+        parts = [None] * world
+        dist.all_gather_object(parts, host)
+        host = {k: np.concatenate([p[k] for p in parts]) for k in host}
+    if rank != 0:
+        return
+    n = next(iter(host.values())).shape[0]
+    keep = min(n, DUMP_LIMIT_BYTES // sum(v[:1].nbytes for v in host.values()))
+    if keep < n:
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        host = {k: v[rows] for k, v in host.items()}
+    os.makedirs(dirpath, exist_ok=True)
+    for k, v in host.items():
+        np.save(os.path.join(dirpath, k + ".npy"), v)
 
 
 ENC_CLASSES = ("embed", "ln_qkv", "out_proj", "row_qk_gemm", "row_softmax", "row_pv_gemm", "col_attn", "ffn")
@@ -322,7 +349,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip latency_b1 / gpu_eager_baseline / the weak-scaling second measurement")
     ap.add_argument("--cpu-trees", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the merge lists and selected log-probabilities of the last timed step "
+                    "as DIR/<name>.npy (float32, at most 64 MB: a fixed seeded sample of alignments beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the device path computed: it needs --impl ours")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -385,12 +418,14 @@ def main():
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         ms_total = float(ms)
         return {"value": n_global * steps / (ms_total / 1e3), "ms_total": ms_total, "launches": launches, "clocks": clocks, "merges": merges,
-                "data_host": data_host, "mask_host": mask_host, "data": data, "mask": mask, "n_global": n_global}
+                "slp": slp, "data_host": data_host, "mask_host": mask_host, "data": data, "mask": mask, "n_global": n_global}
 
     main_run = timed(args.scaling, args.steps, args.warmup, True)
     value, ms_total, launches, clocks, merges = (main_run[k] for k in ("value", "ms_total", "launches", "clocks", "merges"))
     data_host, mask_host, data, mask = (main_run[k] for k in ("data_host", "mask_host", "data", "mask"))
     B_local = data_host.shape[0]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"merges": merges, "selected_log_ps": main_run["slp"]}, world, rank)
 
     # ---- end to end through the host-buffer C-ABI entry point
     model.rollout_host(data_host, mask_host)       # warm

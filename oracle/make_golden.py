@@ -387,8 +387,8 @@ def main_supervise():
 def main_all50(taxa=50, threads=8):
     """The whole of data_gen/data/test/len1024/taxa50 (128 alignments - the set SURVEY.md 8(d) names for configs[1]) through the
     unmodified reference: merge list, Newick, selected_log_ps and per-step max |logit| / top-2 gap of every file, in ONE record
-    (tests/golden/all50/len1024_taxa50.npz) together with the inputs as bit-packed one-hot tokens (25.6 KB per alignment).
-    `all100` does the same for len1024/taxa100 (tests/golden/all100/len1024_taxa100.npz)."""
+    (tests/golden/all50/len1024_taxa50_part*.npz, 64 alignments per part) together with the inputs as bit-packed one-hot tokens
+    (25.6 KB per alignment).  `all100` does the same for len1024/taxa100 (tests/golden/all100/)."""
     torch.set_num_threads(threads)
     import utils as ref_utils
     import finetune_rl_search as ref_main
@@ -446,10 +446,13 @@ def main_all50(taxa=50, threads=8):
         print(f"[{k:3d}] {fn}: reference rollout {dt:.1f}s, min relative top-2 gap {rel:.2e}", flush=True)
     out_dir = os.path.join(GOLD, f"all{taxa}")
     os.makedirs(out_dir, exist_ok=True)
-    np.savez_compressed(os.path.join(out_dir, f"len1024_taxa{taxa}.npz"), shape=np.array([taxa, 1024, 4]), data_bits=np.stack(rec["bits"]),
-                        seq_keys=np.array(rec["keys"]), merges=np.stack(rec["merges"]), newick=np.array(rec["newick"]),
-                        selected_log_ps=np.stack(rec["slp"]), step_max_abs_logit=np.array(rec["lmax"], dtype=np.float32),
-                        step_top2_gap=np.array(rec["gap"], dtype=np.float32), source=np.array(rec["src"]))
+    for p, lo in enumerate(range(0, len(files), 64)):      # parts of 64 alignments keep every file below 1 MB
+        s = slice(lo, lo + 64)
+        np.savez_compressed(os.path.join(out_dir, f"len1024_taxa{taxa}_part{p}.npz"), shape=np.array([taxa, 1024, 4]),
+                            data_bits=np.stack(rec["bits"][s]), seq_keys=np.array(rec["keys"][s]), merges=np.stack(rec["merges"][s]),
+                            newick=np.array(rec["newick"][s]), selected_log_ps=np.stack(rec["slp"][s]),
+                            step_max_abs_logit=np.array(rec["lmax"][s], dtype=np.float32),
+                            step_top2_gap=np.array(rec["gap"][s], dtype=np.float32), source=np.array(rec["src"][s]))
 
 
 if __name__ == "__main__":

@@ -58,6 +58,27 @@ def test_reference_arm_prints_one_contract_line():
     assert d["cpu_baseline"]["value"] == d["value"] and d["cpu_baseline"]["cores"] >= 1
 
 
+def test_dump_outputs_writes_float32_arrays_and_samples_the_same_rows(tmp_path, monkeypatch):
+    """--dump-outputs: every array as <name>.npy in float32; above the size limit the same seeded rows of every array."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    merges = torch.arange(40 * 3 * 2, dtype=torch.int32).view(40, 3, 2)
+    slp = -torch.rand(40, 3)
+    bench.dump_outputs(str(tmp_path / "all"), {"merges": merges, "selected_log_ps": slp})
+    m, s = np.load(tmp_path / "all" / "merges.npy"), np.load(tmp_path / "all" / "selected_log_ps.npy")
+    assert m.dtype == s.dtype == np.float32 and np.array_equal(m, merges.numpy()) and np.array_equal(s, slp.numpy())
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 10 * (6 + 3) * 4)          # room for 10 of the 40 rows
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"merges": merges, "selected_log_ps": slp})
+    m, s = np.load(tmp_path / "a" / "merges.npy"), np.load(tmp_path / "a" / "selected_log_ps.npy")
+    assert m.shape == (10, 3, 2) and s.shape == (10, 3)
+    rows = (m[:, 0, 0] / 6).astype(int)
+    assert list(rows) == sorted(set(rows)) and np.array_equal(s, slp.numpy()[rows])
+    assert np.array_equal(m, np.load(tmp_path / "b" / "merges.npy"))
+
+
 def test_directory_inference_side_measurement_on_the_oracle_stand_in(tmp_path, monkeypatch):
     """bench.py's `directory_inference` extra: synthetic alignments -> PHYLIP files -> `Argmax_inference` per file and stacked.
     The files must read back as the one-hot batch they were written from, and the measurement's bookkeeping is exercised with the

@@ -64,7 +64,14 @@ def test_wide_reference_goldens(name, prec, sd0, gpu_models, parity_report):
     assert env.states[0].subtrees[0].utree_op_str == str(z["newick"][0])
 
 
-ALL50 = os.path.join(GOLD, "all50", "len1024_taxa50.npz")
+ALL50_DIR = os.path.join(GOLD, "all50")
+
+
+def _load_all50():
+    """The 128-file record, stored as parts of 64 alignments (each file stays below 1 MB), concatenated in file order."""
+    parts = [np.load(os.path.join(ALL50_DIR, f), allow_pickle=False)
+             for f in sorted(os.listdir(ALL50_DIR)) if f.startswith("len1024_taxa50_part")]
+    return {k: parts[0][k] if k == "shape" else np.concatenate([p[k] for p in parts]) for k in parts[0].files}
 
 
 @pytest.mark.parametrize("prec", ["fp32", "bf16x3"])
@@ -73,7 +80,8 @@ def test_all_len1024_taxa50_files_match_reference(prec, sd0, gpu_models, parity_
     the unmodified reference (oracle/make_golden.py all50), run here as one batch of 128: merge list and Newick identical per file;
     a file whose own top-2 gap is below the precision's tie tolerance may pass by teacher-forced replay on the oracle instead."""
     from neuralnj_b200 import PhyInferEnv, inference_config
-    z = np.load(ALL50, allow_pickle=False)
+    z = _load_all50()
+    assert z["merges"].shape[0] == 128
     R, L, V = (int(x) for x in z["shape"])
     N = z["data_bits"].shape[0]
     data = torch.from_numpy(np.unpackbits(z["data_bits"], axis=1)[:, :R * L * V].reshape(N, R, L, V).astype(np.int8))
