@@ -187,6 +187,20 @@ int64_t nnj_rank_loss_workspace_bytes(int B, int R);
 int nnj_rank_loss(const float* logits_trace_dev, const uint8_t* in_set_dev, int B, int R, float margin, double ratio,
                   float* out_dev, void* ws_dev, int64_t ws_bytes, void* stream);
 
+/* ---- Bootstrap branch support (RAxML-NG --bootstrap / --support --bs-metric fbp,tbe; DESIGN.md 11).  No model handle or workspace:
+ * both run on the current device, asynchronously on `stream`.
+ * Replicate r of an alignment with l_eff real columns (the prefix; padded columns are the suffix): output column c < l_eff is input
+ * column (x0 * l_eff) >> 32 (64-bit product), x0 = word 0 of Philox4x32-10 with counter (c, r & 0xffffffff, r >> 32, 0) and key
+ * (seed & 0xffffffff, seed >> 32); columns c >= l_eff are copied unchanged.  A replicate depends only on (seed, r, l_eff).
+ * Bootstrap replicates rep0 .. rep0+B-1 of one alignment: data int8 [R,L,4] -> out int8 [B,R,L,4] (both 4-byte aligned). */
+int nnj_bootstrap_columns(const int8_t* data_dev, int R, int L, int l_eff, uint64_t seed, int64_t rep0, int B,
+                          int8_t* out_dev, void* stream);
+/* Transfer distance of S reference splits (leaf bitsets uint64 [S, ceil(R/64)], either side; bit t of word t/64 = taxon t) to each of
+ * B NJ trees (merges int32 [B,R-1,2], the slot rule of nnj_rollout): dist int32 [B,S],
+ *   dist = min(p-1, min over the tree's R-2 non-root clades c of min(|A ^ c|, R - |A ^ c|)),  p = size of the split's lighter side;
+ * a row of -1 = that merge list is not valid (an entry (i, j) of step t that is not 0 <= i < j < R-t).  4 <= R <= 512, S >= 0. */
+int nnj_split_distances(const int32_t* merges_dev, int B, int R, const uint64_t* splits_dev, int S, int32_t* dist_dev, void* stream);
+
 /* Building block of the tensor-core path (precision NNJ_PREC_BF16X3), exposed for unit tests and reuse:
  * C[z] = A[z] * B[z]^T with fp32 A [Z,M,K], B [Z,N,K], C [Z,M,N]; operands are split into bf16 hi/lo planes and
  * multiplied on tcgen05 as hi*hi + hi*lo + lo*hi with fp32 accumulation in TMEM.  K must be a multiple of 8;

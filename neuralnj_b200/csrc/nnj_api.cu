@@ -463,6 +463,17 @@ int nnj_rank_loss(const float* logits_trace, const uint8_t* in_set, int B, int R
     return run_rank_loss(logits_trace, in_set, B, R, margin, ratio, out, ws, (size_t)ws_bytes, (cudaStream_t)stream);
 }
 
+int nnj_bootstrap_columns(const int8_t* data, int R, int L, int l_eff, uint64_t seed, int64_t rep0, int B, int8_t* out, void* stream) {
+    CHECK_ARGS(data && out && R >= 1 && L >= 1 && l_eff >= 1 && l_eff <= L && B >= 1 && rep0 >= 0 && rep0 <= INT64_MAX - B &&
+               ((uintptr_t)data & 3) == 0 && ((uintptr_t)out & 3) == 0, "bootstrap_columns: bad arguments");
+    return run_bootstrap_columns(data, R, L, l_eff, seed, rep0, B, out, (cudaStream_t)stream);
+}
+
+int nnj_split_distances(const int32_t* merges, int B, int R, const uint64_t* splits, int S, int32_t* dist, void* stream) {
+    CHECK_ARGS(merges && B >= 1 && S >= 0 && (S == 0 || (splits && dist)), "split_distances: bad arguments");
+    return run_split_distances(merges, B, R, splits, S, dist, (cudaStream_t)stream);
+}
+
 int nnj_tc_selftest(const float* A, const float* B, float* Dm, int N, void* stream) {
     CHECK_ARGS(A && B && Dm, "tc_selftest: bad arguments");
     return run_tc_unit(A, B, Dm, N, (cudaStream_t)stream);

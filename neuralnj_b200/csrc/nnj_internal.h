@@ -185,4 +185,8 @@ size_t rank_loss_ws_bytes(int B, int R);
 int run_rank_loss(const float* logits_trace, const uint8_t* in_set, int B, int R, float margin, double ratio, float* out, void* ws, size_t ws_bytes,
                   cudaStream_t st);
 
+// bootstrap support: column resampling and transfer distances of reference splits to NJ trees (nnj_support.cu)
+int run_bootstrap_columns(const int8_t* data, int R, int L, int l_eff, uint64_t seed, int64_t rep0, int B, int8_t* out, cudaStream_t st);
+int run_split_distances(const int32_t* merges, int B, int R, const uint64_t* splits, int S, int32_t* dist, cudaStream_t st);
+
 }  // namespace nnj

@@ -26,6 +26,7 @@ from .config import empty_config
 from .environment import PhyInferEnv
 from .model import PhyloATTN
 from .phydata import load_pi_instance
+from .support import _support
 from .treeutil import normalized_rf, rf_distance
 
 EXPLORE_TEMPERTURE = lambda step: 1.0   # finetune_rl_search.py:39
@@ -173,7 +174,7 @@ def _rank_share(items):
 
 
 def Argmax_inference(test_file_path, write_dir, write_file_name=None, branch_optimize=False, cfgs=None, device=None, precision=None,
-                     files_per_call=1, policy_network=None):
+                     files_per_call=1, policy_network=None, bootstrap=0, bootstrap_seed=0):
     """One `.tre` per `.phy` of a directory (finetune_rl_search.py:478-509).
 
     `files_per_call=1` is the reference's loop: one alignment per call (expanded to `cfgs.env.batch_size` copies, :444).
@@ -181,7 +182,11 @@ def Argmax_inference(test_file_path, write_dir, write_file_name=None, branch_opt
     what the batched kernels are built for (hundreds of trees/s instead of one 15 ms call per file); alignments of other shapes go
     into their own calls, nothing is padded, and the rollout of an alignment does not depend on its batch mates, so the trees
     are the ones the per-file loop writes.  Under an initialised process group every rank takes a contiguous share of the sorted
-    file list and writes its own trees (no collective); the return value lists this rank's files."""
+    file list and writes its own trees (no collective); the return value lists this rank's files.
+
+    `bootstrap=N` (not a reference argument) also writes `<name>.fbp.tre` and `<name>.tbe.tre` beside each `<name>.tre`: the same tree
+    with FBP / TBE support from N bootstrap replicates drawn with `bootstrap_seed` (`neuralnj_b200.support`).  A file's replicates
+    run on the rank that owns the file."""
     c = _cfg(cfgs)
     if device is None:                # one process per GPU under torchrun: the rank's own device
         import torch.distributed as dist
@@ -192,6 +197,15 @@ def Argmax_inference(test_file_path, write_dir, write_file_name=None, branch_opt
     os.makedirs(write_dir, exist_ok=True)
     files = _rank_share(sorted(f for f in os.listdir(test_file_path) if f.endswith(".phy")))
     written = []
+
+    def write_support(file, msa, tree):
+        if bootstrap <= 0:
+            return
+        res = _support(msa, policy, bootstrap, bootstrap_seed, tree, None)     # no replicate sharding: the file is this rank's
+        for kind in ("fbp", "tbe"):
+            with open(os.path.join(write_dir, f"{file[:-4]}.{kind}.tre"), "w") as f:
+                f.write(res["newick_" + kind])
+
     if files_per_call <= 1:
         for file in files:
             res = Agmax_one_instance(c, os.path.join(test_file_path, file), policy, env, branch_optimize=branch_optimize)
@@ -199,6 +213,7 @@ def Argmax_inference(test_file_path, write_dir, write_file_name=None, branch_opt
             with open(dst, "w") as f:
                 f.write(res["best_tree_str"])
             written.append(dst)
+            write_support(file, os.path.join(test_file_path, file), res["best_tree_str"])
         return written
 
     pending = {}                      # (taxa, sites) -> [(file, instance), ...]
@@ -206,9 +221,10 @@ def Argmax_inference(test_file_path, write_dir, write_file_name=None, branch_opt
     def run(items):
         batch = _stack_instances([inst for _, inst in items])
         _, _, _, trees = reinforce_rollout(batch, policy, env, c, eval=True, argmax=True, get_all_tree=True, branch_optimize=branch_optimize)
-        for (file, _), tree in zip(items, trees):
+        for (file, inst), tree in zip(items, trees):
             with open(os.path.join(write_dir, file[:-4] + ".tre"), "w") as f:
                 f.write(tree)
+            write_support(file, inst, tree)
 
     for file in files:
         inst = load_pi_instance(os.path.join(test_file_path, file))
@@ -316,7 +332,12 @@ def main(argv=None):
                     help="arithmetic of the CUDA path (not a reference flag); default bf16x3: tcgen05 split-bf16, topologies identical to fp32")
     ap.add_argument("--files_per_call", type=int, default=1,
                     help="Argmax: alignments of equal shape stacked into one rollout call (not a reference flag); 1 = the reference's per-file loop")
+    ap.add_argument("--bootstrap", type=int, default=0,
+                    help="Argmax: also write <name>.fbp.tre / <name>.tbe.tre with support from N bootstrap replicates (not a reference flag)")
+    ap.add_argument("--bootstrap_seed", type=int, default=0, help="seed of the bootstrap replicates (not a reference flag)")
     args = ap.parse_args(argv)
+    if args.bootstrap and args.infer_opt != "Argmax":
+        raise SystemExit("--bootstrap applies to --infer_opt Argmax")
     PRECISION = args.precision
     cfgs = empty_config()
     if args.config_path:
@@ -325,7 +346,8 @@ def main(argv=None):
     name = os.path.basename(os.path.normpath(cfgs.instance_path))
     write_dir = f"output/{args.infer_opt}_dim{cfgs.model.embed_dim}_patch{cfgs.model.patch_size}/{name}"
     if args.infer_opt == "Argmax":
-        return Argmax_inference(cfgs.instance_path, write_dir, None, branch_optimize=args.branch_optimize, files_per_call=args.files_per_call)
+        return Argmax_inference(cfgs.instance_path, write_dir, None, branch_optimize=args.branch_optimize, files_per_call=args.files_per_call,
+                                bootstrap=args.bootstrap, bootstrap_seed=args.bootstrap_seed)
     if args.infer_opt == "Search":
         return Search_inference(cfgs.instance_path, write_dir, None)
     raise SystemExit(f'--infer_opt {args.infer_opt}: "Finetune" (NeuralNJ-RL) trains the policy and is outside this path')

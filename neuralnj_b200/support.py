@@ -1,0 +1,228 @@
+"""Bootstrap branch support of NJ trees: Felsenstein's bootstrap proportion (FBP) and the transfer bootstrap expectation (TBE,
+Lemoine et al., Nature 2018) on the branches of one reference tree - what RAxML-NG computes with `--bootstrap` and
+`--support --bs-metric fbp,tbe`.
+
+    res = bootstrap_support("alignment.phy", policy_network, n_replicates=1000, seed=0)
+    res["newick_fbp"], res["newick_tbe"], res["fbp"], res["tbe"], res["splits"]
+
+The replicates are drawn on the device (`nnj_bootstrap_columns`), each one is an Argmax rollout (`rollout_fused`), and the
+transfer distances of the reference splits to the replicate trees are computed on the device from the merge lists
+(`nnj_split_distances`); per chunk of CHUNK replicates only the int64 totals [2, S] stay behind, and merge lists never reach the
+host.  Definitions: DESIGN.md section 11.  A replicate depends only on (seed, replicate index, real column count), so the chunk
+size and the number of ranks do not change any result.
+"""
+from __future__ import annotations
+
+import ctypes as C
+import os
+import re
+from typing import List, Optional, Tuple
+
+import numpy as np
+import torch
+
+from ._lib import NnjError, check, lib
+from .config import empty_config
+from .environment import PhyInferEnv
+from .phydata import load_pi_instance
+
+CHUNK = 128            # replicates per device round trip (resample -> rollout -> split distances)
+
+
+def _ptr(t: torch.Tensor):
+    return C.c_void_p(t.data_ptr()) if t.numel() else C.c_void_p(0)
+
+
+def _on_cuda(what: str, *tensors: torch.Tensor) -> torch.device:
+    dev = tensors[0].device
+    if dev.type != "cuda" or any(t.device != dev for t in tensors):
+        raise NnjError(f"{what}: tensors must be on one CUDA device (there is no CPU fallback)")
+    return dev
+
+
+def bootstrap_columns(data: torch.Tensor, l_eff: int, seed: int, rep0: int, n: int) -> torch.Tensor:
+    """Replicates rep0 .. rep0+n-1 of one alignment (nnj_bootstrap_columns): data int8 [R,L,4] on the device -> int8 [n,R,L,4]."""
+    dev = _on_cuda("bootstrap_columns", data)
+    data = data.to(torch.int8).contiguous()
+    R, L = data.shape[:2]
+    out = torch.empty(n, R, L, 4, dtype=torch.int8, device=dev)
+    with torch.cuda.device(dev):
+        check(lib().nnj_bootstrap_columns(_ptr(data), R, L, l_eff, seed, rep0, n, _ptr(out),
+                                          C.c_void_p(torch.cuda.current_stream().cuda_stream)), "nnj_bootstrap_columns")
+    return out
+
+
+def split_distances(merges: torch.Tensor, splits: torch.Tensor) -> torch.Tensor:
+    """Transfer distances (nnj_split_distances): merges int32 [B,R-1,2], splits int64 [S,ceil(R/64)] (uint64 bit patterns)
+    -> int32 [B,S]; a row of -1 marks a merge list that is not valid."""
+    dev = _on_cuda("split_distances", merges, splits)
+    merges = merges.to(torch.int32).contiguous()
+    splits = splits.to(torch.int64).contiguous()
+    B, R, S = merges.shape[0], merges.shape[1] + 1, splits.shape[0]
+    out = torch.empty(B, S, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        check(lib().nnj_split_distances(_ptr(merges), B, R, _ptr(splits), S, _ptr(out),
+                                        C.c_void_p(torch.cuda.current_stream().cuda_stream)), "nnj_split_distances")
+    return out
+
+
+# ---------------------------------------------------------------------------------------------------------- Newick side
+
+def internal_clades(newick: str, keys) -> List[Tuple[int, frozenset]]:
+    """(offset just after the `)`, leaf indices below) of every internal node of `newick`, in text order; leaf names are `keys`."""
+    index = {k: i for i, k in enumerate(keys)}
+    stack, out, seen = [set()], [], []
+    s, pos = newick, 0
+    while pos < len(s):
+        ch = s[pos]
+        if ch == "(":
+            stack.append(set())
+            pos += 1
+        elif ch == ")":
+            if len(stack) < 2:
+                raise ValueError(f"bad Newick near position {pos}")
+            clade = stack.pop()
+            stack[-1] |= clade
+            pos += 1
+            out.append((pos, frozenset(clade)))
+            if pos < len(s) and s[pos] not in ":,);" and not s[pos].isspace():
+                raise ValueError("the reference tree already carries internal node labels")
+        elif ch == ":":
+            while pos < len(s) and s[pos] not in ",);":
+                pos += 1
+        elif ch in ",;" or ch.isspace():
+            pos += 1
+        else:
+            st = pos
+            while pos < len(s) and s[pos] not in ":,();":
+                pos += 1
+            name = s[st:pos].strip()
+            if name not in index:
+                raise ValueError(f"taxon {name!r} of the tree is not in the alignment")
+            seen.append(index[name])
+            stack[-1].add(index[name])
+    if len(stack) != 1 or sorted(seen) != list(range(len(keys))):
+        raise ValueError("the tree must name every taxon of the alignment exactly once")
+    return out
+
+
+def reference_splits(newick: str, keys):
+    """Non-trivial splits of `newick`: (light sides as leaf-index frozensets in order of first appearance, split index of each
+    labelled node as (offset, split))."""
+    R = len(keys)
+    everything = frozenset(range(R))
+    splits, where, labelled = [], {}, []
+    for pos, clade in internal_clades(newick, keys):
+        if not 2 <= len(clade) <= R - 2:
+            continue
+        light = min(clade, everything - clade, key=lambda t: (len(t), sorted(keys[i] for i in t)))
+        if light not in where:                   # the two root children of a rooted binary tree are one split
+            where[light] = len(splits)
+            splits.append(light)
+        labelled.append((pos, where[light]))
+    return splits, labelled
+
+
+def split_bitsets(splits, R: int) -> torch.Tensor:
+    """Leaf-index sets -> the bitsets nnj_split_distances reads: int64 [S, ceil(R/64)] holding uint64 bit patterns."""
+    bits = np.zeros((len(splits), (R + 63) // 64), dtype=np.uint64)
+    for k, sp in enumerate(splits):
+        for i in sp:
+            bits[k, i // 64] |= np.uint64(1) << np.uint64(i % 64)
+    return torch.from_numpy(bits.view(np.int64))
+
+
+def label_newick(newick: str, labelled, labels) -> str:
+    """Insert labels[split] after the `)` of every labelled node."""
+    parts, last = [], 0
+    for pos, k in labelled:
+        parts += [newick[last:pos], labels[k]]
+        last = pos
+    return "".join(parts) + newick[last:]
+
+
+def strip_support_labels(newick: str) -> str:
+    """Inverse of the labelling: drop the text between each `)` and the next `:`, `,`, `)` or `;`."""
+    return re.sub(r"\)[^:,;()\s]+", ")", newick)
+
+
+# ---------------------------------------------------------------------------------------------------------- driver
+
+def _process_group():
+    import torch.distributed as dist
+    return dist if dist.is_available() and dist.is_initialized() else None
+
+
+def bootstrap_support(msa, policy_network, n_replicates: int, seed: int = 0, tree: Optional[str] = None) -> dict:
+    """FBP and TBE support of the branches of one tree from `n_replicates` bootstrap replicates of the alignment `msa`.
+
+    `msa` is a path (.phy / .fasta / .aln) or a `load_pi_instance` batch of one alignment.  `tree=None` puts support on the Argmax
+    tree of the original alignment (the Newick string `Argmax_inference` writes); `tree="<newick>"` on a given tree instead (for
+    example the best tree of `RL_Search`), whose taxon names must be the alignment's.  Replicates are drawn, inferred (Argmax
+    rollouts of `policy_network`) and compared on the device.  Under an initialised process group every rank runs a contiguous
+    share of the replicate indices and one all_reduce sums the totals: the result is that of a single process.
+
+    Returns `tree` (unlabelled Newick), `splits` (light sides as frozensets of taxon names), `fbp` [S] (percent), `tbe` [S],
+    `newick_fbp` / `newick_tbe` (labels after the `)` of each internal node with a non-trivial split), `n_replicates`, `seed`."""
+    return _support(msa, policy_network, n_replicates, seed, tree, _process_group())
+
+
+def _support(msa, policy_network, n_replicates: int, seed: int, tree: Optional[str], group) -> dict:
+    if int(n_replicates) < 1:
+        raise ValueError("n_replicates must be >= 1")
+    if not 0 <= int(seed) < 2 ** 64:
+        raise ValueError("seed must be in [0, 2^64)")
+    N, seed = int(n_replicates), int(seed)
+    batch = load_pi_instance(os.fspath(msa)) if isinstance(msa, (str, os.PathLike)) else msa
+    if batch["data"].shape[0] != 1:
+        raise ValueError("bootstrap_support takes one alignment")
+    R, L = batch["data"].shape[1:3]
+    keys = [str(k) for k in batch["seq_keys"][0]]
+    padded = batch["seq_weights"][0] == 0
+    l_eff = int((~padded).sum())
+    if l_eff == 0 or bool(padded[:l_eff].any()):
+        raise NnjError("bootstrap_support: the real columns of the alignment must be a non-empty prefix (padding is the suffix)")
+    device = next(policy_network.parameters()).device
+    data = batch["data"][0].to(device=device, dtype=torch.int8).contiguous()
+    mask = padded.to(device)
+    if tree is None:
+        with torch.no_grad():
+            merges, _, _ = policy_network.rollout_fused(data[None], mask[None])
+        env = PhyInferEnv(empty_config(), device)
+        env.init_states(batch["seqs"], batch["seq_keys"], batch["data"])
+        env.replay_merges(merges)
+        tree = env.states[0].subtrees[0].utree_op_str
+    splits, labelled = reference_splits(tree, keys)
+    S = len(splits)
+    splits_dev = split_bitsets(splits, R).to(device)
+    lo, hi = 0, N
+    if group is not None:
+        from .shard import shard_bounds
+        lo, hi = shard_bounds(N, group.get_rank(), group.get_world_size())
+    # totals[0, :S] = replicates with delta = 0, totals[1, :S] = sum of delta; totals[0, S] counts replicate trees whose merge list
+    # was not valid, so that every rank learns of one after the single all_reduce
+    totals = torch.zeros(2, S + 1, dtype=torch.int64, device=device)
+    if S:
+        with torch.no_grad():
+            for r0 in range(lo, hi, CHUNK):
+                n = min(CHUNK, hi - r0)
+                reps = bootstrap_columns(data, l_eff, seed, r0, n)
+                merges, _, _ = policy_network.rollout_fused(reps, mask.expand(n, L))
+                d = split_distances(merges, splits_dev)
+                totals[0, :S] += (d == 0).sum(0)
+                totals[1, :S] += d.clamp(min=0).sum(0)
+                totals[0, S] += (d < 0).any(1).sum()
+    if group is not None:
+        group.all_reduce(totals)
+    tot = totals.cpu().numpy()
+    if tot[0, S]:
+        raise NnjError(f"bootstrap_support: {int(tot[0, S])} replicate merge lists are not valid")
+    count, dsum = tot[0, :S], tot[1, :S]
+    p = np.array([len(sp) for sp in splits], dtype=np.int64)
+    fbp = 100.0 * count / N
+    tbe = 1.0 - dsum / (N * (p - 1))
+    fbp_labels = [str(int(100 * int(c) / N + 0.5)) for c in count]
+    tbe_labels = [f"{v:.3f}" for v in tbe]
+    return dict(tree=tree, splits=[frozenset(keys[i] for i in sp) for sp in splits], fbp=fbp, tbe=tbe,
+                newick_fbp=label_newick(tree, labelled, fbp_labels), newick_tbe=label_newick(tree, labelled, tbe_labels),
+                n_replicates=N, seed=seed)
