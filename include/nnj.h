@@ -198,7 +198,9 @@ int nnj_bootstrap_columns(const int8_t* data_dev, int R, int L, int l_eff, uint6
 /* Transfer distance of S reference splits (leaf bitsets uint64 [S, ceil(R/64)], either side; bit t of word t/64 = taxon t) to each of
  * B NJ trees (merges int32 [B,R-1,2], the slot rule of nnj_rollout): dist int32 [B,S],
  *   dist = min(p-1, min over the tree's R-2 non-root clades c of min(|A ^ c|, R - |A ^ c|)),  p = size of the split's lighter side;
- * a row of -1 = that merge list is not valid (an entry (i, j) of step t that is not 0 <= i < j < R-t).  4 <= R <= 512, S >= 0. */
+ * a row of -1 = that merge list is not valid (an entry (i, j) of step t that is not 0 <= i < j < R-t).  4 <= R <= 512, S >= 0.
+ * The 512 is this primitive's own limit: it takes merge lists from any source.  Replicate trees from nnj_rollout stop at 400 taxa,
+ * the limit of the encoder's column attention, so a whole bootstrap does too. */
 int nnj_split_distances(const int32_t* merges_dev, int B, int R, const uint64_t* splits_dev, int S, int32_t* dist_dev, void* stream);
 
 /* Building block of the tensor-core path (precision NNJ_PREC_BF16X3), exposed for unit tests and reuse:

@@ -27,6 +27,9 @@ from .environment import PhyInferEnv
 from .phydata import load_pi_instance
 
 CHUNK = 128            # replicates per device round trip (resample -> rollout -> split distances)
+# Every replicate is an Argmax rollout, and the encoder's column attention holds the keys and values of one site column in shared
+# memory (512 bytes a taxon, at most 200 KB): rollouts stop at 400 taxa.  nnj_split_distances alone goes to 512.
+MAX_TAXA = 400
 
 
 def _ptr(t: torch.Tensor):
@@ -156,8 +159,8 @@ def _process_group():
 def bootstrap_support(msa, policy_network, n_replicates: int, seed: int = 0, tree: Optional[str] = None) -> dict:
     """FBP and TBE support of the branches of one tree from `n_replicates` bootstrap replicates of the alignment `msa`.
 
-    `msa` is a path (.phy / .fasta / .aln) or a `load_pi_instance` batch of one alignment.  `tree=None` puts support on the Argmax
-    tree of the original alignment (the Newick string `Argmax_inference` writes); `tree="<newick>"` on a given tree instead (for
+    `msa` is a path (.phy / .fasta / .aln) or a `load_pi_instance` batch of one alignment of at most 400 taxa (MAX_TAXA).  `tree=None`
+    puts support on the Argmax tree of the original alignment (the Newick string `Argmax_inference` writes); `tree="<newick>"` on a given tree instead (for
     example the best tree of `RL_Search`), whose taxon names must be the alignment's.  Replicates are drawn, inferred (Argmax
     rollouts of `policy_network`) and compared on the device.  Under an initialised process group every rank runs a contiguous
     share of the replicate indices and one all_reduce sums the totals: the result is that of a single process.
@@ -177,6 +180,9 @@ def _support(msa, policy_network, n_replicates: int, seed: int, tree: Optional[s
     if batch["data"].shape[0] != 1:
         raise ValueError("bootstrap_support takes one alignment")
     R, L = batch["data"].shape[1:3]
+    if R > MAX_TAXA:
+        raise ValueError(f"bootstrap_support: {R} taxa, at most {MAX_TAXA} are supported: every replicate is an Argmax rollout, and the "
+                         f"encoder's column attention stops at {MAX_TAXA} taxa")
     keys = [str(k) for k in batch["seq_keys"][0]]
     padded = batch["seq_weights"][0] == 0
     l_eff = int((~padded).sum())

@@ -39,19 +39,23 @@ def _min_rel_gap(logits):
     return min(gaps) if gaps else 1.0
 
 
-def _assert_equivalent_trajectory(sd, data, mask, merges, trace, tie_tol, logit_tol=LOGIT_TOL):
+def _assert_equivalent_trajectory(sd, data, mask, merges, trace, tie_tol, logit_tol=LOGIT_TOL, pair_chunk=0):
     """`merges` may leave the oracle's trajectory only at tie-ambiguous steps: replay it on the oracle
-    (teacher-forced) and require every chosen action to be an oracle argmax within tie_tol, logits within LOGIT_TOL."""
+    (teacher-forced) and require every chosen action to be an oracle argmax within tie_tol, logits within LOGIT_TOL.
+    Returns the largest relative logit error along the replayed trajectory."""
     import nnj_oracle as O
-    ref = O.rollout(sd, data, mask, forced_merges=merges)
-    off = 0
+    ref = O.rollout(sd, data, mask, forced_merges=merges, pair_chunk=pair_chunk)
+    off, worst = 0, 0.0
     for t, lg in enumerate(ref["logits"]):
         p = lg.shape[1]
-        assert _rel(trace[:, off:off + p], lg) < logit_tol, t
+        err = _rel(trace[:, off:off + p], lg)
+        assert err < logit_tol, t
+        worst = max(worst, err)
         chosen = lg.gather(1, ref["actions"][t].unsqueeze(1)).squeeze(1)
         slack = (lg.max(1).values - chosen) / lg.abs().max(1).values
         assert float(slack.max()) < tie_tol, f"step {t}: chosen pair is not an oracle argmax (slack {float(slack.max()):.2e})"
         off += p
+    return worst
 
 
 @pytest.mark.parametrize("prec", ["fp32", "bf16x3"])

@@ -186,6 +186,44 @@ def test_identical_replicates_give_full_support(cpu_primitives):
     assert SUP.bootstrap_support(batch, FixedAgent(mg), 7, tree=star)["newick_fbp"] == star
 
 
+class CountingFixedAgent(FixedAgent):
+    """FixedAgent that records the batch size of every rollout call."""
+
+    def __init__(self, merges):
+        super().__init__(merges)
+        self.batches = []
+
+    def rollout_fused(self, data, mask, gumbel=None, want_logits=False):
+        self.batches.append(data.shape[0])
+        return super().rollout_fused(data, mask, gumbel, want_logits)
+
+
+def _random_batch(R, L, seed):
+    rng = np.random.default_rng(seed)
+    data = torch.from_numpy(np.eye(4, dtype=np.int8)[rng.integers(0, 4, (1, R, L))])
+    keys = [f"t{i}" for i in range(R)]
+    mg = np.array([sorted(rng.choice(R - t, 2, replace=False)) for t in range(R - 1)], dtype=np.int32)
+    return {"data": data, "seq_weights": torch.ones(1, L), "seqs": [["A" * L] * R], "seq_keys": [keys]}, mg
+
+
+def test_more_than_400_taxa_raise_before_any_rollout(cpu_primitives):
+    """Every replicate is an Argmax rollout, and the encoder's column attention stops at 400 taxa: 401 taxa are refused before the
+    first rollout (the reference tree's, or the first replicate's when a tree is given), 400 taxa are accepted."""
+    batch, mg = _random_batch(401, 16, 0)
+    agent = CountingFixedAgent(mg)
+    with pytest.raises(ValueError, match="at most 400"):
+        SUP.bootstrap_support(batch, agent, 3)
+    tree = "(" + ", ".join(f"({a}, {b})" for a, b in zip(batch["seq_keys"][0][0:400:2], batch["seq_keys"][0][1:400:2])) + ", t400);"
+    with pytest.raises(ValueError, match="at most 400"):
+        SUP.bootstrap_support(batch, agent, 3, tree=tree)
+    assert agent.batches == []
+    batch, mg = _random_batch(400, 16, 1)
+    agent = CountingFixedAgent(mg)
+    res = SUP.bootstrap_support(batch, agent, 2)
+    assert agent.batches == [1, 2] and len(res["splits"]) == 397
+    assert (res["fbp"] == 100.0).all() and (res["tbe"] == 1.0).all()
+
+
 def test_invalid_merges_and_padding_raise(cpu_primitives):
     from neuralnj_b200 import NnjError
     batch, _ = _golden_batch("t20x256_10")
