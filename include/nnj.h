@@ -148,7 +148,11 @@ int nnj_rollout_host(nnj_model* m, const int8_t* data_host, const uint8_t* seq_m
 /* ---- Tree likelihood (SURVEY.md 8 f2): what Search / branch_optimize=True use to score a topology.
  * Replaces the reference's native binding raxmlpy.compute_llh / raxmlpy.optimize_brlen
  * (RAxMLpy/raxmlpy/core.py:6-12 -> RAxMLpy/cpp/raxmlpy.cpp:1790-1805, 1854-1872; call sites environment.py:365-379, 625-670).
- * Model GTR+I+G4 (raxmlpy's model string "GTR+I+G"); one CTA per tree, fp64.
+ * Model GTR+I+G4 (raxmlpy's model string "GTR+I+G"); one CTA per tree, fp64.  3 <= R <= 4096 taxa (others: NNJ_ERR_INVALID).
+ * Every branch length, and the root branch brlen[c1] + brlen[c2] as a whole, is clamped to [1e-6, 100] in evaluation and
+ * optimisation alike, so zero or negative input lengths score as 1e-6.  Conditional likelihood vectors are rescaled per
+ * (node, pattern) by 2^256 when all their entries fall below 2^-256, with an int32 count per (node, pattern) in the workspace:
+ * no site underflows fp64 at any R in range, and where no vector is rescaled the results are those of unscaled pruning, bit for bit.
  *   tips_dev      uint8 [B,R,L]   4-bit state masks per taxon and alignment pattern (bit a = state a possible; gap / N = 15)
  *   weights_dev   double [B,L]    pattern multiplicities (1 for uncompressed columns)
  *   children_host int32 [B,R-1,2] topology in join order: leaves 0..R-1, inner node R+k = (children[k][0], children[k][1]),

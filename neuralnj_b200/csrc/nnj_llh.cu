@@ -13,6 +13,12 @@
 // traversal, so the only block-wide steps are the 4 x 4 transition matrices of an operation (64 threads, then a barrier) and
 // the reductions of the Newton iteration (fixed order: results are bit-reproducible).
 // Node numbering: leaves 0..R-1, inner node R+k = k-th join (children[k]), root = the last; brlen[v] = branch above v.
+// Scaling: site likelihoods of a few hundred taxa and more underflow fp64.  When all 16 entries of a freshly combined
+// (node, pattern) vector are below 2^-256 the vector is multiplied by 2^256 and an int32 count of that (node, pattern) goes
+// up by one; counts add along the tree like the vectors (D(v) = D(a) + D(b) + own, U(c) = U(parent) + D(sibling) + own) and
+// copies carry theirs.  The root takes log(wk l) - 256 n ln 2, or log(ldexp(wk l, -256 n) + p_inv inv) where there is an
+// invariant term; Newton scales the invariant term up by 2^(256 n) instead.  Powers of two are exact, so wherever n = 0 the
+// arithmetic is the unscaled one, bit for bit.  The CPU restatement (oracle/llh_oracle.py) applies the same rule.
 #include "nnj_internal.h"
 
 namespace nnj {
@@ -20,7 +26,9 @@ namespace nnj {
 constexpr int LLH_THREADS = 512;
 constexpr int LLH_MODEL = 64;      // lam 4 | U 16 | Uinv 16 | freqs 4 | class rates 4 | p_inv | alpha | flags (1 GTR rates free, 2 +G, 4 +I) | pad | 6 GTR rates | pad 10
 constexpr double RATE_LO = 1e-3, RATE_HI = 1e3, ALPHA_LO = 0.02, ALPHA_HI = 100.0, PINV_HI = 0.99, GOLD = 0.3819660112501051;   // as in oracle/llh_oracle.py
-constexpr double BRLEN_MIN = 1e-6, BRLEN_MAX = 100.0;
+constexpr double BRLEN_MIN = 1e-6, BRLEN_MAX = 100.0;    // every length, in evaluation and optimisation, is clamped to this range
+constexpr int SCALE_EXP = 256;
+constexpr double SCALE_BELOW = 0x1p-256, SCALE_UP = 0x1p256, SCALE_LN = 256.0 * 0.69314718055994530942;
 enum { OP_OPT = 0, OP_UP = 1, OP_DOWN = 2, OP_SWAPROOT = 3 };
 
 struct LlhArgs {
@@ -31,6 +39,7 @@ struct LlhArgs {
     double* brlen;              // [B][2R-2] in / out
     const double* model;        // [B][LLH_MODEL]
     double *D, *U, *S, *inv;    // workspace: [B][R-1][L][16], [B][2R-2][L][16], [B][L][16], [B][L]
+    int32_t *Dn, *Un, *Sn;      // scale counts of D, U and the Newton sumtable: [B][R-1][L], [B][2R-2][L], [B][L]
     double* llh;                // [B][2]: before, after
     int B, R, L, n_ops, max_passes, optimise;     // optimise: 0 evaluate, 1 branch lengths, 2 branch lengths + model parameters
     double eps;
@@ -67,6 +76,7 @@ __device__ __forceinline__ void clv_load(const LlhArgs& a, const double* Dt, con
         for (int i = 0; i < 8; ++i) { const double2 d = p[i]; x[2 * i] = d.x; x[2 * i + 1] = d.y; }
     }
 }
+__device__ __forceinline__ int cnt_load(const LlhArgs& a, const int32_t* Dnt, int v, int s) { return v < a.R ? 0 : Dnt[(size_t)(v - a.R) * a.L + s]; }
 __device__ __forceinline__ void vec_load(const double* p, double (&x)[16]) {
     const double2* q = reinterpret_cast<const double2*>(p);
 #pragma unroll
@@ -213,14 +223,14 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh(const LlhArgs a) {
     double* Ut = a.U + (size_t)b * (2 * R - 2) * L * 16;
     double* St = a.S + (size_t)b * L * 16;
     double* invt = a.inv + (size_t)b * L;
+    int32_t* Dnt = a.Dn + (size_t)b * (R - 1) * L;
+    int32_t* Unt = a.Un + (size_t)b * (2 * R - 2) * L;
+    int32_t* Snt = a.Sn + (size_t)b * L;
     if (tid < LLH_MODEL) mdl[tid] = a.model[(size_t)b * LLH_MODEL + tid];
-    for (int v = tid; v < 2 * R - 2; v += LLH_THREADS) t[v] = clampd(a.brlen[(size_t)b * (2 * R - 2) + v], 0.0, BRLEN_MAX);
+    for (int v = tid; v < 2 * R - 2; v += LLH_THREADS) t[v] = clampd(a.brlen[(size_t)b * (2 * R - 2) + v], BRLEN_MIN, BRLEN_MAX);
     __syncthreads();
     const int c1 = ch[(R - 2) * 2], c2 = ch[(R - 2) * 2 + 1];
-    if (tid == 0) { const double t0 = clampd(t[c1] + t[c2], a.optimise ? BRLEN_MIN : 0.0, BRLEN_MAX); t[c1] = t0; t[c2] = t0; }   // the root branch, stored at both ends
-    __syncthreads();
-    if (a.optimise)
-        for (int v = tid; v < 2 * R - 2; v += LLH_THREADS) t[v] = clampd(t[v], BRLEN_MIN, BRLEN_MAX);
+    if (tid == 0) { const double t0 = clampd(t[c1] + t[c2], BRLEN_MIN, BRLEN_MAX); t[c1] = t0; t[c2] = t0; }   // the root branch, stored at both ends
     __syncthreads();
     double pinv = mdl[44], wk = (1.0 - pinv) * 0.25;            // re-read after every change of the model (optimise = 2)
     // invariant-site term: pi_x where every tip of the pattern is compatible with exactly one state x
@@ -230,21 +240,32 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh(const LlhArgs a) {
         invt[s] = (m != 0 && (m & (m - 1)) == 0) ? mdl[36 + (31 - __clz(m))] : 0.0;      // times p_inv where it is used
     }
     // ---- subtree vectors, children before parents (join order); the virtual root itself is never needed
-    auto combine = [&](int x, int y, double* dst_base /* [L][16] */, const double* xsrc_U /* non-null: take U[x] instead of D[x] */) {
+    // dst = (P(t_x) X) * (P(t_y) D[y]) with X = D[x], or U[x] when xsrc_U is given; scaled as described at the top
+    auto combine = [&](int x, int y, double* dst_base /* [L][16] */, int32_t* dst_n /* [L] */, const double* xsrc_U, const int32_t* xsrc_Un) {
         pmat2(Pm, mdl, t[x], t[y]);
         for (int s = tid; s < L; s += LLH_THREADS) {
             double vx[16], vy[16], px[16], py[16];
             if (xsrc_U) vec_load(xsrc_U + (size_t)s * 16, vx); else clv_load(a, Dt, tips, x, s, vx);
             clv_load(a, Dt, tips, y, s, vy);
+            int n = (xsrc_U ? xsrc_Un[s] : cnt_load(a, Dnt, x, s)) + cnt_load(a, Dnt, y, s);
             pm_apply(Pm, vx, px);
             pm_apply(Pm + 64, vy, py);
+            double mx = 0.0;
 #pragma unroll
-            for (int i = 0; i < 16; ++i) px[i] *= py[i];
+            for (int i = 0; i < 16; ++i) { px[i] *= py[i]; mx = fmax(mx, px[i]); }
+            if (mx < SCALE_BELOW) {
+#pragma unroll
+                for (int i = 0; i < 16; ++i) px[i] *= SCALE_UP;          // exact: a power of two
+                ++n;
+            }
             vec_store(dst_base + (size_t)s * 16, px);
+            dst_n[s] = n;
         }
         __syncthreads();      // Pm is rewritten by the next operation
     };
-    auto down_pass = [&]() { for (int k = 0; k < R - 2; ++k) combine(ch[2 * k], ch[2 * k + 1], Dt + (size_t)k * L * 16, nullptr); };
+    auto down_pass = [&]() {
+        for (int k = 0; k < R - 2; ++k) combine(ch[2 * k], ch[2 * k + 1], Dt + (size_t)k * L * 16, Dnt + (size_t)k * L, nullptr, nullptr);
+    };
     down_pass();
     auto root_loglik = [&]() {
         pmat2(Pm, mdl, t[c1], 0.0);
@@ -259,7 +280,12 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh(const LlhArgs a) {
             for (int k = 0; k < 4; ++k)
 #pragma unroll
                 for (int c = 0; c < 4; ++c) l = fma(mdl[36 + c] * p1[k * 4 + c], v2[k * 4 + c], l);
-            acc += wts[s] * log(wk * l + pinv * invt[s]);
+            const int n = cnt_load(a, Dnt, c1, s) + cnt_load(a, Dnt, c2, s);
+            double site;
+            if (n == 0) site = log(wk * l + pinv * invt[s]);
+            else if (pinv * invt[s] == 0.0) site = log(wk * l) - n * SCALE_LN;
+            else site = log(ldexp(wk * l, -SCALE_EXP * n) + pinv * invt[s]);
+            acc += wts[s] * site;
         }
         block_sum2(acc, dummy, red);
         return acc;
@@ -275,18 +301,20 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh(const LlhArgs a) {
                 double v2[16];
                 clv_load(a, Dt, tips, c2, s, v2);
                 vec_store(Ut + ((size_t)c1 * L + s) * 16, v2);
+                Unt[(size_t)c1 * L + s] = cnt_load(a, Dnt, c2, s);
             }
             for (int oi = 0; oi < a.n_ops; ++oi) {
                 const int op = ops[oi * 4], v = ops[oi * 4 + 1], x = ops[oi * 4 + 2], y = ops[oi * 4 + 3];
                 if (op == OP_UP) {
-                    combine(x, y, Ut + (size_t)v * L * 16, Ut + (size_t)x * L * 16);
+                    combine(x, y, Ut + (size_t)v * L * 16, Unt + (size_t)v * L, Ut + (size_t)x * L * 16, Unt + (size_t)x * L);
                 } else if (op == OP_DOWN) {
-                    combine(x, y, Dt + (size_t)(v - R) * L * 16, nullptr);
+                    combine(x, y, Dt + (size_t)(v - R) * L * 16, Dnt + (size_t)(v - R) * L, nullptr, nullptr);
                 } else if (op == OP_SWAPROOT) {
                     for (int s = tid; s < L; s += LLH_THREADS) {
                         double v1[16];
                         clv_load(a, Dt, tips, x, s, v1);
                         vec_store(Ut + ((size_t)v * L + s) * 16, v1);
+                        Unt[(size_t)v * L + s] = cnt_load(a, Dnt, x, s);
                     }
                 } else {
                     // ---- Newton-Raphson on the branch above v.  Sumtable S[s][k][j] = (sum_a pi_a U[a] Umat[a][j]) (sum_b Uinv[j][b] D[b])
@@ -307,6 +335,7 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh(const LlhArgs a) {
                                 sv[k * 4 + j] = A * Bm;
                             }
                         vec_store(St + (size_t)s * 16, sv);
+                        Snt[s] = Unt[(size_t)v * L + s] + cnt_load(a, Dnt, v, s);
                     }
                     double tv = t[v], lo = BRLEN_MIN, hi = BRLEN_MAX;
                     for (int it = 0; it < 32; ++it) {
@@ -325,7 +354,10 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh(const LlhArgs a) {
                                 const double se = sv[i] * ek[i];
                                 l0 += se; l1 = fma(se, ek[16 + i], l1); l2 = fma(se, ek[32 + i], l2);
                             }
-                            const double L0 = wk * l0 + pinv * invt[s], g = wk * l1 / L0;
+                            // a scaled pattern: its invariant term scaled up to match (inf where that overflows: then g = 0, and no 0 * inf)
+                            const int n = Snt[s];
+                            const double L0 = n == 0 ? wk * l0 + pinv * invt[s] : wk * l0 + (invt[s] > 0.0 ? ldexp(pinv * invt[s], SCALE_EXP * n) : 0.0);
+                            const double g = wk * l1 / L0;
                             f1 = fma(wts[s], g, f1);
                             f2 = fma(wts[s], wk * l2 / L0 - g * g, f2);
                         }
@@ -391,18 +423,21 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh(const LlhArgs a) {
 
 // ---- host side
 static inline size_t up256(size_t v) { return (v + 255) & ~(size_t)255; }
-struct LlhLayout { size_t tipsz, D, U, S, inv, small, total; };
+struct LlhLayout { size_t tipsz, D, U, S, inv, Dn, Un, Sn, small, total; };
 static LlhLayout llh_layout(int B, int R, int L, int n_ops) {
     LlhLayout l;
     l.D = up256((size_t)B * (R - 1) * L * 16 * 8);
     l.U = up256((size_t)B * (2 * R - 2) * L * 16 * 8);
     l.S = up256((size_t)B * L * 16 * 8);
     l.inv = up256((size_t)B * L * 8);
+    l.Dn = up256((size_t)B * (R - 1) * L * 4);
+    l.Un = up256((size_t)B * (2 * R - 2) * L * 4);
+    l.Sn = up256((size_t)B * L * 4);
     // staged host arrays: children, ops, brlen, model, llh
     l.small = up256((size_t)B * (R - 1) * 2 * 4) + up256((size_t)B * n_ops * 4 * 4) + up256((size_t)B * (2 * R - 2) * 8) + up256((size_t)B * LLH_MODEL * 8) +
               up256((size_t)B * 2 * 8);
     l.tipsz = 0;
-    l.total = l.D + l.U + l.S + l.inv + l.small + 256;
+    l.total = l.D + l.U + l.S + l.inv + l.Dn + l.Un + l.Sn + l.small + 256;
     return l;
 }
 
@@ -476,6 +511,9 @@ int run_llh(const uint8_t* tips, const double* weights, const int32_t* children_
     a.U = reinterpret_cast<double*>(p); p += lay.U;
     a.S = reinterpret_cast<double*>(p); p += lay.S;
     a.inv = reinterpret_cast<double*>(p); p += lay.inv;
+    a.Dn = reinterpret_cast<int32_t*>(p); p += lay.Dn;
+    a.Un = reinterpret_cast<int32_t*>(p); p += lay.Un;
+    a.Sn = reinterpret_cast<int32_t*>(p); p += lay.Sn;
     int32_t* d_ch = reinterpret_cast<int32_t*>(p); p += up256((size_t)B * (R - 1) * 2 * 4);
     int32_t* d_ops = reinterpret_cast<int32_t*>(p); p += up256((size_t)B * n_ops * 4 * 4);
     double* d_br = reinterpret_cast<double*>(p); p += up256((size_t)B * (2 * R - 2) * 8);
@@ -489,7 +527,11 @@ int run_llh(const uint8_t* tips, const double* weights, const int32_t* children_
     a.children = d_ch; a.ops = d_ops; a.brlen = d_br; a.model = d_md; a.llh = d_ll;
     a.B = B; a.R = R; a.L = L; a.n_ops = n_ops; a.max_passes = max_passes; a.optimise = optimise; a.eps = eps;
     a.lh_eps = lh_eps; a.max_rounds = max_rounds; a.golden_iters = golden_iters; a.model_out = d_md;
-    const size_t smem = (LLH_MODEL + 128 + 66 + 48 + 2 * (size_t)R) * sizeof(double);
+    const size_t smem = (LLH_MODEL + 128 + 66 + 48 + 2 * (size_t)R) * sizeof(double);      // 67 968 bytes at R = 4096
+    if (smem > 48 * 1024) {       // above the default limit the kernel must opt in (from R = 2920 on)
+        e = cudaFuncSetAttribute(k_llh, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
+    }
     prof_begin(KC_LLH, st);
     k_llh<<<B, LLH_THREADS, smem, st>>>(a);
     ++g_launches;

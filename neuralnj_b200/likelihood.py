@@ -12,7 +12,10 @@ this module holds what is host logic in any implementation: Newick <-> join-orde
 parametrisation and the outer loop over model parameters.  There is no CPU fallback.
 
 Model: GTR (or JC) + optional invariant sites (+I) + optional discrete gamma, 4 classes (+G), empirical base
-frequencies.  RAxML-NG itself is not available (the reference git-clones it at install time): parity with its numbers is
+frequencies.  Branch lengths are clamped to [BRLEN_MIN, BRLEN_MAX] = [1e-6, 100] everywhere, evaluation included, and so is
+the root branch (the two root edges, one branch of the unrooted tree): zero or negative lengths, which Newick files and the
+zero branches that resolve a multifurcation bring, score as 1e-6.  Per-pattern scaling of the conditional likelihood vectors
+keeps trees of 3 to 4096 taxa free of fp64 underflow.  RAxML-NG itself is not available (the reference git-clones it at install time): parity with its numbers is
 UNPINNED; tests pin this implementation against an independent CPU restatement and brute-force enumeration
 (oracle/llh_oracle.py).  The optimiser is this repo's own (coordinate golden-section over 5 rates, alpha, p_inv between
 branch-length sweeps, stopping when a round gains < 1 log-unit like `optimize_model(treeinfo, 1.0)`, raxmlpy.cpp:1721-1746) and
@@ -31,6 +34,7 @@ from . import _lib
 from .treeutil import treestr_to_tuples
 
 BRLEN_DEFAULT = 0.1                    # raxml-ng's RAXML_BRLEN_DEFAULT: trees without lengths start here
+BRLEN_MIN, BRLEN_MAX = 1e-6, 100.0     # every length is clamped to this range, when evaluated as when optimised
 PLACEHOLDER = 0.12345                  # environment.py:287 prints missing lengths like this; treated as "no length"
 RATE_LO, RATE_HI, ALPHA_LO, ALPHA_HI, PINV_HI = 1e-3, 1e3, 0.02, 100.0, 0.99
 _GOLD = 0.3819660112501051

@@ -10,12 +10,21 @@ and RAxMLpy/test/*.py only print.  What pins this file instead (tests/test_llh_o
   * the discrete-gamma mean rates vs the published table value (Yang 1994: alpha 0.5, 4 categories ->
     0.0334, 0.2519, 0.8203, 2.8944);
   * JC69 two-taxon closed form: d = -3/4 ln(1 - 4p/3) maximises the likelihood;
-  * the optimiser never decreases the likelihood, and a numerical gradient at its fixed point vanishes.
+  * the optimiser never decreases the likelihood, and a numerical gradient at its fixed point vanishes;
+  * for trees whose site likelihoods underflow fp64 (a few hundred taxa and up), `loglik_logspace`: pruning on
+    log-CLVs with logsumexp and transition matrices from scipy.linalg.expm - no eigen form and no rescaling.
 The published algorithm restated: Felsenstein (1981) pruning; Yang (1994) discrete gamma, mean of each quantile
 class; invariant-site mixture L = (1-p) L_gamma + p * pi_x for columns whose tips share one state x; per-branch
 Newton-Raphson on the eigen-space "sumtable" with the other branches fixed, swept in depth-first order with the
 conditional likelihood vectors refreshed on the way (the scheme of libpll's pllmod_algo_opt_brlen_treeinfo);
-branch lengths in [1e-6, 100], default 0.1 (raxml-ng's RAXML_BRLEN_MIN / MAX / DEFAULT).
+branch lengths in [1e-6, 100], default 0.1 (raxml-ng's RAXML_BRLEN_MIN / MAX / DEFAULT): evaluation and optimisation
+both clamp every length, and the root branch brlen[c1] + brlen[c2], into that range.
+
+Scaling (the rule of csrc/nnj_llh.cu, applied everywhere a CLV is formed): when all 16 entries of a (node, pattern)
+vector are below 2^-256, the vector is multiplied by 2^256 and the pattern's integer count of that node goes up by one.
+Counts add along the tree: D(v) = D(a) + D(b) + own, U(c) = U(parent) + D(sibling) + own, and copies keep theirs.  A
+site likelihood is ldexp(wk * l, -256 n) + p_inv * inv; its log is taken as log(wk * l) - 256 n ln 2 when p_inv * inv
+is 0.  Powers of two are exact: where nothing is scaled, every result is bit-identical to unscaled pruning.
 
 Tree encoding shared with the CUDA path: leaves 0..R-1, inner node R+k = k-th join, children[k] = (left, right);
 the last inner node is the (virtual) root.  brlen[v] = length of the edge above node v (v < 2R-2); the two root
@@ -29,6 +38,9 @@ import numpy as np
 from scipy import special
 
 BRLEN_MIN, BRLEN_MAX, BRLEN_DEFAULT = 1e-6, 100.0, 0.1
+SCALE_EXP = 256                        # a CLV whose entries are all below 2^-SCALE_EXP is multiplied by 2^SCALE_EXP
+SCALE_THRESHOLD = 2.0 ** -SCALE_EXP
+LN2 = float(np.log(2.0))
 NCAT = 4
 OP_OPT, OP_UP, OP_DOWN, OP_SWAPROOT = 0, 1, 2, 3
 
@@ -117,24 +129,113 @@ def invariant_term(tips: np.ndarray, freqs: np.ndarray) -> np.ndarray:
     return np.where(single & (m > 0), freqs[np.minimum(idx, 3)], 0.0)
 
 
-def down_clvs(children, brlen, tips, model: Model):
-    R = tips.shape[0]
+def _scale(x: np.ndarray, n: np.ndarray, scaling: bool):
+    """The kernel's rule on one freshly combined CLV x [L, ncat, 4] with the summed counts n [L] of its inputs."""
+    if scaling:
+        small = (x < SCALE_THRESHOLD).all(axis=(1, 2))
+        if small.any():
+            x[small] = np.ldexp(x[small], SCALE_EXP)
+            n = n + small
+    return x, n
+
+
+def _combine(Px, x, nx, Py, y, ny, scaling: bool):
+    z = np.einsum("kxy,sky->skx", Px, x) * np.einsum("kxy,sky->skx", Py, y)
+    return _scale(z, nx + ny, scaling)
+
+
+def down_clvs(children, brlen, tips, model: Model, scaling: bool = True):
+    """Subtree CLVs of every node -> (D [2R-1] of [L, ncat, 4], counts [2R-1] of int [L])."""
+    R, L = tips.shape
     D = [tip_clv(tips[v], model.ncat) for v in range(R)]
-    for k, (a, b) in enumerate(children):
-        Pa, Pb = model.pmats(brlen[a]), model.pmats(brlen[b])
-        D.append(np.einsum("kxy,sky->skx", Pa, D[a]) * np.einsum("kxy,sky->skx", Pb, D[b]))
-    return D
+    N = [np.zeros(L, dtype=np.int64) for _ in range(R)]
+    for a, b in children:
+        d, n = _combine(model.pmats(brlen[a]), D[a], N[a], model.pmats(brlen[b]), D[b], N[b], scaling)
+        D.append(d)
+        N.append(n)
+    return D, N
 
 
-def site_likelihoods(children, brlen, tips, model: Model) -> np.ndarray:
-    D = down_clvs(children, brlen, tips, model)
-    root = D[-1]
-    lg = np.einsum("ska,a->s", root, model.freqs) / model.ncat
-    return (1.0 - model.pinv) * lg + model.pinv * invariant_term(tips, model.freqs)
+def clamp_lengths(children, brlen) -> np.ndarray:
+    """The lengths every computation uses: each clamped to [BRLEN_MIN, BRLEN_MAX], and the root branch (the two root
+    edges, one branch of the unrooted tree) clamped as a whole and stored at both ends."""
+    t = np.clip(np.array(brlen, dtype=np.float64), BRLEN_MIN, BRLEN_MAX)
+    c1, c2 = (int(v) for v in children[-1])
+    t[c1] = t[c2] = min(max(t[c1] + t[c2], BRLEN_MIN), BRLEN_MAX)
+    return t
 
 
-def loglik(children, brlen, tips, weights, model: Model) -> float:
-    return float((weights * np.log(site_likelihoods(children, brlen, tips, model))).sum())
+def log_sites(lw: np.ndarray, n: np.ndarray, iv: np.ndarray) -> np.ndarray:
+    """log(ldexp(lw, -256 n) + iv) per pattern; log(lw) - 256 n ln 2 where iv (= p_inv * inv) is 0 and n > 0."""
+    with np.errstate(divide="ignore"):
+        out = np.log(np.ldexp(lw, -SCALE_EXP * n) + iv)
+        sc = (n > 0) & (iv == 0)
+        if sc.any():
+            out[sc] = np.log(lw[sc]) - n[sc] * (SCALE_EXP * LN2)
+    return out
+
+
+def root_terms(children, brlen, tips, model: Model, scaling: bool = True):
+    """-> (wk * l, n, p_inv * inv) per pattern: the site likelihood is ldexp(wk * l, -256 n) + p_inv * inv.  The root branch
+    is one branch of length t[c1] (clamp_lengths), between D[c1] and D[c2]."""
+    children = np.asarray(children)
+    t = clamp_lengths(children, brlen)
+    c1, c2 = (int(v) for v in children[-1])
+    D, N = down_clvs(children[:-1], t, tips, model, scaling)
+    x = np.einsum("kxy,sky->skx", model.pmats(t[c1]), D[c1]) * D[c2]
+    lw = (1.0 - model.pinv) * (np.einsum("ska,a->s", x, model.freqs) / model.ncat)
+    return lw, N[c1] + N[c2], model.pinv * invariant_term(tips, model.freqs)
+
+
+def site_likelihoods(children, brlen, tips, model: Model, scaling: bool = False) -> np.ndarray:
+    """Plain site likelihoods.  Unscaled (the default) they underflow to subnormals or 0 on large trees - which is what
+    tests use this for; scaled, the result is exact up to the final ldexp, which may underflow the same way."""
+    lw, n, iv = root_terms(children, brlen, tips, model, scaling)
+    return np.ldexp(lw, -SCALE_EXP * n) + iv
+
+
+def site_logliks(children, brlen, tips, model: Model, scaling: bool = True) -> np.ndarray:
+    return log_sites(*root_terms(children, brlen, tips, model, scaling))
+
+
+def loglik(children, brlen, tips, weights, model: Model, scaling: bool = True) -> float:
+    return float((weights * site_logliks(children, brlen, tips, model, scaling)).sum())
+
+
+def loglik_logspace(children, brlen, tips, weights, model: Model) -> float:
+    """Independent reference for trees of any size: pruning on log-CLVs (scipy.special.logsumexp), transition matrices
+    scipy.linalg.expm(Q r_k t) of the normalised GTR matrix built here again - neither the eigen form nor any rescaling.
+    Slow; it exists to pin the scaled pruning above."""
+    from scipy import linalg
+    children = np.asarray(children)
+    R = tips.shape[0]
+    t = clamp_lengths(children, brlen)
+    c1, c2 = (int(v) for v in children[-1])
+    pi = np.asarray(model.freqs, dtype=np.float64)
+    Q = np.zeros((4, 4))
+    for (a, b), v in zip(itertools.combinations(range(4), 2), model.rates6):
+        Q[a, b], Q[b, a] = v * pi[b], v * pi[a]
+    Q -= np.diag(Q.sum(1))
+    Q /= -(pi * np.diag(Q)).sum()
+    cat = model.cat
+
+    def logp(tv):                                                         # [ncat, 4, 4]
+        with np.errstate(divide="ignore"):
+            return np.log(np.stack([linalg.expm(Q * r * tv) for r in cat]))
+
+    def move(lp, x):                                                      # log sum_y P[k, a, y] exp(x[s, k, y])
+        return special.logsumexp(lp[None, :, :, :] + x[:, :, None, :], axis=3)
+
+    with np.errstate(divide="ignore"):
+        logD = [np.log(tip_clv(tips[v], model.ncat)) for v in range(R)]
+    for a, b in children[:-1]:
+        logD.append(move(logp(t[a]), logD[a]) + move(logp(t[b]), logD[b]))
+    x = move(logp(t[c1]), logD[c1]) + logD[c2]                              # [L, ncat, 4]
+    with np.errstate(divide="ignore"):
+        lg = special.logsumexp(x + np.log(pi)[None, None, :], axis=(1, 2)) - np.log(model.ncat)
+        iv = np.log(model.pinv * invariant_term(tips, pi))
+        site = np.logaddexp(np.log1p(-model.pinv) + lg, iv)
+    return float((weights * site).sum())
 
 
 def loglik_bruteforce(children, brlen, tips, weights, model: Model) -> float:
@@ -204,7 +305,8 @@ def build_ops(children, R: int):
 
 def _newton(S, lam, cat, wk, inv, weights, t0):
     """Safeguarded Newton-Raphson on f(t) = sum_s w_s log L_s(t), L_s = sum_kj S[s,k,j] exp(lam_j r_k t) * wk + inv_s.
-    Same arithmetic and control flow as nr_branch in csrc/nnj_llh.cu."""
+    Same arithmetic and control flow as the Newton loop in csrc/nnj_llh.cu; S is scaled by 2^(-256 n_s), inv_s by the
+    caller to match."""
     rate = lam[None, :] * cat[:, None]                                    # [k, j]
     t, lo, hi = min(max(t0, BRLEN_MIN), BRLEN_MAX), BRLEN_MIN, BRLEN_MAX
     for _ in range(32):
@@ -232,45 +334,45 @@ def _newton(S, lam, cat, wk, inv, weights, t0):
     return t
 
 
-def optimize_branches(children, brlen, tips, weights, model: Model, max_passes=32, eps=1e-3):
+def optimize_branches(children, brlen, tips, weights, model: Model, max_passes=32, eps=1e-3, scaling: bool = True):
     """Returns (brlen_opt, loglik_before, loglik_after).  A pass = one sweep of build_ops; passes stop when the
     log-likelihood gain of a pass is below eps."""
     children = np.asarray(children)
     R = tips.shape[0]
-    t = np.array(brlen, dtype=np.float64).copy()
-    root = R + len(children) - 1
+    t = clamp_lengths(children, brlen)                                    # the root branch is stored at both ends
     c1, c2 = (int(v) for v in children[-1])
-    t[c1] = t[c2] = min(max(t[c1] + t[c2], BRLEN_MIN), BRLEN_MAX)       # one branch, stored at both ends
-    t = np.clip(t, BRLEN_MIN, BRLEN_MAX)
     ops = build_ops(children, R)
     inv = model.pinv * invariant_term(tips, model.freqs)
     wk = (1.0 - model.pinv) / model.ncat
 
-    def root_loglik(D):
+    def root_loglik(D, N):
         x = np.einsum("kxy,sky->skx", model.pmats(t[c1]), D[c1]) * D[c2]
-        return float((weights * np.log(wk * np.einsum("ska,a->s", x, model.freqs) + inv)).sum())
+        return float((weights * log_sites(wk * np.einsum("ska,a->s", x, model.freqs), N[c1] + N[c2], inv)).sum())
 
     tt = t.copy()
     tt[c2] = 0.0
-    D = down_clvs(children, tt, tips, model)
-    U = [None] * (2 * R - 1)
-    ll0 = ll = root_loglik(D)
+    D, N = down_clvs(children, tt, tips, model, scaling)
+    U, NU = [None] * (2 * R - 1), [None] * (2 * R - 1)
+    ll0 = ll = root_loglik(D, N)
     for _ in range(max_passes):
-        U[c1] = D[c2]
+        U[c1], NU[c1] = D[c2], N[c2]
         for op, v, x, y in ops:
             if op == OP_OPT:
                 A = np.einsum("ska,a,aj->skj", U[v], model.freqs, model.U)
                 Bm = np.einsum("jb,skb->skj", model.Uinv, D[v])
-                t[v] = _newton(A * Bm, model.lam, model.cat, wk, inv, weights, t[v])
+                n = NU[v] + N[v]
+                with np.errstate(over="ignore"):                          # 2^(256 n) p_inv pi_x may be inf: then g = 0, exactly enough
+                    invs = np.where((inv > 0) & (n > 0), np.ldexp(inv, SCALE_EXP * n), inv)
+                t[v] = _newton(A * Bm, model.lam, model.cat, wk, invs, weights, t[v])
                 if v == c1:
                     t[c2] = t[c1]
             elif op == OP_UP:
-                U[v] = np.einsum("kxy,sky->skx", model.pmats(t[x]), U[x]) * np.einsum("kxy,sky->skx", model.pmats(t[y]), D[y])
+                U[v], NU[v] = _combine(model.pmats(t[x]), U[x], NU[x], model.pmats(t[y]), D[y], N[y], scaling)
             elif op == OP_DOWN:
-                D[v] = np.einsum("kxy,sky->skx", model.pmats(t[x]), D[x]) * np.einsum("kxy,sky->skx", model.pmats(t[y]), D[y])
+                D[v], N[v] = _combine(model.pmats(t[x]), D[x], N[x], model.pmats(t[y]), D[y], N[y], scaling)
             else:
-                U[v] = D[x]
-        new = root_loglik(D)
+                U[v], NU[v] = D[x], N[x]
+        new = root_loglik(D, N)
         gain, ll = new - ll, new
         if gain < eps:
             break
@@ -300,10 +402,10 @@ def golden_max(f, lo, hi, iters=24):
     return (x1, f1) if f1 > f2 else (x2, f2)
 
 
-def optimize_all(children, brlen, tips, weights, model: Model, lh_eps=1.0, max_rounds=10):
+def optimize_all(children, brlen, tips, weights, model: Model, lh_eps=1.0, max_rounds=10, scaling: bool = True):
     """Branch lengths, then rounds of (5 free GTR rates, alpha, pinv, branch lengths) until a round gains < lh_eps
     (raxmlpy.cpp:1721-1746 `optimize_model(treeinfo, 1.0)` has this loop shape; its inner optimisers differ)."""
-    t, ll0, ll = optimize_branches(children, brlen, tips, weights, model)
+    t, ll0, ll = optimize_branches(children, brlen, tips, weights, model, scaling=scaling)
     for _ in range(max_rounds):
         start = ll
 
@@ -311,7 +413,7 @@ def optimize_all(children, brlen, tips, weights, model: Model, lh_eps=1.0, max_r
             def f(x):
                 setter(x)
                 model.refresh()
-                return loglik(children, t, tips, weights, model)
+                return loglik(children, t, tips, weights, model, scaling)
             return f
 
         for i in range(5):
@@ -328,7 +430,7 @@ def optimize_all(children, brlen, tips, weights, model: Model, lh_eps=1.0, max_r
         x, _ = golden_max(with_param(set_pinv), 0.0, PINV_HI)
         set_pinv(x)
         model.refresh()
-        t, _, ll = optimize_branches(children, t, tips, weights, model)
+        t, _, ll = optimize_branches(children, t, tips, weights, model, scaling=scaling)
         if ll - start < lh_eps:
             break
     return t, ll0, ll

@@ -49,7 +49,109 @@ def test_pruning_equals_bruteforce(R, seed):
     tips = O.simulate(ch, bl, R, 25, m, rng, gap_frac=0.15)
     tips[0, :3] = 5            # an ambiguity code (A or G)
     w = rng.integers(1, 4, size=25).astype(float)
-    assert abs(O.loglik(ch, bl, tips, w, m) - O.loglik_bruteforce(ch, bl, tips, w, m)) < 1e-9
+    brute = O.loglik_bruteforce(ch, bl, tips, w, m)
+    for scaling in (True, False):
+        assert abs(O.loglik(ch, bl, tips, w, m, scaling=scaling) - brute) < 1e-9
+    assert abs(O.loglik_logspace(ch, bl, tips, w, m) - brute) < 1e-9
+
+
+def _iid(R, L, rng):
+    return (1 << rng.integers(0, 4, size=(R, L))).astype(np.uint8)
+
+
+def _underflows(ch, bl, tips, m):
+    """Patterns whose unscaled site likelihood is 0 or subnormal in fp64."""
+    with np.errstate(all="ignore"):
+        s = O.site_likelihoods(ch, bl, tips, m, scaling=False)
+    return int((s < np.finfo(np.float64).tiny).sum())
+
+
+@pytest.mark.parametrize("R,L", [(3, 40), (12, 200), (50, 300), (130, 300)])
+def test_scaling_changes_nothing_where_it_does_not_trigger(R, L):
+    rng = np.random.default_rng(R)
+    m = _model()
+    ch, bl = O.random_tree(R, rng)
+    tips = O.simulate(ch, bl, R, L, m, rng, gap_frac=0.05)
+    pat, w = O.compress_patterns(tips)
+    assert not O.root_terms(ch, bl, pat, m)[1].any()
+    a, b = O.loglik(ch, bl, pat, w, m), O.loglik(ch, bl, pat, w, m, scaling=False)
+    assert a == b and abs(a - O.loglik_logspace(ch, bl, pat, w, m)) < 1e-12 * abs(a)
+
+
+# Each case underflows fp64 without scaling (asserted), so it pins the scaled pruning against the log-space one.
+SCALED_CASES = [(300, 300, "iid", 0.1, 50.0), (512, 300, "iid", 1.0, 0.5), (1000, 200, "sim", 1.0, None), (4096, 64, "sim", 1.0, None)]
+
+
+@pytest.mark.parametrize("R,L,kind,scale,alpha", SCALED_CASES)
+def test_scaled_pruning_matches_logspace(R, L, kind, scale, alpha):
+    rng = np.random.default_rng(R)
+    gen = _model()
+    ch, bl = O.random_tree(R, rng)
+    tips = O.simulate(ch, bl, R, L, gen, rng, gap_frac=0.05) if kind == "sim" else _iid(R, L, rng)
+    pat, w = O.compress_patterns(tips)
+    m = gen if alpha is None else O.Model(alpha=alpha)
+    bl = bl * scale
+    assert _underflows(ch, bl, pat, m) > 0
+    with np.errstate(divide="ignore"):
+        assert not np.isfinite(O.loglik(ch, bl, pat, w, m, scaling=False)) or _underflows(ch, bl, pat, m) > 0
+    got = O.loglik(ch, bl, pat, w, m)
+    assert np.isfinite(got) and O.root_terms(ch, bl, pat, m)[1].max() >= 1
+    assert abs(got - O.loglik_logspace(ch, bl, pat, w, m)) < 1e-10 * abs(got)
+
+
+def test_scaled_optimiser_equals_unscaled_where_nothing_scales():
+    rng = np.random.default_rng(12)
+    m = _model()
+    ch, bl = O.random_tree(30, rng)
+    tips = O.simulate(ch, bl, 30, 300, m, rng, gap_frac=0.05)
+    pat, w = O.compress_patterns(tips)
+    start = np.full(58, O.BRLEN_DEFAULT)
+    t1, b1, a1 = O.optimize_branches(ch, start, pat, w, m)
+    t2, b2, a2 = O.optimize_branches(ch, start, pat, w, m, scaling=False)
+    assert abs(a1 - a2) < 1e-12 * abs(a2) and abs(b1 - b2) < 1e-12 * abs(b2) and np.allclose(t1, t2, rtol=1e-12, atol=0)
+
+
+def test_scaled_optimiser_on_an_underflowing_tree():
+    """300 iid taxa at 0.1x lengths: every site underflows unscaled at the start; the optimiser climbs, and the log-space
+    pruning reproduces its reported maximum at the returned lengths."""
+    R, L = 300, 60
+    rng = np.random.default_rng(30)
+    ch, bl = O.random_tree(R, rng)
+    tips = _iid(R, L, rng)
+    m = O.Model(alpha=50.0)
+    start = bl * 0.1
+    assert _underflows(ch, start, tips, m) == L
+    t, before, after = O.optimize_branches(ch, start, tips, np.ones(L), m, max_passes=2)
+    assert np.isfinite(before) and after > before
+    assert abs(O.loglik_logspace(ch, start, tips, np.ones(L), m) - before) < 1e-10 * abs(before)
+    assert abs(O.loglik_logspace(ch, t, tips, np.ones(L), m) - after) < 1e-10 * abs(after)
+
+
+def test_lengths_are_clamped_in_evaluation():
+    """Zero, negative and huge lengths score as the clamped lengths [BRLEN_MIN, BRLEN_MAX]; the root branch is clamped as one."""
+    rng = np.random.default_rng(6)
+    m = _model()
+    ch, bl = O.random_tree(8, rng)
+    tips = O.simulate(ch, bl, 8, 50, m, rng)
+    w = np.ones(50)
+    c1, c2 = ch[-1]
+    odd = bl.copy()
+    odd[[0, 3]] = 0.0
+    odd[5] = -0.3
+    odd[7] = 250.0
+    odd[c1], odd[c2] = 70.0, 60.0
+    ref = bl.copy()
+    ref[[0, 3, 5]] = O.BRLEN_MIN
+    ref[7] = O.BRLEN_MAX
+    ref[c1], ref[c2] = O.BRLEN_MAX, 0.0
+    got = O.loglik(ch, odd, tips, w, m)
+    assert np.isfinite(got) and got == O.loglik(ch, ref, tips, w, m)
+    assert abs(got - O.loglik_logspace(ch, odd, tips, w, m)) < 1e-10 * abs(got)
+    # two different tips on zero-length branches: the true site likelihood at length 0 is 0; clamped it is tiny and positive
+    ch3 = np.array([[0, 1], [3, 2]], dtype=np.int32)
+    tips3 = np.array([[1], [2], [1]], dtype=np.uint8)
+    s = O.site_likelihoods(ch3, np.array([0.0, 0.0, 0.1, 0.1]), tips3, O.Model(pinv=0.0))
+    assert s[0] > 0 and abs(s[0] - O.site_likelihoods(ch3, np.array([1e-6, 1e-6, 0.1, 0.1]), tips3, O.Model(pinv=0.0))[0]) == 0
 
 
 def test_jc69_two_taxon_closed_form():
