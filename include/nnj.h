@@ -175,6 +175,28 @@ int nnj_llh_optimize_brlen(const uint8_t* tips_dev, const double* weights_dev, c
 int nnj_llh_optimize_all(const uint8_t* tips_dev, const double* weights_dev, const int32_t* children_host, double* brlen_host,
                          double* model_host, int B, int R, int L, int max_passes, double eps, double lh_eps, int max_rounds,
                          double* llh_before_host, double* llh_after_host, void* ws_dev, int64_t ws_bytes, void* stream);
+/* Likelihood branch support of a fixed tree (IQ-TREE -alrt / -abayes, PhyML aLRT; DESIGN.md 12): for each of the R-3 internal
+ * branches (in increasing v: the branch above inner node v, the root branch once at the first root child and only when both root
+ * children are inner) the two NNI alternatives of its quartet, each with its central and four outer lengths optimised by rounds of
+ * Newton (model fixed; a round optimises central, A, B, C, D; rounds stop after one gains < 1e-3, or after 8), and RELL replicates
+ * rep0 .. rep0+n_rell-1 of the per-pattern log-likelihoods.  Inputs as nnj_llh_eval; 3 <= R <= 4096 (R = 3: no branches, nothing
+ * written).  The pattern weights must be non-negative integers (their sum n is the site count the replicates draw from).
+ * Draw i of replicate r is the site u = (x0 * n) >> 32, x0 = word 0 of Philox4x32-10 with counter (i, r & 0xffffffff, r >> 32, 0)
+ * and key (seed & 0xffffffff, seed >> 32) (the rule of nnj_bootstrap_columns); pattern p takes the sites cum[p] <= u < cum[p+1].
+ *   branch_node_host int32  [B,R-3]      v of each internal branch
+ *   llh_host         double [B,R-3,3]    L0 (the tree), L1 (AC|BD), L2 (AD|BC)
+ *   nni_brlen_host   double [B,R-3,2,5]  optimised central, A, B, C, D lengths of each alternative
+ *   sh_count_host    int32  [B,R-3]      replicates with delta > (largest - second largest of Lk* - Lk) + 0.05 (SH-aLRT = 100 count / n_rell)
+ *   lbp_count_host   int32  [B,R-3]      replicates with L0* >= max(L1*, L2*) (local bootstrap probability)
+ *   site_llh_dev     double [B,R-3,3,L]  per-pattern log-likelihoods l0, l1, l2 (device; may be NULL)
+ * In the RELL statistics Lk = sum_p w[p] lk[p], Lk* = sum_p c_r[p] lk[p] (pattern order, a multiply then an add) and delta = L0 - max(L1, L2)
+ * from those sums.  A replicate depends only on (seed, r, n): counts over disjoint rep0 ranges add.  Bad weights, an invalid tree:
+ * NNJ_ERR_INVALID; a workspace smaller than nnj_llh_support_workspace_bytes(B, R, L, n_rell): NNJ_ERR_WORKSPACE.  Synchronises `stream`. */
+int64_t nnj_llh_support_workspace_bytes(int B, int R, int L, int n_rell);
+int nnj_llh_branch_support(const uint8_t* tips_dev, const double* weights_dev, const int32_t* children_host, const double* brlen_host,
+                           const double* model_host, int B, int R, int L, uint64_t seed, int64_t rep0, int n_rell,
+                           int32_t* branch_node_host, double* llh_host, double* nni_brlen_host, int32_t* sh_count_host,
+                           int32_t* lbp_count_host, double* site_llh_dev, void* ws_dev, int64_t ws_bytes, void* stream);
 /* Mean rates of the ncat equal-probability classes of Gamma(alpha, alpha) (Yang 1994): rates_host double [ncat]. */
 int nnj_gamma_rates(double alpha, int ncat, double* rates_host);
 

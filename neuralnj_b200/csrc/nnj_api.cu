@@ -450,6 +450,19 @@ int nnj_llh_optimize_all(const uint8_t* tips, const double* weights, const int32
     return rc;
 }
 
+int64_t nnj_llh_support_workspace_bytes(int B, int R, int L, int n_rell) {
+    return (B >= 1 && R >= 3 && L >= 1 && n_rell >= 0) ? (int64_t)llh_support_ws_bytes(B, R, L, n_rell) : -1;
+}
+
+int nnj_llh_branch_support(const uint8_t* tips, const double* weights, const int32_t* children_h, const double* brlen_h, const double* model_h, int B, int R,
+                           int L, uint64_t seed, int64_t rep0, int n_rell, int32_t* branch_node_h, double* llh_h, double* nni_brlen_h, int32_t* sh_count_h,
+                           int32_t* lbp_count_h, double* site_llh_dev, void* ws, int64_t ws_bytes, void* stream) {
+    CHECK_ARGS(tips && weights && children_h && brlen_h && model_h && ws && B >= 1 && R >= 3 && R <= 4096 && L >= 1 && n_rell >= 0 && rep0 >= 0 &&
+               (R == 3 || (branch_node_h && llh_h && nni_brlen_h && sh_count_h && lbp_count_h)), "llh_branch_support: bad arguments");
+    return run_llh_support(tips, weights, children_h, brlen_h, model_h, B, R, L, seed, rep0, n_rell, branch_node_h, llh_h, nni_brlen_h, sh_count_h,
+                           lbp_count_h, site_llh_dev, ws, (size_t)ws_bytes, (cudaStream_t)stream);
+}
+
 int nnj_gamma_rates(double alpha, int ncat, double* rates_h) {
     CHECK_ARGS(rates_h, "gamma_rates: bad arguments");
     return gamma_rates(alpha, ncat, rates_h);

@@ -196,6 +196,23 @@ __device__ __forceinline__ float reduce16(float v) {
     return v;
 }
 
+// Philox4x32-10 (Salmon et al., SC 2011; the constants of Random123), word 0 of the output block: the resampling draws of the bootstrap
+// (nnj_support.cu) and of the RELL replicates (nnj_llh_nni.cu).
+__device__ __forceinline__ uint32_t philox_x0(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1) {
+#pragma unroll
+    for (int round = 0; round < 10; ++round) {
+        const uint32_t lo0 = 0xD2511F53u * c0, hi0 = __umulhi(0xD2511F53u, c0);
+        const uint32_t lo1 = 0xCD9E8D57u * c2, hi1 = __umulhi(0xCD9E8D57u, c2);
+        c0 = hi1 ^ c1 ^ k0;
+        c1 = lo1;
+        c2 = hi0 ^ c3 ^ k1;
+        c3 = lo0;
+        k0 += 0x9E3779B9u;
+        k1 += 0xBB67AE85u;
+    }
+    return c0;
+}
+
 // position of pair (i<j) among combinations(range(n), 2)  (environment.py:458)
 __host__ __device__ __forceinline__ int pair_index(int i, int j, int n) { return i * n - i * (i + 1) / 2 + (j - i - 1); }
 

@@ -175,9 +175,17 @@ int run_gemm_split_bf16(const float* A, const float* B, float* Cm, int Z, int M,
 
 // tree likelihood / branch-length optimisation (nnj_llh.cu)
 size_t llh_ws_bytes(int B, int R, int L);
+struct LlhState { const double *D, *U, *inv; const int32_t *Dn, *Un; };    // where run_llh leaves the vectors of the trees in the workspace
+int llh_check_tree(const int32_t* ch, int R);     // 0 when children is a binary tree in join order
+// optimise 3 (evaluate and fill U at the given lengths) also writes the per-pattern log-likelihoods to site_dev [B][L]
 int run_llh(const uint8_t* tips, const double* weights, const int32_t* children_h, double* brlen_h, double* model_h, int B, int R, int L,
             int optimise, int max_passes, double eps, double lh_eps, int max_rounds, int golden_iters, double* llh_h, void* ws, size_t ws_bytes,
-            cudaStream_t st);
+            cudaStream_t st, double* site_dev = nullptr, LlhState* state = nullptr);
+// likelihood branch support (nnj_llh_nni.cu): NNI quartets of every internal branch, RELL replicates
+size_t llh_support_ws_bytes(int B, int R, int L, int n_rell);
+int run_llh_support(const uint8_t* tips, const double* weights, const int32_t* children_h, const double* brlen_h, const double* model_h, int B, int R,
+                    int L, uint64_t seed, int64_t rep0, int n_rell, int32_t* branch_node_h, double* llh_h, double* nni_brlen_h, int32_t* sh_h,
+                    int32_t* lbp_h, double* site_dev, void* ws, size_t ws_bytes, cudaStream_t st);
 int gamma_rates(double alpha, int ncat, double* out);
 
 // pre-training loss over a teacher-forced rollout's logits trace (nnj_rankloss.cu)

@@ -20,102 +20,30 @@
 // invariant term; Newton scales the invariant term up by 2^(256 n) instead.  Powers of two are exact, so wherever n = 0 the
 // arithmetic is the unscaled one, bit for bit.  The CPU restatement (oracle/llh_oracle.py) applies the same rule.
 #include "nnj_internal.h"
+#include "nnj_llh.cuh"
 
 namespace nnj {
 
-constexpr int LLH_THREADS = 512;
-constexpr int LLH_MODEL = 64;      // lam 4 | U 16 | Uinv 16 | freqs 4 | class rates 4 | p_inv | alpha | flags (1 GTR rates free, 2 +G, 4 +I) | pad | 6 GTR rates | pad 10
 constexpr double RATE_LO = 1e-3, RATE_HI = 1e3, ALPHA_LO = 0.02, ALPHA_HI = 100.0, PINV_HI = 0.99, GOLD = 0.3819660112501051;   // as in oracle/llh_oracle.py
-constexpr double BRLEN_MIN = 1e-6, BRLEN_MAX = 100.0;    // every length, in evaluation and optimisation, is clamped to this range
-constexpr int SCALE_EXP = 256;
-constexpr double SCALE_BELOW = 0x1p-256, SCALE_UP = 0x1p256, SCALE_LN = 256.0 * 0.69314718055994530942;
 enum { OP_OPT = 0, OP_UP = 1, OP_DOWN = 2, OP_SWAPROOT = 3 };
 
 struct LlhArgs {
     const uint8_t* tips;        // [B][R][L] 4-bit state masks
     const double* weights;      // [B][L] pattern multiplicities
     const int32_t* children;    // [B][R-1][2]
-    const int32_t* ops;         // [B][n_ops][4] (optimise only)
+    const int32_t* ops;         // [B][n_ops][4] (optimise 1, 2: the build_ops schedule; 3: its UP and SWAPROOT rows)
     double* brlen;              // [B][2R-2] in / out
     const double* model;        // [B][LLH_MODEL]
     double *D, *U, *S, *inv;    // workspace: [B][R-1][L][16], [B][2R-2][L][16], [B][L][16], [B][L]
     int32_t *Dn, *Un, *Sn;      // scale counts of D, U and the Newton sumtable: [B][R-1][L], [B][2R-2][L], [B][L]
     double* llh;                // [B][2]: before, after
-    int B, R, L, n_ops, max_passes, optimise;     // optimise: 0 evaluate, 1 branch lengths, 2 branch lengths + model parameters
+    double* site;               // [B][L] per-pattern log-likelihood at the given lengths (optimise = 3), else null
+    int B, R, L, n_ops, max_passes, optimise;     // optimise: 0 evaluate, 1 branch lengths, 2 branch lengths + model parameters,
+                                                  // 3 evaluate and fill U for every branch (the NNI quartets of nnj_llh_nni.cu)
     double eps;
     double lh_eps; int max_rounds, golden_iters;  // optimise = 2: rounds of (free parameters one at a time, branch sweeps) until a round gains < lh_eps
     double* model_out;                            // [B][LLH_MODEL] optimised model (optimise = 2)
 };
-
-__device__ __forceinline__ double clampd(double v, double lo, double hi) { return v < lo ? lo : (v > hi ? hi : v); }
-
-// P(t)[k][a][b] = sum_j U[a][j] exp(lam_j r_k t) Uinv[j][b] for two branch lengths at once (threads 0..127), then a barrier
-__device__ __forceinline__ void pmat2(double* Pm, const double* mdl, double t0, double t1) {
-    const int i = threadIdx.x;
-    if (i < 128) {
-        const int w = i >> 6, k = (i >> 4) & 3, a = (i >> 2) & 3, b = i & 3;
-        const double t = w ? t1 : t0;
-        double s = 0.0;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) s += mdl[4 + a * 4 + j] * exp(mdl[j] * mdl[40 + k] * t) * mdl[20 + j * 4 + b];
-        Pm[i] = s;
-    }
-    __syncthreads();
-}
-
-__device__ __forceinline__ void clv_load(const LlhArgs& a, const double* Dt, const uint8_t* tips, int v, int s, double (&x)[16]) {
-    if (v < a.R) {
-        const int m = tips[(size_t)v * a.L + s];
-#pragma unroll
-        for (int k = 0; k < 4; ++k)
-#pragma unroll
-            for (int c = 0; c < 4; ++c) x[k * 4 + c] = (double)((m >> c) & 1);
-    } else {
-        const double2* p = reinterpret_cast<const double2*>(Dt + ((size_t)(v - a.R) * a.L + s) * 16);
-#pragma unroll
-        for (int i = 0; i < 8; ++i) { const double2 d = p[i]; x[2 * i] = d.x; x[2 * i + 1] = d.y; }
-    }
-}
-__device__ __forceinline__ int cnt_load(const LlhArgs& a, const int32_t* Dnt, int v, int s) { return v < a.R ? 0 : Dnt[(size_t)(v - a.R) * a.L + s]; }
-__device__ __forceinline__ void vec_load(const double* p, double (&x)[16]) {
-    const double2* q = reinterpret_cast<const double2*>(p);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) { const double2 d = q[i]; x[2 * i] = d.x; x[2 * i + 1] = d.y; }
-}
-__device__ __forceinline__ void vec_store(double* p, const double (&x)[16]) {
-    double2* q = reinterpret_cast<double2*>(p);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) q[i] = make_double2(x[2 * i], x[2 * i + 1]);
-}
-// y[k][a] = sum_b P[k][a][b] x[k][b]
-__device__ __forceinline__ void pm_apply(const double* P, const double (&x)[16], double (&y)[16]) {
-#pragma unroll
-    for (int k = 0; k < 4; ++k)
-#pragma unroll
-        for (int c = 0; c < 4; ++c) {
-            double s = 0.0;
-#pragma unroll
-            for (int b = 0; b < 4; ++b) s = fma(P[k * 16 + c * 4 + b], x[k * 4 + b], s);
-            y[k * 4 + c] = s;
-        }
-}
-
-// block-wide sums of two values in a fixed order; every thread returns with the totals.  red: 2 * 32 + 2 doubles.
-__device__ __forceinline__ void block_sum2(double& v0, double& v1, double* red) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) { v0 += __shfl_xor_sync(0xffffffffu, v0, o); v1 += __shfl_xor_sync(0xffffffffu, v1, o); }
-    const int warp = threadIdx.x >> 5;
-    if ((threadIdx.x & 31) == 0) { red[warp] = v0; red[32 + warp] = v1; }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double s0 = 0.0, s1 = 0.0;
-        for (int w = 0; w < LLH_THREADS / 32; ++w) { s0 += red[w]; s1 += red[32 + w]; }
-        red[64] = s0; red[65] = s1;
-    }
-    __syncthreads();
-    v0 = red[64]; v1 = red[65];
-    __syncthreads();
-}
 
 // ---- model parameters on the device (optimise = 2): one thread rebuilds the eigen-system and the class rates of its tree
 // regularised lower incomplete gamma P(a, x): series / continued fraction (Lentz), as gammp below on the host
@@ -245,19 +173,12 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh(const LlhArgs a) {
         pmat2(Pm, mdl, t[x], t[y]);
         for (int s = tid; s < L; s += LLH_THREADS) {
             double vx[16], vy[16], px[16], py[16];
-            if (xsrc_U) vec_load(xsrc_U + (size_t)s * 16, vx); else clv_load(a, Dt, tips, x, s, vx);
-            clv_load(a, Dt, tips, y, s, vy);
-            int n = (xsrc_U ? xsrc_Un[s] : cnt_load(a, Dnt, x, s)) + cnt_load(a, Dnt, y, s);
+            if (xsrc_U) vec_load(xsrc_U + (size_t)s * 16, vx); else clv_load(R, L, Dt, tips, x, s, vx);
+            clv_load(R, L, Dt, tips, y, s, vy);
+            int n = (xsrc_U ? xsrc_Un[s] : cnt_load(R, L, Dnt, x, s)) + cnt_load(R, L, Dnt, y, s);
             pm_apply(Pm, vx, px);
             pm_apply(Pm + 64, vy, py);
-            double mx = 0.0;
-#pragma unroll
-            for (int i = 0; i < 16; ++i) { px[i] *= py[i]; mx = fmax(mx, px[i]); }
-            if (mx < SCALE_BELOW) {
-#pragma unroll
-                for (int i = 0; i < 16; ++i) px[i] *= SCALE_UP;          // exact: a power of two
-                ++n;
-            }
+            n += mul_scaled(px, py);
             vec_store(dst_base + (size_t)s * 16, px);
             dst_n[s] = n;
         }
@@ -272,20 +193,21 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh(const LlhArgs a) {
         double acc = 0.0, dummy = 0.0;
         for (int s = tid; s < L; s += LLH_THREADS) {
             double v1[16], v2[16], p1[16];
-            clv_load(a, Dt, tips, c1, s, v1);
-            clv_load(a, Dt, tips, c2, s, v2);
+            clv_load(R, L, Dt, tips, c1, s, v1);
+            clv_load(R, L, Dt, tips, c2, s, v2);
             pm_apply(Pm, v1, p1);
             double l = 0.0;
 #pragma unroll
             for (int k = 0; k < 4; ++k)
 #pragma unroll
                 for (int c = 0; c < 4; ++c) l = fma(mdl[36 + c] * p1[k * 4 + c], v2[k * 4 + c], l);
-            const int n = cnt_load(a, Dnt, c1, s) + cnt_load(a, Dnt, c2, s);
+            const int n = cnt_load(R, L, Dnt, c1, s) + cnt_load(R, L, Dnt, c2, s);
             double site;
             if (n == 0) site = log(wk * l + pinv * invt[s]);
             else if (pinv * invt[s] == 0.0) site = log(wk * l) - n * SCALE_LN;
             else site = log(ldexp(wk * l, -SCALE_EXP * n) + pinv * invt[s]);
             acc += wts[s] * site;
+            if (a.site) a.site[(size_t)b * L + s] = site;
         }
         block_sum2(acc, dummy, red);
         return acc;
@@ -299,9 +221,9 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh(const LlhArgs a) {
             // U[c1] = D[c2]
             for (int s = tid; s < L; s += LLH_THREADS) {
                 double v2[16];
-                clv_load(a, Dt, tips, c2, s, v2);
+                clv_load(R, L, Dt, tips, c2, s, v2);
                 vec_store(Ut + ((size_t)c1 * L + s) * 16, v2);
-                Unt[(size_t)c1 * L + s] = cnt_load(a, Dnt, c2, s);
+                Unt[(size_t)c1 * L + s] = cnt_load(R, L, Dnt, c2, s);
             }
             for (int oi = 0; oi < a.n_ops; ++oi) {
                 const int op = ops[oi * 4], v = ops[oi * 4 + 1], x = ops[oi * 4 + 2], y = ops[oi * 4 + 3];
@@ -312,63 +234,21 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh(const LlhArgs a) {
                 } else if (op == OP_SWAPROOT) {
                     for (int s = tid; s < L; s += LLH_THREADS) {
                         double v1[16];
-                        clv_load(a, Dt, tips, x, s, v1);
+                        clv_load(R, L, Dt, tips, x, s, v1);
                         vec_store(Ut + ((size_t)v * L + s) * 16, v1);
-                        Unt[(size_t)v * L + s] = cnt_load(a, Dnt, x, s);
+                        Unt[(size_t)v * L + s] = cnt_load(R, L, Dnt, x, s);
                     }
                 } else {
                     // ---- Newton-Raphson on the branch above v.  Sumtable S[s][k][j] = (sum_a pi_a U[a] Umat[a][j]) (sum_b Uinv[j][b] D[b])
                     for (int s = tid; s < L; s += LLH_THREADS) {
                         double u[16], d[16], sv[16];
                         vec_load(Ut + ((size_t)v * L + s) * 16, u);
-                        clv_load(a, Dt, tips, v, s, d);
-#pragma unroll
-                        for (int k = 0; k < 4; ++k)
-#pragma unroll
-                            for (int j = 0; j < 4; ++j) {
-                                double A = 0.0, Bm = 0.0;
-#pragma unroll
-                                for (int c = 0; c < 4; ++c) {
-                                    A = fma(mdl[36 + c] * u[k * 4 + c], mdl[4 + c * 4 + j], A);
-                                    Bm = fma(mdl[20 + j * 4 + c], d[k * 4 + c], Bm);
-                                }
-                                sv[k * 4 + j] = A * Bm;
-                            }
+                        clv_load(R, L, Dt, tips, v, s, d);
+                        sumtable_row(mdl, u, d, sv);
                         vec_store(St + (size_t)s * 16, sv);
-                        Snt[s] = Unt[(size_t)v * L + s] + cnt_load(a, Dnt, v, s);
+                        Snt[s] = Unt[(size_t)v * L + s] + cnt_load(R, L, Dnt, v, s);
                     }
-                    double tv = t[v], lo = BRLEN_MIN, hi = BRLEN_MAX;
-                    for (int it = 0; it < 32; ++it) {
-                        if (tid < 16) {
-                            const double rate = mdl[tid & 3] * mdl[40 + (tid >> 2)];
-                            ek[tid] = exp(rate * tv); ek[16 + tid] = rate; ek[32 + tid] = rate * rate;
-                        }
-                        __syncthreads();
-                        double f1 = 0.0, f2 = 0.0;
-                        for (int s = tid; s < L; s += LLH_THREADS) {
-                            double sv[16];
-                            vec_load(St + (size_t)s * 16, sv);
-                            double l0 = 0.0, l1 = 0.0, l2 = 0.0;
-#pragma unroll
-                            for (int i = 0; i < 16; ++i) {
-                                const double se = sv[i] * ek[i];
-                                l0 += se; l1 = fma(se, ek[16 + i], l1); l2 = fma(se, ek[32 + i], l2);
-                            }
-                            // a scaled pattern: its invariant term scaled up to match (inf where that overflows: then g = 0, and no 0 * inf)
-                            const int n = Snt[s];
-                            const double L0 = n == 0 ? wk * l0 + pinv * invt[s] : wk * l0 + (invt[s] > 0.0 ? ldexp(pinv * invt[s], SCALE_EXP * n) : 0.0);
-                            const double g = wk * l1 / L0;
-                            f1 = fma(wts[s], g, f1);
-                            f2 = fma(wts[s], wk * l2 / L0 - g * g, f2);
-                        }
-                        block_sum2(f1, f2, red);
-                        if (f1 > 0.0) lo = tv; else hi = tv;
-                        double tn = f2 < 0.0 ? tv - f1 / f2 : (f1 > 0.0 ? tv * 4.0 : tv * 0.25);
-                        if (!(tn > lo && tn < hi)) tn = 0.5 * (lo + hi);
-                        const bool done = fabs(tn - tv) < 1e-9 + 1e-7 * tv;
-                        tv = tn;
-                        if (done) break;
-                    }
+                    const double tv = newton_brlen(St, Snt, mdl, ek, red, wts, invt, pinv, wk, L, t[v]);
                     if (tid == 0) { t[v] = tv; if (v == c1) t[c2] = tv; }
                     __syncthreads();
                 }
@@ -379,7 +259,9 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh(const LlhArgs a) {
             if (gain < a.eps) break;
         }
     };
-    if (a.optimise) {
+    if (a.optimise == 3) {
+        sweeps();             // max_passes = 1 and only UP / SWAPROOT rows: one pass fills U[v] for every v at the given lengths
+    } else if (a.optimise) {
         sweeps();
         if (a.optimise == 2) {
             // ---- model parameters: rounds of (every free parameter by golden section, all else fixed; branch sweeps) until a round
@@ -476,7 +358,7 @@ static int build_ops(const int32_t* ch, int R, std::vector<int32_t>& ops) {
     return (int)(ops.size() / 4);
 }
 
-static int check_tree(const int32_t* ch, int R) {
+int llh_check_tree(const int32_t* ch, int R) {
     std::vector<char> used(2 * R - 1, 0);
     for (int k = 0; k < R - 1; ++k)
         for (int e = 0; e < 2; ++e) {
@@ -489,14 +371,21 @@ static int check_tree(const int32_t* ch, int R) {
 
 int run_llh(const uint8_t* tips, const double* weights, const int32_t* children_h, double* brlen_h, double* model_h, int B, int R, int L,
             int optimise, int max_passes, double eps, double lh_eps, int max_rounds, int golden_iters, double* llh_h, void* ws, size_t ws_bytes,
-            cudaStream_t st) {
+            cudaStream_t st, double* site_dev, LlhState* state) {
     std::vector<int32_t> ops_all;
     int n_ops = 0;
     for (int b = 0; b < B; ++b) {
-        if (check_tree(children_h + (size_t)b * (R - 1) * 2, R)) return set_error(NNJ_ERR_INVALID, "llh: children is not a binary tree in join order");
+        if (llh_check_tree(children_h + (size_t)b * (R - 1) * 2, R)) return set_error(NNJ_ERR_INVALID, "llh: children is not a binary tree in join order");
         if (optimise) {
             std::vector<int32_t> ops;
-            const int n = build_ops(children_h + (size_t)b * (R - 1) * 2, R, ops);
+            int n = build_ops(children_h + (size_t)b * (R - 1) * 2, R, ops);
+            if (optimise == 3) {           // the U pass alone: UP and SWAPROOT rows, no Newton, no refreshed subtree vectors
+                std::vector<int32_t> keep;
+                for (int i = 0; i < n; ++i)
+                    if (ops[4 * i] == OP_UP || ops[4 * i] == OP_SWAPROOT) keep.insert(keep.end(), ops.begin() + 4 * i, ops.begin() + 4 * i + 4);
+                ops.swap(keep);
+                n = (int)(ops.size() / 4);
+            }
             if (b == 0) n_ops = n;
             if (n != n_ops) return set_error(NNJ_ERR_INVALID, "llh: internal error (schedule length differs between trees)");
             ops_all.insert(ops_all.end(), ops.begin(), ops.end());
@@ -524,7 +413,9 @@ int run_llh(const uint8_t* tips, const double* weights, const int32_t* children_
     if (e == cudaSuccess) e = cudaMemcpyAsync(d_br, brlen_h, (size_t)B * (2 * R - 2) * 8, cudaMemcpyHostToDevice, st);
     if (e == cudaSuccess) e = cudaMemcpyAsync(d_md, model_h, (size_t)B * LLH_MODEL * 8, cudaMemcpyHostToDevice, st);
     if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
-    a.children = d_ch; a.ops = d_ops; a.brlen = d_br; a.model = d_md; a.llh = d_ll;
+    a.children = d_ch; a.ops = d_ops; a.brlen = d_br; a.model = d_md; a.llh = d_ll; a.site = optimise == 3 ? site_dev : nullptr;
+    if (optimise == 3) max_passes = 1;
+    if (state) { state->D = a.D; state->U = a.U; state->inv = a.inv; state->Dn = a.Dn; state->Un = a.Un; }
     a.B = B; a.R = R; a.L = L; a.n_ops = n_ops; a.max_passes = max_passes; a.optimise = optimise; a.eps = eps;
     a.lh_eps = lh_eps; a.max_rounds = max_rounds; a.golden_iters = golden_iters; a.model_out = d_md;
     const size_t smem = (LLH_MODEL + 128 + 66 + 48 + 2 * (size_t)R) * sizeof(double);      // 67 968 bytes at R = 4096
@@ -538,7 +429,7 @@ int run_llh(const uint8_t* tips, const double* weights, const int32_t* children_
     prof_end(st);
     e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaMemcpyAsync(llh_h, d_ll, (size_t)B * 2 * 8, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess && optimise) e = cudaMemcpyAsync(brlen_h, d_br, (size_t)B * (2 * R - 2) * 8, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess && (optimise == 1 || optimise == 2)) e = cudaMemcpyAsync(brlen_h, d_br, (size_t)B * (2 * R - 2) * 8, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess && optimise == 2) e = cudaMemcpyAsync(model_h, d_md, (size_t)B * LLH_MODEL * 8, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);       // the small results are host values: the call returns them
     if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);

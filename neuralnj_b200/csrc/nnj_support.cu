@@ -27,22 +27,6 @@ constexpr int SPLIT_THREADS = 256;
 constexpr int SPLIT_MAX_WORDS = 8;                   // R <= 512
 constexpr int SPLIT_MAX_TAXA = 64 * SPLIT_MAX_WORDS;
 
-// Philox4x32-10 (Salmon et al., SC 2011; the constants of Random123), word 0 of the output block.
-__device__ __forceinline__ uint32_t philox_x0(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1) {
-#pragma unroll
-    for (int round = 0; round < 10; ++round) {
-        const uint32_t lo0 = 0xD2511F53u * c0, hi0 = __umulhi(0xD2511F53u, c0);
-        const uint32_t lo1 = 0xCD9E8D57u * c2, hi1 = __umulhi(0xCD9E8D57u, c2);
-        c0 = hi1 ^ c1 ^ k0;
-        c1 = lo1;
-        c2 = hi0 ^ c3 ^ k1;
-        c3 = lo0;
-        k0 += 0x9E3779B9u;
-        k1 += 0xBB67AE85u;
-    }
-    return c0;
-}
-
 // out[b][t][c] (4-byte one-hot words) = data[t][src(rep0 + b, c)][:]; one thread per (replicate, column), writes coalesced along c
 __global__ void __launch_bounds__(BOOT_THREADS) k_boot_columns(const uint32_t* __restrict__ data, int R, int L, int l_eff, uint64_t seed,
                                                               int64_t rep0, int B, uint32_t* __restrict__ out) {

@@ -230,6 +230,75 @@ def tuples_to_newick(t) -> str:
     return fmt(t) + ";"
 
 
+# ------------------------------------------------------------------ NNI quartets (DESIGN.md 12)
+def internal_branches(children) -> List[int]:
+    """The R-3 internal branches of a tree as the inner node v below each, in increasing v: every inner node but the root, where
+    the root branch counts once, at the first root child c1, and only when both root children are inner."""
+    children = np.asarray(children)
+    R = len(children) + 1
+    c1, c2 = (int(c) for c in children[-1])
+    return [v for v in range(R, 2 * R - 2) if v not in (c1, c2) or (v == c1 and c2 >= R)]
+
+
+def quartet(children, v: int) -> Tuple[Tuple[int, int, int, int], Tuple[int, int, int, int, int]]:
+    """The quartet around the branch above v -> ((a, b, c, d), edges).  a, b are v's children, c its sibling and d its parent p,
+    whose outer vector is U[p] (the rest of the tree); for the root branch (v = c1) c and d are the children of c2.  `edges` are the
+    nodes whose brlen entries hold the central, A, B, C and D lengths (v, a, b, c, p; the root branch is brlen[c1] + brlen[c2])."""
+    children = np.asarray(children)
+    R = len(children) + 1
+    c1, c2 = (int(c) for c in children[-1])
+    a, b = (int(c) for c in children[v - R])
+    if v == c1:
+        c, d = (int(x) for x in children[c2 - R])
+        return (a, b, c, d), (v, a, b, c, d)
+    p = next(R + k for k, pair in enumerate(children.tolist()) if v in pair)
+    pa, pb = (int(x) for x in children[p - R])
+    c = pb if pa == v else pa
+    return (a, b, c, p), (v, a, b, c, p)
+
+
+def nni_tree(children, v: int, k: int, brlen=None):
+    """Alternative k (1: AC|BD, 2: AD|BC) of the branch above v as a join-order children array; k = 0 is the tree itself (renumbered
+    the same way).  Alternative 1 swaps B and C, alternative 2 swaps A and C.  With `brlen`, also returns the lengths carried over:
+    the branch above every node keeps its length (the nodes are renumbered, their edges are not)."""
+    children = np.asarray(children)
+    R = len(children) + 1
+    kids = {R + j: [int(x), int(y)] for j, (x, y) in enumerate(children.tolist())}
+    (a, b, c, _), _ = quartet(children, v)
+    c1, c2 = (int(x) for x in children[-1])
+    holder = c2 if v == c1 else next(u for u, pair in kids.items() if v in pair)      # the node c hangs below
+    if k in (1, 2):
+        mine = b if k == 1 else a
+        kids[v][kids[v].index(mine)] = c
+        kids[holder][kids[holder].index(c)] = mine
+    elif k != 0:
+        raise ValueError("k must be 0, 1 or 2")
+    new_id, out = {u: u for u in range(R)}, []
+
+    def visit(u):
+        stack = [(u, False)]
+        while stack:
+            x, done = stack.pop()
+            if x < R:
+                continue
+            if done:
+                new_id[x] = R + len(out)
+                out.append((new_id[kids[x][0]], new_id[kids[x][1]]))
+            else:
+                stack.append((x, True))
+                stack.append((kids[x][1], False))
+                stack.append((kids[x][0], False))
+
+    visit(2 * R - 2)
+    ch = np.asarray(out, dtype=np.int32)
+    if brlen is None:
+        return ch
+    bl = np.zeros(2 * R - 2)
+    for u in range(2 * R - 2):
+        bl[new_id[u]] = brlen[u]
+    return ch, bl
+
+
 # ------------------------------------------------------------------ engine
 class TreeLikelihood:
     """B trees over alignments of one shape, scored together (one CTA per tree)."""
@@ -309,6 +378,44 @@ class TreeLikelihood:
         < lh_eps - per tree, entirely inside the kernel (nnj_llh_optimize_all: eigen-system and class rates are rebuilt on the
         device, no host round trips).  Updates `model` in place.  -> (brlen_opt, llh_before, llh_after)"""
         return self._call("all", children, brlen, model, max_passes, eps, lh_eps, max_rounds)
+
+
+    def nni_support(self, children, brlen, model: SubstModel, n_rell: int, seed: int, rep0: int = 0, site_llh: bool = False) -> dict:
+        """Likelihood support of the R-3 internal branches of B trees (nnj_llh_branch_support, DESIGN.md 12) at the given lengths and
+        model, which should be optimised already (optimize_all).  -> dict of numpy arrays: branch_node [B, R-3], llh [B, R-3, 3]
+        (L0, L1, L2), nni_brlen [B, R-3, 2, 5], sh_count and lbp_count [B, R-3] over replicates rep0 .. rep0+n_rell-1, and with
+        site_llh=True the per-pattern log-likelihoods [B, R-3, 3, L] as a device tensor."""
+        children = np.ascontiguousarray(children, dtype=np.int32)
+        B, R, L = children.shape[0], self.R, self.L
+        brlen = np.ascontiguousarray(brlen, dtype=np.float64)
+        if children.shape != (B, R - 1, 2) or brlen.shape != (B, 2 * R - 2) or model.B != B:
+            raise ValueError("children must be [B, R-1, 2], brlen [B, 2R-2], one model row per tree")
+        if not 0 <= int(seed) < 2 ** 64 or int(rep0) < 0 or int(n_rell) < 0:
+            raise ValueError("need 0 <= seed < 2^64, rep0 >= 0, n_rell >= 0")
+        nb = max(R - 3, 0)
+        tips, w = self._staged(B)
+        lib = _lib.lib()
+        need = int(lib.nnj_llh_support_workspace_bytes(B, R, L, int(n_rell)))
+        if need < 0:
+            raise _lib.NnjError("nnj_llh_support_workspace_bytes: bad shape")
+        if self._ws is None or self._ws.numel() < need:
+            self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+        ws = self._ws
+        packed = model.pack()
+        out = dict(branch_node=np.zeros((B, nb), dtype=np.int32), llh=np.zeros((B, nb, 3)), nni_brlen=np.zeros((B, nb, 2, 5)),
+                   sh_count=np.zeros((B, nb), dtype=np.int32), lbp_count=np.zeros((B, nb), dtype=np.int32))
+        site = torch.empty((B, nb, 3, L), dtype=torch.float64, device=self.device) if site_llh and nb else None
+        vp = C.c_void_p
+        ptr = [out[k].ctypes.data_as(vp) for k in ("branch_node", "llh", "nni_brlen", "sh_count", "lbp_count")]
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream(self.device).cuda_stream
+            rc = lib.nnj_llh_branch_support(vp(tips.data_ptr()), vp(w.data_ptr()), children.ctypes.data_as(vp), brlen.ctypes.data_as(vp),
+                                            packed.ctypes.data_as(vp), B, R, L, C.c_uint64(int(seed)), int(rep0), int(n_rell), *ptr,
+                                            vp(site.data_ptr() if site is not None else 0), vp(ws.data_ptr()), ws.numel(), vp(stream))
+        _lib.check(rc, "nnj_llh_branch_support")
+        if site_llh:
+            out["site_llh"] = site if site is not None else torch.empty((B, 0, 3, L), dtype=torch.float64, device=self.device)
+        return out
 
 
 # ------------------------------------------------------------------ raxmlpy-compatible entry points

@@ -174,7 +174,8 @@ def _rank_share(items):
 
 
 def Argmax_inference(test_file_path, write_dir, write_file_name=None, branch_optimize=False, cfgs=None, device=None, precision=None,
-                     files_per_call=1, policy_network=None, bootstrap=0, bootstrap_seed=0):
+                     files_per_call=1, policy_network=None, bootstrap=0, bootstrap_seed=0,
+                     alrt=0, alrt_seed=0):
     """One `.tre` per `.phy` of a directory (finetune_rl_search.py:478-509).
 
     `files_per_call=1` is the reference's loop: one alignment per call (expanded to `cfgs.env.batch_size` copies, :444).
@@ -186,7 +187,10 @@ def Argmax_inference(test_file_path, write_dir, write_file_name=None, branch_opt
 
     `bootstrap=N` (not a reference argument) also writes `<name>.fbp.tre` and `<name>.tbe.tre` beside each `<name>.tre`: the same tree
     with FBP / TBE support from N bootstrap replicates drawn with `bootstrap_seed` (`neuralnj_b200.support`).  A file's replicates
-    run on the rank that owns the file."""
+    run on the rank that owns the file.
+
+    `alrt=N` (not a reference argument) also writes `<name>.alrt.tre` (SH-aLRT from N RELL replicates drawn with `alrt_seed`) and
+    `<name>.abayes.tre` (aBayes): the tree with its branch lengths and model optimised (`neuralnj_b200.support.likelihood_support`)."""
     c = _cfg(cfgs)
     if device is None:                # one process per GPU under torchrun: the rank's own device
         import torch.distributed as dist
@@ -199,6 +203,12 @@ def Argmax_inference(test_file_path, write_dir, write_file_name=None, branch_opt
     written = []
 
     def write_support(file, msa, tree):
+        if alrt > 0:
+            from .support import likelihood_support
+            res = likelihood_support(msa, policy, tree=tree, n_rell=alrt, seed=alrt_seed)
+            for kind in ("alrt", "abayes"):
+                with open(os.path.join(write_dir, f"{file[:-4]}.{kind}.tre"), "w") as f:
+                    f.write(res["newick_" + kind])
         if bootstrap <= 0:
             return
         res = _support(msa, policy, bootstrap, bootstrap_seed, tree, None)     # no replicate sharding: the file is this rank's
@@ -335,9 +345,14 @@ def main(argv=None):
     ap.add_argument("--bootstrap", type=int, default=0,
                     help="Argmax: also write <name>.fbp.tre / <name>.tbe.tre with support from N bootstrap replicates (not a reference flag)")
     ap.add_argument("--bootstrap_seed", type=int, default=0, help="seed of the bootstrap replicates (not a reference flag)")
+    ap.add_argument("--alrt", type=int, default=0,
+                    help="Argmax: also write <name>.alrt.tre / <name>.abayes.tre with SH-aLRT from N RELL replicates and aBayes (not a reference flag)")
+    ap.add_argument("--alrt_seed", type=int, default=0, help="seed of the RELL replicates (not a reference flag)")
     args = ap.parse_args(argv)
     if args.bootstrap and args.infer_opt != "Argmax":
         raise SystemExit("--bootstrap applies to --infer_opt Argmax")
+    if args.alrt and args.infer_opt != "Argmax":
+        raise SystemExit("--alrt applies to --infer_opt Argmax")
     PRECISION = args.precision
     cfgs = empty_config()
     if args.config_path:
@@ -347,7 +362,7 @@ def main(argv=None):
     write_dir = f"output/{args.infer_opt}_dim{cfgs.model.embed_dim}_patch{cfgs.model.patch_size}/{name}"
     if args.infer_opt == "Argmax":
         return Argmax_inference(cfgs.instance_path, write_dir, None, branch_optimize=args.branch_optimize, files_per_call=args.files_per_call,
-                                bootstrap=args.bootstrap, bootstrap_seed=args.bootstrap_seed)
+                                bootstrap=args.bootstrap, bootstrap_seed=args.bootstrap_seed, alrt=args.alrt, alrt_seed=args.alrt_seed)
     if args.infer_opt == "Search":
         return Search_inference(cfgs.instance_path, write_dir, None)
     raise SystemExit(f'--infer_opt {args.infer_opt}: "Finetune" (NeuralNJ-RL) trains the policy and is outside this path')

@@ -10,6 +10,9 @@ transfer distances of the reference splits to the replicate trees are computed o
 (`nnj_split_distances`); per chunk of CHUNK replicates only the int64 totals [2, S] stay behind, and merge lists never reach the
 host.  Definitions: DESIGN.md section 11.  A replicate depends only on (seed, replicate index, real column count), so the chunk
 size and the number of ranks do not change any result.
+
+`likelihood_support` puts aLRT, SH-aLRT, aBayes and the local bootstrap probability on the branches of one tree instead (DESIGN.md
+section 12): no rollouts, the NNI alternatives of every branch and RELL replicates on the device, trees up to 4096 taxa.
 """
 from __future__ import annotations
 
@@ -232,3 +235,90 @@ def _support(msa, policy_network, n_replicates: int, seed: int, tree: Optional[s
     return dict(tree=tree, splits=[frozenset(keys[i] for i in sp) for sp in splits], fbp=fbp, tbe=tbe,
                 newick_fbp=label_newick(tree, labelled, fbp_labels), newick_tbe=label_newick(tree, labelled, tbe_labels),
                 n_replicates=N, seed=seed)
+
+
+# ---------------------------------------------------------------------------------------------------------- likelihood support
+
+def likelihood_support(msa, policy_network=None, tree: Optional[str] = None, n_rell: int = 1000, seed: int = 0, model: str = "GTR+I+G") -> dict:
+    """Likelihood branch support (DESIGN.md 12) of one tree: aLRT, SH-aLRT, aBayes and the local bootstrap probability (LBP) of
+    every internal branch - what IQ-TREE reports with `-alrt 1000 -abayes`.
+
+    `msa` is a path or a `load_pi_instance` batch of one alignment.  `tree=None` builds the Argmax tree of `policy_network` (at most
+    400 taxa, the rollout's limit); a given Newick `tree` may have up to 4096 taxa.  The branch lengths and model parameters are
+    optimised first (`TreeLikelihood.optimize_all`), then the two NNI alternatives of every internal branch are optimised and
+    n_rell RELL replicates drawn with `seed` (`TreeLikelihood.nni_support`), all on the device.
+
+    Returns `tree` (unrooted Newick with the optimised lengths), `splits` (light sides as frozensets of taxon names), per split
+    `alrt` (2 delta), `sh_alrt` and `lbp` (percent), `abayes`, `llh_nni` [S, 2] (L1, L2), and `llh` (L0), `n_better_nni` (splits
+    where an NNI has the higher likelihood, delta < 0), `newick_alrt` (SH-aLRT, %.1f) and `newick_abayes` (%.3f), `n_rell`, `seed`."""
+    from . import likelihood as LH
+    from .treeutil import treestr_to_tuples
+    if int(n_rell) < 1:
+        raise ValueError("n_rell must be >= 1")
+    if not 0 <= int(seed) < 2 ** 64:
+        raise ValueError("seed must be in [0, 2^64)")
+    N, seed = int(n_rell), int(seed)
+    batch = load_pi_instance(os.fspath(msa)) if isinstance(msa, (str, os.PathLike)) else msa
+    if batch["data"].shape[0] != 1:
+        raise ValueError("likelihood_support takes one alignment")
+    R = batch["data"].shape[1]
+    if R > 4096:
+        raise ValueError(f"likelihood_support: {R} taxa, the tree likelihood supports at most 4096")
+    keys = [str(k) for k in batch["seq_keys"][0]]
+    real = (batch["seq_weights"][0] != 0).cpu().numpy()
+    if tree is None:
+        if policy_network is None:
+            raise ValueError("likelihood_support: tree=None needs a policy_network to build the Argmax tree")
+        device = next(policy_network.parameters()).device
+        data = batch["data"][0].to(device=device, dtype=torch.int8).contiguous()
+        with torch.no_grad():
+            merges, _, _ = policy_network.rollout_fused(data[None], torch.from_numpy(~real).to(device)[None])
+        env = PhyInferEnv(empty_config(), device)
+        env.init_states(batch["seqs"], batch["seq_keys"], batch["data"])
+        env.replay_merges(merges)
+        tree = env.states[0].subtrees[0].utree_op_str
+    else:
+        device = next(policy_network.parameters()).device if policy_network is not None else torch.device("cuda")
+    masks = LH.onehot_to_masks(batch["data"][0])[:, real]
+    pats, w = LH.compress_patterns(masks)
+    children, brlen = LH.tree_arrays_from_tuples(treestr_to_tuples(tree), keys)
+    ch = children[None]
+    eng = LH.TreeLikelihood(pats, w, device=device)
+    sm = LH.SubstModel(model, LH.empirical_freqs(masks), 1)
+    t, _, ll = eng.optimize_all(ch, brlen[None], sm)
+    res = eng.nni_support(ch, t, sm, N, seed)
+    out_tree = LH.tuples_to_newick(LH.tuples_with_lengths(children, t[0], keys, unrooted=True))
+    splits, labelled = reference_splits(out_tree, keys)
+    S = len(splits)
+    where = {sp: k for k, sp in enumerate(splits)}
+    everything = frozenset(range(R))
+    order = np.zeros(S, dtype=np.int64)
+    nodes = res["branch_node"][0]
+    if len(nodes) != S:
+        raise NnjError(f"likelihood_support: {len(nodes)} internal branches but {S} splits in the tree")
+    for i, v in enumerate(nodes.tolist()):
+        clade = frozenset(_leaves_below(children, int(v)))
+        light = min(clade, everything - clade, key=lambda x: (len(x), sorted(keys[j] for j in x)))
+        order[where[light]] = i
+    llh3 = res["llh"][0][order]
+    delta = llh3[:, 0] - np.maximum(llh3[:, 1], llh3[:, 2])
+    with np.errstate(over="ignore"):
+        abayes = 1.0 / (1.0 + np.exp(llh3[:, 1] - llh3[:, 0]) + np.exp(llh3[:, 2] - llh3[:, 0]))
+    sh = 100.0 * res["sh_count"][0][order] / N
+    lbp = 100.0 * res["lbp_count"][0][order] / N
+    return dict(tree=out_tree, splits=[frozenset(keys[i] for i in sp) for sp in splits], alrt=2.0 * delta, sh_alrt=sh, abayes=abayes, lbp=lbp,
+                llh_nni=llh3[:, 1:].copy(), llh=float(ll[0]), n_better_nni=int((delta < 0).sum()),
+                newick_alrt=label_newick(out_tree, labelled, [f"{x:.1f}" for x in sh]),
+                newick_abayes=label_newick(out_tree, labelled, [f"{x:.3f}" for x in abayes]), n_rell=N, seed=seed)
+
+
+def _leaves_below(children, v: int) -> List[int]:
+    R = len(children) + 1
+    out, stack = [], [v]
+    while stack:
+        x = stack.pop()
+        if x < R:
+            out.append(x)
+        else:
+            stack.extend(int(c) for c in children[x - R])
+    return out
