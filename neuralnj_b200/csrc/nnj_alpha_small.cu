@@ -1,4 +1,4 @@
-// nnj_alpha_small.cu — pair blend + global-attention logits for the LATE steps of the NJ loop (<= 32 pairs, <= 32 live nodes).
+// nnj_alpha_small.cu — pair blend + global-attention logits for the LATE steps of the NJ loop (<= 16 pairs, <= 16 live nodes).
 //
 // Same arithmetic as k_alpha_v3 (model.py:105-118):
 //     z = sigmoid(Y_i - Y_j + b_h),   x = z x_i + (1 - z) x_j                         per listed pair and site
@@ -10,7 +10,7 @@
 // pair-score kernel reads), K' rows are the B fragments (4-byte loads), and the [pairs x slots] accumulator stays in the warp's
 // registers across all its sites (3-term bf16 split, fp32 accumulate).  The warps' accumulators are summed in fixed order into the
 // ONE partial of the site group (bit-reproducible), indexed by physical slot like k_alpha_v3's.
-// CTA = (tree, 128-site group); T = 1: <= 16 pairs / slots, 16 warps; T = 2: <= 32, 8 warps.
+// CTA = (tree, 128-site group), 16 warps; T = 1 row tile of 16 pairs over 16 slots.
 #include "nnj_internal.h"
 #include "nnj_tc.cuh"
 
@@ -171,23 +171,10 @@ __global__ void __launch_bounds__(WARPS * 32, 1) k_alpha_small(const AlphaSmallA
     }
 }
 
-template <int T, int W>
-static int launch_alpha_small_t(const AlphaSmallArgs& a, int groups, int B, cudaStream_t st) {
-    constexpr size_t smem = 1024 + 1024 + (size_t)W * (16 * T * 768);
-    static DevOnce once;      // per device, not per process
-    if (once.need()) {
-        cudaError_t e = cudaFuncSetAttribute(k_alpha_small<T, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
-        once.done();
-    }
-    k_alpha_small<T, W><<<dim3(groups, B), W * 32, smem, st>>>(a);
-    return 0;
-}
-
 int launch_alpha_small(const Model* m, const float* X, const float* Y, size_t tree_stride, const int32_t* slot_of, int slot_stride, const int32_t* pair_i,
                        const int32_t* pair_j, int pair_stride, int n0, int nc, int S, int n_live, int C, int B, const void* kp_h, const void* kp_l, float* xf,
                        int pc, float* alpha_part, int alpha_pairs, int nSG, int RP, int* n_part, cudaStream_t st) {
-    if (nc > 32 || n_live > 32 || nc < 1 || nc > pc) return set_error(NNJ_ERR_INVALID, "alpha_small: at most 32 pairs over 32 live nodes");
+    if (nc > 16 || n_live > 16 || nc < 1 || nc > pc) return set_error(NNJ_ERR_INVALID, "alpha_small: at most 16 pairs over 16 live nodes");
     const int groups = (C + AS_SITES - 1) / AS_SITES;
     *n_part = groups;
     if (groups > nSG) return set_error(NNJ_ERR_INVALID, "alpha_small: partial buffer too small");
@@ -195,11 +182,17 @@ int launch_alpha_small(const Model* m, const float* X, const float* Y, size_t tr
     a.X = X; a.Y = Y; a.tree_stride = tree_stride; a.kph = (const __nv_bfloat16*)kp_h; a.kpl = (const __nv_bfloat16*)kp_l; a.S = S;
     a.slot_of = slot_of; a.slot_stride = slot_stride; a.pair_i = pair_i; a.pair_j = pair_j; a.pair_stride = pair_stride; a.n0 = n0; a.nc = nc;
     a.Rp = n_live; a.C = C; a.bh = m->nj.bh; a.xf = xf; a.pc = pc; a.alpha_part = alpha_part; a.alpha_pairs = alpha_pairs; a.nSG = nSG; a.RP = RP;
+    constexpr size_t smem = 1024 + 1024 + 16 * (16 * 768);      // alignment | biases, pair slots | 16 warps x one site buffer (X, Y, K' hi / lo)
+    static DevOnce once;      // per device, not per process
+    if (once.need()) {
+        cudaError_t e = cudaFuncSetAttribute(k_alpha_small<1, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
+        once.done();
+    }
     prof_begin(KC_ALPHA, st);
-    const int rc = (nc <= 16 && n_live <= 16) ? launch_alpha_small_t<1, 16>(a, groups, B, st) : launch_alpha_small_t<2, 8>(a, groups, B, st);
+    k_alpha_small<1, 16><<<dim3(groups, B), 16 * 32, smem, st>>>(a);
     ++g_launches;
     prof_end(st);
-    if (rc) return rc;
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
     return 0;

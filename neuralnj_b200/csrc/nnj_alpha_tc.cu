@@ -328,73 +328,41 @@ k_alpha_v3(const __grid_constant__ CUtensorMap mapX, const __grid_constant__ CUt
 }
 
 // ------------------------------------------------------------------ host side
-typedef CUresult (*PFN_enc)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                            const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static PFN_enc get_enc() {
-    static PFN_enc enc = nullptr;
-    if (!enc) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-            enc = reinterpret_cast<PFN_enc>(p);
-    }
-    return enc;
-}
-
 // fp32 node pool [B][S][C][64] (tree stride given) as a 4-D tensor (d, site, slot, tree); box = 32 channels of all slots at one site
 static int make_tmap_pool_f32(CUtensorMap* map, const float* base, size_t tree_stride, int S, int C, int B, int box_rows) {
-    PFN_enc enc = get_enc();
-    if (!enc) return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
-    cuuint64_t gdim[4] = {64, (cuuint64_t)C, (cuuint64_t)S, (cuuint64_t)B};
-    cuuint64_t gstr[3] = {256, (cuuint64_t)C * 256, (cuuint64_t)tree_stride * 4};
-    cuuint32_t box[4] = {32, 1, (cuuint32_t)box_rows, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled failed for the fp32 node pool");
-    return 0;
+    const cuuint64_t gdim[4] = {64, (cuuint64_t)C, (cuuint64_t)S, (cuuint64_t)B};
+    const cuuint64_t gstr[3] = {256, (cuuint64_t)C * 256, (cuuint64_t)tree_stride * 4};
+    const cuuint32_t box[4] = {32, 1, (cuuint32_t)box_rows, 1};
+    return encode_tmap(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, base, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                       "the fp32 node pool");
 }
 
 // x planes [B][pc][C][64] fp32 as a 4-D tensor (d, site, pair, tree); store box = 16 channels of 32 pairs at one site (SWIZZLE_64B)
 static int make_tmap_xplanes(CUtensorMap* map, float* base, int pc, int nrows, int C, int B) {
-    PFN_enc enc = get_enc();
-    if (!enc) return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
-    cuuint64_t gdim[4] = {64, (cuuint64_t)C, (cuuint64_t)nrows, (cuuint64_t)B};   // rows past the pair list are clipped by the map
-    cuuint64_t gstr[3] = {256, (cuuint64_t)C * 256, (cuuint64_t)pc * C * 256};
-    cuuint32_t box[4] = {16, 1, 32, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, base, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled failed for the x planes");
-    return 0;
+    const cuuint64_t gdim[4] = {64, (cuuint64_t)C, (cuuint64_t)nrows, (cuuint64_t)B};   // rows past the pair list are clipped by the map
+    const cuuint64_t gstr[3] = {256, (cuuint64_t)C * 256, (cuuint64_t)pc * C * 256};
+    const cuuint32_t box[4] = {16, 1, 32, 1};
+    return encode_tmap(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, base, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
+                       "the x planes");
 }
 
 // K' planes [B][S][C][64] bf16 as a 4-D tensor (d, site, slot, tree); box = all slots of one site: [64 slots][64 d]
 static int make_tmap_kprime(CUtensorMap* map, const void* base, int S, int n_live, int C, int B, int box_rows) {
-    PFN_enc enc = get_enc();
-    if (!enc) return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
-    cuuint64_t gdim[4] = {64, (cuuint64_t)C, (cuuint64_t)n_live, (cuuint64_t)B};   // slots >= n_live are dead: never loaded (zero-filled)
-    cuuint64_t gstr[3] = {128, (cuuint64_t)C * 128, (cuuint64_t)S * C * 128};
-    cuuint32_t box[4] = {64, 1, (cuuint32_t)box_rows, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled failed for the K' planes");
-    return 0;
+    const cuuint64_t gdim[4] = {64, (cuuint64_t)C, (cuuint64_t)n_live, (cuuint64_t)B};   // slots >= n_live are dead: never loaded (zero-filled)
+    const cuuint64_t gstr[3] = {128, (cuuint64_t)C * 128, (cuuint64_t)S * C * 128};
+    const cuuint32_t box[4] = {64, 1, (cuuint32_t)box_rows, 1};
+    return encode_tmap(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                       "the K' planes");
 }
 
 // writes the x planes of pairs [n0, n0+nc) and alpha_part[b][n][partial][slot]; returns the number of partials per pair in *n_part
 int launch_alpha_tc(const Model* m, const float* X, const float* Y, size_t tree_stride, const int32_t* slot_of, int slot_stride, const int32_t* pair_i,
                     const int32_t* pair_j, int pair_stride, int n0, int nc, int S, int n_live, int C, int B, const void* kp_h, const void* kp_l, float* xf,
                     int pc, float* alpha_part, int alpha_pairs, int nSG, int RP, int* n_part, cudaStream_t st) {
-    {   // late steps (<= 16 pairs over <= 16 live nodes): the register-fragment kernel, whose cost follows the number of live pairs (nnj_alpha_small.cu)
-        static int small_on = -1;
-        if (small_on < 0) { const char* ev = getenv("NNJ_ALPHA_SMALL"); small_on = ev ? atoi(ev) : 1; }
-        const int lim = small_on > 1 ? 32 : 16;          // NNJ_ALPHA_SMALL=2: the 32-row variant as well (slower than k_alpha_v3's 4-way split below 25 pairs)
-        if (small_on && nc <= lim && n_live <= lim && !(C & 7))
-            return launch_alpha_small(m, X, Y, tree_stride, slot_of, slot_stride, pair_i, pair_j, pair_stride, n0, nc, S, n_live, C, B, kp_h, kp_l, xf, pc,
-                                      alpha_part, alpha_pairs, nSG, RP, n_part, st);
-    }
+    // late steps (<= 16 pairs over <= 16 live nodes): the register-fragment kernel, whose cost follows the number of live pairs (nnj_alpha_small.cu)
+    if (nc <= 16 && n_live <= 16 && !(C & 7))
+        return launch_alpha_small(m, X, Y, tree_stride, slot_of, slot_stride, pair_i, pair_j, pair_stride, n0, nc, S, n_live, C, B, kp_h, kp_l, xf, pc,
+                                  alpha_part, alpha_pairs, nSG, RP, n_part, st);
     static DevOnce once;      // per device, not per process
     if (once.need()) {
         cudaError_t e = cudaFuncSetAttribute(k_alpha_v3, cudaFuncAttributeMaxDynamicSharedMemorySize, AV_SMEM_MAX);
@@ -406,8 +374,7 @@ int launch_alpha_tc(const Model* m, const float* X, const float* Y, size_t tree_
     if (nc > AV_MAXT * 128 || nc > pc) return set_error(NNJ_ERR_INVALID, "alpha_tc: at most 512 pairs per launch");
     const int groups = (C + AV_SITES - 1) / AV_SITES;
     const bool dup = nc <= 64;
-    static const int quad_on = getenv("NNJ_ALPHA_QUAD") ? atoi(getenv("NNJ_ALPHA_QUAD")) : 1;
-    const int ways = !dup ? 1 : (nc <= 32 && quad_on && 4 * groups <= nSG) ? 4 : 2;
+    const int ways = !dup ? 1 : (nc <= 32 && 4 * groups <= nSG) ? 4 : 2;
     *n_part = ways * groups;
     if (*n_part > nSG) return set_error(NNJ_ERR_INVALID, "alpha_tc: partial buffer too small");
     // the live nodes occupy physical slots [0, n_live) (k_select keeps them compact): only those rows are streamed

@@ -12,7 +12,6 @@
 //   k_out_proj       out_proj + residual add (:116,236; msa_modules.py:120)
 //   k_ffn            LN + fc1 + GELU + fc2 + residual (msa_modules.py:144-151)
 #include <cuda_bf16.h>
-#include <cstdlib>
 
 #include "nnj_internal.h"
 #include "nnj_tc.cuh"
@@ -425,82 +424,6 @@ __device__ __forceinline__ void split_bf16(float v, __nv_bfloat16& hi, __nv_bflo
     lo = NNJ_LO_BF16(__float2bfloat16_rn(v - __bfloat162float(hi)));
 }
 
-// LN + q/k/v projections of the tied row attention, written as bf16 hi/lo planes for the tcgen05 GEMMs:
-//   Q, K : [B,H,C,R*8]   (K-major operands of S = Q K^T, contraction over (taxon, head-dim))
-//   V^T  : [B,H,R*8,C]   (K-major B operand of ctx = P V, contraction over key sites)
-// NATURAL token order (one taxon, 128 consecutive sites per tile) so V^T rows are written 8 sites (16 B) at a time.
-__global__ void __launch_bounds__(NTHREADS) k_ln_qkv_rowtc(const float* __restrict__ x, size_t x_tree_stride, int R, int C, AttnW w,
-                                                           float q_scale, const uint8_t* __restrict__ mask,
-                                                           __nv_bfloat16* __restrict__ qh, __nv_bfloat16* __restrict__ ql,
-                                                           __nv_bfloat16* __restrict__ kh, __nv_bfloat16* __restrict__ kl,
-                                                           __nv_bfloat16* __restrict__ vth, __nv_bfloat16* __restrict__ vtl, int xsm) {
-    extern __shared__ __align__(16) float smem[];
-    float* xs = smem;
-    float* Ws = smem + TILE_ROWS * LDA;
-    const int b = blockIdx.y, tile = blockIdx.x;
-    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-    const int T = R * C, KD = R * DH;
-    load_x_tile<false>(xs, x + (size_t)b * x_tree_stride, tile, R, C, xsm);
-    __syncthreads();
-    tile_layernorm(xs, w.ln_g, w.ln_b);
-    __syncthreads();
-    const float* wt[3] = {w.qt, w.kt, w.vt};
-    const float* bs[3] = {w.qb, w.kb, w.vb};
-    const int h = tx >> 1, d0 = (tx & 1) * 4;
-#pragma unroll
-    for (int p = 0; p < 3; ++p) {
-        load_w64(Ws, wt[p]);
-        __syncthreads();
-        float acc[8][4];
-        acc_set_bias(acc, bs[p], tx);
-        tile_mma64(acc, xs, Ws, ty, tx);
-        const int t0 = tile * TILE_ROWS + ty * 8;
-        if (p < 2) {
-            __nv_bfloat16* oh = p == 0 ? qh : kh;
-            __nv_bfloat16* ol = p == 0 ? ql : kl;
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                int t = t0 + i;
-                if (t >= T) continue;
-                int r = t / C, c = t - r * C;
-                float s = 1.0f;
-                if (p == 0) s = (mask && mask[(size_t)b * C + c]) ? 0.f : q_scale;   // axial_attention.py:81-82
-                __align__(8) __nv_bfloat16 hv[4], lv[4];
-#pragma unroll
-                for (int j = 0; j < 4; ++j) split_bf16(acc[i][j] * s, hv[j], lv[j]);
-                size_t off = (((size_t)b * H + h) * C + c) * KD + r * DH + d0;
-                *reinterpret_cast<uint2*>(oh + off) = *reinterpret_cast<uint2*>(hv);
-                *reinterpret_cast<uint2*>(ol + off) = *reinterpret_cast<uint2*>(lv);
-            }
-        } else {
-            const int r0 = t0 / C, c0 = t0 - r0 * C;
-            const bool fast = (t0 + 7 < T) && (c0 + 7 < C) && ((c0 & 7) == 0) && ((C & 7) == 0);
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                if (fast) {
-                    __align__(16) __nv_bfloat16 hv[8], lv[8];
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) split_bf16(acc[i][j], hv[i], lv[i]);
-                    size_t off = (((size_t)b * H + h) * KD + r0 * DH + d0 + j) * C + c0;
-                    *reinterpret_cast<uint4*>(vth + off) = *reinterpret_cast<uint4*>(hv);
-                    *reinterpret_cast<uint4*>(vtl + off) = *reinterpret_cast<uint4*>(lv);
-                } else {
-                    for (int i = 0; i < 8; ++i) {
-                        int t = t0 + i;
-                        if (t >= T) continue;
-                        int r = t / C, c = t - r * C;
-                        __nv_bfloat16 hv, lv;
-                        split_bf16(acc[i][j], hv, lv);
-                        size_t off = (((size_t)b * H + h) * KD + r * DH + d0 + j) * C + c;
-                        vth[off] = hv; vtl[off] = lv;
-                    }
-                }
-            }
-        }
-        __syncthreads();
-    }
-}
-
 // softmax over key sites of S [Z, C, C] (fp32) -> probabilities as bf16 hi/lo planes; one warp per row; C even.
 __global__ void __launch_bounds__(NTHREADS) k_softmax_rows_split(const float* __restrict__ S, __nv_bfloat16* __restrict__ Ph,
                                                                  __nv_bfloat16* __restrict__ Pl, int C, const uint8_t* __restrict__ mask) {
@@ -604,25 +527,17 @@ __global__ void __launch_bounds__(NTHREADS) k_softmax_rows_split_reg(const float
 // ------------------------------------------------------------------ host-side driver
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+// The tensor-core path works on the site-major residual stream: LN1 + row q|k|v, the row GEMMs and the feed-forward block run on
+// tcgen05 (nnj_encoder_tc.cu, nnj_tc.cu), and so does the fused column block up to 128 taxa; above that the CUDA-core column
+// stages below run on the same stream.
 static bool use_tc(const Model* m, int C) { return m->cfg.precision != NNJ_PREC_FP32 && (C % 8) == 0; }
-
-// Which per-token stages run on tcgen05 over the site-major residual stream (nnj_encoder_tc.cu): bit 0 LN1 + row q|k|v,
-// bit 1 the fused column block (at most 128 taxa), bit 2 the feed-forward block.  NNJ_ENC_TC overrides the default (all) for bisecting.
-static int enc_tc_mask(const Model* m, int R, int C) {
-    if (!use_tc(m, C)) return 0;
-    static int env = -1;
-    if (env < 0) { const char* e = getenv("NNJ_ENC_TC"); env = e ? (atoi(e) & 7) : 7; }
-    int mk = env;
-    if (R > 128) mk &= ~2;
-    return mk;
-}
 
 // per-tree workspace floats for the encoder
 static size_t enc_tree_floats(const Model* m, int R, int C) {
     size_t act = (size_t)R * C * D;
     size_t s = (size_t)H * C * C;         // row-attention logits; also holds the column-attention context
     size_t p = use_tc(m, C) ? s : 0;      // probabilities as bf16 hi/lo planes (tensor-core path)
-    size_t xs = enc_tc_mask(m, R, C) ? xs_tree_floats(R * C) : 0;   // site-major residual stream (tile-planar, whole 128-token tiles)
+    size_t xs = use_tc(m, C) ? xs_tree_floats(R * C) : 0;   // site-major residual stream (tile-planar, whole 128-token tiles)
     return 3 * act + (s > act ? s : act) + p + xs; // q (row ctx), k, v, S [, P] [, xs]
 }
 
@@ -660,8 +575,8 @@ int run_encoder(Model* m, const int8_t* data, const uint8_t* mask, int B, int R,
     float* v = k + act * chunk;
     float* S = v + act * chunk;   // region of chunk * max(H*C*C, act) floats
     const bool tc = use_tc(m, C);
-    const int mk = enc_tc_mask(m, R, C);
-    const int xsm = mk ? 1 : 0;
+    const bool col_tc = tc && R <= 128;       // the fused column block (k_enc_colblock_tc) holds at most 128 taxa
+    const int xsm = tc ? 1 : 0;
     const size_t s_floats = (size_t)H * C * C > act ? (size_t)H * C * C : act;
     __nv_bfloat16* P = reinterpret_cast<__nv_bfloat16*>(S + s_floats * chunk);   // [2 planes][chunk*H][C][C] (tensor-core path only)
     float* xs_ws = S + s_floats * chunk + (tc ? (size_t)H * C * C * chunk : 0);  // site-major residual stream [chunk][tiles of 128 tokens t = c R + r][16 chunks][128][4]
@@ -675,13 +590,12 @@ int run_encoder(Model* m, const int8_t* data, const uint8_t* mask, int B, int R,
         cudaFuncSetAttribute(k_ffn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_ffn);
         cudaFuncSetAttribute(k_ln_qkv<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_qkv);
         cudaFuncSetAttribute(k_ln_qkv<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_qkv);
-        cudaFuncSetAttribute(k_ln_qkv_rowtc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_qkv);
         cudaFuncSetAttribute(k_out_proj<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_qkv);
         cudaFuncSetAttribute(k_out_proj<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_qkv);
         cudaFuncSetAttribute(k_col_attn, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         attr_once.done();
     }
-    if (!(mk & 2) && smem_col > 200 * 1024) return set_error(NNJ_ERR_INVALID, "encode: too many taxa for the column-attention kernel (max 400)");
+    if (!col_tc && smem_col > 200 * 1024) return set_error(NNJ_ERR_INVALID, "encode: too many taxa for the column-attention kernel (max 400)");
     if (R == 1) return set_error(NNJ_ERR_INVALID, "encode: R == 1 is not supported");
     const float row_scale = (1.0f / sqrtf((float)DH)) / sqrtf((float)R);   // align_scaling, axial_attention.py:31-33
     const float col_scale = 1.0f / sqrtf((float)DH);
@@ -705,37 +619,24 @@ int run_encoder(Model* m, const int8_t* data, const uint8_t* mask, int B, int R,
                 __nv_bfloat16 *vh = reinterpret_cast<__nv_bfloat16*>(v), *vl = vh + pl;
                 const size_t pp = (size_t)chunk * H * C * C;   // elements per plane of P
                 const int KD = R * DH;
-                if (mk & 1) {      // V as [B,H,C,R*8]: the MN-major B operand of ctx = P V
-                    if (int e = launch_enc_rowqkv_tc(m, l, xb, xstr, nb, R, C, row_scale, mb, qh, ql, kh, kl, vh, vl, st)) return e;
-                } else {           // V^T as [B,H,R*8,C]
-                    prof_begin(KC_LN_QKV, st);
-                    k_ln_qkv_rowtc<<<dim3(tiles, nb), NTHREADS, smem_qkv, st>>>(xb, xstr, R, C, lw.row, row_scale, mb, qh, ql, kh, kl, vh, vl, xsm);
-                    LAUNCH_CHECK();
-                }
+                // V as [B,H,C,R*8]: the MN-major B operand of ctx = P V
+                if (int e = launch_enc_rowqkv_tc(m, l, xb, xstr, nb, R, C, row_scale, mb, qh, ql, kh, kl, vh, vl, st)) return e;
                 const int products = m->cfg.precision == NNJ_PREC_BF16 ? 1 : 3;
                 __nv_bfloat16* Plo = products == 1 ? nullptr : P + pp;      // one-product mode: the register softmax writes the hi plane only
-                const bool fused = (mk & 1) && row_qk_softmax_ok(C, products);   // softmax in the Q K^T epilogue: S never leaves the chip
-                if (fused) {
-                    float* rowsum = S;                                            // [nb * H][C]: the logits buffer is free in this form
+                float* rowsum = nullptr;
+                if (row_qk_softmax_ok(C, products)) {      // softmax in the Q K^T epilogue: S never leaves the chip
+                    rowsum = S;                             // [nb * H][C]: the logits buffer is free in this form
                     if (int e = launch_row_qk_softmax(KC_ROW_QK, qh, ql, kh, kl, P, P + pp, rowsum, mb, H, nb * H, C, KD, st)) return e;
-                    if (int e = launch_tc_gemm_bmn(KC_ROW_PV, P, P + pp, vh, vl, q /*ctx fp32 [B,H,C,R*8]*/, nb * H, C, KD, C, C, (size_t)C * C, KD,
-                                                   (size_t)C * KD, KD, (size_t)C * KD, st, products, rowsum)) return e;
                 } else {
-                if (int e = launch_tc_gemm(KC_ROW_QK, qh, ql, kh, kl, S, nb * H, C, C, KD, KD, (size_t)C * KD, KD, (size_t)C * KD, C, (size_t)C * C, st, products)) return e;
-                prof_begin(KC_ROW_SOFTMAX, st);
-                if (C <= 512) k_softmax_rows_split_reg<2><<<dim3((C + 7) / 8, nb * H), NTHREADS, 0, st>>>(S, P, Plo, C, mb);
-                else if (C <= 1024) k_softmax_rows_split_reg<4><<<dim3((C + 7) / 8, nb * H), NTHREADS, 0, st>>>(S, P, Plo, C, mb);
-                else k_softmax_rows_split<<<dim3((C + 7) / 8, nb * H), NTHREADS, 0, st>>>(S, P, P + pp, C, mb);
-                LAUNCH_CHECK();
+                    if (int e = launch_tc_gemm(KC_ROW_QK, qh, ql, kh, kl, S, nb * H, C, C, KD, KD, (size_t)C * KD, KD, (size_t)C * KD, C, (size_t)C * C, st, products)) return e;
+                    prof_begin(KC_ROW_SOFTMAX, st);
+                    if (C <= 512) k_softmax_rows_split_reg<2><<<dim3((C + 7) / 8, nb * H), NTHREADS, 0, st>>>(S, P, Plo, C, mb);
+                    else if (C <= 1024) k_softmax_rows_split_reg<4><<<dim3((C + 7) / 8, nb * H), NTHREADS, 0, st>>>(S, P, Plo, C, mb);
+                    else k_softmax_rows_split<<<dim3((C + 7) / 8, nb * H), NTHREADS, 0, st>>>(S, P, P + pp, C, mb);
+                    LAUNCH_CHECK();
                 }
-                if (fused) {
-                } else if (mk & 1) {
-                    if (int e = launch_tc_gemm_bmn(KC_ROW_PV, P, P + pp, vh, vl, q /*ctx fp32 [B,H,C,R*8]*/, nb * H, C, KD, C, C, (size_t)C * C, KD,
-                                                   (size_t)C * KD, KD, (size_t)C * KD, st, products)) return e;
-                } else {
-                    if (int e = launch_tc_gemm(KC_ROW_PV, P, P + pp, vh, vl, q /*ctx fp32 [B,H,C,R*8]*/, nb * H, C, KD, C, C, (size_t)C * C, C,
-                                               (size_t)KD * C, KD, (size_t)C * KD, st, products)) return e;
-                }
+                if (int e = launch_tc_gemm_bmn(KC_ROW_PV, P, P + pp, vh, vl, q /*ctx fp32 [B,H,C,R*8]*/, nb * H, C, KD, C, C, (size_t)C * C, KD,
+                                               (size_t)C * KD, KD, (size_t)C * KD, st, products, rowsum)) return e;
             } else {
                 prof_begin(KC_LN_QKV, st);
                 k_ln_qkv<true><<<dim3(tiles, nb), NTHREADS, smem_qkv, st>>>(xb, xstr, R, C, lw.row, row_scale, mb, q, k, v, xsm);
@@ -752,7 +653,7 @@ int run_encoder(Model* m, const int8_t* data, const uint8_t* mask, int B, int R,
                     S, v, q /*ctx*/, C, R * DH, C, (size_t)C * C, (size_t)C * R * DH, (size_t)C * R * DH, C, R * DH, R * DH);
                 LAUNCH_CHECK();
             }
-            if (mk & 2) {
+            if (col_tc) {
                 // --- row out_proj + residual, LN2, column attention, column out_proj + residual: one kernel
                 if (int e = launch_enc_colblock_tc(m, l, xb, xstr, q, nb, R, C, mb, st)) return e;
             } else {
@@ -771,7 +672,7 @@ int run_encoder(Model* m, const int8_t* data, const uint8_t* mask, int B, int R,
                 LAUNCH_CHECK();
             }
             // --- feed forward (per token: the memory order of the stream does not matter)
-            if (mk & 4) {
+            if (tc) {
                 if (int e = launch_enc_ffn_tc(m, l, xb, xstr, nb, R, C, st)) return e;
             } else {
                 prof_begin(KC_FFN, st);

@@ -1,5 +1,6 @@
 // nnj_internal.h — host-side structures shared by the libnnj translation units.
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <stddef.h>
 #include <stdint.h>
@@ -158,6 +159,15 @@ int launch_tc_gemm_ex(int cls, const void* Ah, const void* Al, const void* Bh, c
                       cudaStream_t st, int products = 3);
 int launch_tc_gemm_bmn(int cls, const void* Ah, const void* Al, const void* Bh, const void* Bl, float* Cm, int Z, int M, int N, int K, size_t lda,
                        size_t sA, size_t ldb, size_t sB, int ldc, size_t sC, cudaStream_t st, int products = 3, const float* row_div = nullptr);
+// TMA tensor maps (nnj_tc.cu).  encode_tmap: cuTensorMapEncodeTiled through the runtime's driver entry point, element strides 1, no
+// interleave, no out-of-bounds fill; dims / strides / box as that call takes them.  Returns 0, or NNJ_ERR_CUDA with a message naming `what`.
+int encode_tmap(CUtensorMap* map, CUtensorMapDataType dtype, int rank, const void* base, const cuuint64_t* dims, const cuuint64_t* strides,
+                const cuuint32_t* box, CUtensorMapSwizzle swizzle, CUtensorMapL2promotion l2, const char* what);
+// node planes [B*C][S][128] bf16 ([X | W_g X] per slot), box 64 channels x box_rows slots of one site; slots >= n_live (when > 0) read as 0
+// (nnj_score_tc.cu)
+int make_tmap_nodes(CUtensorMap* map, const void* base, int S, int BC, int box_rows = 64, int n_live = -1);
+// x planes [B][pc][C][64] fp32 as (d, site, pair, tree), box 32 channels x box_rows pairs at one site; pairs >= nrows read as 0 (nnj_score_tc.cu)
+int make_tmap_xtile(CUtensorMap* map, const float* base, int pc, int nrows, int C, int B, int box_rows = 64);
 // S = Q K^T of the tied row attention with the softmax in the epilogue: unnormalised exp(s - max) as bf16 hi / lo planes + the row sums, which the
 // P V launch takes as `row_div` (k_tc_gemm2s, CTA pairs; site count a multiple of 256)
 bool row_qk_softmax_ok(int C, int products);

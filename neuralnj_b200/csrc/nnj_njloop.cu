@@ -1128,12 +1128,6 @@ static NjBuffers nj_layout(char* base, int B, int S, int R, int C, bool X_in_ws,
 static inline char* ws_align(void* ws) { return reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(ws) + 255) / 256 * 256); }
 
 static size_t smem_score(int Rp) { return (2 * 4096 + 2 * TILE_ROWS * LDA + 128 + 64 + ((Rp + 3) & ~3) + (size_t)Rp * 32) * sizeof(float); }
-// NNJ_MERGE_TC=0: keep the 64 x 64 products of the merge / node-derive kernels on the CUDA cores in the tensor-core modes too (A/B runs)
-static bool merge_tc_enabled() {
-    static const bool on = [] { const char* v = getenv("NNJ_MERGE_TC"); return !(v && v[0] == '0'); }();
-    return on;
-}
-
 static size_t smem_merge(int Rp) { return (2 * TILE_ROWS * LDA + 4096 + 128 + 2 * ((Rp + 3) & ~3) + 8) * sizeof(float); }
 static const size_t smem_derive = (2 * TILE_ROWS * LDA + 4096 + 128) * sizeof(float);
 
@@ -1237,7 +1231,6 @@ static int score_pairs(const Model* m, const Pool& pool, const NjBuffers& nb, co
 static int merge_pair(const Model* m, const Pool& pool, const NjBuffers& nb, float* Xw, const int32_t* slot, int Rp, int C,
                       const int32_t* ij, int ij_stride, int B, float* out_x, size_t out_stride, bool derive, cudaStream_t st) {
     const float inv_scale = 1.0f / sqrtf((float)D * (float)C);
-    const bool mtc = nb.tc && merge_tc_enabled();      // the 64 x 64 products on mma.sync (tensor-core precision modes)
     auto launch_merge = [&](bool glob) {
         uint2* nh = (derive && nb.tc) ? (uint2*)nb.nodes_h : nullptr; uint2* nl = (derive && nb.tc) ? (uint2*)nb.nodes_l : nullptr;
         uint2* kh = (derive && nb.tc) ? (uint2*)nb.kp_h : nullptr;    uint2* kl = (derive && nb.tc) ? (uint2*)nb.kp_l : nullptr;
@@ -1245,8 +1238,9 @@ static int merge_pair(const Model* m, const Pool& pool, const NjBuffers& nb, flo
         const dim3 grid(nb.nCT, B);
         const size_t sm = smem_merge(Rp);
 #define NNJ_MERGE_ARGS pool, Xw, nb.Y, nb.K, nb.kap, slot, nb.S, Rp, C, ij, ij_stride, nb.alpha, nb.RP, m->nj, m->nj_frag, out_x, out_stride, nb.new_slot, derive ? 1 : 0, nh, nl, kh, kl, mv
-        if (glob) { if (mtc) k_merge<true, true><<<grid, NTHREADS, sm, st>>>(NNJ_MERGE_ARGS); else k_merge<true, false><<<grid, NTHREADS, sm, st>>>(NNJ_MERGE_ARGS); }
-        else      { if (mtc) k_merge<false, true><<<grid, NTHREADS, sm, st>>>(NNJ_MERGE_ARGS); else k_merge<false, false><<<grid, NTHREADS, sm, st>>>(NNJ_MERGE_ARGS); }
+        // second template argument: the 64 x 64 products on mma.sync (tensor-core precision modes)
+        if (glob) { if (nb.tc) k_merge<true, true><<<grid, NTHREADS, sm, st>>>(NNJ_MERGE_ARGS); else k_merge<true, false><<<grid, NTHREADS, sm, st>>>(NNJ_MERGE_ARGS); }
+        else      { if (nb.tc) k_merge<false, true><<<grid, NTHREADS, sm, st>>>(NNJ_MERGE_ARGS); else k_merge<false, false><<<grid, NTHREADS, sm, st>>>(NNJ_MERGE_ARGS); }
 #undef NNJ_MERGE_ARGS
     };
     if (Rp > 2) {
@@ -1271,13 +1265,12 @@ static int merge_pair(const Model* m, const Pool& pool, const NjBuffers& nb, flo
 
 static int derive_all(const Model* m, const float* X, const NjBuffers& nb, int B, int S, int nodes, int C, cudaStream_t st) {
     prof_begin(KC_DERIVE, st);
-    if (nb.tc && merge_tc_enabled())
+    if (nb.tc)
         k_node_derive<true><<<dim3(nb.nCT, nodes, B), NTHREADS, smem_derive, st>>>(X, nb.Y, nb.K, nb.kap, (size_t)S * C * D, S, C, nb.nCT, nullptr, 0, m->nj, m->nj_frag,
                                                                                    (uint2*)nb.kp_h, (uint2*)nb.kp_l, (uint2*)nb.nodes_h, (uint2*)nb.nodes_l);
     else
         k_node_derive<false><<<dim3(nb.nCT, nodes, B), NTHREADS, smem_derive, st>>>(X, nb.Y, nb.K, nb.kap, (size_t)S * C * D, S, C, nb.nCT, nullptr, 0, m->nj, m->nj_frag,
-                                                                                    nb.tc ? (uint2*)nb.kp_h : nullptr, nb.tc ? (uint2*)nb.kp_l : nullptr,
-                                                                                    nb.tc ? (uint2*)nb.nodes_h : nullptr, nb.tc ? (uint2*)nb.nodes_l : nullptr);
+                                                                                    nullptr, nullptr, nullptr, nullptr);
     LAUNCH_CHECK();
     return 0;
 }
@@ -1430,13 +1423,12 @@ int run_rollout(Model* m, const int8_t* data, const float* state0, const uint8_t
             cudaError_t e1 = cudaMemsetAsync(nb.nodes_h, 0, npb, st), e2 = cudaMemsetAsync(nb.nodes_l, 0, npb, st);
             if (e1 != cudaSuccess || e2 != cudaSuccess) return set_cuda_error(e1 != cudaSuccess ? e1 : e2, __FILE__, __LINE__);
         }
-        if (nb.tc && merge_tc_enabled())
+        if (nb.tc)
             k_node_derive<true><<<dim3(nb.nCT, R, nbt), NTHREADS, smem_derive, st>>>(nb.X, nb.Y, nb.K, nb.kap, tree_stride, S, C, nb.nCT, nullptr, 0, m->nj, m->nj_frag,
                                                                                      (uint2*)nb.kp_h, (uint2*)nb.kp_l, (uint2*)nb.nodes_h, (uint2*)nb.nodes_l);
         else
             k_node_derive<false><<<dim3(nb.nCT, R, nbt), NTHREADS, smem_derive, st>>>(nb.X, nb.Y, nb.K, nb.kap, tree_stride, S, C, nb.nCT, nullptr, 0, m->nj, m->nj_frag,
-                                                                                      nb.tc ? (uint2*)nb.kp_h : nullptr, nb.tc ? (uint2*)nb.kp_l : nullptr,
-                                                                                      nb.tc ? (uint2*)nb.nodes_h : nullptr, nb.tc ? (uint2*)nb.nodes_l : nullptr);
+                                                                                      nullptr, nullptr, nullptr, nullptr);
         LAUNCH_CHECK();
         Pool pool = make_pool(nb.X, nb, S, C);
         int32_t* mg = merges + (size_t)b0 * (R - 1) * 2;

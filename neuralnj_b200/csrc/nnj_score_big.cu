@@ -331,19 +331,6 @@ __global__ void __launch_bounds__(256) k_blend_planes(const float* __restrict__ 
 }
 
 // ------------------------------------------------------------------ host side
-typedef CUresult (*PFN_encb)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                             const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static PFN_encb get_encb() {
-    static PFN_encb enc = nullptr;
-    if (!enc) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-            enc = reinterpret_cast<PFN_encb>(p);
-    }
-    return enc;
-}
-
 int launch_blend_planes(const Model* m, const float* X, const float* Y, size_t tree_stride, int C, int B, const int32_t* slot_of, int slot_stride,
                         const int32_t* pair_i, const int32_t* pair_j, int pair_stride, int n0, int nc, float* xf, void* xh, void* xl, int pc,
                         cudaStream_t st) {
@@ -368,29 +355,10 @@ int launch_score_big(const Model* m, const float* xf, int pc, const void* nodes_
     }
     if (Rp > 256 || S > 256) return set_error(NNJ_ERR_INVALID, "score_big: at most 256 node slots");
     if (C & 7) return set_error(NNJ_ERR_INVALID, "score_big: site count must be a multiple of 8");
-    PFN_encb enc = get_encb();
-    if (!enc) return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
-    CUtensorMap mh, ml, mx;
-    {   // node planes [B*C][S][128] bf16 ([X | W_g X] per slot): box = 64 channels x 64 slots of one site; slots >= Rp are dead (zero-filled)
-        cuuint64_t gdim[3] = {128, (cuuint64_t)Rp, (cuuint64_t)B * C};
-        cuuint64_t gstr[2] = {256, (cuuint64_t)S * 256};
-        cuuint32_t box[3] = {64, 64, 1};
-        cuuint32_t estr[3] = {1, 1, 1};
-        CUresult r1 = enc(&mh, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(nodes_h), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                          CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        CUresult r2 = enc(&ml, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(nodes_l), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                          CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r1 != CUDA_SUCCESS || r2 != CUDA_SUCCESS) return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled failed for the node planes (score_big)");
-    }
-    {   // x planes [B][pc][C][64] fp32 as (d, site, pair, tree); box = 32 channels of 64 pairs at one site (pairs >= nc read as 0)
-        cuuint64_t gdim[4] = {64, (cuuint64_t)C, (cuuint64_t)nc, (cuuint64_t)B};
-        cuuint64_t gstr[3] = {256, (cuuint64_t)C * 256, (cuuint64_t)pc * C * 256};
-        cuuint32_t box[4] = {32, 1, 64, 1};
-        cuuint32_t estr[4] = {1, 1, 1, 1};
-        CUresult r = enc(&mx, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(xf), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                         CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled failed for the x tiles (score_big)");
-    }
+    CUtensorMap mh, ml, mx;      // node planes: 64 slots of one site per box, slots >= Rp dead (zero-filled); x tiles: 64 pairs, pairs >= nc read as 0
+    if (int e = make_tmap_nodes(&mh, nodes_h, S, B * C, 64, Rp)) return e;
+    if (int e = make_tmap_nodes(&ml, nodes_l, S, B * C, 64, Rp)) return e;
+    if (int e = make_tmap_xtile(&mx, xf, pc, nc, C, B)) return e;
     ScoreBigArgs a;
     a.alpha = alpha; a.RP = RP; a.alpha_pairs = alpha_pairs;
     a.slot_of = slot_of; a.slot_stride = slot_stride; a.pair_i = pair_i; a.pair_stride = pair_stride; a.n0 = n0; a.nc = nc;

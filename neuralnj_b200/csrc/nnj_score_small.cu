@@ -1,4 +1,4 @@
-// nnj_score_small.cu — pair scoring for the LATE steps of the NJ loop (<= 32 pairs over <= 32 live nodes per tree).
+// nnj_score_small.cu — pair scoring for the LATE steps of the NJ loop (<= 16 pairs over <= 16 live nodes per tree).
 //
 // Same arithmetic as k_score_inc (model.py:90-99, 148-153), per (pair p, site c):
 //     [x_glob | g] = alpha[p, :] . [X | W_g X][:, c, :]                 GEMM 1, K = live slots
@@ -7,13 +7,13 @@
 //     score[p]    += w2 . GELU(s + b_s) + b2 over unmasked sites
 // k_score_inc puts pairs on TMEM lanes: a work item costs the same ~2 950 clocks whether a tree has 32 live pairs or 2
 // (profiles/r02_ncu_launches: 715 us per launch of 128 trees at n = 2, 770 us at n = 32), because a tcgen05 tile is 128 rows and
-// every epilogue instruction is a full warp.  With 16 / 32 rows the natural tile is the 16 x 8 x 16 register-fragment instruction
+// every epilogue instruction is a full warp.  With 16 rows the natural tile is the 16 x 8 x 16 register-fragment instruction
 // (mma.sync, 8 clocks per sub-partition, scratch/hmma_bench.cu): one warp owns one site at a time, the alpha operand of the tree
 // lives in its registers as A fragments for all sites, the site's node rows come through ldmatrix.trans as B fragments, the C
 // fragments of GEMM 1 turn into the A fragments of GEMM 2 without leaving the registers (same trick as the column attention), and
 // the GELU / w2 epilogue runs on the C fragments of GEMM 2.  Every product is the 3-term bf16 split, accumulated in fp32.
-// 144 (<= 16 pairs) / 384 (<= 32) tensor instructions per site instead of a fixed ~1 500 clocks.
-// CTA = (tree, 128-site group), 8 warps x 16 sites; a warp streams its sites through a private double buffer with cp.async.
+// 144 tensor instructions per site instead of a fixed ~1 500 clocks.
+// CTA = (tree, 128-site group), 16 warps x 8 sites; a warp streams its sites through a private buffer with cp.async.
 // Partial scores per site group go to the same buffer k_score_inc fills (fixed-order reduction: bit-reproducible).
 #include "nnj_internal.h"
 #include "nnj_tc.cuh"
@@ -47,14 +47,13 @@ __device__ __forceinline__ void ss_cp16(uint32_t dst, const void* src) {
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
 }
 
-// T = 16-row / 16-slot tiles: 1 (<= 16 pairs and slots) or 2 (<= 32); SS_WARPS warps with NBUF private tile buffers each.
-// Measured (128 trees, profiles/r02_score_small.txt): T = 2 is bound by its 384 tensor instructions per site (8 clocks each and
-// sub-partition: 770 clocks per site and SM) and loses to k_score_inc's narrow mode (860 vs 770 us per launch) - it is kept for
-// reference but not dispatched; T = 1 with 8 warps ran at 43 % of the legacy tensor pipe (two warps per sub-partition cannot
-// cover the 20-clock dependent instruction chains and the gate math between the two GEMMs; an 8-warp double-buffered
-// variant measured 355 vs 340 us), hence 16 warps with one buffer each.
-// HALF (T = 1 only): at most 8 listed pairs - rows 8..15 of the tile are padding and their gate / GELU math is compiled out.
-template <int T, int SS_WARPS, int NBUF, bool HALF>
+// T = 1 16-row / 16-slot tile (<= 16 pairs and slots); SS_WARPS warps with one private tile buffer each.
+// Measured (128 trees, DESIGN 4.6): a 32-row form (17-32 pairs) is bound by its 384 tensor instructions per site (8 clocks each and
+// sub-partition: 770 clocks per site and SM) and loses to k_score_inc's narrow mode (860 vs 770 us per launch); the 16-row tile with
+// 8 warps ran at 43 % of the legacy tensor pipe (two warps per sub-partition cannot cover the 20-clock dependent instruction chains
+// and the gate math between the two GEMMs; an 8-warp double-buffered variant measured 355 vs 340 us), hence 16 warps with one buffer each.
+// HALF: at most 8 listed pairs - rows 8..15 of the tile are padding and their gate / GELU math is compiled out.
+template <int T, int SS_WARPS, bool HALF>
 __global__ void __launch_bounds__(SS_WARPS * 32, 1) k_score_small(const ScoreSmallArgs a) {
     constexpr int ROWS = 16 * T;
     constexpr int NODE_B = ROWS * 256;                  // one node plane of a site: [slot][128 ch] bf16, 16-byte chunk c stored at c ^ (slot & 7)
@@ -80,7 +79,7 @@ __global__ void __launch_bounds__(SS_WARPS * 32, 1) k_score_small(const ScoreSma
     }
     if (tid < 64) { s_bias[tid] = a.bg[tid]; s_bias[64 + tid] = a.bs[tid]; s_bias[128 + tid] = a.w2[tid]; }
     for (int i = tid; i < 32 * 33; i += SS_WARPS * 32) tab[i] = 0.f;
-    for (int i = tid; i < (SS_WARPS * NBUF * BUF) >> 4; i += SS_WARPS * 32) reinterpret_cast<uint4*>(bufs)[i] = make_uint4(0u, 0u, 0u, 0u);
+    for (int i = tid; i < (SS_WARPS * BUF) >> 4; i += SS_WARPS * 32) reinterpret_cast<uint4*>(bufs)[i] = make_uint4(0u, 0u, 0u, 0u);
     __syncthreads();
     {
         const int32_t* so = a.slot_of + (size_t)b * a.slot_stride;
@@ -105,14 +104,14 @@ __global__ void __launch_bounds__(SS_WARPS * 32, 1) k_score_small(const ScoreSma
         }
     __syncthreads();                                     // tab is reused for the partial scores below
 
-    uint8_t* mybuf = bufs + warp * NBUF * BUF;
+    uint8_t* mybuf = bufs + warp * BUF;
     const uint32_t mybuf_u = smem_u32(mybuf);
     const uint32_t wsm_u = smem_u32(wsm);
     const size_t node_site_stride = (size_t)a.S * 128;  // bf16 elements per site in a node plane
-    // this warp's sites: warp, warp + 8, ...
-    auto issue = [&](int site, int buf) {
+    // this warp's sites: warp, warp + SS_WARPS, ...
+    auto issue = [&](int site) {
         const int c = c_base + site;
-        const uint32_t dst = mybuf_u + buf * BUF;
+        const uint32_t dst = mybuf_u;
         const uint8_t* nh = reinterpret_cast<const uint8_t*>(a.nodes_h + ((size_t)b * a.C + c) * node_site_stride);
         const uint8_t* nl = reinterpret_cast<const uint8_t*>(a.nodes_l + ((size_t)b * a.C + c) * node_site_stride);
         {   // live node rows (contiguous in both planes): lane = (slot parity, 16-byte chunk), two slots per pass
@@ -136,15 +135,12 @@ __global__ void __launch_bounds__(SS_WARPS * 32, 1) k_score_small(const ScoreSma
 #pragma unroll
     for (int m = 0; m < T; ++m) { part[m][0] = 0.f; part[m][1] = 0.f; }
     int n_unmasked = 0;
-    int buf = 0;
-    if (NBUF == 2 && warp < n_sites) issue(warp, 0);
-    for (int site = warp; site < n_sites; site += SS_WARPS, buf ^= (NBUF - 1)) {
-        if (NBUF == 2 && site + SS_WARPS < n_sites) { issue(site + SS_WARPS, buf ^ 1); asm volatile("cp.async.wait_group 1;" ::: "memory"); }
-        else { if (NBUF == 1) issue(site, 0); asm volatile("cp.async.wait_group 0;" ::: "memory"); }
+    for (int site = warp; site < n_sites; site += SS_WARPS) {
+        issue(site);
+        asm volatile("cp.async.wait_group 0;" ::: "memory");
         __syncwarp();
         const bool unmasked = !(a.mask && a.mask[(size_t)b * a.C + c_base + site]);
-        const uint32_t nb_u = mybuf_u + buf * BUF;
-        const uint8_t* xt = mybuf + buf * BUF + 2 * NODE_B;
+        const uint8_t* xt = mybuf + 2 * NODE_B;
         float sacc[T][8][4];
 #pragma unroll
         for (int m = 0; m < T; ++m)
@@ -163,7 +159,7 @@ __global__ void __launch_bounds__(SS_WARPS * 32, 1) k_score_small(const ScoreSma
                 for (int k = 0; k < T; ++k) {
                     // four 8 x 8 matrices: slots 16k + 0..7 / 8..15 of chunk j (x_glob), the same of chunk 8 + j (g); lane l supplies row l & 7 of matrix l >> 3
                     const int slot = 16 * k + ((lane >> 3) & 1) * 8 + (lane & 7);
-                    const uint32_t ad = nb_u + slot * 256 + ((((lane >> 4) * 8 + j) ^ (lane & 7)) << 4);
+                    const uint32_t ad = mybuf_u + slot * 256 + ((((lane >> 4) * 8 + j) ^ (lane & 7)) << 4);
                     uint32_t bh[4], bl[4];
                     ss_ldsm4t(bh, ad);
                     ss_ldsm4t(bl, ad + NODE_B);
@@ -226,7 +222,7 @@ __global__ void __launch_bounds__(SS_WARPS * 32, 1) k_score_small(const ScoreSma
                 part[m][1] += acc1.x + acc1.y;
             }
         }
-        __syncwarp();                                    // everybody done with this buffer before the loads two sites ahead land in it
+        __syncwarp();                                    // everybody done with this buffer before the next site's loads land in it
     }
     // ---- partial score of this site group: quad sum, then the warps in fixed order
 #pragma unroll
@@ -248,24 +244,23 @@ __global__ void __launch_bounds__(SS_WARPS * 32, 1) k_score_small(const ScoreSma
     }
 }
 
-template <int T, int W, int NB, bool HALF = false>
+template <bool HALF>
 static int launch_small_t(const ScoreSmallArgs& a, int groups, int B, cudaStream_t st) {
-    constexpr size_t smem = 1024 + 2 * 64 * SS_WPITCH + (32 * 33 + 192) * 4 + 1024 + (size_t)W * NB * (3 * 16 * T * 256);
+    constexpr size_t smem = 1024 + 2 * 64 * SS_WPITCH + (32 * 33 + 192) * 4 + 1024 + (size_t)16 * (3 * 16 * 256);
     static DevOnce once;      // per device, not per process
     if (once.need()) {
-        cudaError_t e = cudaFuncSetAttribute(k_score_small<T, W, NB, HALF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(k_score_small<1, 16, HALF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
         once.done();
     }
-    k_score_small<T, W, NB, HALF><<<dim3(groups, B), W * 32, smem, st>>>(a);
+    k_score_small<1, 16, HALF><<<dim3(groups, B), 16 * 32, smem, st>>>(a);
     return 0;
 }
 
 int launch_score_small(const Model* m, const float* xf, int pc, const void* nodes_h, const void* nodes_l, const float* alpha, int RP, int alpha_pairs,
                        const int32_t* slot_of, int slot_stride, const int32_t* pair_i, int pair_stride, int n0, int nc, int Rp, int S, int C, int B,
                        const uint8_t* mask, float* score_part, int nSG, int* n_part, cudaStream_t st) {
-    const int T = (nc <= 16 && Rp <= 16) ? 1 : 2;
-    if (nc > 32 || Rp > 32 || nc < 1) return set_error(NNJ_ERR_INVALID, "score_small: at most 32 pairs over 32 live nodes");
+    if (nc > 16 || Rp > 16 || nc < 1) return set_error(NNJ_ERR_INVALID, "score_small: at most 16 pairs over 16 live nodes");
     ScoreSmallArgs a;
     a.xf = xf; a.pc = pc; a.nodes_h = (const __nv_bfloat16*)nodes_h; a.nodes_l = (const __nv_bfloat16*)nodes_l; a.S = S;
     a.alpha = alpha; a.RP = RP; a.alpha_pairs = alpha_pairs; a.slot_of = slot_of; a.slot_stride = slot_stride;
@@ -277,8 +272,7 @@ int launch_score_small(const Model* m, const float* xf, int pc, const void* node
     *n_part = groups;
     if (groups > nSG) return set_error(NNJ_ERR_INVALID, "score_small: partial buffer too small");
     prof_begin(KC_SCORE, st);
-    const int rc = T == 1 ? (nc <= 8 ? launch_small_t<1, 16, 1, true>(a, groups, B, st) : launch_small_t<1, 16, 1>(a, groups, B, st))
-                          : launch_small_t<2, 8, 1>(a, groups, B, st);
+    const int rc = nc <= 8 ? launch_small_t<true>(a, groups, B, st) : launch_small_t<false>(a, groups, B, st);
     ++g_launches;
     prof_end(st);
     if (rc) return rc;

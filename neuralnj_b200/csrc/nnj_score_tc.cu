@@ -11,11 +11,12 @@
 // One CTA = 128 pairs x 64 sites.  Sites alternate between two pipelines, each with its own TMEM accumulators
 // ([x_glob | g]: 128 columns, s: 64), operand buffers and a group of 8 epilogue warps (4 TMEM lane quarters x 2 column
 // halves); two control warps issue TMA + tcgen05.mma, so the tensor core works on one site while the CUDA cores run
-// the sigmoid / blend / GELU epilogue of the other.  With <= 64 pairs (every step after the first) the pairs are
-// duplicated into rows 64..127 so that all four lane quarters - hence all 16 epilogue warps - have work.  Every product is split-bf16 (hi*hi + hi*lo + lo*hi, fp32
-// accumulate); operands produced on the fly are written by the epilogue threads straight into SWIZZLE_128B shared
-// memory (validated by nnj_tc_selftest).  Node state for UMMA 1 comes from site-major bf16 planes [B][C][S][128]
-// [X | W_g X], indexed by PHYSICAL slot, so alpha is scattered to slot order and dead / free slots simply get weight 0.
+// the sigmoid / blend / GELU epilogue of the other.  A tile of <= 64 pairs (the tail tile of step 0, e.g. 136 = 128 + 8 pairs at
+// 17 taxa; later steps go to k_score_inc) has its pairs duplicated into rows 64..127 so that all four lane quarters - hence all
+// 16 epilogue warps - have work.  Every product is split-bf16 (hi*hi + hi*lo + lo*hi, fp32 accumulate); operands produced on
+// the fly are written by the epilogue threads straight into SWIZZLE_128B shared memory (validated by nnj_tc_selftest).  Node state
+// for UMMA 1 comes from site-major bf16 planes [B][C][S][128] [X | W_g X], indexed by PHYSICAL slot, so alpha is scattered to slot
+// order and dead / free slots simply get weight 0.
 #include <cstdio>
 #include <cstdlib>
 
@@ -739,58 +740,30 @@ k_score_inc(const __grid_constant__ CUtensorMap mapXh, const __grid_constant__ C
 
 // ------------------------------------------------------------------ host side
 
-// box {64, 64, 1} over site-major node planes [B*C][S][128]  ([X | W_g X] per slot)
-static int make_tmap_nodes(CUtensorMap* map, const void* base, int S, int BC, int box_rows = 64, int n_live = -1) {
-    typedef CUresult (*PFN)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                            const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-    static PFN enc = nullptr;
-    if (!enc) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) != cudaSuccess || qres != cudaDriverEntryPointSuccess)
-            return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
-        enc = reinterpret_cast<PFN>(p);
-    }
-    cuuint64_t gdim[3] = {128, (cuuint64_t)(n_live > 0 ? n_live : S), (cuuint64_t)BC};   // slots >= n_live are dead: zero-filled, never loaded
-    cuuint64_t gstr[2] = {256, (cuuint64_t)S * 256};
-    cuuint32_t box[3] = {64, (cuuint32_t)box_rows, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled failed for the node planes");
-    return 0;
+int make_tmap_nodes(CUtensorMap* map, const void* base, int S, int BC, int box_rows, int n_live) {
+    const cuuint64_t gdim[3] = {128, (cuuint64_t)(n_live > 0 ? n_live : S), (cuuint64_t)BC};   // slots >= n_live are dead: zero-filled, never loaded
+    const cuuint64_t gstr[2] = {256, (cuuint64_t)S * 256};
+    const cuuint32_t box[3] = {64, (cuuint32_t)box_rows, 1};
+    return encode_tmap(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, base, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                       "the node planes");
 }
 
-// x planes [B][pc][C][64] fp32 as a 4-D tensor (d, site, pair, tree); box = 32 channels of 64 pairs at one site (pairs >= nc read as 0)
-static int make_tmap_xtile(CUtensorMap* map, const float* base, int pc, int nrows, int C, int B, int box_rows = 64) {
-    typedef CUresult (*PFN)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                            const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) != cudaSuccess || qres != cudaDriverEntryPointSuccess)
-        return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
-    cuuint64_t gdim[4] = {64, (cuuint64_t)C, (cuuint64_t)nrows, (cuuint64_t)B};
-    cuuint64_t gstr[3] = {256, (cuuint64_t)C * 256, (cuuint64_t)pc * C * 256};
-    cuuint32_t box[4] = {32, 1, (cuuint32_t)box_rows, 1};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = reinterpret_cast<PFN>(p)(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), gdim, gstr, box, estr,
-                                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled failed for the x tiles");
-    return 0;
+int make_tmap_xtile(CUtensorMap* map, const float* base, int pc, int nrows, int C, int B, int box_rows) {
+    const cuuint64_t gdim[4] = {64, (cuuint64_t)C, (cuuint64_t)nrows, (cuuint64_t)B};
+    const cuuint64_t gstr[3] = {256, (cuuint64_t)C * 256, (cuuint64_t)pc * C * 256};
+    const cuuint32_t box[4] = {32, 1, (cuuint32_t)box_rows, 1};
+    return encode_tmap(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, base, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                       "the x tiles");
 }
 
 // <= 64 pairs per tree: the persistent site-parity kernel
 static int launch_score_inc(const Model* m, const float* xf, int pc, const void* nodes_h, const void* nodes_l, const float* alpha, int RP,
                             int alpha_pairs, const int32_t* slot_of, int slot_stride, const int32_t* pair_i, int pair_stride, int n0, int nc, int Rp,
                             int S, int C, int B, const uint8_t* mask, float* score_part, int nSG, int* n_part, cudaStream_t st) {
-    {   // late steps (<= 16 pairs over <= 16 live nodes; NNJ_SCORE_SMALL=2: <= 32, slower than the narrow mode below): the register-fragment kernel, whose cost follows the number of live pairs (nnj_score_small.cu)
-        static int small_on = -1;
-        if (small_on < 0) { const char* ev = getenv("NNJ_SCORE_SMALL"); small_on = ev ? atoi(ev) : 1; }
-        if (small_on && nc <= (small_on > 1 ? 32 : 16) && Rp <= (small_on > 1 ? 32 : 16) && !(C & 7))
-            return launch_score_small(m, xf, pc, nodes_h, nodes_l, alpha, RP, alpha_pairs, slot_of, slot_stride, pair_i, pair_stride, n0, nc, Rp, S, C, B, mask,
-                                      score_part, nSG, n_part, st);
-    }
+    // late steps (<= 16 pairs over <= 16 live nodes): the register-fragment kernel, whose cost follows the number of live pairs (nnj_score_small.cu)
+    if (nc <= 16 && Rp <= 16 && !(C & 7))
+        return launch_score_small(m, xf, pc, nodes_h, nodes_l, alpha, RP, alpha_pairs, slot_of, slot_stride, pair_i, pair_stride, n0, nc, Rp, S, C, B, mask,
+                                  score_part, nSG, n_part, st);
     static DevOnce once;      // per device, not per process
     if (once.need()) {
         cudaError_t e = cudaFuncSetAttribute(k_score_inc, cudaFuncAttributeMaxDynamicSharedMemorySize, SI_SMEM_MAX);
@@ -806,8 +779,8 @@ static int launch_score_inc(const Model* m, const float* xf, int pc, const void*
     if (trace_state > 0 && nc == trace_state) { if (!trace_buf) cudaMalloc(&trace_buf, 32 * 600 * 8); cudaMemsetAsync(trace_buf, 0, 32 * 600 * 8, st); a.trace = trace_buf; }
     { static int dbg = -1; if (dbg < 0) { const char* ev = getenv("NNJ_SCORE_DBG"); dbg = ev ? atoi(ev) : 0; } a.dbg = dbg; }
 #endif
+    a.narrow = nc <= 32 ? 1 : 0;
     // the live nodes occupy physical slots [0, Rp) (k_select keeps them compact): only those rows are streamed / contracted
-    { static int nw = -1; if (nw < 0) { const char* ev = getenv("NNJ_SCORE_NARROW"); nw = ev ? atoi(ev) : 1; } a.narrow = (nw && nc <= 32) ? 1 : 0; }
     a.node_rows = (Rp + 7) & ~7; a.x_rows = (nc + 7) & ~7;
     const int stage = 4 * a.node_rows * 128 + 2 * a.x_rows * 128;
     a.nst = (SI_SMEM_MAX - 1024 - SI_RING - 1024 - SI_MISC_BYTES) / stage;
@@ -858,13 +831,9 @@ int launch_score_tc(const Model* m, const float* xf, int pc, const void* nodes_h
         once.done();
     }
     if (S > 64) return set_error(NNJ_ERR_INVALID, "score_tc: at most 63 taxa on the tensor-core pair-score path");
-    {
-        static int inc = -1;
-        if (inc < 0) { const char* ev = getenv("NNJ_SCORE_INC"); inc = ev ? atoi(ev) : 1; }
-        if (inc && nc <= 64)
-            return launch_score_inc(m, xf, pc, nodes_h, nodes_l, alpha, RP, alpha_pairs, slot_of, slot_stride, pair_i, pair_stride, n0, nc, Rp, S, C, B,
-                                    mask, score_part, nSG, n_part, st);
-    }
+    if (nc <= 64)
+        return launch_score_inc(m, xf, pc, nodes_h, nodes_l, alpha, RP, alpha_pairs, slot_of, slot_stride, pair_i, pair_stride, n0, nc, Rp, S, C, B,
+                                mask, score_part, nSG, n_part, st);
     *n_part = (C + ST_SITES - 1) / ST_SITES;
     CUtensorMap mh, ml, mx;
     if (int e = make_tmap_xtile(&mx, xf, pc, nc, C, B)) return e;

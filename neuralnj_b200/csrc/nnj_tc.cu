@@ -13,7 +13,7 @@
 // Every mbarrier wait is bounded (trap after ~20 s) so that a protocol bug surfaces as an error, not a hang.
 //
 // CTA-pair kernels (cta_group::2, clusters of two CTAs on one TPC; further down): k_tc_gemm2 (256 x 256 tiles, half the B tile per SM),
-// k_tc_gemm2s (Q K^T with the row softmax in the epilogue - the default of the tied row attention), k_tc_gemm2w (P V in one pass over P).
+// k_tc_gemm2s (Q K^T with the row softmax in the epilogue - the tied row attention where row_qk_softmax_ok holds), k_tc_gemm2w (P V in one pass over P).
 // The single-CTA k_tc_gemm serves shapes without an even number of 128-row blocks, split-K launches, the 64 / 128-column tiles and the
 // one-product mode (NNJ_PREC_BF16).
 #include "nnj_internal.h"
@@ -1061,61 +1061,52 @@ typedef CUresult (*PFN_tmapEncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuin
                                         const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                         CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-static PFN_tmapEncodeTiled tmap_encoder() {
-    static PFN_tmapEncodeTiled fn = nullptr;
-    if (!fn) {
+int encode_tmap(CUtensorMap* map, CUtensorMapDataType dtype, int rank, const void* base, const cuuint64_t* dims, const cuuint64_t* strides,
+                const cuuint32_t* box, CUtensorMapSwizzle swizzle, CUtensorMapL2promotion l2, const char* what) {
+    static PFN_tmapEncodeTiled enc = nullptr;
+    if (!enc) {
         void* p = nullptr;
         cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_tmapEncodeTiled>(p);
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) != cudaSuccess || qres != cudaDriverEntryPointSuccess)
+            return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
+        enc = reinterpret_cast<PFN_tmapEncodeTiled>(p);
     }
-    return fn;
-}
-
-// 3-D bf16 tensor [Z][rows][K] (K contiguous, row pitch ld elements, batch stride sz elements), box 64 x 128 x 1, SWIZZLE_128B.
-int make_tmap_k_major(CUtensorMap* map, const void* base, int K, int rows, int Z, size_t ld, size_t sz, int box_rows) {
-    PFN_tmapEncodeTiled enc = tmap_encoder();
-    if (!enc) return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
-    if ((ld * 2) % 16 != 0 || (sz * 2) % 16 != 0 || (reinterpret_cast<uintptr_t>(base) & 15))
-        return set_error(NNJ_ERR_INVALID, "tensor-core path: operand rows must be 16-byte aligned (K and site count multiples of 8)");
-    cuuint64_t gdim[3] = {(cuuint64_t)K, (cuuint64_t)rows, (cuuint64_t)Z};
-    cuuint64_t gstr[2] = {(cuuint64_t)ld * 2, (cuuint64_t)sz * 2};
-    cuuint32_t box[3] = {(cuuint32_t)TC_BK, (cuuint32_t)box_rows, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+    CUresult r = enc(map, dtype, (cuuint32_t)rank, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, l2,
+                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) {
-        char msg[96];
-        snprintf(msg, sizeof(msg), "cuTensorMapEncodeTiled failed (CUresult %d)", (int)r);
+        char msg[128];
+        snprintf(msg, sizeof(msg), "cuTensorMapEncodeTiled failed for %s (CUresult %d)", what, (int)r);
         return set_error(NNJ_ERR_CUDA, msg);
     }
     return 0;
 }
 
+// 3-D bf16 tensor [Z][rows][K] (K contiguous, row pitch ld elements, batch stride sz elements), box 64 x 128 x 1, SWIZZLE_128B.
+int make_tmap_k_major(CUtensorMap* map, const void* base, int K, int rows, int Z, size_t ld, size_t sz, int box_rows) {
+    if ((ld * 2) % 16 != 0 || (sz * 2) % 16 != 0 || (reinterpret_cast<uintptr_t>(base) & 15))
+        return set_error(NNJ_ERR_INVALID, "tensor-core path: operand rows must be 16-byte aligned (K and site count multiples of 8)");
+    const cuuint64_t gdim[3] = {(cuuint64_t)K, (cuuint64_t)rows, (cuuint64_t)Z};
+    const cuuint64_t gstr[2] = {(cuuint64_t)ld * 2, (cuuint64_t)sz * 2};
+    const cuuint32_t box[3] = {(cuuint32_t)TC_BK, (cuuint32_t)box_rows, 1};
+    return encode_tmap(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, base, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                       "a K-major operand");
+}
+
 // 3-D bf16 tensor [Z][K][N] (N contiguous, pitch ld elements), box 64 (N) x 64 (K) x 1, SWIZZLE_128B: MN-major B operand tiles.
 static int make_tmap_mn_major(CUtensorMap* map, const void* base, int N, int K, int Z, size_t ld, size_t sz) {
-    PFN_tmapEncodeTiled enc = tmap_encoder();
-    if (!enc) return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
     if ((ld * 2) % 16 != 0 || (sz * 2) % 16 != 0 || (reinterpret_cast<uintptr_t>(base) & 15))
         return set_error(NNJ_ERR_INVALID, "tensor-core path: operand rows must be 16-byte aligned");
-    cuuint64_t gdim[3] = {(cuuint64_t)N, (cuuint64_t)K, (cuuint64_t)Z};
-    cuuint64_t gstr[2] = {(cuuint64_t)ld * 2, (cuuint64_t)sz * 2};
-    cuuint32_t box[3] = {64, 64, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return set_error(NNJ_ERR_CUDA, "cuTensorMapEncodeTiled failed (MN-major operand)");
-    return 0;
+    const cuuint64_t gdim[3] = {(cuuint64_t)N, (cuuint64_t)K, (cuuint64_t)Z};
+    const cuuint64_t gstr[2] = {(cuuint64_t)ld * 2, (cuuint64_t)sz * 2};
+    const cuuint32_t box[3] = {64, 64, 1};
+    return encode_tmap(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, base, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                       "an MN-major operand");
 }
 
 static int tc_sm_count() { return sm_count(); }    // of the current device (cached per device, nnj_api.cu)
 
-// ---- CTA-pair GEMM (k_tc_gemm2).  NNJ_GEMM_2SM: bit 0 = the K-major instantiation (Q K^T), bit 1 = the MN-major one (P V), bit 2 = the
-// one-pass form of P V for 256 < N <= 512 (k_tc_gemm2w); default all.
-static int gemm2_mask() {
-    static const int mk = [] { const char* v = getenv("NNJ_GEMM_2SM"); return v ? (atoi(v) & 7) : 7; }();
-    return mk;
-}
+// ---- CTA-pair GEMM (k_tc_gemm2)
 template <bool BMN>
 static int gemm2_clusters() {      // CTA pairs that can be resident at once on the current device (cached per device)
     static std::atomic<int> cache[64];
@@ -1153,7 +1144,7 @@ static int launch_tc_gemm2(int cls, const CUtensorMap& mAh, const CUtensorMap& m
     if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
     return 0;
 }
-// one pass over A for 256 < N <= 512 (NNJ_GEMM_2SM bit 2 = off switch: value 3 keeps the two-tile form)
+// one pass over A for 256 < N <= 512
 static int launch_tc_gemm2w(int cls, const CUtensorMap& mAh, const CUtensorMap& mAl, const CUtensorMap& mBh, const CUtensorMap& mBl, const TcGemmArgs& g,
                             cudaStream_t st) {
     static DevOnce once;
@@ -1173,14 +1164,13 @@ static int launch_tc_gemm2w(int cls, const CUtensorMap& mAh, const CUtensorMap& 
     if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
     return 0;
 }
-static bool gemm2_ok(int bit, int M, int N, int bn, int nsplit, int products) {
-    return (gemm2_mask() >> bit & 1) && bn == 256 && nsplit == 1 && products == 3 && M % (2 * TC_BM) == 0 && N >= 256;
+static bool gemm2_ok(int M, int N, int bn, int nsplit, int products) {
+    return bn == 256 && nsplit == 1 && products == 3 && M % (2 * TC_BM) == 0 && N >= 256;
 }
 
-// S = Q K^T with the softmax in the epilogue (k_tc_gemm2s).  NNJ_ROW_FUSED=0 keeps the three-kernel form (GEMM, softmax pass, GEMM).
+// S = Q K^T with the softmax in the epilogue (k_tc_gemm2s)
 bool row_qk_softmax_ok(int C, int products) {
-    static const int on = [] { const char* v = getenv("NNJ_ROW_FUSED"); return v ? atoi(v) : 1; }();
-    return on && products == 3 && (gemm2_mask() & 1) && C >= 256 && C % 256 == 0 && C <= 4096;
+    return products == 3 && C % 256 == 0 && C >= 256 && C <= 4096;
 }
 int launch_row_qk_softmax(int cls, const void* Qh, const void* Ql, const void* Kh, const void* Kl, void* Ph, void* Pl, float* rowsum, const uint8_t* mask,
                           int heads, int Z, int C, int K, cudaStream_t st) {
@@ -1232,8 +1222,10 @@ int launch_tc_gemm_bmn(int cls, const void* Ah, const void* Al, const void* Bh, 
     TcGemmArgs g{Cm, M, N, K, ldc, sC, Z, 1, (K + TC_BK - 1) / TC_BK, 0};
     g.row_div = row_div;
     const int bn = N > 128 ? 256 : 128;         // 128 x 256 tiles: a UMMA with N = 256 runs at 75 % of the tensor peak, N = 128 at 60 %
-    if (gemm2_ok(1, M, N, bn, 1, products) && (gemm2_mask() & 4) && N > 256 && N <= 512) return launch_tc_gemm2w(cls, mAh, mAl, mBh, mBl, g, st);
-    if (gemm2_ok(1, M, N, bn, 1, products)) return launch_tc_gemm2<true>(cls, mAh, mAl, mBh, mBl, g, st);
+    if (gemm2_ok(M, N, bn, 1, products)) {
+        if (N > 256 && N <= 512) return launch_tc_gemm2w(cls, mAh, mAl, mBh, mBl, g, st);
+        return launch_tc_gemm2<true>(cls, mAh, mAl, mBh, mBl, g, st);
+    }
     const int n_tiles = ((N + bn - 1) / bn) * ((M + TC_BM - 1) / TC_BM) * Z;
     const dim3 grid(n_tiles < tc_sm_count() ? n_tiles : tc_sm_count());
     prof_begin(cls, st);
@@ -1272,7 +1264,7 @@ int launch_tc_gemm_ex(int cls, const void* Ah, const void* Al, const void* Bh, c
     if (int e = make_tmap_k_major(&mBh, Bh, K, N, Z, ldb, sB, bn)) return e;
     if (int e = make_tmap_k_major(&mBl, Bl, K, N, Z, ldb, sB, bn)) return e;
     TcGemmArgs g{Cm, M, N, K, ldc, sC, Z, nsplit, chunks_per_split, split_stride};
-    if (gemm2_ok(0, M, N, bn, nsplit, products) && N % 256 == 0) {
+    if (gemm2_ok(M, N, bn, nsplit, products) && N % 256 == 0) {
         CUtensorMap mBh2, mBl2;      // half an N tile per CTA of the pair
         if (int e = make_tmap_k_major(&mBh2, Bh, K, N, Z, ldb, sB, 128)) return e;
         if (int e = make_tmap_k_major(&mBl2, Bl, K, N, Z, ldb, sB, 128)) return e;

@@ -14,8 +14,9 @@ pytestmark = pytest.mark.gpu
 
 
 # taxa -> step-0 pairs: 12 -> 66 (one full tile), 17 -> 136 (128 + 8: second score tile duplicated), 24 -> 276 (second
-# alpha launch of 20 pairs: parity split at step 0), 33 -> 528 (two launches + 16), 63 -> 1953 (largest tensor-core size)
-@pytest.mark.parametrize("R,L", [(12, 128), (17, 192), (24, 128), (33, 64), (63, 72), (64, 64), (49, 136)])
+# alpha launch of 20 pairs: parity split at step 0), 33 -> 528 (two launches + 16), 63 -> 1953 (largest tensor-core size); 40 x 256:
+# the late steps (33-64 pairs: 2-way site split, <= 32: lane quarters, <= 16: register-fragment kernels) over two 128-site groups
+@pytest.mark.parametrize("R,L", [(12, 128), (17, 192), (24, 128), (33, 64), (63, 72), (64, 64), (49, 136), (40, 256)])
 def test_tile_shapes_match_oracle(R, L, sd0, gpu_models):
     import nnj_oracle as O
     data = O.evolved_msa(2, R, L, seed=100 + R)
@@ -127,55 +128,6 @@ def test_large_alignment_200x4096(gpu_models):
     assert bool(torch.isfinite(s2).all())
 
 
-_TOGGLE_SCRIPT = r"""
-import sys, torch
-sys.path.insert(0, sys.argv[1]); sys.path.insert(0, sys.argv[1] + "/oracle")
-import nnj_oracle as O
-from neuralnj_b200 import PhyloATTN, inference_config
-torch.manual_seed(0)
-m = PhyloATTN(inference_config(), precision="bf16x3").cuda().eval()
-data = O.evolved_msa(2, 40, 256, seed=11)
-mask = torch.zeros(2, 256, dtype=torch.bool)
-merges, slp, trace = m.rollout_fused(data.cuda(), mask.cuda(), want_logits=True)
-torch.save({"merges": merges.cpu(), "trace": trace.cpu()}, sys.argv[2])
-"""
-
-
-def test_lane_quarter_modes_agree_with_the_two_way_split(tmp_path):
-    """<= 32 pairs: k_alpha_v3 splits the tile over four sites (NNJ_ALPHA_QUAD) and k_score_inc splits a pair's channels over
-    two warps (NNJ_SCORE_NARROW); <= 16 pairs: the register-fragment kernels k_alpha_small / k_score_small take over
-    (NNJ_ALPHA_SMALL, NNJ_SCORE_SMALL).  All must reproduce the 2-way site-parity tcgen05 kernels they replace: same merges, logits
-    within the tolerance of the oracle comparison (the partial sums are grouped differently, nothing else changes).  The switches
-    are read once per process, hence the two subprocesses."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    outs = []
-    for tag, env in (("new", {}), ("old", {"NNJ_ALPHA_QUAD": "0", "NNJ_SCORE_NARROW": "0", "NNJ_SCORE_SMALL": "0", "NNJ_ALPHA_SMALL": "0"})):
-        path = str(tmp_path / f"{tag}.pt")
-        subprocess.run([sys.executable, "-c", _TOGGLE_SCRIPT, root, path], check=True, env={**os.environ, **env}, timeout=300)
-        outs.append(torch.load(path))
-    # Same merges - or, where the two groupings of the partial sums break a numerical tie differently, both choices within the logit
-    # tolerance of each other in BOTH runs (the trajectories part there, so only the steps up to that one are compared).
-    m0, m1, t0, t1 = outs[0]["merges"].long(), outs[1]["merges"].long(), outs[0]["trace"], outs[1]["trace"]
-    R = m0.shape[1] + 1
-    for b in range(m0.shape[0]):
-        diff = (m0[b] != m1[b]).any(dim=1).nonzero()
-        t_end = int(diff[0]) if len(diff) else R - 1
-        off = 0
-        for t in range(min(t_end + 1, R - 1)):
-            n = R - t
-            P = n * (n - 1) // 2
-            a0, a1 = t0[b, off:off + P], t1[b, off:off + P]
-            scale = float(a0.abs().max())
-            assert float((a0 - a1).abs().max()) / scale < LOGIT_TOL
-            if t == t_end:
-                idx = [i * n - i * (i + 1) // 2 + (j - i - 1) for i, j in (m0[b, t].tolist(), m1[b, t].tolist())]
-                assert abs(float(a0[idx[0]] - a0[idx[1]])) / scale < LOGIT_TOL and abs(float(a1[idx[0]] - a1[idx[1]])) / scale < LOGIT_TOL
-            off += P
-
-
 # Row-attention GEMM dispatch (nnj_tc.cu): ctx = P V has N = 8 R columns and M = C rows.  C % 256 == 0 selects the CTA-pair kernels:
 # N <= 256 (R <= 32) k_tc_gemm2<true> with one (ragged) N tile, 256 < N <= 512 the one-pass k_tc_gemm2w (second UMMA of 16 .. 256 columns:
 # R = 33 -> 16, 45 -> 112, 50 -> 144, 64 -> 256), N > 512 k_tc_gemm2<true> with three N tiles; C = 384 (odd number of 128-row blocks) stays on
@@ -190,42 +142,3 @@ def test_row_gemm_variants_encoder_matches_oracle(R, C, sd0, gpu_models):
     got = gpu_models["bf16x3"].encode_zxr(data.cuda(), mask.cuda()).cpu()
     err = float((got - ref).abs().max() / ref.abs().max())
     assert err < 5e-5, err
-
-
-_ENC_SCRIPT = r"""
-import sys, torch
-root, out = sys.argv[1], sys.argv[2]
-sys.path.insert(0, root); sys.path.insert(0, root + "/oracle")
-import nnj_oracle as O
-from neuralnj_b200 import PhyloATTN, inference_config
-torch.manual_seed(0)
-model = PhyloATTN(inference_config(), precision="bf16x3").to("cuda:0").eval()
-res = {}
-for R, C in ((50, 512), (20, 256)):
-    data = O.evolved_msa(2, R, C, seed=R + C)
-    mask = torch.zeros(2, C, dtype=torch.bool); mask[1, C - 40:] = True
-    res[(R, C)] = model.encode_zxr(data.cuda(), mask.cuda()).cpu()
-torch.save(res, out)
-"""
-
-
-@pytest.mark.parametrize("env", [{"NNJ_ROW_FUSED": "0"}, {"NNJ_ROW_FUSED": "0", "NNJ_GEMM_2SM": "3"}, {"NNJ_GEMM_2SM": "0"}, {"NNJ_MERGE_TC": "0"}],
-                         ids=["softmax_pass", "two_tile_pv", "single_cta_gemms", "merge_cuda_cores"])
-def test_row_attention_fallback_forms_match_oracle(env, sd0, tmp_path):
-    """The diagnostic switches of the row attention select the forms the fused CTA-pair kernels replaced (three-kernel softmax, two-N-tile
-    P V, single-CTA GEMMs); each must still meet the encoder tolerance against the oracle.  Switches are read once per process."""
-    import os
-    import subprocess
-    import sys
-    import nnj_oracle as O
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    path = str(tmp_path / "enc.pt")
-    subprocess.run([sys.executable, "-c", _ENC_SCRIPT, root, path], check=True, env={**os.environ, **env}, timeout=300)
-    res = torch.load(path)
-    for (R, C), got in res.items():
-        data = O.evolved_msa(2, R, C, seed=R + C)
-        mask = torch.zeros(2, C, dtype=torch.bool)
-        mask[1, C - 40:] = True
-        ref = O.encode(sd0, data, mask)
-        err = float((got - ref).abs().max() / ref.abs().max())
-        assert err < 5e-5, (env, R, C, err)
