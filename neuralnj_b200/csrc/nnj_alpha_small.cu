@@ -29,14 +29,6 @@ struct AlphaSmallArgs {
     float* alpha_part; int alpha_pairs; int nSG; int RP;
 };
 
-__device__ __forceinline__ void as_mma(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3]) : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ void as_cp16(uint32_t dst, const void* src) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-}
-
 template <int T, int WARPS>
 __global__ void __launch_bounds__(WARPS * 32, 1) k_alpha_small(const AlphaSmallArgs a) {
     constexpr int ROWS = 16 * T;
@@ -95,16 +87,16 @@ __global__ void __launch_bounds__(WARPS * 32, 1) k_alpha_small(const AlphaSmallA
             const float* py = a.Y + tb + ((size_t)ld_slot0 * a.C + c) * 64 + ld_ch * 4;
             for (int slot = ld_slot0; slot < a.Rp; slot += 2, px += ld_stride_x, py += ld_stride_x) {
                 const uint32_t off = mybuf_u + slot * 256 + ((ld_ch ^ (slot & 7)) << 4);
-                as_cp16(off, px);
-                as_cp16(off + XB, py);
+                cp_async16(off, px);
+                cp_async16(off + XB, py);
             }
             // K' rows (hi, lo): lane = (slot mod 4, chunk), four slots per pass
             const __nv_bfloat16* ph = a.kph + (((size_t)b * a.S + (lane >> 3)) * a.C + c) * 64 + (lane & 7) * 8;
             const __nv_bfloat16* pl = a.kpl + (((size_t)b * a.S + (lane >> 3)) * a.C + c) * 64 + (lane & 7) * 8;
             for (int slot = lane >> 3; slot < a.Rp; slot += 4, ph += ld_stride_k, pl += ld_stride_k) {
                 const uint32_t off = mybuf_u + 2 * XB + slot * 128 + (((lane & 7) ^ (slot & 7)) << 4);
-                as_cp16(off, ph);
-                as_cp16(off + KB, pl);
+                cp_async16(off, ph);
+                cp_async16(off + KB, pl);
             }
         }
         asm volatile("cp.async.commit_group;" ::: "memory");
@@ -141,9 +133,9 @@ __global__ void __launch_bounds__(WARPS * 32, 1) k_alpha_small(const AlphaSmallA
                 const uint32_t kl0 = *reinterpret_cast<const uint32_t*>(kr + KB + (((2 * kk) ^ g) << 4)), kl1 = *reinterpret_cast<const uint32_t*>(kr + KB + (((2 * kk + 1) ^ g) << 4));
 #pragma unroll
                 for (int m = 0; m < T; ++m) {
-                    as_mma(acc[m][j], xl[m], kh0, kh1);      // small terms first
-                    as_mma(acc[m][j], xh[m], kl0, kl1);
-                    as_mma(acc[m][j], xh[m], kh0, kh1);
+                    mma_m16n8k16(acc[m][j], xl[m], kh0, kh1);      // small terms first
+                    mma_m16n8k16(acc[m][j], xh[m], kl0, kl1);
+                    mma_m16n8k16(acc[m][j], xh[m], kh0, kh1);
                 }
             }
         }
@@ -171,30 +163,22 @@ __global__ void __launch_bounds__(WARPS * 32, 1) k_alpha_small(const AlphaSmallA
     }
 }
 
-int launch_alpha_small(const Model* m, const float* X, const float* Y, size_t tree_stride, const int32_t* slot_of, int slot_stride, const int32_t* pair_i,
-                       const int32_t* pair_j, int pair_stride, int n0, int nc, int S, int n_live, int C, int B, const void* kp_h, const void* kp_l, float* xf,
-                       int pc, float* alpha_part, int alpha_pairs, int nSG, int RP, int* n_part, cudaStream_t st) {
-    if (nc > 16 || n_live > 16 || nc < 1 || nc > pc) return set_error(NNJ_ERR_INVALID, "alpha_small: at most 16 pairs over 16 live nodes");
-    const int groups = (C + AS_SITES - 1) / AS_SITES;
+int launch_alpha_small(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st) {
+    if (c.nc > 16 || c.Rp > 16 || c.nc < 1 || c.nc > c.pc) return set_error(NNJ_ERR_INVALID, "alpha_small: at most 16 pairs over 16 live nodes");
+    const int groups = (c.C + AS_SITES - 1) / AS_SITES;
     *n_part = groups;
-    if (groups > nSG) return set_error(NNJ_ERR_INVALID, "alpha_small: partial buffer too small");
+    if (groups > c.nAP) return set_error(NNJ_ERR_INVALID, "alpha_small: partial buffer too small");
     AlphaSmallArgs a;
-    a.X = X; a.Y = Y; a.tree_stride = tree_stride; a.kph = (const __nv_bfloat16*)kp_h; a.kpl = (const __nv_bfloat16*)kp_l; a.S = S;
-    a.slot_of = slot_of; a.slot_stride = slot_stride; a.pair_i = pair_i; a.pair_j = pair_j; a.pair_stride = pair_stride; a.n0 = n0; a.nc = nc;
-    a.Rp = n_live; a.C = C; a.bh = m->nj.bh; a.xf = xf; a.pc = pc; a.alpha_part = alpha_part; a.alpha_pairs = alpha_pairs; a.nSG = nSG; a.RP = RP;
+    a.X = c.X; a.Y = c.Y; a.tree_stride = c.tree_stride; a.kph = (const __nv_bfloat16*)c.kp_h; a.kpl = (const __nv_bfloat16*)c.kp_l; a.S = c.S;
+    a.slot_of = c.slot_of; a.slot_stride = c.slot_stride; a.pair_i = c.pair_i; a.pair_j = c.pair_j; a.pair_stride = c.pair_stride; a.n0 = c.n0;
+    a.nc = c.nc; a.Rp = c.Rp; a.C = c.C; a.bh = m->nj.bh; a.xf = c.xf; a.pc = c.pc;
+    a.alpha_part = c.alpha_part; a.alpha_pairs = c.alpha_pairs; a.nSG = c.nAP; a.RP = c.RP;
     constexpr size_t smem = 1024 + 1024 + 16 * (16 * 768);      // alignment | biases, pair slots | 16 warps x one site buffer (X, Y, K' hi / lo)
     static DevOnce once;      // per device, not per process
-    if (once.need()) {
-        cudaError_t e = cudaFuncSetAttribute(k_alpha_small<1, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
-        once.done();
-    }
+    if (int e = smem_opt_in(once, k_alpha_small<1, 16>, smem)) return e;
     prof_begin(KC_ALPHA, st);
-    k_alpha_small<1, 16><<<dim3(groups, B), 16 * 32, smem, st>>>(a);
-    ++g_launches;
-    prof_end(st);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
+    k_alpha_small<1, 16><<<dim3(groups, c.B), 16 * 32, smem, st>>>(a);
+    LAUNCH_CHECK();
     return 0;
 }
 

@@ -356,52 +356,40 @@ static int make_tmap_kprime(CUtensorMap* map, const void* base, int S, int n_liv
 }
 
 // writes the x planes of pairs [n0, n0+nc) and alpha_part[b][n][partial][slot]; returns the number of partials per pair in *n_part
-int launch_alpha_tc(const Model* m, const float* X, const float* Y, size_t tree_stride, const int32_t* slot_of, int slot_stride, const int32_t* pair_i,
-                    const int32_t* pair_j, int pair_stride, int n0, int nc, int S, int n_live, int C, int B, const void* kp_h, const void* kp_l, float* xf,
-                    int pc, float* alpha_part, int alpha_pairs, int nSG, int RP, int* n_part, cudaStream_t st) {
-    // late steps (<= 16 pairs over <= 16 live nodes): the register-fragment kernel, whose cost follows the number of live pairs (nnj_alpha_small.cu)
-    if (nc <= 16 && n_live <= 16 && !(C & 7))
-        return launch_alpha_small(m, X, Y, tree_stride, slot_of, slot_stride, pair_i, pair_j, pair_stride, n0, nc, S, n_live, C, B, kp_h, kp_l, xf, pc,
-                                  alpha_part, alpha_pairs, nSG, RP, n_part, st);
+int launch_alpha_v3(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st) {
     static DevOnce once;      // per device, not per process
-    if (once.need()) {
-        cudaError_t e = cudaFuncSetAttribute(k_alpha_v3, cudaFuncAttributeMaxDynamicSharedMemorySize, AV_SMEM_MAX);
-        if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
-        once.done();
-    }
+    if (int e = smem_opt_in(once, k_alpha_v3, AV_SMEM_MAX)) return e;
     const int n_sm = sm_count();
-    if (S > 64) return set_error(NNJ_ERR_INVALID, "alpha_tc: at most 63 taxa on the tensor-core path");
-    if (nc > AV_MAXT * 128 || nc > pc) return set_error(NNJ_ERR_INVALID, "alpha_tc: at most 512 pairs per launch");
-    const int groups = (C + AV_SITES - 1) / AV_SITES;
-    const bool dup = nc <= 64;
-    const int ways = !dup ? 1 : (nc <= 32 && 4 * groups <= nSG) ? 4 : 2;
+    if (c.S > 64) return set_error(NNJ_ERR_INVALID, "alpha_v3: at most 63 taxa on the tensor-core path");
+    if (c.nc > AV_MAXT * 128 || c.nc > c.pc) return set_error(NNJ_ERR_INVALID, "alpha_v3: at most 512 pairs per launch");
+    const int groups = (c.C + AV_SITES - 1) / AV_SITES;
+    const bool dup = c.nc <= 64;
+    const int ways = !dup ? 1 : (c.nc <= 32 && 4 * groups <= c.nAP) ? 4 : 2;
     *n_part = ways * groups;
-    if (*n_part > nSG) return set_error(NNJ_ERR_INVALID, "alpha_tc: partial buffer too small");
-    // the live nodes occupy physical slots [0, n_live) (k_select keeps them compact): only those rows are streamed
-    const int rows8 = (n_live + 7) & ~7;
+    if (*n_part > c.nAP) return set_error(NNJ_ERR_INVALID, "alpha_v3: partial buffer too small");
+    // the live nodes occupy physical slots [0, Rp) (k_select keeps them compact): only those rows are streamed
+    const int rows8 = (c.Rp + 7) & ~7;
     AlphaV3Args a;
     a.tile_bytes = rows8 * 128;
     a.nmma = (rows8 + 15) & ~15;
     a.nst = (AV_SMEM_MAX - 1024 - AV_XS_BYTES - AV_MISC_BYTES) / (6 * a.tile_bytes);
     if (a.nst > AV_MAXST) a.nst = AV_MAXST;
     CUtensorMap mx, my, mh, ml, mo;
-    if (int e = make_tmap_xplanes(&mo, xf, pc, nc, C, B)) return e;
-    if (int e = make_tmap_pool_f32(&mx, X, tree_stride, n_live, C, B, rows8)) return e;
-    if (int e = make_tmap_pool_f32(&my, Y, tree_stride, n_live, C, B, rows8)) return e;
-    if (int e = make_tmap_kprime(&mh, kp_h, S, n_live, C, B, rows8)) return e;
-    if (int e = make_tmap_kprime(&ml, kp_l, S, n_live, C, B, rows8)) return e;
-    a.slot_of = slot_of; a.slot_stride = slot_stride;
-    a.pair_i = pair_i; a.pair_j = pair_j; a.pair_stride = pair_stride; a.n0 = n0; a.nc = nc; a.C = C; a.B = B; a.groups = groups; a.bh = m->nj.bh;
+    if (int e = make_tmap_xplanes(&mo, c.xf, c.pc, c.nc, c.C, c.B)) return e;
+    if (int e = make_tmap_pool_f32(&mx, c.X, c.tree_stride, c.Rp, c.C, c.B, rows8)) return e;
+    if (int e = make_tmap_pool_f32(&my, c.Y, c.tree_stride, c.Rp, c.C, c.B, rows8)) return e;
+    if (int e = make_tmap_kprime(&mh, c.kp_h, c.S, c.Rp, c.C, c.B, rows8)) return e;
+    if (int e = make_tmap_kprime(&ml, c.kp_l, c.S, c.Rp, c.C, c.B, rows8)) return e;
+    a.slot_of = c.slot_of; a.slot_stride = c.slot_stride;
+    a.pair_i = c.pair_i; a.pair_j = c.pair_j; a.pair_stride = c.pair_stride; a.n0 = c.n0; a.nc = c.nc; a.C = c.C; a.B = c.B; a.groups = groups;
+    a.bh = m->nj.bh;
     a.dup = dup ? 1 : 0; a.ways = ways;
-    a.alpha_part = alpha_part; a.alpha_pairs = alpha_pairs; a.nSG = nSG; a.RP = RP;
-    const int n_work = B * groups;
+    a.alpha_part = c.alpha_part; a.alpha_pairs = c.alpha_pairs; a.nSG = c.nAP; a.RP = c.RP;
+    const int n_work = c.B * groups;
     const size_t smem = 1024 + (size_t)a.nst * 6 * a.tile_bytes + AV_XS_BYTES + AV_MISC_BYTES;
     prof_begin(KC_ALPHA, st);
     k_alpha_v3<<<n_work < n_sm ? n_work : n_sm, AV_THREADS, smem, st>>>(mx, my, mh, ml, mo, a);
-    ++g_launches;
-    prof_end(st);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
+    LAUNCH_CHECK();
     return 0;
 }
 

@@ -555,14 +555,6 @@ size_t encoder_ws_bytes(const Model* m, int B, int R, int C) {
     return align_up(enc_tree_floats(m, R, C) * sizeof(float) * encoder_chunk(m, B, R, C), 256) + 256;
 }
 
-#define LAUNCH_CHECK()                                                         \
-    do {                                                                       \
-        ++g_launches;                                                          \
-        prof_end(st);                                                          \
-        cudaError_t e_ = cudaGetLastError();                                   \
-        if (e_ != cudaSuccess) return set_cuda_error(e_, __FILE__, __LINE__);  \
-    } while (0)
-
 int run_encoder(Model* m, const int8_t* data, const uint8_t* mask, int B, int R, int L, float* x, size_t x_tree_stride,
                 void* ws, size_t ws_bytes, cudaStream_t st) {
     const int C = L;  // patch_size == 1

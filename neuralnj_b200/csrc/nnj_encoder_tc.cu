@@ -494,19 +494,6 @@ __device__ __forceinline__ void col_attend(const float* __restrict__ qb, const f
 // ---- tensor-path attention (R <= 64).  q | k | v of the tile sit in shared memory as bf16 hi / lo planes [128 rows][64] (128 B per row,
 // the 16-byte chunk of head h stored at h ^ (row & 7): the A-operand swizzle, conflict-free for the fragment loads below).
 constexpr int K2_PLANE = 128 * 128;
-// D[16 x 8] += A[16 x 16] . B[16 x 8] on register fragments (bf16 operands, fp32 accumulate).  Lane (g = lane >> 2, t = lane & 3):
-// a0 = A[g][2t, 2t+1], a1 = A[g+8][2t, 2t+1], a2 = A[g][8+2t, 9+2t], a3 = A[g+8][8+2t, 9+2t]; b0 = B[2t, 2t+1][g], b1 = B[8+2t, 9+2t][g];
-// d0 d1 = D[g][2t, 2t+1], d2 d3 = D[g+8][2t, 2t+1].  Measured on B200 (scratch/hmma_bench.cu): one m16n8k16 and one m16n8k8 both hold a
-// sub-partition's legacy tensor pipe for 8 clocks (20 clocks latency), so the K = 16 form is used throughout.
-__device__ __forceinline__ void mma_m16n8k16(float (&d)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3]) : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
-}
-// four 8 x 8 b16 matrices (rows of 16 B, lane l supplies the address of row l & 7 of matrix l >> 3), transposed on the way in:
-// lane (g, t) receives M[2t, 2t+1][g] of every matrix = a B fragment half for a row-major [k][n] operand
-__device__ __forceinline__ void ldsm_x4_t(uint32_t (&r)[4], uint32_t addr) {
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
-}
 // One (site, head, 16-query-row block): S = Q K^T [16 x 8 NT], softmax over the R keys in registers (the C fragments of two key blocks
 // ARE the A fragment of the next m16n8k16), O = P V, normalised and written as bf16 hi / lo into the A operand of the column
 // out-projection.  The 3-product bf16 split costs two instructions per 8 keys in Q K^T - the head dimension is 8, so the K = 16 of one
@@ -527,8 +514,8 @@ __device__ __forceinline__ void col_attend_mma(const uint8_t* __restrict__ pl, u
     for (int n = 0; n < NT; ++n) {
         const uint32_t kh = *reinterpret_cast<const uint32_t*>(kp + n * 1024), kl = *reinterpret_cast<const uint32_t*>(kp + K2_PLANE + n * 1024);
         sc[n][0] = 0.f; sc[n][1] = 0.f; sc[n][2] = 0.f; sc[n][3] = 0.f;
-        mma_m16n8k16(sc[n], qh0, qh1, 0u, 0u, kl, 0u);        // q_hi . k_lo (small term first)
-        mma_m16n8k16(sc[n], qh0, qh1, ql0, ql1, kh, kh);      // q_hi . k_hi + q_lo . k_hi
+        mma_m16n8k16(sc[n], {qh0, qh1, 0u, 0u}, kl, 0u);        // q_hi . k_lo (small term first)
+        mma_m16n8k16(sc[n], {qh0, qh1, ql0, ql1}, kh, kh);      // q_hi . k_hi + q_lo . k_hi
     }
     {   // keys >= R do not exist (only the last key block can hold them)
         const int j = (NT - 1) * 8 + 2 * t;
@@ -563,9 +550,9 @@ __device__ __forceinline__ void col_attend_mma(const uint8_t* __restrict__ pl, u
             }
         }
         float (&o)[4] = (n2 & 1) ? o1 : o0;
-        mma_m16n8k16(o, pw[0], pw[1], pw[2], pw[3], vf[0], vf[1]);      // P_lo . V_hi
-        mma_m16n8k16(o, ph[0], ph[1], ph[2], ph[3], vf[2], vf[3]);      // P_hi . V_lo
-        mma_m16n8k16(o, ph[0], ph[1], ph[2], ph[3], vf[0], vf[1]);      // P_hi . V_hi
+        mma_m16n8k16(o, pw, vf[0], vf[1]);      // P_lo . V_hi
+        mma_m16n8k16(o, ph, vf[2], vf[3]);      // P_hi . V_lo
+        mma_m16n8k16(o, ph, vf[0], vf[1]);      // P_hi . V_hi
     }
     float s_a = l_a.x + l_a.y, s_b = l_b.x + l_b.y;
     s_a += __shfl_xor_sync(0xffffffffu, s_a, 1); s_a += __shfl_xor_sync(0xffffffffu, s_a, 2);
@@ -825,14 +812,6 @@ static int enc_tc_attrs() {
     return 0;
 }
 
-#define ETC_DONE()                                                             \
-    do {                                                                       \
-        ++g_launches;                                                          \
-        prof_end(st);                                                          \
-        cudaError_t e_ = cudaGetLastError();                                   \
-        if (e_ != cudaSuccess) return set_cuda_error(e_, __FILE__, __LINE__);  \
-    } while (0)
-
 int launch_enc_rowqkv_tc(const Model* m, int layer, const float* xs, size_t xs_tree_stride, int B, int R, int C, float q_scale, const uint8_t* mask,
                          void* qh, void* ql, void* kh, void* kl, void* vh, void* vl, cudaStream_t st) {
     if (int e = enc_tc_attrs()) return e;
@@ -848,7 +827,7 @@ int launch_enc_rowqkv_tc(const Model* m, int layer, const float* xs, size_t xs_t
     const int grid = work < 2 * sm_count() ? work : 2 * sm_count();
     prof_begin(KC_LN_QKV, st);
     k_enc_rowqkv_tc<<<grid, ET_THREADS, K1_SMEM, st>>>(a);
-    ETC_DONE();
+    LAUNCH_CHECK();
     return 0;
 }
 
@@ -879,7 +858,7 @@ int launch_enc_colblock_tc(const Model* m, int layer, float* xs, size_t xs_tree_
         case 8: k_enc_colblock_tc<2, 8><<<grid, K2_THREADS, K2_SMEM, st>>>(a); break;
         default: k_enc_colblock_tc<4, 0><<<grid, K2_THREADS, K2_SMEM, st>>>(a); break;
     }
-    ETC_DONE();
+    LAUNCH_CHECK();
     return 0;
 }
 
@@ -895,14 +874,14 @@ int launch_enc_ffn_tc(const Model* m, int layer, float* xs, size_t xs_tree_strid
     const int grid = work < sm_count() ? work : sm_count();
     prof_begin(KC_FFN, st);
     k_enc_ffn_tc<<<grid, K3_THREADS, K3_SMEM, st>>>(a);
-    ETC_DONE();
+    LAUNCH_CHECK();
     return 0;
 }
 
 int launch_sm_to_nm(const float* xs, size_t xs_tree_stride, float* out, size_t out_tree_stride, int B, int R, int C, cudaStream_t st) {
     prof_begin(KC_MISC, st);
     k_sm_to_nm<<<dim3(64, B), 256, 0, st>>>(xs, xs_tree_stride, out, out_tree_stride, R, C);
-    ETC_DONE();
+    LAUNCH_CHECK();
     return 0;
 }
 

@@ -90,6 +90,16 @@ void prof_end(cudaStream_t st);
 int set_error(int code, const char* msg);
 int set_cuda_error(cudaError_t e, const char* file, int line);
 
+// Tail of every kernel launch inside a function returning an NNJ error code, with the stream in `st`: count the launch, close the
+// profiler window prof_begin opened, and return the launch error, if any.
+#define LAUNCH_CHECK()                                                         \
+    do {                                                                       \
+        ++g_launches;                                                          \
+        prof_end(st);                                                          \
+        cudaError_t e_ = cudaGetLastError();                                   \
+        if (e_ != cudaSuccess) return set_cuda_error(e_, __FILE__, __LINE__);  \
+    } while (0)
+
 // ---- per-device state.  cudaFuncSetAttribute and the SM count belong to a DEVICE, not to the process: a second model on another
 // GPU of the same process must raise the shared-memory limits there too.  `DevOnce` is a bit mask of initialised devices (the
 // initialisers are idempotent, so two threads racing on the same device both succeed).
@@ -100,6 +110,16 @@ struct DevOnce {
     bool need() const { return !((mask.load(std::memory_order_acquire) >> (current_device() & 63)) & 1ull); }
     void done() { mask.fetch_or(1ull << (current_device() & 63), std::memory_order_release); }
 };
+// Raise `kernel`'s dynamic shared-memory limit to `bytes` on the current device, once per device: `once` is the call site's own
+// static DevOnce.
+template <typename Kernel>
+int smem_opt_in(DevOnce& once, Kernel* kernel, size_t bytes) {
+    if (!once.need()) return 0;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
+    once.done();
+    return 0;
+}
 // RAII: make the model's device current for the duration of an entry point, restore the caller's device afterwards
 struct DeviceGuard {
     int prev = -1; bool switched = false; cudaError_t err = cudaSuccess;
@@ -132,28 +152,36 @@ int run_rollout(Model* m, const int8_t* data, const float* state0, const uint8_t
                 const float* gumbel, int32_t* merges, float* logits_trace, float* selected_logp, void* ws, size_t ws_bytes,
                 cudaStream_t st);
 
+// One launch of the NJ pair-score step: pairs [n0, n0 + nc) of the pair lists of B trees, against the Rp live nodes that occupy physical
+// slots [0, Rp) of S, over C sites.  score_pairs (nnj_njloop.cu) fills it from its workspace; nj_path there picks the launchers below.
+struct PairChunk {
+    int B, Rp, S, C, n0, nc;
+    const int32_t* slot_of; int slot_stride;                  // logical node -> physical slot, per tree
+    const int32_t *pair_i, *pair_j; int pair_stride;          // pair lists by logical node (pair_i < 0: no pair)
+    const uint8_t* mask;                                      // [B][C], nonzero = masked site; or null
+    const float *X, *Y; size_t tree_stride;                   // fp32 node pools [B][S][C][64]
+    const void *kp_h, *kp_l;                                  // K' planes [B][S][C][64] bf16 hi / lo
+    const void *nodes_h, *nodes_l;                            // node planes [B][C][S][128] bf16 hi / lo = [X | W_g X]
+    float* xf; int pc;                                        // x planes of the chunk [B][pc][C][64] fp32, pc pairs per tree
+    void *xh, *xl;                                            // large-slot path: the x planes as K-major bf16 hi / lo
+    float* alpha_part; int nAP;                               // alpha partials [B][alpha_pairs][nAP][RP], by physical slot
+    float* alpha; int RP; int alpha_pairs;                    // softmaxed alpha [B][alpha_pairs][RP]
+    float* score_part; int nSB;                               // score partials [B][alpha_pairs][nSB]
+};
+// Tensor-core pair-score launchers.  The alpha launchers write the chunk's x planes and alpha_part, the score launchers score_part;
+// *n_part: the partials per pair they wrote.  A chunk outside a launcher's range is refused with NNJ_ERR_INVALID.
+int launch_alpha_v3(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st);        // nnj_alpha_tc.cu
+int launch_alpha_small(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st);     // nnj_alpha_small.cu
+int launch_score_tc(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st);        // nnj_score_tc.cu
+int launch_score_inc(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st);       // nnj_score_tc.cu
+int launch_score_small(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st);     // nnj_score_small.cu
+int launch_score_big(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st);       // nnj_score_big.cu
+int launch_blend_planes(const Model* m, const PairChunk& c, cudaStream_t st);                 // nnj_score_big.cu: x planes, fp32 and bf16
+
 // tcgen05 split-bf16 GEMM (nnj_tc.cu)
 // products: 3 = hi*hi + hi*lo + lo*hi (NNJ_PREC_BF16X3), 1 = hi*hi only (NNJ_PREC_BF16: plain bf16 operands, the lo planes are not read)
 int launch_tc_gemm(int cls, const void* Ah, const void* Al, const void* Bh, const void* Bl, float* Cm, int Z, int M, int N, int K, size_t lda,
                    size_t sA, size_t ldb, size_t sB, int ldc, size_t sC, cudaStream_t st, int products = 3);
-int launch_alpha_tc(const Model* m, const float* X, const float* Y, size_t tree_stride, const int32_t* slot_of, int slot_stride, const int32_t* pair_i,
-                    const int32_t* pair_j, int pair_stride, int n0, int nc, int S, int n_live, int C, int B, const void* kp_h, const void* kp_l, float* xf,
-                    int pc, float* alpha_part, int alpha_pairs, int nSG, int RP, int* n_part, cudaStream_t st);
-int launch_score_tc(const Model* m, const float* xf, int pc, const void* nodes_h, const void* nodes_l, const float* alpha, int RP,
-                    int alpha_pairs, const int32_t* slot_of, int slot_stride, const int32_t* pair_i, int pair_stride, int n0, int nc, int Rp,
-                    int S, int C, int B, const uint8_t* mask, float* score_part, int nSG, int* n_part, cudaStream_t st);
-int launch_blend_planes(const Model* m, const float* X, const float* Y, size_t tree_stride, int C, int B, const int32_t* slot_of, int slot_stride,
-                        const int32_t* pair_i, const int32_t* pair_j, int pair_stride, int n0, int nc, float* xf, void* xh, void* xl, int pc,
-                        cudaStream_t st);
-int launch_alpha_small(const Model* m, const float* X, const float* Y, size_t tree_stride, const int32_t* slot_of, int slot_stride, const int32_t* pair_i,
-                       const int32_t* pair_j, int pair_stride, int n0, int nc, int S, int n_live, int C, int B, const void* kp_h, const void* kp_l, float* xf,
-                       int pc, float* alpha_part, int alpha_pairs, int nSG, int RP, int* n_part, cudaStream_t st);
-int launch_score_small(const Model* m, const float* xf, int pc, const void* nodes_h, const void* nodes_l, const float* alpha, int RP, int alpha_pairs,
-                       const int32_t* slot_of, int slot_stride, const int32_t* pair_i, int pair_stride, int n0, int nc, int Rp, int S, int C, int B,
-                       const uint8_t* mask, float* score_part, int nSG, int* n_part, cudaStream_t st);
-int launch_score_big(const Model* m, const float* xf, int pc, const void* nodes_h, const void* nodes_l, const float* alpha, int RP, int alpha_pairs,
-                     const int32_t* slot_of, int slot_stride, const int32_t* pair_i, int pair_stride, int n0, int nc, int Rp, int S, int C, int B,
-                     const uint8_t* mask, float* score_part, int nSG, int* n_part, cudaStream_t st);
 int launch_tc_gemm_ex(int cls, const void* Ah, const void* Al, const void* Bh, const void* Bl, float* Cm, int Z, int M, int N, int K, size_t lda,
                       size_t sA, size_t ldb, size_t sB, int ldc, size_t sC, int bn, int nsplit, int chunks_per_split, size_t split_stride,
                       cudaStream_t st, int products = 3);

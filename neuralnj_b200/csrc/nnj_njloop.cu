@@ -32,10 +32,6 @@ struct Pool {
 // that does not shrink with the number of live nodes.  In the tensor-core precision mode they run on mma.sync.m16n8k16 bf16 register
 // fragments - A split into hi / lo on the fly from the fp32 tile in shared memory, B from the fragment-packed weights (NjFrag),
 // hi*hi + hi*lo + lo*hi with fp32 accumulation like every other contraction of that mode.  Warp w owns tile rows 16w .. 16w+15.
-__device__ __forceinline__ void nj_mma(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3]) : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
 __device__ __forceinline__ void load_wfrag(float* __restrict__ Ws, const uint4* __restrict__ Wf) {
 #pragma unroll
     for (int it = 0; it < 4; ++it) {
@@ -58,9 +54,9 @@ __device__ __forceinline__ void warp_mma64(float (&c)[8][4], const float* __rest
 #pragma unroll
         for (int nt = 0; nt < 8; ++nt) {
             const uint4 wv = wf[(ks * 8 + nt) * 32];
-            nj_mma(c[nt], al, wv.x, wv.y);       // lo * hi
-            nj_mma(c[nt], ah, wv.z, wv.w);       // hi * lo
-            nj_mma(c[nt], ah, wv.x, wv.y);       // hi * hi
+            mma_m16n8k16(c[nt], al, wv.x, wv.y);       // lo * hi
+            mma_m16n8k16(c[nt], ah, wv.z, wv.w);       // hi * lo
+            mma_m16n8k16(c[nt], ah, wv.x, wv.y);       // hi * hi
         }
     }
 }
@@ -1052,14 +1048,6 @@ __global__ void k_reindex_copy(const float* __restrict__ in, const float* __rest
 }
 
 // ------------------------------------------------------------------ host side
-#define LAUNCH_CHECK()                                                         \
-    do {                                                                       \
-        ++g_launches;                                                          \
-        prof_end(st);                                                          \
-        cudaError_t e_ = cudaGetLastError();                                   \
-        if (e_ != cudaSuccess) return set_cuda_error(e_, __FILE__, __LINE__);  \
-    } while (0)
-
 static inline size_t aup(size_t v) { return (v + 255) / 256 * 256; }
 
 struct NjBuffers {
@@ -1070,22 +1058,22 @@ struct NjBuffers {
     void *xh, *xl;            // large-slot tensor-core path: the same rows as K-major bf16 hi / lo planes (A operand of the alpha-logit GEMM)
     void *nodes_h, *nodes_l;  // tensor-core path: site-major node planes [B][C][S][128] bf16 = [X | W_g X]
     void *kp_h, *kp_l;        // tensor-core path: K' planes [B][S][C][64] bf16 (B operand of the alpha GEMM)
-    bool tc;                  // tcgen05 NJ kernels: 1 = fused kernels (<= 64 slots), 2 handled via `big`
-    bool big;                 // 65 .. 256 slots: blend -> split-K alpha GEMM -> k_score_big
+    bool tc;                  // nj_use_tc: tensor-core NJ kernels, the merge / node-derive products on mma.sync
+    bool big;                 // tc and 65 .. 256 slots: the large-slot pair-score path (nj_path)
     int pc;                   // pairs per launch on the tensor-core path (capacity of the x planes)
     int S, nCT, nSB, nAP, RP, pair_stride, P0;   // nSB: 32-site groups (fp32 kernels); nAP: alpha partials allocated per pair (stride)
     size_t total;
 };
 
-// carve the NJ workspace; X_in_ws: the node pool X lives in the workspace too (rollout)
 constexpr int TC_PAIRS = 256;   // pairs per launch on the tensor-core pair-score path
 
-// The tcgen05 NJ kernels (k_alpha_v3, k_score_tc, k_score_inc) take at most 64 physical slots and - like the tensor-core encoder
-// (use_tc in nnj_encoder.cu) - need C % 8 == 0: their TMA boxes and the two-sites-per-item ring assume 16-byte rows and an even
-// site count.  Every other shape runs the fp32 CUDA-core kernels of this file, whatever the precision mode.
+// The tensor-core NJ kernels take at most 256 physical slots (the fused kernels up to 64, the large-slot path 65 .. 256; nj_path) and -
+// like the tensor-core encoder (use_tc in nnj_encoder.cu) - need C % 8 == 0: their TMA boxes and the two-sites-per-item ring assume
+// 16-byte rows and an even site count.  Every other shape runs the fp32 CUDA-core kernels of this file, whatever the precision mode.
 static bool nj_use_tc(const Model* m, int S, int C) { return m->cfg.precision != NNJ_PREC_FP32 && S <= 256 && (C % 8) == 0; }
 constexpr int BIG_PAIRS = 512;  // pairs per launch of the large-slot path (4 pair tiles share one pass over the K' planes in the alpha GEMM)
 
+// carve the NJ workspace; X_in_ws: the node pool X lives in the workspace too (rollout)
 static NjBuffers nj_layout(char* base, int B, int S, int R, int C, bool X_in_ws, bool need_newx, bool tc) {
     NjBuffers nb{};
     nb.S = S; nb.nCT = (C + TILE_ROWS - 1) / TILE_ROWS; nb.nSB = (C + SB_SITES - 1) / SB_SITES;
@@ -1155,50 +1143,58 @@ static int check_dims(int Rp, int C) {
     return 0;
 }
 
+// Kernels of the pair-score step for a chunk of nc pairs over Rp live nodes.  The rules are checked in order; S is the physical slot
+// count of the workspace (R + 1 in the rollout, Rp in the step-wise API), so a rollout keeps the path S gives it down to its last step.
+//   rule                    alpha                                                         pair score
+//   Rp <= 2                 (none: no global attention, model.py:111)                     k_score<false>
+//   !nj_use_tc(m, S, C)     k_alpha + k_alpha_softmax                                     k_score<true>
+//   S > 64 (nj_layout: big) k_blend_planes + split-K k_tc_gemm + k_alpha_softmax_wide     k_score_big
+//   nc <= 16 and Rp <= 16   k_alpha_small + k_alpha_softmax                               k_score_small
+//   nc <= 64                k_alpha_v3 (2- or 4-way site split) + k_alpha_softmax         k_score_inc
+//   otherwise               k_alpha_v3 + k_alpha_softmax                                  k_score_tc
+// The first three rules do not depend on nc, so they also fix the pairs per launch: PAIR_CHUNK on the fp32 kernels, nb.pc (BIG_PAIRS on
+// the large-slot path, TC_PAIRS otherwise) on the tensor-core ones.
+enum class NjPath { NoGlobal, Fp32, Big, Small, Inc, Tc };
+static NjPath nj_path(const NjBuffers& nb, int Rp, int nc) {
+    if (Rp <= 2) return NjPath::NoGlobal;
+    if (!nb.tc) return NjPath::Fp32;
+    if (nb.big) return NjPath::Big;
+    if (nc <= 16 && Rp <= 16) return NjPath::Small;
+    if (nc <= 64) return NjPath::Inc;
+    return NjPath::Tc;
+}
+
 // scores of N listed pairs per tree against Rp nodes; pool tensors must be derived already.
 static int score_pairs(const Model* m, const Pool& pool, const NjBuffers& nb, const int32_t* slot, int Rp, int C, int N,
                        const uint8_t* mask, int B, float* scores, int score_stride, cudaStream_t st) {
-    const bool glob = Rp > 2;     // model.py:111
-    const bool tc = nb.tc && glob;
-    const int step = tc ? nb.pc : PAIR_CHUNK;
+    const NjPath first = nj_path(nb, Rp, N);
+    const int step = (first == NjPath::NoGlobal || first == NjPath::Fp32) ? PAIR_CHUNK : nb.pc;
     const float inv_scale = 1.0f / sqrtf((float)D * (float)C);   // model.py:118 (patch_num == C)
+    PairChunk c;
+    c.B = B; c.Rp = Rp; c.S = nb.S; c.C = C;
+    c.slot_of = slot; c.slot_stride = nb.S;
+    c.pair_i = nb.pair_i; c.pair_j = nb.pair_j; c.pair_stride = nb.pair_stride;
+    c.mask = mask;
+    c.X = pool.X; c.Y = pool.Y; c.tree_stride = pool.tree_stride;
+    c.kp_h = nb.kp_h; c.kp_l = nb.kp_l; c.nodes_h = nb.nodes_h; c.nodes_l = nb.nodes_l;
+    c.xf = nb.xf; c.pc = nb.pc; c.xh = nb.xh; c.xl = nb.xl;
+    c.alpha_part = nb.alpha_part; c.nAP = nb.nAP;
+    c.alpha = nb.alpha; c.RP = nb.RP; c.alpha_pairs = PAIR_CHUNK;
+    c.score_part = nb.score_part; c.nSB = nb.nSB;
     for (int n0 = 0; n0 < N; n0 += step) {
         const int nc = (N - n0 < step) ? (N - n0) : step;
-        int tc_parts = 0;       // score partials per pair written by the tensor-core kernel of this launch
-        if (glob && tc && nb.big) {
-            // 65 .. 256 slots: pair blend -> x planes (fp32 + bf16 hi / lo), alpha logits as a split-K tcgen05 GEMM
-            // [pairs x C*64] . [slots x C*64]^T over the K' planes (one 64-element K chunk = one site; partials per split, indexed by
-            // physical slot), softmax, then the K-blocked fused score kernel
-            if (int e = launch_blend_planes(m, pool.X, pool.Y, pool.tree_stride, C, B, slot, nb.S, nb.pair_i, nb.pair_j, nb.pair_stride, n0, nc, nb.xf,
-                                            nb.xh, nb.xl, nb.pc, st)) return e;
-            const int bn = Rp <= 64 ? 64 : (Rp <= 128 ? 128 : 256);
-            // K splits: a function of the site count only (NOT of the batch or the pair count), so that a tree's logits do not depend on
-            // what else is in the batch: >= 32 sites per split, <= 64 partials per pair
-            const int cps = (C + 63) / 64 > 32 ? (C + 63) / 64 : 32;
-            const int nsplit = (C + cps - 1) / cps;
-            if (nsplit > nb.nAP) return set_error(NNJ_ERR_INVALID, "large-slot alpha: partial buffer too small");
-            const size_t K = (size_t)C * D;
-            if (int e = launch_tc_gemm_ex(KC_ALPHA, nb.xh, nb.xl, nb.kp_h, nb.kp_l, nb.alpha_part, B, nc, Rp, (int)K, K, (size_t)nb.pc * K, K, (size_t)nb.S * K,
-                                          nb.nAP * nb.RP, (size_t)PAIR_CHUNK * nb.nAP * nb.RP, bn, nsplit, cps, (size_t)nb.RP, st)) return e;
-            prof_begin(KC_ALPHA_SOFTMAX, st);
-            k_alpha_softmax_wide<<<dim3(nc, B), NTHREADS, 0, st>>>(nb.alpha_part, pool.kap, slot, nb.S, nb.S, nb.nCT, Rp, nb.pair_i,
-                                                                   nb.pair_j, nb.pair_stride, n0, nc, nb.nAP, nb.RP, inv_scale, nb.alpha, nsplit);
+        c.n0 = n0; c.nc = nc;
+        int n_part = nb.nSB;    // score partials per pair, summed by k_score_reduce
+        const NjPath path = nj_path(nb, Rp, nc);
+        switch (path) {
+        case NjPath::NoGlobal:
+            prof_begin(KC_SCORE, st);
+            k_score<false><<<dim3(nb.nSB, (nc + 31) / 32, B), NTHREADS, smem_score(Rp), st>>>(pool, slot, nb.S, Rp, C, nb.pair_i, nb.pair_j,
+                                                                                             nb.pair_stride, n0, nc, nb.alpha, nb.RP, m->nj, mask,
+                                                                                             nb.score_part, nb.nSB);
             LAUNCH_CHECK();
-            if (int e = launch_score_big(m, nb.xf, nb.pc, nb.nodes_h, nb.nodes_l, nb.alpha, nb.RP, PAIR_CHUNK, slot, nb.S, nb.pair_i, nb.pair_stride, n0, nc,
-                                         Rp, nb.S, C, B, mask, nb.score_part, nb.nSB, &tc_parts, st)) return e;
-        } else if (glob && tc) {
-            // blend + alpha partials in one tcgen05 kernel (fp32 x planes written on the way, partials per 64-site group - two when the
-            // tile is split by site parity - indexed by physical slot) -> softmax -> fused score kernel
-            int n_part = 0;
-            if (int e = launch_alpha_tc(m, pool.X, pool.Y, pool.tree_stride, slot, nb.S, nb.pair_i, nb.pair_j, nb.pair_stride, n0, nc, nb.S, Rp, C, B,
-                                        nb.kp_h, nb.kp_l, nb.xf, TC_PAIRS, nb.alpha_part, PAIR_CHUNK, nb.nAP, nb.RP, &n_part, st)) return e;
-            prof_begin(KC_ALPHA_SOFTMAX, st);
-            k_alpha_softmax<<<dim3((nc + 7) / 8, B), NTHREADS, 0, st>>>(nb.alpha_part, pool.kap, slot, nb.S, nb.S, nb.nCT, Rp, nb.pair_i,
-                                                                        nb.pair_j, nb.pair_stride, n0, nc, nb.nAP, nb.RP, inv_scale, nb.alpha, 1, n_part);
-            LAUNCH_CHECK();
-            if (int e = launch_score_tc(m, nb.xf, TC_PAIRS, nb.nodes_h, nb.nodes_l, nb.alpha, nb.RP, PAIR_CHUNK, slot, nb.S, nb.pair_i,
-                                        nb.pair_stride, n0, nc, Rp, nb.S, C, B, mask, nb.score_part, nb.nSB, &tc_parts, st)) return e;
-        } else if (glob) {
+            break;
+        case NjPath::Fp32: {
             const int node_tiles = (Rp + 63) / 64, pair_tiles = (nc + 63) / 64;
             prof_begin(KC_ALPHA, st);
             k_alpha<<<dim3(nb.nSB, pair_tiles * node_tiles, B), NTHREADS, 0, st>>>(pool, slot, nb.S, Rp, C, nb.pair_i, nb.pair_j, nb.pair_stride,
@@ -1213,15 +1209,45 @@ static int score_pairs(const Model* m, const Pool& pool, const NjBuffers& nb, co
                                                                                             nb.pair_stride, n0, nc, nb.alpha, nb.RP, m->nj, mask,
                                                                                             nb.score_part, nb.nSB);
             LAUNCH_CHECK();
-        } else {
-            prof_begin(KC_SCORE, st);
-            k_score<false><<<dim3(nb.nSB, (nc + 31) / 32, B), NTHREADS, smem_score(Rp), st>>>(pool, slot, nb.S, Rp, C, nb.pair_i, nb.pair_j,
-                                                                                             nb.pair_stride, n0, nc, nb.alpha, nb.RP, m->nj, mask,
-                                                                                             nb.score_part, nb.nSB);
+            break;
+        }
+        case NjPath::Big: {
+            // pair blend -> x planes (fp32 + bf16 hi / lo), alpha logits as a split-K tcgen05 GEMM [pairs x C*64] . [slots x C*64]^T over the
+            // K' planes (one 64-element K chunk = one site; partials per split, indexed by physical slot), softmax, then the K-blocked fused
+            // score kernel
+            if (int e = launch_blend_planes(m, c, st)) return e;
+            const int bn = Rp <= 64 ? 64 : (Rp <= 128 ? 128 : 256);
+            // K splits: a function of the site count only (NOT of the batch or the pair count), so that a tree's logits do not depend on
+            // what else is in the batch: >= 32 sites per split, <= 64 partials per pair
+            const int cps = (C + 63) / 64 > 32 ? (C + 63) / 64 : 32;
+            const int nsplit = (C + cps - 1) / cps;
+            if (nsplit > nb.nAP) return set_error(NNJ_ERR_INVALID, "large-slot alpha: partial buffer too small");
+            const size_t K = (size_t)C * D;
+            if (int e = launch_tc_gemm_ex(KC_ALPHA, nb.xh, nb.xl, nb.kp_h, nb.kp_l, nb.alpha_part, B, nc, Rp, (int)K, K, (size_t)nb.pc * K, K, (size_t)nb.S * K,
+                                          nb.nAP * nb.RP, (size_t)PAIR_CHUNK * nb.nAP * nb.RP, bn, nsplit, cps, (size_t)nb.RP, st)) return e;
+            prof_begin(KC_ALPHA_SOFTMAX, st);
+            k_alpha_softmax_wide<<<dim3(nc, B), NTHREADS, 0, st>>>(nb.alpha_part, pool.kap, slot, nb.S, nb.S, nb.nCT, Rp, nb.pair_i,
+                                                                   nb.pair_j, nb.pair_stride, n0, nc, nb.nAP, nb.RP, inv_scale, nb.alpha, nsplit);
             LAUNCH_CHECK();
+            if (int e = launch_score_big(m, c, &n_part, st)) return e;
+            break;
+        }
+        case NjPath::Small: case NjPath::Inc: case NjPath::Tc: {
+            // blend + alpha partials in one kernel (fp32 x planes written on the way, partials per site group, indexed by physical slot)
+            // -> softmax -> fused score kernel
+            int a_part = 0;
+            if (int e = (path == NjPath::Small ? launch_alpha_small : launch_alpha_v3)(m, c, &a_part, st)) return e;
+            prof_begin(KC_ALPHA_SOFTMAX, st);
+            k_alpha_softmax<<<dim3((nc + 7) / 8, B), NTHREADS, 0, st>>>(nb.alpha_part, pool.kap, slot, nb.S, nb.S, nb.nCT, Rp, nb.pair_i,
+                                                                        nb.pair_j, nb.pair_stride, n0, nc, nb.nAP, nb.RP, inv_scale, nb.alpha, 1, a_part);
+            LAUNCH_CHECK();
+            if (int e = (path == NjPath::Small ? launch_score_small : path == NjPath::Inc ? launch_score_inc : launch_score_tc)(m, c, &n_part, st))
+                return e;
+            break;
+        }
         }
         prof_begin(KC_MISC, st);
-        k_score_reduce<<<dim3((nc + 127) / 128, B), 128, 0, st>>>(nb.score_part, nb.nSB, (glob && tc) ? tc_parts : nb.nSB, nc, scores, score_stride, n0);
+        k_score_reduce<<<dim3((nc + 127) / 128, B), 128, 0, st>>>(nb.score_part, nb.nSB, n_part, nc, scores, score_stride, n0);
         LAUNCH_CHECK();
     }
     return 0;
@@ -1263,8 +1289,14 @@ static int merge_pair(const Model* m, const Pool& pool, const NjBuffers& nb, flo
     return 0;
 }
 
+// Y, K, kappa (and on the tensor-core path the K' and node planes) of `nodes` nodes in slots [0, nodes) of S
 static int derive_all(const Model* m, const float* X, const NjBuffers& nb, int B, int S, int nodes, int C, cudaStream_t st) {
     prof_begin(KC_DERIVE, st);
+    if (nb.tc && nodes < S) {   // the spare slots' rows are read (with weight 0) by the pair-score UMMA: they must be finite
+        const size_t npb = (size_t)B * C * S * 2 * D * 2;
+        cudaError_t e1 = cudaMemsetAsync(nb.nodes_h, 0, npb, st), e2 = cudaMemsetAsync(nb.nodes_l, 0, npb, st);
+        if (e1 != cudaSuccess || e2 != cudaSuccess) return set_cuda_error(e1 != cudaSuccess ? e1 : e2, __FILE__, __LINE__);
+    }
     if (nb.tc)
         k_node_derive<true><<<dim3(nb.nCT, nodes, B), NTHREADS, smem_derive, st>>>(X, nb.Y, nb.K, nb.kap, (size_t)S * C * D, S, C, nb.nCT, nullptr, 0, m->nj, m->nj_frag,
                                                                                    (uint2*)nb.kp_h, (uint2*)nb.kp_l, (uint2*)nb.nodes_h, (uint2*)nb.nodes_l);
@@ -1417,19 +1449,7 @@ int run_rollout(Model* m, const int8_t* data, const float* state0, const uint8_t
         prof_begin(KC_MISC, st);
         k_fill_pairs_full<<<dim3((P0 + 127) / 128, nbt < 64 ? nbt : 64), 128, 0, st>>>(nb.pair_i, nb.pair_j, nb.pair_stride, R, nbt);
         LAUNCH_CHECK();
-        prof_begin(KC_DERIVE, st);
-        if (nb.tc) {   // the free slot's rows are read (with weight 0) by the pair-score UMMA: they must be finite
-            const size_t npb = (size_t)nbt * C * S * 2 * D * 2;
-            cudaError_t e1 = cudaMemsetAsync(nb.nodes_h, 0, npb, st), e2 = cudaMemsetAsync(nb.nodes_l, 0, npb, st);
-            if (e1 != cudaSuccess || e2 != cudaSuccess) return set_cuda_error(e1 != cudaSuccess ? e1 : e2, __FILE__, __LINE__);
-        }
-        if (nb.tc)
-            k_node_derive<true><<<dim3(nb.nCT, R, nbt), NTHREADS, smem_derive, st>>>(nb.X, nb.Y, nb.K, nb.kap, tree_stride, S, C, nb.nCT, nullptr, 0, m->nj, m->nj_frag,
-                                                                                     (uint2*)nb.kp_h, (uint2*)nb.kp_l, (uint2*)nb.nodes_h, (uint2*)nb.nodes_l);
-        else
-            k_node_derive<false><<<dim3(nb.nCT, R, nbt), NTHREADS, smem_derive, st>>>(nb.X, nb.Y, nb.K, nb.kap, tree_stride, S, C, nb.nCT, nullptr, 0, m->nj, m->nj_frag,
-                                                                                      nullptr, nullptr, nullptr, nullptr);
-        LAUNCH_CHECK();
+        if (int e = derive_all(m, nb.X, nb, nbt, S, R, C, st)) return e;
         Pool pool = make_pool(nb.X, nb, S, C);
         int32_t* mg = merges + (size_t)b0 * (R - 1) * 2;
         float* slp = selected_logp ? selected_logp + (size_t)b0 * (R - 1) : nullptr;

@@ -331,49 +331,36 @@ __global__ void __launch_bounds__(256) k_blend_planes(const float* __restrict__ 
 }
 
 // ------------------------------------------------------------------ host side
-int launch_blend_planes(const Model* m, const float* X, const float* Y, size_t tree_stride, int C, int B, const int32_t* slot_of, int slot_stride,
-                        const int32_t* pair_i, const int32_t* pair_j, int pair_stride, int n0, int nc, float* xf, void* xh, void* xl, int pc,
-                        cudaStream_t st) {
+int launch_blend_planes(const Model* m, const PairChunk& c, cudaStream_t st) {
     prof_begin(KC_BLEND, st);
-    k_blend_planes<<<dim3((C + 63) / 64, (nc + BP_PAIRS - 1) / BP_PAIRS, B), 256, 0, st>>>(X, Y, tree_stride, C, slot_of, slot_stride, pair_i, pair_j, pair_stride, n0, nc, m->nj.bh, xf,
-                                                              (uint2*)xh, (uint2*)xl, pc);
-    ++g_launches;
-    prof_end(st);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
+    k_blend_planes<<<dim3((c.C + 63) / 64, (c.nc + BP_PAIRS - 1) / BP_PAIRS, c.B), 256, 0, st>>>(c.X, c.Y, c.tree_stride, c.C, c.slot_of, c.slot_stride,
+                                                                                            c.pair_i, c.pair_j, c.pair_stride, c.n0, c.nc, m->nj.bh,
+                                                                                            c.xf, (uint2*)c.xh, (uint2*)c.xl, c.pc);
+    LAUNCH_CHECK();
     return 0;
 }
 
-int launch_score_big(const Model* m, const float* xf, int pc, const void* nodes_h, const void* nodes_l, const float* alpha, int RP, int alpha_pairs,
-                     const int32_t* slot_of, int slot_stride, const int32_t* pair_i, int pair_stride, int n0, int nc, int Rp, int S, int C, int B,
-                     const uint8_t* mask, float* score_part, int nSG, int* n_part, cudaStream_t st) {
+int launch_score_big(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st) {
     static DevOnce once;      // per device, not per process
-    if (once.need()) {
-        cudaError_t e = cudaFuncSetAttribute(k_score_big, cudaFuncAttributeMaxDynamicSharedMemorySize, SB_SMEM);
-        if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
-        once.done();
-    }
-    if (Rp > 256 || S > 256) return set_error(NNJ_ERR_INVALID, "score_big: at most 256 node slots");
-    if (C & 7) return set_error(NNJ_ERR_INVALID, "score_big: site count must be a multiple of 8");
+    if (int e = smem_opt_in(once, k_score_big, SB_SMEM)) return e;
+    if (c.Rp > 256 || c.S > 256) return set_error(NNJ_ERR_INVALID, "score_big: at most 256 node slots");
+    if (c.C & 7) return set_error(NNJ_ERR_INVALID, "score_big: site count must be a multiple of 8");
     CUtensorMap mh, ml, mx;      // node planes: 64 slots of one site per box, slots >= Rp dead (zero-filled); x tiles: 64 pairs, pairs >= nc read as 0
-    if (int e = make_tmap_nodes(&mh, nodes_h, S, B * C, 64, Rp)) return e;
-    if (int e = make_tmap_nodes(&ml, nodes_l, S, B * C, 64, Rp)) return e;
-    if (int e = make_tmap_xtile(&mx, xf, pc, nc, C, B)) return e;
+    if (int e = make_tmap_nodes(&mh, c.nodes_h, c.S, c.B * c.C, 64, c.Rp)) return e;
+    if (int e = make_tmap_nodes(&ml, c.nodes_l, c.S, c.B * c.C, 64, c.Rp)) return e;
+    if (int e = make_tmap_xtile(&mx, c.xf, c.pc, c.nc, c.C, c.B)) return e;
     ScoreBigArgs a;
-    a.alpha = alpha; a.RP = RP; a.alpha_pairs = alpha_pairs;
-    a.slot_of = slot_of; a.slot_stride = slot_stride; a.pair_i = pair_i; a.pair_stride = pair_stride; a.n0 = n0; a.nc = nc;
-    a.Rp = Rp; a.C = C; a.KB = (Rp + 63) / 64;
+    a.alpha = c.alpha; a.RP = c.RP; a.alpha_pairs = c.alpha_pairs;
+    a.slot_of = c.slot_of; a.slot_stride = c.slot_stride; a.pair_i = c.pair_i; a.pair_stride = c.pair_stride; a.n0 = c.n0; a.nc = c.nc;
+    a.Rp = c.Rp; a.C = c.C; a.KB = (c.Rp + 63) / 64;
     a.wsh = (const uint4*)m->nj_bf.wsh; a.wsl = (const uint4*)m->nj_bf.wsl;
     a.bg = m->nj.bg; a.bs = m->nj.bs; a.w2 = m->nj.w2; a.b2 = m->nj.b2;
-    a.mask = mask; a.score_part = score_part; a.nSG = nSG;
-    *n_part = (C + SB_SITES - 1) / SB_SITES;
-    if (*n_part > nSG) return set_error(NNJ_ERR_INVALID, "score_big: partial buffer too small");
+    a.mask = c.mask; a.score_part = c.score_part; a.nSG = c.nSB;
+    *n_part = (c.C + SB_SITES - 1) / SB_SITES;
+    if (*n_part > c.nSB) return set_error(NNJ_ERR_INVALID, "score_big: partial buffer too small");
     prof_begin(KC_SCORE, st);
-    k_score_big<<<dim3(*n_part, (nc + 127) / 128, B), SB_THREADS, SB_SMEM, st>>>(mh, ml, mx, a);
-    ++g_launches;
-    prof_end(st);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
+    k_score_big<<<dim3(*n_part, (c.nc + 127) / 128, c.B), SB_THREADS, SB_SMEM, st>>>(mh, ml, mx, a);
+    LAUNCH_CHECK();
     return 0;
 }
 

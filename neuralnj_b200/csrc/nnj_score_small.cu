@@ -36,17 +36,6 @@ struct ScoreSmallArgs {
     float* score_part; int nSG;
 };
 
-__device__ __forceinline__ void ss_mma(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3]) : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ void ss_ldsm4t(uint32_t (&r)[4], uint32_t addr) {
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
-}
-__device__ __forceinline__ void ss_cp16(uint32_t dst, const void* src) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-}
-
 // T = 1 16-row / 16-slot tile (<= 16 pairs and slots); SS_WARPS warps with one private tile buffer each.
 // Measured (128 trees, DESIGN 4.6): a 32-row form (17-32 pairs) is bound by its 384 tensor instructions per site (8 clocks each and
 // sub-partition: 770 clocks per site and SM) and loses to k_score_inc's narrow mode (860 vs 770 us per launch); the 16-row tile with
@@ -120,14 +109,14 @@ __global__ void __launch_bounds__(SS_WARPS * 32, 1) k_score_small(const ScoreSma
             const uint8_t* pl = nl + lane * 16;
             for (int slot = lane >> 4; slot < a.Rp; slot += 2, ph += 512, pl += 512) {
                 const uint32_t off = dst + slot * 256 + ((ch ^ (slot & 7)) << 4);
-                ss_cp16(off, ph);
-                ss_cp16(off + NODE_B, pl);
+                cp_async16(off, ph);
+                cp_async16(off + NODE_B, pl);
             }
             // x rows of the listed pairs at this site (one 256-byte row per pair, C rows apart)
             const float* px = a.xf + (((size_t)b * a.pc + (lane >> 4)) * a.C + c) * 64 + ch * 4;
             const size_t xstride = (size_t)2 * a.C * 64;
             for (int row = lane >> 4; row < a.nc; row += 2, px += xstride)
-                ss_cp16(dst + 2 * NODE_B + row * 256 + ((ch ^ (row & 7)) << 4), px);
+                cp_async16(dst + 2 * NODE_B + row * 256 + ((ch ^ (row & 7)) << 4), px);
         }
         asm volatile("cp.async.commit_group;" ::: "memory");
     };
@@ -161,16 +150,16 @@ __global__ void __launch_bounds__(SS_WARPS * 32, 1) k_score_small(const ScoreSma
                     const int slot = 16 * k + ((lane >> 3) & 1) * 8 + (lane & 7);
                     const uint32_t ad = mybuf_u + slot * 256 + ((((lane >> 4) * 8 + j) ^ (lane & 7)) << 4);
                     uint32_t bh[4], bl[4];
-                    ss_ldsm4t(bh, ad);
-                    ss_ldsm4t(bl, ad + NODE_B);
+                    ldsm_x4_t(bh, ad);
+                    ldsm_x4_t(bl, ad + NODE_B);
 #pragma unroll
                     for (int m = 0; m < T; ++m) {
-                        ss_mma(xg[m], al[m][k], bh[0], bh[1]);      // small terms first
-                        ss_mma(xg[m], ah[m][k], bl[0], bl[1]);
-                        ss_mma(xg[m], ah[m][k], bh[0], bh[1]);
-                        ss_mma(gg[m], al[m][k], bh[2], bh[3]);
-                        ss_mma(gg[m], ah[m][k], bl[2], bl[3]);
-                        ss_mma(gg[m], ah[m][k], bh[2], bh[3]);
+                        mma_m16n8k16(xg[m], al[m][k], bh[0], bh[1]);      // small terms first
+                        mma_m16n8k16(xg[m], ah[m][k], bl[0], bl[1]);
+                        mma_m16n8k16(xg[m], ah[m][k], bh[0], bh[1]);
+                        mma_m16n8k16(gg[m], al[m][k], bh[2], bh[3]);
+                        mma_m16n8k16(gg[m], ah[m][k], bl[2], bl[3]);
+                        mma_m16n8k16(gg[m], ah[m][k], bh[2], bh[3]);
                     }
                 }
                 // gate on this thread's elements: rows 16m + g and 16m + g + 8, channels 8j + 2t, 8j + 2t + 1
@@ -200,9 +189,9 @@ __global__ void __launch_bounds__(SS_WARPS * 32, 1) k_score_small(const ScoreSma
                 asm volatile("ld.shared.b32 %0, [%1];" : "=r"(wl1) : "r"(wa + 64 * SS_WPITCH + 16));
 #pragma unroll
                 for (int m = 0; m < T; ++m) {
-                    ss_mma(sacc[m][f], xl[m], wh0, wh1);
-                    ss_mma(sacc[m][f], xh[m], wl0, wl1);
-                    ss_mma(sacc[m][f], xh[m], wh0, wh1);
+                    mma_m16n8k16(sacc[m][f], xl[m], wh0, wh1);
+                    mma_m16n8k16(sacc[m][f], xh[m], wl0, wl1);
+                    mma_m16n8k16(sacc[m][f], xh[m], wh0, wh1);
                 }
             }
         }
@@ -248,37 +237,26 @@ template <bool HALF>
 static int launch_small_t(const ScoreSmallArgs& a, int groups, int B, cudaStream_t st) {
     constexpr size_t smem = 1024 + 2 * 64 * SS_WPITCH + (32 * 33 + 192) * 4 + 1024 + (size_t)16 * (3 * 16 * 256);
     static DevOnce once;      // per device, not per process
-    if (once.need()) {
-        cudaError_t e = cudaFuncSetAttribute(k_score_small<1, 16, HALF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
-        once.done();
-    }
+    if (int e = smem_opt_in(once, k_score_small<1, 16, HALF>, smem)) return e;
+    prof_begin(KC_SCORE, st);
     k_score_small<1, 16, HALF><<<dim3(groups, B), 16 * 32, smem, st>>>(a);
+    LAUNCH_CHECK();
     return 0;
 }
 
-int launch_score_small(const Model* m, const float* xf, int pc, const void* nodes_h, const void* nodes_l, const float* alpha, int RP, int alpha_pairs,
-                       const int32_t* slot_of, int slot_stride, const int32_t* pair_i, int pair_stride, int n0, int nc, int Rp, int S, int C, int B,
-                       const uint8_t* mask, float* score_part, int nSG, int* n_part, cudaStream_t st) {
-    if (nc > 16 || Rp > 16 || nc < 1) return set_error(NNJ_ERR_INVALID, "score_small: at most 16 pairs over 16 live nodes");
+int launch_score_small(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st) {
+    if (c.nc > 16 || c.Rp > 16 || c.nc < 1) return set_error(NNJ_ERR_INVALID, "score_small: at most 16 pairs over 16 live nodes");
     ScoreSmallArgs a;
-    a.xf = xf; a.pc = pc; a.nodes_h = (const __nv_bfloat16*)nodes_h; a.nodes_l = (const __nv_bfloat16*)nodes_l; a.S = S;
-    a.alpha = alpha; a.RP = RP; a.alpha_pairs = alpha_pairs; a.slot_of = slot_of; a.slot_stride = slot_stride;
-    a.pair_i = pair_i; a.pair_stride = pair_stride; a.n0 = n0; a.nc = nc; a.Rp = Rp; a.C = C;
+    a.xf = c.xf; a.pc = c.pc; a.nodes_h = (const __nv_bfloat16*)c.nodes_h; a.nodes_l = (const __nv_bfloat16*)c.nodes_l; a.S = c.S;
+    a.alpha = c.alpha; a.RP = c.RP; a.alpha_pairs = c.alpha_pairs; a.slot_of = c.slot_of; a.slot_stride = c.slot_stride;
+    a.pair_i = c.pair_i; a.pair_stride = c.pair_stride; a.n0 = c.n0; a.nc = c.nc; a.Rp = c.Rp; a.C = c.C;
     a.wsh = (const uint4*)m->nj_bf.wsh; a.wsl = (const uint4*)m->nj_bf.wsl;
     a.bg = m->nj.bg; a.bs = m->nj.bs; a.w2 = m->nj.w2; a.b2 = m->nj.b2;
-    a.mask = mask; a.score_part = score_part; a.nSG = nSG;
-    const int groups = (C + SS_SITES - 1) / SS_SITES;
+    a.mask = c.mask; a.score_part = c.score_part; a.nSG = c.nSB;
+    const int groups = (c.C + SS_SITES - 1) / SS_SITES;
     *n_part = groups;
-    if (groups > nSG) return set_error(NNJ_ERR_INVALID, "score_small: partial buffer too small");
-    prof_begin(KC_SCORE, st);
-    const int rc = nc <= 8 ? launch_small_t<true>(a, groups, B, st) : launch_small_t<false>(a, groups, B, st);
-    ++g_launches;
-    prof_end(st);
-    if (rc) return rc;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
-    return 0;
+    if (groups > c.nSB) return set_error(NNJ_ERR_INVALID, "score_small: partial buffer too small");
+    return c.nc <= 8 ? launch_small_t<true>(a, groups, c.B, st) : launch_small_t<false>(a, groups, c.B, st);
 }
 
 }  // namespace nnj

@@ -757,55 +757,45 @@ int make_tmap_xtile(CUtensorMap* map, const float* base, int pc, int nrows, int 
 }
 
 // <= 64 pairs per tree: the persistent site-parity kernel
-static int launch_score_inc(const Model* m, const float* xf, int pc, const void* nodes_h, const void* nodes_l, const float* alpha, int RP,
-                            int alpha_pairs, const int32_t* slot_of, int slot_stride, const int32_t* pair_i, int pair_stride, int n0, int nc, int Rp,
-                            int S, int C, int B, const uint8_t* mask, float* score_part, int nSG, int* n_part, cudaStream_t st) {
-    // late steps (<= 16 pairs over <= 16 live nodes): the register-fragment kernel, whose cost follows the number of live pairs (nnj_score_small.cu)
-    if (nc <= 16 && Rp <= 16 && !(C & 7))
-        return launch_score_small(m, xf, pc, nodes_h, nodes_l, alpha, RP, alpha_pairs, slot_of, slot_stride, pair_i, pair_stride, n0, nc, Rp, S, C, B, mask,
-                                  score_part, nSG, n_part, st);
+int launch_score_inc(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st) {
     static DevOnce once;      // per device, not per process
-    if (once.need()) {
-        cudaError_t e = cudaFuncSetAttribute(k_score_inc, cudaFuncAttributeMaxDynamicSharedMemorySize, SI_SMEM_MAX);
-        if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
-        once.done();
-    }
+    if (int e = smem_opt_in(once, k_score_inc, SI_SMEM_MAX)) return e;
+    if (c.S > 64 || c.nc > 64) return set_error(NNJ_ERR_INVALID, "score_inc: at most 64 pairs over 63 taxa");
     const int n_sm = sm_count();
     ScoreIncArgs a;
 #ifdef NNJ_DEBUG_TOOLS
     a.trace = nullptr;
     static long long* trace_buf = nullptr; static int trace_state = -1;
     if (trace_state < 0) { const char* ev = getenv("NNJ_SCORE_TRACE"); trace_state = ev ? atoi(ev) : 0; }
-    if (trace_state > 0 && nc == trace_state) { if (!trace_buf) cudaMalloc(&trace_buf, 32 * 600 * 8); cudaMemsetAsync(trace_buf, 0, 32 * 600 * 8, st); a.trace = trace_buf; }
+    if (trace_state > 0 && c.nc == trace_state) { if (!trace_buf) cudaMalloc(&trace_buf, 32 * 600 * 8); cudaMemsetAsync(trace_buf, 0, 32 * 600 * 8, st); a.trace = trace_buf; }
     { static int dbg = -1; if (dbg < 0) { const char* ev = getenv("NNJ_SCORE_DBG"); dbg = ev ? atoi(ev) : 0; } a.dbg = dbg; }
 #endif
-    a.narrow = nc <= 32 ? 1 : 0;
+    a.narrow = c.nc <= 32 ? 1 : 0;
     // the live nodes occupy physical slots [0, Rp) (k_select keeps them compact): only those rows are streamed / contracted
-    a.node_rows = (Rp + 7) & ~7; a.x_rows = (nc + 7) & ~7;
+    a.node_rows = (c.Rp + 7) & ~7; a.x_rows = (c.nc + 7) & ~7;
     const int stage = 4 * a.node_rows * 128 + 2 * a.x_rows * 128;
     a.nst = (SI_SMEM_MAX - 1024 - SI_RING - 1024 - SI_MISC_BYTES) / stage;
     if (a.nst > SI_MAXST) a.nst = SI_MAXST;
     a.nst &= ~1;                      // even: the two half-pipelines own the even / odd ring stages (see the kernel)
     if (a.nst < 2) return set_error(NNJ_ERR_INVALID, "score_inc: ring does not fit");
-    if (C & 7) return set_error(NNJ_ERR_INVALID, "score_inc: the tensor-core NJ kernels need a site count that is a multiple of 8 (nj_use_tc routes other shapes to the fp32 kernels)");
+    if (c.C & 7) return set_error(NNJ_ERR_INVALID, "score_inc: the tensor-core NJ kernels need a site count that is a multiple of 8 (nj_use_tc routes other shapes to the fp32 kernels)");
     CUtensorMap mh, ml, mx;
-    if (int e = make_tmap_xtile(&mx, xf + (size_t)0, pc, nc, C, B, a.x_rows)) return e;
-    if (int e = make_tmap_nodes(&mh, nodes_h, S, B * C, a.node_rows, Rp)) return e;
-    if (int e = make_tmap_nodes(&ml, nodes_l, S, B * C, a.node_rows, Rp)) return e;
-    a.alpha = alpha; a.RP = RP; a.alpha_pairs = alpha_pairs;
-    a.slot_of = slot_of; a.slot_stride = slot_stride; a.pair_i = pair_i; a.pair_stride = pair_stride; a.n0 = n0; a.nc = nc;
-    a.Rp = Rp; a.S = Rp; a.C = C; a.B = B; a.groups = (C + SI_SITES - 1) / SI_SITES;   // a.S: slots contracted by UMMA 1
+    if (int e = make_tmap_xtile(&mx, c.xf, c.pc, c.nc, c.C, c.B, a.x_rows)) return e;
+    if (int e = make_tmap_nodes(&mh, c.nodes_h, c.S, c.B * c.C, a.node_rows, c.Rp)) return e;
+    if (int e = make_tmap_nodes(&ml, c.nodes_l, c.S, c.B * c.C, a.node_rows, c.Rp)) return e;
+    a.alpha = c.alpha; a.RP = c.RP; a.alpha_pairs = c.alpha_pairs;
+    a.slot_of = c.slot_of; a.slot_stride = c.slot_stride; a.pair_i = c.pair_i; a.pair_stride = c.pair_stride; a.n0 = c.n0; a.nc = c.nc;
+    a.Rp = c.Rp; a.S = c.Rp; a.C = c.C; a.B = c.B; a.groups = (c.C + SI_SITES - 1) / SI_SITES;   // a.S: slots contracted by UMMA 1
     *n_part = a.groups;
-    if (a.groups > nSG) return set_error(NNJ_ERR_INVALID, "score_inc: partial buffer too small");
+    if (a.groups > c.nSB) return set_error(NNJ_ERR_INVALID, "score_inc: partial buffer too small");
     a.wsh = (const uint4*)m->nj_bf.wsh; a.wsl = (const uint4*)m->nj_bf.wsl;
     a.bg = m->nj.bg; a.bs = m->nj.bs; a.w2 = m->nj.w2; a.b2 = m->nj.b2;
-    a.mask = mask; a.score_part = score_part; a.nSG = nSG;
-    const int n_work = B * a.groups;
+    a.mask = c.mask; a.score_part = c.score_part; a.nSG = c.nSB;
+    const int n_work = c.B * a.groups;
     const size_t smem = 1024 + SI_RING + (size_t)a.nst * stage + 1024 + SI_MISC_BYTES;
     prof_begin(KC_SCORE, st);
     k_score_inc<<<n_work < n_sm ? n_work : n_sm, SI_THREADS, smem, st>>>(mh, ml, mx, a);
-    ++g_launches;
-    prof_end(st);
+    LAUNCH_CHECK();
 #ifdef NNJ_DEBUG_TOOLS
     if (a.trace) {
         cudaStreamSynchronize(st);
@@ -816,43 +806,29 @@ static int launch_score_inc(const Model* m, const float* xf, int pc, const void*
         trace_state = 0;
     }
 #endif
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
     return 0;
 }
 
-int launch_score_tc(const Model* m, const float* xf, int pc, const void* nodes_h, const void* nodes_l, const float* alpha, int RP,
-                    int alpha_pairs, const int32_t* slot_of, int slot_stride, const int32_t* pair_i, int pair_stride, int n0, int nc, int Rp,
-                    int S, int C, int B, const uint8_t* mask, float* score_part, int nSG, int* n_part, cudaStream_t st) {
+int launch_score_tc(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st) {
     static DevOnce once;      // per device, not per process
-    if (once.need()) {
-        cudaError_t e = cudaFuncSetAttribute(k_score_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, ST_SMEM);
-        if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
-        once.done();
-    }
-    if (S > 64) return set_error(NNJ_ERR_INVALID, "score_tc: at most 63 taxa on the tensor-core pair-score path");
-    if (nc <= 64)
-        return launch_score_inc(m, xf, pc, nodes_h, nodes_l, alpha, RP, alpha_pairs, slot_of, slot_stride, pair_i, pair_stride, n0, nc, Rp, S, C, B,
-                                mask, score_part, nSG, n_part, st);
-    *n_part = (C + ST_SITES - 1) / ST_SITES;
+    if (int e = smem_opt_in(once, k_score_tc, ST_SMEM)) return e;
+    if (c.S > 64) return set_error(NNJ_ERR_INVALID, "score_tc: at most 63 taxa on the tensor-core pair-score path");
+    *n_part = (c.C + ST_SITES - 1) / ST_SITES;
     CUtensorMap mh, ml, mx;
-    if (int e = make_tmap_xtile(&mx, xf, pc, nc, C, B)) return e;
-    if (int e = make_tmap_nodes(&mh, nodes_h, S, B * C)) return e;
-    if (int e = make_tmap_nodes(&ml, nodes_l, S, B * C)) return e;
+    if (int e = make_tmap_xtile(&mx, c.xf, c.pc, c.nc, c.C, c.B)) return e;
+    if (int e = make_tmap_nodes(&mh, c.nodes_h, c.S, c.B * c.C)) return e;
+    if (int e = make_tmap_nodes(&ml, c.nodes_l, c.S, c.B * c.C)) return e;
     ScoreTcArgs a;
-    a.xf = (const float4*)xf; a.pc = pc;
-    a.alpha = alpha; a.RP = RP; a.alpha_pairs = alpha_pairs;
-    a.slot_of = slot_of; a.slot_stride = slot_stride; a.pair_i = pair_i; a.pair_stride = pair_stride; a.n0 = n0; a.nc = nc;
-    a.Rp = Rp; a.S = S; a.C = C;
+    a.xf = (const float4*)c.xf; a.pc = c.pc;
+    a.alpha = c.alpha; a.RP = c.RP; a.alpha_pairs = c.alpha_pairs;
+    a.slot_of = c.slot_of; a.slot_stride = c.slot_stride; a.pair_i = c.pair_i; a.pair_stride = c.pair_stride; a.n0 = c.n0; a.nc = c.nc;
+    a.Rp = c.Rp; a.S = c.S; a.C = c.C;
     a.wsh = (const uint4*)m->nj_bf.wsh; a.wsl = (const uint4*)m->nj_bf.wsl;
     a.bg = m->nj.bg; a.bs = m->nj.bs; a.w2 = m->nj.w2; a.b2 = m->nj.b2;
-    a.mask = mask; a.score_part = score_part; a.nSG = nSG;
+    a.mask = c.mask; a.score_part = c.score_part; a.nSG = c.nSB;
     prof_begin(KC_SCORE, st);
-    k_score_tc<<<dim3((C + ST_SITES - 1) / ST_SITES, (nc + 127) / 128, B), ST_THREADS, ST_SMEM, st>>>(mh, ml, mx, a);
-    ++g_launches;
-    prof_end(st);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
+    k_score_tc<<<dim3((c.C + ST_SITES - 1) / ST_SITES, (c.nc + 127) / 128, c.B), ST_THREADS, ST_SMEM, st>>>(mh, ml, mx, a);
+    LAUNCH_CHECK();
     return 0;
 }
 

@@ -1,4 +1,5 @@
-// nnj_tc.cuh — inline-PTX helpers for tcgen05 / TMEM / TMA / mbarrier on sm_100a (shared by the tensor-core kernels).
+// nnj_tc.cuh — inline-PTX helpers for tcgen05 / TMEM / TMA / mbarrier and for mma.sync / ldmatrix / cp.async on sm_100a (shared by the
+// tensor-core kernels).
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
@@ -18,6 +19,24 @@ __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)_
 // 1024-byte aligned start inside the dynamic shared-memory window.  Pure pointer arithmetic on the __shared__ array (no integer
 // round trip), so the compiler keeps the shared address space and emits LDS / STS instead of generic LD / ST.
 __device__ __forceinline__ uint8_t* smem_align1024(uint8_t* raw) { return raw + ((1024u - (smem_u32(raw) & 1023u)) & 1023u); }
+
+// D[16 x 8] += A[16 x 16] . B[16 x 8] on register fragments (bf16 operands, fp32 accumulate).  Lane (g = lane >> 2, t = lane & 3):
+// a0 = A[g][2t, 2t+1], a1 = A[g+8][2t, 2t+1], a2 = A[g][8+2t, 9+2t], a3 = A[g+8][8+2t, 9+2t]; b0 = B[2t, 2t+1][g], b1 = B[8+2t, 9+2t][g];
+// d0 d1 = D[g][2t, 2t+1], d2 d3 = D[g+8][2t, 2t+1].  Measured on B200 (scratch/hmma_bench.cu): one m16n8k16 and one m16n8k8 both hold a
+// sub-partition's legacy tensor pipe for 8 clocks (20 clocks latency), so the K = 16 form is used throughout.
+__device__ __forceinline__ void mma_m16n8k16(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
+    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+                 : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3]) : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+}
+// four 8 x 8 b16 matrices (rows of 16 B, lane l supplies the address of row l & 7 of matrix l >> 3), transposed on the way in:
+// lane (g, t) receives M[2t, 2t+1][g] of every matrix = a B fragment half for a row-major [k][n] operand
+__device__ __forceinline__ void ldsm_x4_t(uint32_t (&r)[4], uint32_t addr) {
+    asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
+}
+// 16-byte global -> shared copy, bypassing L1 (cp.async.cg); completes at the next commit_group / wait_group
+__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
+}
 
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));

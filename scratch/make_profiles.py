@@ -67,7 +67,7 @@ def klass(k):
     if k.startswith("k_tc_gemm2<"): return "row_pv_gemm" if k.startswith("k_tc_gemm2<1") else "row_qk_gemm"
     if k.startswith("k_tc_gemm<"):      # <BN, BMN, ONE>: MN-major B = the P V GEMM
         return "row_pv_gemm" if k.split(",")[1].strip().startswith("1") else "row_qk_gemm"
-    for pre, c in (("k_merge<", "merge"), ("k_node_derive", "node_derive"), ("k_score_small", "pair_score"), ("k_alpha_small", "alpha"), ("k_enc_colblock_tc", "col_attn"), ("k_score_big", "pair_score"), ("k_pair_blend", "pair_blend")):
+    for pre, c in (("k_merge<", "merge"), ("k_node_derive", "node_derive"), ("k_score_small", "pair_score"), ("k_alpha_small", "alpha"), ("k_enc_colblock_tc", "col_attn"), ("k_score_big", "pair_score"), ("k_blend_planes", "pair_blend")):
         if k.startswith(pre): return c
     return "misc"
 for k, a in agg.items(): byc[klass(k)] += a[1]

@@ -108,8 +108,8 @@ def test_full_size_properties_tensor_core(gpu_models):
 
 
 def test_large_alignment_200x4096(gpu_models):
-    """BASELINE config 4 (200 taxa x 4096 sites, Argmax): above 63 taxa the NJ loop runs on the fp32 CUDA-core kernels, the encoder
-    stays on tcgen05.  The CPU oracle needs minutes at this size, so the check is by properties: valid merge lists, finite
+    """BASELINE config 4 (200 taxa x 4096 sites, Argmax): 201 node slots put the NJ loop on the large-slot tensor-core path (k_blend_planes,
+    split-K alpha GEMM, k_score_big; DESIGN 4.4), the encoder stays on tcgen05.  The CPU oracle needs minutes at this size, so the check is by properties: valid merge lists, finite
     log-probabilities, bit-exact rerun, and batch independence (B = 2 against its own B = 1 halves)."""
     import nnj_oracle as O
     model = gpu_models["bf16x3"]

@@ -4,7 +4,7 @@ The kernels change with the taxon count R (the NJ pool has S = R + 1 slots):
 * R > 128: the encoder runs the row attention on tcgen05 and the rest of the layer on the fp32 tile-planar kernels (k_out_proj,
   k_ln_qkv<false>, k_col_attn); C % 256 == 0 selects the CTA-pair row GEMMs (ceil(8R / 256) N tiles, ragged at 129, 333, 400) and the
   fused Q K^T softmax, C = 200 the single-CTA GEMMs, C = 250 (not a multiple of 8) the fp32 encoder.
-* R <= 255: the bf16x3 NJ loop stays on the large-slot path (k_pair_blend, split-K alpha, k_alpha_softmax_wide, k_score_big with
+* R <= 255: the bf16x3 NJ loop stays on the large-slot path (k_blend_planes, split-K alpha, k_alpha_softmax_wide, k_score_big with
   bn = 64 / 128 / 256 by live nodes).  R >= 256 (S > 256): both precisions run the fp32 NJ kernels (k_alpha, k_alpha_softmax,
   k_score<GLOB>, k_merge).
 * R > 400: k_col_attn would need more than 200 KB of shared memory; the encoder refuses the shape, and so does bootstrap_support.
