@@ -420,22 +420,16 @@ int64_t nnj_llh_workspace_bytes(int B, int R, int L) { return (B >= 1 && R >= 3 
 int nnj_llh_eval(const uint8_t* tips, const double* weights, const int32_t* children_h, const double* brlen_h, const double* model_h, int B, int R, int L,
                  double* llh_h, void* ws, int64_t ws_bytes, void* stream) {
     CHECK_ARGS(tips && weights && children_h && brlen_h && model_h && llh_h && ws && B >= 1 && R >= 3 && R <= 4096 && L >= 1, "llh_eval: bad arguments");
-    std::vector<double> both((size_t)B * 2);
-    int rc = run_llh(tips, weights, children_h, const_cast<double*>(brlen_h), const_cast<double*>(model_h), B, R, L, 0, 0, 0.0, 0.0, 0, 0, both.data(), ws,
-                     (size_t)ws_bytes, (cudaStream_t)stream);
-    if (rc == 0) for (int b = 0; b < B; ++b) llh_h[b] = both[2 * b + 1];
-    return rc;
+    const LlhTrees in{tips, weights, children_h, const_cast<double*>(brlen_h), const_cast<double*>(model_h), B, R, L};
+    return run_llh(in, LlhMode::Eval, {}, nullptr, llh_h, ws, (size_t)ws_bytes, (cudaStream_t)stream);
 }
 
 int nnj_llh_optimize_brlen(const uint8_t* tips, const double* weights, const int32_t* children_h, double* brlen_h, const double* model_h, int B, int R, int L,
                            int max_passes, double eps, double* llh_before_h, double* llh_after_h, void* ws, int64_t ws_bytes, void* stream) {
     CHECK_ARGS(tips && weights && children_h && brlen_h && model_h && llh_after_h && ws && B >= 1 && R >= 3 && R <= 4096 && L >= 1 && max_passes >= 1,
                "llh_optimize_brlen: bad arguments");
-    std::vector<double> both((size_t)B * 2);
-    int rc = run_llh(tips, weights, children_h, brlen_h, const_cast<double*>(model_h), B, R, L, 1, max_passes, eps, 0.0, 0, 0, both.data(), ws, (size_t)ws_bytes,
-                     (cudaStream_t)stream);
-    if (rc == 0) for (int b = 0; b < B; ++b) { if (llh_before_h) llh_before_h[b] = both[2 * b]; llh_after_h[b] = both[2 * b + 1]; }
-    return rc;
+    const LlhTrees in{tips, weights, children_h, brlen_h, const_cast<double*>(model_h), B, R, L};
+    return run_llh(in, LlhMode::Brlen, {max_passes, eps, 0.0, 0}, llh_before_h, llh_after_h, ws, (size_t)ws_bytes, (cudaStream_t)stream);
 }
 
 int nnj_llh_optimize_all(const uint8_t* tips, const double* weights, const int32_t* children_h, double* brlen_h, double* model_h, int B, int R, int L,
@@ -443,11 +437,8 @@ int nnj_llh_optimize_all(const uint8_t* tips, const double* weights, const int32
                          void* stream) {
     CHECK_ARGS(tips && weights && children_h && brlen_h && model_h && llh_after_h && ws && B >= 1 && R >= 3 && R <= 4096 && L >= 1 && max_passes >= 1 && max_rounds >= 1,
                "llh_optimize_all: bad arguments");
-    std::vector<double> both((size_t)B * 2);
-    int rc = run_llh(tips, weights, children_h, brlen_h, model_h, B, R, L, 2, max_passes, eps, lh_eps, max_rounds, 24, both.data(), ws, (size_t)ws_bytes,
-                     (cudaStream_t)stream);
-    if (rc == 0) for (int b = 0; b < B; ++b) { if (llh_before_h) llh_before_h[b] = both[2 * b]; llh_after_h[b] = both[2 * b + 1]; }
-    return rc;
+    const LlhTrees in{tips, weights, children_h, brlen_h, model_h, B, R, L};
+    return run_llh(in, LlhMode::All, {max_passes, eps, lh_eps, max_rounds}, llh_before_h, llh_after_h, ws, (size_t)ws_bytes, (cudaStream_t)stream);
 }
 
 int64_t nnj_llh_support_workspace_bytes(int B, int R, int L, int n_rell) {
@@ -459,8 +450,9 @@ int nnj_llh_branch_support(const uint8_t* tips, const double* weights, const int
                            int32_t* lbp_count_h, double* site_llh_dev, void* ws, int64_t ws_bytes, void* stream) {
     CHECK_ARGS(tips && weights && children_h && brlen_h && model_h && ws && B >= 1 && R >= 3 && R <= 4096 && L >= 1 && n_rell >= 0 && rep0 >= 0 &&
                (R == 3 || (branch_node_h && llh_h && nni_brlen_h && sh_count_h && lbp_count_h)), "llh_branch_support: bad arguments");
-    return run_llh_support(tips, weights, children_h, brlen_h, model_h, B, R, L, seed, rep0, n_rell, branch_node_h, llh_h, nni_brlen_h, sh_count_h,
-                           lbp_count_h, site_llh_dev, ws, (size_t)ws_bytes, (cudaStream_t)stream);
+    const LlhTrees in{tips, weights, children_h, const_cast<double*>(brlen_h), const_cast<double*>(model_h), B, R, L};
+    return run_llh_support(in, seed, rep0, n_rell, branch_node_h, llh_h, nni_brlen_h, sh_count_h, lbp_count_h, site_llh_dev, ws, (size_t)ws_bytes,
+                           (cudaStream_t)stream);
 }
 
 int nnj_gamma_rates(double alpha, int ncat, double* rates_h) {
@@ -504,10 +496,20 @@ int nnj_rollout_host(nnj_model* m, const int8_t* data_h, const uint8_t* mask_h, 
     const size_t ws_bytes = nj_rollout_ws_bytes(m, chunk, R, L);
     const size_t P0 = (size_t)R * (R - 1) / 2;
     const size_t t_data = (size_t)R * L * 4, t_mask = (size_t)L, t_mg = (size_t)(R - 1) * 2, t_gum = gumbel_h ? (size_t)(R - 1) * P0 : 0;
-    auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    const size_t io_bytes = up(B * t_data) + up(B * t_mask) + up(B * t_mg * 4) + up(B * t_mg * 2) + up(B * t_gum * 4) + 256;
     // workspace + staging buffers live in one grow-only allocation owned by the model (no cudaMalloc on the steady-state path)
-    const size_t need = up(ws_bytes) + io_bytes;
+    auto staging = [&](char* base) {
+        WsCarver c(base);
+        c.take<char>(ws_bytes);                                   // the rollout workspace
+        struct { int8_t* data; uint8_t* mask; int32_t* mg; float *slp, *gum; size_t end; } io;
+        io.data = c.take<int8_t>(B * t_data);
+        io.mask = c.take<uint8_t>(B * t_mask);
+        io.mg = c.take<int32_t>(B * t_mg);
+        io.slp = c.take<float>((size_t)B * (R - 1));
+        io.gum = c.take<float>(B * t_gum);
+        io.end = c.off + 256;
+        return io;
+    };
+    const size_t need = staging(nullptr).end;
     if (m->host_ws_bytes < need) {
         if (m->host_ws) { CUDA_TRY(cudaDeviceSynchronize()); cudaFree(m->host_ws); m->host_ws = nullptr; m->host_ws_bytes = 0; }
         CUDA_TRY(cudaMalloc(&m->host_ws, need));
@@ -521,12 +523,12 @@ int nnj_rollout_host(nnj_model* m, const int8_t* data_h, const uint8_t* mask_h, 
         m->host_events.push_back(ev);
     }
     char* ws = reinterpret_cast<char*>(m->host_ws);
-    char* io = ws + up(ws_bytes);
-    int8_t* d_data = (int8_t*)io;
-    uint8_t* d_mask = (uint8_t*)(io + up(B * t_data));
-    int32_t* d_mg = (int32_t*)((char*)d_mask + up(B * t_mask));
-    float* d_slp = (float*)((char*)d_mg + up(B * t_mg * 4));
-    float* d_gum = gumbel_h ? (float*)((char*)d_slp + up(B * t_mg * 2)) : nullptr;
+    const auto io = staging(ws);
+    int8_t* d_data = io.data;
+    uint8_t* d_mask = io.mask;
+    int32_t* d_mg = io.mg;
+    float* d_slp = io.slp;
+    float* d_gum = gumbel_h ? io.gum : nullptr;
     cudaStream_t cs = m->host_compute, xs = m->host_copy;
     cudaError_t e = cudaSuccess;
     int rc = NNJ_OK;

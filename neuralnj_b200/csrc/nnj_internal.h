@@ -120,6 +120,18 @@ int smem_opt_in(DevOnce& once, Kernel* kernel, size_t bytes) {
     once.done();
     return 0;
 }
+// Workspace layout: regions taken one after another, each rounded up to 256 bytes.  The same lines size a workspace (null base: the
+// pointers are null, `off` ends as the bytes the regions need) and carve it (base from ws_align), so the two cannot drift apart.
+inline char* ws_align(void* ws) { return reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255); }
+struct WsCarver {
+    char* base; size_t off = 0;
+    explicit WsCarver(char* b = nullptr) : base(b) {}
+    template <typename T> T* take(size_t count) {
+        T* p = base ? reinterpret_cast<T*>(base + off) : nullptr;
+        off += (count * sizeof(T) + 255) & ~(size_t)255;
+        return p;
+    }
+};
 // RAII: make the model's device current for the duration of an entry point, restore the caller's device afterwards
 struct DeviceGuard {
     int prev = -1; bool switched = false; cudaError_t err = cudaSuccess;
@@ -212,18 +224,33 @@ int run_tc_unit(const float* A, const float* B, float* Dm, int bn, cudaStream_t 
 int run_gemm_split_bf16(const float* A, const float* B, float* Cm, int Z, int M, int N, int K, void* ws, size_t ws_bytes, cudaStream_t st);
 
 // tree likelihood / branch-length optimisation (nnj_llh.cu)
+// The inputs of every likelihood entry point: tips [B][R][L] (4-bit state masks) and pattern weights [B][L] on the device; children
+// [B][R-1][2] in join order, brlen [B][2R-2] and the packed model [B][LLH_MODEL] on the host.  The modes that optimise branch
+// lengths write them back to brlen, LlhMode::All the optimised model to model.
+struct LlhTrees {
+    const uint8_t* tips; const double* weights;
+    const int32_t* children; double* brlen; double* model;
+    int B, R, L;
+};
+// Eval: log L at the given lengths; Brlen: branch-length sweeps; All: branch lengths and model parameters; Prepare: llh_prepare
+enum class LlhMode : int { Eval = 0, Brlen = 1, All = 2, Prepare = 3 };
+struct LlhOptions {
+    int max_passes; double eps;        // branch-length sweeps until one gains < eps (Brlen, All)
+    double lh_eps; int max_rounds;     // rounds of (model parameters, sweeps) until one gains < lh_eps (All)
+};
 size_t llh_ws_bytes(int B, int R, int L);
-struct LlhState { const double *D, *U, *inv; const int32_t *Dn, *Un; };    // where run_llh leaves the vectors of the trees in the workspace
 int llh_check_tree(const int32_t* ch, int R);     // 0 when children is a binary tree in join order
-// optimise 3 (evaluate and fill U at the given lengths) also writes the per-pattern log-likelihoods to site_dev [B][L]
-int run_llh(const uint8_t* tips, const double* weights, const int32_t* children_h, double* brlen_h, double* model_h, int B, int R, int L,
-            int optimise, int max_passes, double eps, double lh_eps, int max_rounds, int golden_iters, double* llh_h, void* ws, size_t ws_bytes,
-            cudaStream_t st, double* site_dev = nullptr, LlhState* state = nullptr);
+// modes Eval, Brlen, All; llh_before / llh_after [B] (host) may be null
+int run_llh(const LlhTrees& in, LlhMode mode, const LlhOptions& opt, double* llh_before, double* llh_after, void* ws, size_t ws_bytes, cudaStream_t st);
+// First step of branch support, for trees the caller has checked: the subtree vectors D and, for every branch, the vector U of the
+// rest of the tree, at the given lengths; the per-pattern log-likelihoods to site_dev [B][L] (device) and log L to llh_h [B] (host).
+// rc is 0 or an error code; the vectors and their scale counts stay in ws.
+struct LlhPrepared { int rc; const double *D, *U, *inv; const int32_t *Dn, *Un; };
+LlhPrepared llh_prepare(const LlhTrees& in, double* site_dev, double* llh_h, void* ws, size_t ws_bytes, cudaStream_t st);
 // likelihood branch support (nnj_llh_nni.cu): NNI quartets of every internal branch, RELL replicates
 size_t llh_support_ws_bytes(int B, int R, int L, int n_rell);
-int run_llh_support(const uint8_t* tips, const double* weights, const int32_t* children_h, const double* brlen_h, const double* model_h, int B, int R,
-                    int L, uint64_t seed, int64_t rep0, int n_rell, int32_t* branch_node_h, double* llh_h, double* nni_brlen_h, int32_t* sh_h,
-                    int32_t* lbp_h, double* site_dev, void* ws, size_t ws_bytes, cudaStream_t st);
+int run_llh_support(const LlhTrees& in, uint64_t seed, int64_t rep0, int n_rell, int32_t* branch_node_h, double* llh_h, double* nni_brlen_h,
+                    int32_t* sh_h, int32_t* lbp_h, double* site_dev, void* ws, size_t ws_bytes, cudaStream_t st);
 int gamma_rates(double alpha, int ncat, double* out);
 
 // pre-training loss over a teacher-forced rollout's logits trace (nnj_rankloss.cu)

@@ -25,29 +25,30 @@
 namespace nnj {
 
 constexpr double RATE_LO = 1e-3, RATE_HI = 1e3, ALPHA_LO = 0.02, ALPHA_HI = 100.0, PINV_HI = 0.99, GOLD = 0.3819660112501051;   // as in oracle/llh_oracle.py
+constexpr int GOLDEN_ITERS = 24;          // golden-section steps per model parameter and round (LlhMode::All)
 enum { OP_OPT = 0, OP_UP = 1, OP_DOWN = 2, OP_SWAPROOT = 3 };
 
 struct LlhArgs {
     const uint8_t* tips;        // [B][R][L] 4-bit state masks
     const double* weights;      // [B][L] pattern multiplicities
     const int32_t* children;    // [B][R-1][2]
-    const int32_t* ops;         // [B][n_ops][4] (optimise 1, 2: the build_ops schedule; 3: its UP and SWAPROOT rows)
+    const int32_t* ops;         // [B][n_ops][4] (Brlen, All: the build_ops schedule; Prepare: its UP and SWAPROOT rows)
     double* brlen;              // [B][2R-2] in / out
     const double* model;        // [B][LLH_MODEL]
     double *D, *U, *S, *inv;    // workspace: [B][R-1][L][16], [B][2R-2][L][16], [B][L][16], [B][L]
     int32_t *Dn, *Un, *Sn;      // scale counts of D, U and the Newton sumtable: [B][R-1][L], [B][2R-2][L], [B][L]
     double* llh;                // [B][2]: before, after
-    double* site;               // [B][L] per-pattern log-likelihood at the given lengths (optimise = 3), else null
-    int B, R, L, n_ops, max_passes, optimise;     // optimise: 0 evaluate, 1 branch lengths, 2 branch lengths + model parameters,
-                                                  // 3 evaluate and fill U for every branch (the NNI quartets of nnj_llh_nni.cu)
+    double* site;               // [B][L] per-pattern log-likelihood at the given lengths (Prepare), else null
+    int B, R, L, n_ops, max_passes;
+    LlhMode mode;
     double eps;
-    double lh_eps; int max_rounds, golden_iters;  // optimise = 2: rounds of (free parameters one at a time, branch sweeps) until a round gains < lh_eps
-    double* model_out;                            // [B][LLH_MODEL] optimised model (optimise = 2)
+    double lh_eps; int max_rounds, golden_iters;  // All: rounds of (free parameters one at a time, branch sweeps) until a round gains < lh_eps
+    double* model_out;                            // [B][LLH_MODEL] optimised model (All)
 };
 
-// ---- model parameters on the device (optimise = 2): one thread rebuilds the eigen-system and the class rates of its tree
-// regularised lower incomplete gamma P(a, x): series / continued fraction (Lentz), as gammp below on the host
-__device__ double gammp_dev(double a, double x) {
+// ---- discrete gamma (Yang 1994), on the host (gamma_rates) and, for LlhMode::All, on the device (rebuild_model)
+// regularised lower incomplete gamma P(a, x): series / continued fraction (Lentz)
+__host__ __device__ double gammp(double a, double x) {
     if (x <= 0.0) return 0.0;
     const double gln = lgamma(a);
     if (x < a + 1.0) {
@@ -68,14 +69,15 @@ __device__ double gammp_dev(double a, double x) {
     }
     return 1.0 - exp(-x + a * log(x) - gln) * h;
 }
-// class i (0..3) boundary quantile of Gamma(alpha, 1) at (i + 1) / 4, then P(alpha + 1, .) - what gamma_rates() does on the host
-__device__ double gamma_cdf1_dev(double alpha, int i) {
-    const double target = (double)(i + 1) * 0.25, gln = lgamma(alpha);
+// class boundary: the quantile x of Gamma(alpha, 1) at q (Newton on P(alpha, x), monotone with a known density, kept inside a
+// bracket: a bisection step whenever Newton leaves it), then P(alpha + 1, x), the share of the mean below x
+__host__ __device__ double gamma_class_cdf(double alpha, double q) {
+    const double gln = lgamma(alpha);
     double lo = 0.0, hi = alpha + 1.0;
-    while (gammp_dev(alpha, hi) < target) hi *= 2.0;
+    while (gammp(alpha, hi) < q) hi *= 2.0;
     double x = 0.5 * (lo + hi);
     for (int it = 0; it < 200; ++it) {
-        const double f = gammp_dev(alpha, x) - target;
+        const double f = gammp(alpha, x) - q;
         if (f < 0.0) lo = x; else hi = x;
         const double pdf = exp((alpha - 1.0) * log(x) - x - gln);
         double xn = pdf > 0.0 ? x - f / pdf : 0.5 * (lo + hi);
@@ -84,15 +86,18 @@ __device__ double gamma_cdf1_dev(double alpha, int i) {
         x = xn;
         if (done) break;
     }
-    return gammp_dev(alpha + 1.0, x);
+    return gammp(alpha + 1.0, x);
 }
-// mdl: raw parameters (rates [48..53], freqs [36..39], alpha [45]) -> eigenvalues [0..3], U [4..19], U^-1 [20..35], class rates [40..43].
+
+// ---- model parameters on the device (LlhMode::All): one thread rebuilds the eigen-system and the class rates of its tree
+// mdl: raw parameters (GTR rates, freqs, alpha) -> eigenvalues, U, U^-1, class rates.
 // Threads 0 (eigen-system: cyclic Jacobi on the symmetrised rate matrix) and 1..3 (class boundaries) work, then a barrier.
 __device__ void rebuild_model(double* mdl, double* scratch /* 4 doubles */, bool eigen, bool gamma) {
     const int tid = threadIdx.x;
     if (tid == 0 && eigen) {
-        const double* pi = mdl + 36;
-        double r[4][4] = {{0, mdl[48], mdl[49], mdl[50]}, {mdl[48], 0, mdl[51], mdl[52]}, {mdl[49], mdl[51], 0, mdl[53]}, {mdl[50], mdl[52], mdl[53], 0}};
+        const double* pi = mdl + MDL_FREQ;
+        const double* g = mdl + MDL_GTR;
+        double r[4][4] = {{0, g[0], g[1], g[2]}, {g[0], 0, g[3], g[4]}, {g[1], g[3], 0, g[5]}, {g[2], g[4], g[5], 0}};
         double Q[4][4], S[4][4], V[4][4];
         double norm = 0.0;
         for (int a = 0; a < 4; ++a) {
@@ -122,16 +127,17 @@ __device__ void rebuild_model(double* mdl, double* scratch /* 4 doubles */, bool
                     for (int k = 0; k < 4; ++k) { const double vkp = V[k][p], vkq = V[k][q]; V[k][p] = cs * vkp - sn * vkq; V[k][q] = sn * vkp + cs * vkq; }
                 }
         }
-        for (int j = 0; j < 4; ++j) mdl[j] = S[j][j];
+        for (int j = 0; j < 4; ++j) mdl[MDL_LAM + j] = S[j][j];
         for (int a = 0; a < 4; ++a)
-            for (int j = 0; j < 4; ++j) { mdl[4 + a * 4 + j] = V[a][j] / sqrt(pi[a]); mdl[20 + j * 4 + a] = V[a][j] * sqrt(pi[a]); }
+            for (int j = 0; j < 4; ++j) { mdl[MDL_U + a * 4 + j] = V[a][j] / sqrt(pi[a]); mdl[MDL_UINV + j * 4 + a] = V[a][j] * sqrt(pi[a]); }
     }
-    if (gamma && tid >= 1 && tid <= 3) scratch[tid] = gamma_cdf1_dev(mdl[45], tid - 1);
+    if (gamma && tid >= 1 && tid <= 3) scratch[tid] = gamma_class_cdf(mdl[MDL_ALPHA], (double)tid * 0.25);   // boundaries of classes 0..2
     __syncthreads();
     if (gamma && tid == 0) {
         scratch[0] = 0.0;
         const double c4 = 1.0;
-        mdl[40] = 4.0 * (scratch[1] - 0.0); mdl[41] = 4.0 * (scratch[2] - scratch[1]); mdl[42] = 4.0 * (scratch[3] - scratch[2]); mdl[43] = 4.0 * (c4 - scratch[3]);
+        double* rate = mdl + MDL_RATE;
+        rate[0] = 4.0 * (scratch[1] - 0.0); rate[1] = 4.0 * (scratch[2] - scratch[1]); rate[2] = 4.0 * (scratch[3] - scratch[2]); rate[3] = 4.0 * (c4 - scratch[3]);
     }
     __syncthreads();
 }
@@ -160,12 +166,12 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh(const LlhArgs a) {
     const int c1 = ch[(R - 2) * 2], c2 = ch[(R - 2) * 2 + 1];
     if (tid == 0) { const double t0 = clampd(t[c1] + t[c2], BRLEN_MIN, BRLEN_MAX); t[c1] = t0; t[c2] = t0; }   // the root branch, stored at both ends
     __syncthreads();
-    double pinv = mdl[44], wk = (1.0 - pinv) * 0.25;            // re-read after every change of the model (optimise = 2)
+    double pinv = mdl[MDL_PINV], wk = (1.0 - pinv) * 0.25;      // re-read after every change of the model (All)
     // invariant-site term: pi_x where every tip of the pattern is compatible with exactly one state x
     for (int s = tid; s < L; s += LLH_THREADS) {
         int m = 15;
         for (int v = 0; v < R; ++v) m &= tips[(size_t)v * L + s];
-        invt[s] = (m != 0 && (m & (m - 1)) == 0) ? mdl[36 + (31 - __clz(m))] : 0.0;      // times p_inv where it is used
+        invt[s] = (m != 0 && (m & (m - 1)) == 0) ? mdl[MDL_FREQ + (31 - __clz(m))] : 0.0;      // times p_inv where it is used
     }
     // ---- subtree vectors, children before parents (join order); the virtual root itself is never needed
     // dst = (P(t_x) X) * (P(t_y) D[y]) with X = D[x], or U[x] when xsrc_U is given; scaled as described at the top
@@ -196,16 +202,8 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh(const LlhArgs a) {
             clv_load(R, L, Dt, tips, c1, s, v1);
             clv_load(R, L, Dt, tips, c2, s, v2);
             pm_apply(Pm, v1, p1);
-            double l = 0.0;
-#pragma unroll
-            for (int k = 0; k < 4; ++k)
-#pragma unroll
-                for (int c = 0; c < 4; ++c) l = fma(mdl[36 + c] * p1[k * 4 + c], v2[k * 4 + c], l);
             const int n = cnt_load(R, L, Dnt, c1, s) + cnt_load(R, L, Dnt, c2, s);
-            double site;
-            if (n == 0) site = log(wk * l + pinv * invt[s]);
-            else if (pinv * invt[s] == 0.0) site = log(wk * l) - n * SCALE_LN;
-            else site = log(ldexp(wk * l, -SCALE_EXP * n) + pinv * invt[s]);
+            const double site = site_loglik(mdl, p1, v2, n, wk, pinv, invt[s]);
             acc += wts[s] * site;
             if (a.site) a.site[(size_t)b * L + s] = site;
         }
@@ -259,21 +257,21 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh(const LlhArgs a) {
             if (gain < a.eps) break;
         }
     };
-    if (a.optimise == 3) {
-        sweeps();             // max_passes = 1 and only UP / SWAPROOT rows: one pass fills U[v] for every v at the given lengths
-    } else if (a.optimise) {
+    if (a.mode == LlhMode::Prepare) {
+        sweeps();             // one pass over the UP / SWAPROOT rows (llh_prepare) fills U[v] for every v at the given lengths
+    } else if (a.mode != LlhMode::Eval) {
         sweeps();
-        if (a.optimise == 2) {
+        if (a.mode == LlhMode::All) {
             // ---- model parameters: rounds of (every free parameter by golden section, all else fixed; branch sweeps) until a round
             //      gains < lh_eps - the loop of oracle/llh_oracle.py optimize_all, one tree per CTA, no host round trips
-            const int flags = (int)mdl[46];
+            const int flags = (int)mdl[MDL_FLAGS];
             auto objective = [&](int prm, double x) {            // set parameter prm to x (log scale for rates / alpha), rebuild, evaluate
                 if (tid == 0) {
-                    if (prm < 5) mdl[48 + prm] = exp(x); else if (prm == 5) mdl[45] = exp(x); else mdl[44] = x;
+                    if (prm < 5) mdl[MDL_GTR + prm] = exp(x); else if (prm == 5) mdl[MDL_ALPHA] = exp(x); else mdl[MDL_PINV] = x;
                 }
                 __syncthreads();
                 rebuild_model(mdl, ek, prm < 5, prm == 5);
-                pinv = mdl[44]; wk = (1.0 - pinv) * 0.25;
+                pinv = mdl[MDL_PINV]; wk = (1.0 - pinv) * 0.25;
                 down_pass();
                 return root_loglik();
             };
@@ -304,29 +302,38 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh(const LlhArgs a) {
 }
 
 // ---- host side
-static inline size_t up256(size_t v) { return (v + 255) & ~(size_t)255; }
-struct LlhLayout { size_t tipsz, D, U, S, inv, Dn, Un, Sn, small, total; };
-static LlhLayout llh_layout(int B, int R, int L, int n_ops) {
-    LlhLayout l;
-    l.D = up256((size_t)B * (R - 1) * L * 16 * 8);
-    l.U = up256((size_t)B * (2 * R - 2) * L * 16 * 8);
-    l.S = up256((size_t)B * L * 16 * 8);
-    l.inv = up256((size_t)B * L * 8);
-    l.Dn = up256((size_t)B * (R - 1) * L * 4);
-    l.Un = up256((size_t)B * (2 * R - 2) * L * 4);
-    l.Sn = up256((size_t)B * L * 4);
-    // staged host arrays: children, ops, brlen, model, llh
-    l.small = up256((size_t)B * (R - 1) * 2 * 4) + up256((size_t)B * n_ops * 4 * 4) + up256((size_t)B * (2 * R - 2) * 8) + up256((size_t)B * LLH_MODEL * 8) +
-              up256((size_t)B * 2 * 8);
-    l.tipsz = 0;
-    l.total = l.D + l.U + l.S + l.inv + l.Dn + l.Un + l.Sn + l.small + 256;
-    return l;
+struct LlhBuffers {
+    double *D, *U, *S, *inv;
+    int32_t *Dn, *Un, *Sn;
+    int32_t *ch, *ops; double *br, *md, *ll;     // staged host arrays: children, schedule, brlen, model, llh (before, after)
+    size_t total;
+};
+static LlhBuffers llh_layout(char* base, int B, int R, int L, int n_ops) {
+    WsCarver c(base);
+    LlhBuffers w;
+    const size_t inner = (size_t)B * (R - 1), edges = (size_t)B * (2 * R - 2);
+    w.D = c.take<double>(inner * L * 16);
+    w.U = c.take<double>(edges * L * 16);
+    w.S = c.take<double>((size_t)B * L * 16);
+    w.inv = c.take<double>((size_t)B * L);
+    w.Dn = c.take<int32_t>(inner * L);
+    w.Un = c.take<int32_t>(edges * L);
+    w.Sn = c.take<int32_t>((size_t)B * L);
+    w.ch = c.take<int32_t>(inner * 2);
+    w.ops = c.take<int32_t>((size_t)B * n_ops * 4);
+    w.br = c.take<double>(edges);
+    w.md = c.take<double>((size_t)B * LLH_MODEL);
+    w.ll = c.take<double>((size_t)B * 2);
+    w.total = c.off + 256;
+    return w;
 }
 
-size_t llh_ws_bytes(int B, int R, int L) { return llh_layout(B, R, L, 5 * R).total; }
+// build_ops emits 5R - 8 rows for every binary tree: OPT for each of the 2R - 3 branches, two UP rows and one DOWN row for each of the
+// R - 2 inner nodes below the root, and SWAPROOT.  5R rows bound every mode's schedule.
+size_t llh_ws_bytes(int B, int R, int L) { return llh_layout(nullptr, B, R, L, 5 * R).total; }
 
 // depth-first schedule of oracle/llh_oracle.py build_ops (same order: the two implementations visit the branches identically)
-static int build_ops(const int32_t* ch, int R, std::vector<int32_t>& ops) {
+static void build_ops(const int32_t* ch, int R, std::vector<int32_t>& ops) {
     struct Item { int what, v, x, y; };   // 0 enter(optimise = x), 1 up, 2 down
     auto is_inner = [&](int v) { return v >= R; };
     std::vector<Item> st;
@@ -355,7 +362,19 @@ static int build_ops(const int32_t* ch, int R, std::vector<int32_t>& ops) {
     run(c1, 1);
     ops.insert(ops.end(), {OP_SWAPROOT, c2, c1, 0});
     run(c2, 0);
-    return (int)(ops.size() / 4);
+}
+
+// the build_ops schedules of the B trees, one after another -> rows per tree, or an error code (< 0)
+static int schedule(const LlhTrees& in, std::vector<int32_t>& all) {
+    int n_ops = 0;
+    for (int b = 0; b < in.B; ++b) {
+        const size_t start = all.size();
+        build_ops(in.children + (size_t)b * (in.R - 1) * 2, in.R, all);
+        const int n = (int)((all.size() - start) / 4);
+        if (b == 0) n_ops = n;
+        if (n != n_ops) return set_error(NNJ_ERR_INVALID, "llh: internal error (schedule length differs between trees)");
+    }
+    return n_ops;
 }
 
 int llh_check_tree(const int32_t* ch, int R) {
@@ -369,55 +388,24 @@ int llh_check_tree(const int32_t* ch, int R) {
     return 0;
 }
 
-int run_llh(const uint8_t* tips, const double* weights, const int32_t* children_h, double* brlen_h, double* model_h, int B, int R, int L,
-            int optimise, int max_passes, double eps, double lh_eps, int max_rounds, int golden_iters, double* llh_h, void* ws, size_t ws_bytes,
-            cudaStream_t st, double* site_dev, LlhState* state) {
-    std::vector<int32_t> ops_all;
-    int n_ops = 0;
-    for (int b = 0; b < B; ++b) {
-        if (llh_check_tree(children_h + (size_t)b * (R - 1) * 2, R)) return set_error(NNJ_ERR_INVALID, "llh: children is not a binary tree in join order");
-        if (optimise) {
-            std::vector<int32_t> ops;
-            int n = build_ops(children_h + (size_t)b * (R - 1) * 2, R, ops);
-            if (optimise == 3) {           // the U pass alone: UP and SWAPROOT rows, no Newton, no refreshed subtree vectors
-                std::vector<int32_t> keep;
-                for (int i = 0; i < n; ++i)
-                    if (ops[4 * i] == OP_UP || ops[4 * i] == OP_SWAPROOT) keep.insert(keep.end(), ops.begin() + 4 * i, ops.begin() + 4 * i + 4);
-                ops.swap(keep);
-                n = (int)(ops.size() / 4);
-            }
-            if (b == 0) n_ops = n;
-            if (n != n_ops) return set_error(NNJ_ERR_INVALID, "llh: internal error (schedule length differs between trees)");
-            ops_all.insert(ops_all.end(), ops.begin(), ops.end());
-        }
-    }
-    const LlhLayout lay = llh_layout(B, R, L, n_ops);
-    if (ws_bytes < lay.total) return set_error(NNJ_ERR_WORKSPACE, "llh: workspace too small (nnj_llh_workspace_bytes)");
-    char* p = reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
-    LlhArgs a;
-    a.tips = tips; a.weights = weights;
-    a.D = reinterpret_cast<double*>(p); p += lay.D;
-    a.U = reinterpret_cast<double*>(p); p += lay.U;
-    a.S = reinterpret_cast<double*>(p); p += lay.S;
-    a.inv = reinterpret_cast<double*>(p); p += lay.inv;
-    a.Dn = reinterpret_cast<int32_t*>(p); p += lay.Dn;
-    a.Un = reinterpret_cast<int32_t*>(p); p += lay.Un;
-    a.Sn = reinterpret_cast<int32_t*>(p); p += lay.Sn;
-    int32_t* d_ch = reinterpret_cast<int32_t*>(p); p += up256((size_t)B * (R - 1) * 2 * 4);
-    int32_t* d_ops = reinterpret_cast<int32_t*>(p); p += up256((size_t)B * n_ops * 4 * 4);
-    double* d_br = reinterpret_cast<double*>(p); p += up256((size_t)B * (2 * R - 2) * 8);
-    double* d_md = reinterpret_cast<double*>(p); p += up256((size_t)B * LLH_MODEL * 8);
-    double* d_ll = reinterpret_cast<double*>(p);
-    cudaError_t e = cudaMemcpyAsync(d_ch, children_h, (size_t)B * (R - 1) * 2 * 4, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess && n_ops) e = cudaMemcpyAsync(d_ops, ops_all.data(), (size_t)B * n_ops * 4 * 4, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_br, brlen_h, (size_t)B * (2 * R - 2) * 8, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_md, model_h, (size_t)B * LLH_MODEL * 8, cudaMemcpyHostToDevice, st);
+// one k_llh launch over B checked trees with the schedule ops (n_ops rows per tree); llh_before / llh_after / site_dev may be null.
+// w: where the workspace holds the buffers.
+static int launch_llh(const LlhTrees& in, LlhMode mode, const LlhOptions& opt, const std::vector<int32_t>& ops, int n_ops, double* llh_before,
+                      double* llh_after, double* site_dev, void* ws, size_t ws_bytes, cudaStream_t st, LlhBuffers& w) {
+    const int B = in.B, R = in.R, L = in.L;
+    if (ws_bytes < llh_layout(nullptr, B, R, L, n_ops).total) return set_error(NNJ_ERR_WORKSPACE, "llh: workspace too small (nnj_llh_workspace_bytes)");
+    w = llh_layout(ws_align(ws), B, R, L, n_ops);
+    cudaError_t e = cudaMemcpyAsync(w.ch, in.children, (size_t)B * (R - 1) * 2 * 4, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess && n_ops) e = cudaMemcpyAsync(w.ops, ops.data(), (size_t)B * n_ops * 4 * 4, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(w.br, in.brlen, (size_t)B * (2 * R - 2) * 8, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(w.md, in.model, (size_t)B * LLH_MODEL * 8, cudaMemcpyHostToDevice, st);
     if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
-    a.children = d_ch; a.ops = d_ops; a.brlen = d_br; a.model = d_md; a.llh = d_ll; a.site = optimise == 3 ? site_dev : nullptr;
-    if (optimise == 3) max_passes = 1;
-    if (state) { state->D = a.D; state->U = a.U; state->inv = a.inv; state->Dn = a.Dn; state->Un = a.Un; }
-    a.B = B; a.R = R; a.L = L; a.n_ops = n_ops; a.max_passes = max_passes; a.optimise = optimise; a.eps = eps;
-    a.lh_eps = lh_eps; a.max_rounds = max_rounds; a.golden_iters = golden_iters; a.model_out = d_md;
+    LlhArgs a;
+    a.tips = in.tips; a.weights = in.weights; a.children = w.ch; a.ops = w.ops; a.brlen = w.br; a.model = w.md;
+    a.D = w.D; a.U = w.U; a.S = w.S; a.inv = w.inv; a.Dn = w.Dn; a.Un = w.Un; a.Sn = w.Sn;
+    a.llh = w.ll; a.site = site_dev;
+    a.B = B; a.R = R; a.L = L; a.n_ops = n_ops; a.max_passes = opt.max_passes; a.mode = mode; a.eps = opt.eps;
+    a.lh_eps = opt.lh_eps; a.max_rounds = opt.max_rounds; a.golden_iters = GOLDEN_ITERS; a.model_out = w.md;
     const size_t smem = (LLH_MODEL + 128 + 66 + 48 + 2 * (size_t)R) * sizeof(double);      // 67 968 bytes at R = 4096
     if (smem > 48 * 1024) {       // above the default limit the kernel must opt in (from R = 2920 on)
         e = cudaFuncSetAttribute(k_llh, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -427,61 +415,49 @@ int run_llh(const uint8_t* tips, const double* weights, const int32_t* children_
     k_llh<<<B, LLH_THREADS, smem, st>>>(a);
     ++g_launches;
     prof_end(st);
+    std::vector<double> ll((size_t)B * 2);
+    const bool brlen_out = mode == LlhMode::Brlen || mode == LlhMode::All;
     e = cudaGetLastError();
-    if (e == cudaSuccess) e = cudaMemcpyAsync(llh_h, d_ll, (size_t)B * 2 * 8, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess && (optimise == 1 || optimise == 2)) e = cudaMemcpyAsync(brlen_h, d_br, (size_t)B * (2 * R - 2) * 8, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess && optimise == 2) e = cudaMemcpyAsync(model_h, d_md, (size_t)B * LLH_MODEL * 8, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(ll.data(), w.ll, ll.size() * 8, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess && brlen_out) e = cudaMemcpyAsync(in.brlen, w.br, (size_t)B * (2 * R - 2) * 8, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess && mode == LlhMode::All) e = cudaMemcpyAsync(in.model, w.md, (size_t)B * LLH_MODEL * 8, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);       // the small results are host values: the call returns them
     if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
+    for (int b = 0; b < B; ++b) {
+        if (llh_before) llh_before[b] = ll[2 * b];
+        if (llh_after) llh_after[b] = ll[2 * b + 1];
+    }
     return 0;
 }
 
-// ---- discrete gamma (Yang 1994): mean rate of each of ncat equal-probability classes of Gamma(alpha, alpha)
-static double gammp(double a, double x) {     // regularised lower incomplete gamma P(a, x): series / continued fraction (Lentz)
-    if (x <= 0.0) return 0.0;
-    const double gln = lgamma(a);
-    if (x < a + 1.0) {
-        double ap = a, sum = 1.0 / a, del = sum;
-        for (int n = 0; n < 2000; ++n) { ap += 1.0; del *= x / ap; sum += del; if (fabs(del) < fabs(sum) * 1e-17) break; }
-        return sum * exp(-x + a * log(x) - gln);
-    }
-    double b = x + 1.0 - a, c = 1e300, d = 1.0 / b, h = d;
-    for (int i = 1; i < 2000; ++i) {
-        const double an = -i * (i - a);
-        b += 2.0;
-        d = an * d + b; if (fabs(d) < 1e-300) d = 1e-300;
-        c = b + an / c; if (fabs(c) < 1e-300) c = 1e-300;
-        d = 1.0 / d;
-        const double del = d * c;
-        h *= del;
-        if (fabs(del - 1.0) < 1e-17) break;
-    }
-    return 1.0 - exp(-x + a * log(x) - gln) * h;
+int run_llh(const LlhTrees& in, LlhMode mode, const LlhOptions& opt, double* llh_before, double* llh_after, void* ws, size_t ws_bytes, cudaStream_t st) {
+    for (int b = 0; b < in.B; ++b)
+        if (llh_check_tree(in.children + (size_t)b * (in.R - 1) * 2, in.R)) return set_error(NNJ_ERR_INVALID, "llh: children is not a binary tree in join order");
+    std::vector<int32_t> ops;
+    const int n_ops = mode == LlhMode::Eval ? 0 : schedule(in, ops);
+    if (n_ops < 0) return n_ops;
+    LlhBuffers w;
+    return launch_llh(in, mode, opt, ops, n_ops, llh_before, llh_after, nullptr, ws, ws_bytes, st, w);
+}
+
+LlhPrepared llh_prepare(const LlhTrees& in, double* site_dev, double* llh_h, void* ws, size_t ws_bytes, cudaStream_t st) {
+    std::vector<int32_t> ops, u_pass;
+    const int n = schedule(in, ops);
+    if (n < 0) return {n, nullptr, nullptr, nullptr, nullptr, nullptr};
+    // the U pass alone: UP and SWAPROOT rows (2R - 3 per tree), no Newton, no refreshed subtree vectors; one pass fills U[v] for every v
+    for (size_t i = 0; i < ops.size(); i += 4)
+        if (ops[i] == OP_UP || ops[i] == OP_SWAPROOT) u_pass.insert(u_pass.end(), ops.begin() + i, ops.begin() + i + 4);
+    const LlhOptions one_pass{1, 0.0, 0.0, 0};
+    LlhBuffers w{};
+    const int rc = launch_llh(in, LlhMode::Prepare, one_pass, u_pass, (int)(u_pass.size() / 4 / in.B), nullptr, llh_h, site_dev, ws, ws_bytes, st, w);
+    return {rc, w.D, w.U, w.inv, w.Dn, w.Un};
 }
 
 int gamma_rates(double alpha, int ncat, double* out) {
     if (!(alpha > 0.0) || ncat < 1 || ncat > 64) return set_error(NNJ_ERR_INVALID, "gamma_rates: alpha must be > 0 and 1 <= ncat <= 64");
     std::vector<double> cdf(ncat + 1, 0.0);
     cdf[ncat] = 1.0;
-    for (int i = 1; i < ncat; ++i) {
-        // quantile x of Gamma(alpha, 1) at i / ncat: Newton on P(alpha, x) (monotone, density known) kept inside a bracket, a bisection
-        // step whenever Newton leaves it
-        const double target = (double)i / ncat, gln = lgamma(alpha);
-        double lo = 0.0, hi = alpha + 1.0;
-        while (gammp(alpha, hi) < target) hi *= 2.0;
-        double x = 0.5 * (lo + hi);
-        for (int it = 0; it < 200; ++it) {
-            const double f = gammp(alpha, x) - target;
-            if (f < 0.0) lo = x; else hi = x;
-            const double pdf = exp((alpha - 1.0) * log(x) - x - gln);
-            double xn = pdf > 0.0 ? x - f / pdf : 0.5 * (lo + hi);
-            if (!(xn > lo && xn < hi)) xn = 0.5 * (lo + hi);
-            const bool done = fabs(xn - x) <= 1e-15 * x || hi - lo <= 1e-300;
-            x = xn;
-            if (done) break;
-        }
-        cdf[i] = gammp(alpha + 1.0, x);
-    }
+    for (int i = 1; i < ncat; ++i) cdf[i] = gamma_class_cdf(alpha, (double)i / ncat);
     for (int i = 0; i < ncat; ++i) out[i] = ncat * (cdf[i + 1] - cdf[i]);
     return 0;
 }

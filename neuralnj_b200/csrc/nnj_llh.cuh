@@ -7,7 +7,15 @@
 namespace nnj {
 
 constexpr int LLH_THREADS = 512;
-constexpr int LLH_MODEL = 64;      // lam 4 | U 16 | Uinv 16 | freqs 4 | class rates 4 | p_inv | alpha | flags (1 GTR rates free, 2 +G, 4 +I) | pad | 6 GTR rates | pad 10
+constexpr int LLH_MODEL = 64;      // doubles per tree of the packed model; its slots below (likelihood.py SubstModel.pack writes the same layout)
+constexpr int MDL_LAM = 0;         // 4 eigenvalues of the normalised rate matrix
+constexpr int MDL_U = 4;           // U [4][4] and U^-1 [4][4]: Q = U diag(lam) U^-1
+constexpr int MDL_UINV = 20;
+constexpr int MDL_FREQ = 36;       // 4 base frequencies
+constexpr int MDL_RATE = 40;       // 4 gamma class rates
+constexpr int MDL_PINV = 44, MDL_ALPHA = 45;
+constexpr int MDL_FLAGS = 46;      // free parameters: 1 GTR rates, 2 alpha (+G), 4 p_inv (+I); slot 47 is padding
+constexpr int MDL_GTR = 48;        // 6 GTR exchangeabilities AC AG AT CG CT GT; slots 54..63 are padding
 constexpr double BRLEN_MIN = 1e-6, BRLEN_MAX = 100.0;    // every length, in evaluation and optimisation, is clamped to this range
 constexpr int SCALE_EXP = 256;
 constexpr double SCALE_BELOW = 0x1p-256, SCALE_UP = 0x1p256, SCALE_LN = 256.0 * 0.69314718055994530942;
@@ -22,7 +30,7 @@ __device__ __forceinline__ void pmat2(double* Pm, const double* mdl, double t0, 
         const double t = w ? t1 : t0;
         double s = 0.0;
 #pragma unroll
-        for (int j = 0; j < 4; ++j) s += mdl[4 + a * 4 + j] * exp(mdl[j] * mdl[40 + k] * t) * mdl[20 + j * 4 + b];
+        for (int j = 0; j < 4; ++j) s += mdl[MDL_U + a * 4 + j] * exp(mdl[MDL_LAM + j] * mdl[MDL_RATE + k] * t) * mdl[MDL_UINV + j * 4 + b];
         Pm[i] = s;
     }
     __syncthreads();
@@ -34,7 +42,7 @@ __device__ __forceinline__ void pmat1(double* Pm, const double* mdl, double t) {
         const int k = (i >> 4) & 3, a = (i >> 2) & 3, b = i & 3;
         double s = 0.0;
 #pragma unroll
-        for (int j = 0; j < 4; ++j) s += mdl[4 + a * 4 + j] * exp(mdl[j] * mdl[40 + k] * t) * mdl[20 + j * 4 + b];
+        for (int j = 0; j < 4; ++j) s += mdl[MDL_U + a * 4 + j] * exp(mdl[MDL_LAM + j] * mdl[MDL_RATE + k] * t) * mdl[MDL_UINV + j * 4 + b];
         Pm[i] = s;
     }
     __syncthreads();
@@ -117,11 +125,25 @@ __device__ __forceinline__ void sumtable_row(const double* mdl, const double (&u
             double A = 0.0, Bm = 0.0;
 #pragma unroll
             for (int c = 0; c < 4; ++c) {
-                A = fma(mdl[36 + c] * u[k * 4 + c], mdl[4 + c * 4 + j], A);
-                Bm = fma(mdl[20 + j * 4 + c], d[k * 4 + c], Bm);
+                A = fma(mdl[MDL_FREQ + c] * u[k * 4 + c], mdl[MDL_U + c * 4 + j], A);
+                Bm = fma(mdl[MDL_UINV + j * 4 + c], d[k * 4 + c], Bm);
             }
             sv[k * 4 + j] = A * Bm;
         }
+}
+
+// log-likelihood of one pattern at a branch: p = P(t) x on one side, y the other side, n the scale count of the pair.  The site
+// likelihood is the mixture wk l + p_inv inv with l = sum_k sum_c pi_c p[k][c] y[k][c]; with n > 0 the 2^(256 n) scaling is undone
+// (exact: wherever n = 0 the arithmetic is the unscaled one)
+__device__ __forceinline__ double site_loglik(const double* mdl, const double (&p)[16], const double (&y)[16], int n, double wk, double pinv, double inv) {
+    double l = 0.0;
+#pragma unroll
+    for (int k = 0; k < 4; ++k)
+#pragma unroll
+        for (int c = 0; c < 4; ++c) l = fma(mdl[MDL_FREQ + c] * p[k * 4 + c], y[k * 4 + c], l);
+    if (n == 0) return log(wk * l + pinv * inv);
+    if (pinv * inv == 0.0) return log(wk * l) - n * SCALE_LN;
+    return log(ldexp(wk * l, -SCALE_EXP * n) + pinv * inv);
 }
 
 // safeguarded Newton-Raphson on one branch from tv, over the sumtable St [L][16] and its scale counts Snt [L] (the block's own
@@ -132,7 +154,7 @@ __device__ __forceinline__ double newton_brlen(const double* St, const int32_t* 
     double lo = BRLEN_MIN, hi = BRLEN_MAX;
     for (int it = 0; it < 32; ++it) {
         if (tid < 16) {
-            const double rate = mdl[tid & 3] * mdl[40 + (tid >> 2)];
+            const double rate = mdl[MDL_LAM + (tid & 3)] * mdl[MDL_RATE + (tid >> 2)];
             ek[tid] = exp(rate * tv); ek[16 + tid] = rate; ek[32 + tid] = rate * rate;
         }
         __syncthreads();

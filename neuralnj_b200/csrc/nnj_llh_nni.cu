@@ -2,8 +2,8 @@
 // five quartet lengths optimised, and RELL replicates of the per-pattern log-likelihoods for SH-aLRT and the local bootstrap
 // probability.  DESIGN.md section 12 gives the definitions; oracle/alrt_oracle.py restates them in numpy.
 //
-// 1. k_llh mode 3 (nnj_llh.cu), one CTA per tree: subtree vectors D, the U pass of the build_ops schedule (its UP and SWAPROOT
-//    rows) and the per-pattern log-likelihoods l0 at the given lengths.
+// 1. llh_prepare (nnj_llh.cu), k_llh with one CTA per tree: subtree vectors D, the U pass of the build_ops schedule (its UP and
+//    SWAPROOT rows) and the per-pattern log-likelihoods l0 at the given lengths.
 // 2. k_llh_nni, one CTA per (tree, internal branch, alternative), threads over patterns.  The quartet around the branch above v has
 //    the outer vectors A = D[a], B = D[b] (children of v), C = D[s] (sibling of v) and D = U[p] (parent of v), or for the root
 //    branch the two children of the other root child.  Alternative 1 pairs (A, C | B, D), alternative 2 (A, D | B, C).  Rounds of
@@ -29,7 +29,7 @@ struct NniArgs {
     const uint8_t* tips;        // [B][R][L]
     const double* weights;      // [B][L]
     const double* model;        // [B][LLH_MODEL]
-    const double *D, *U, *inv;  // k_llh mode 3 results: [B][R-1][L][16], [B][2R-2][L][16], [B][L]
+    const double *D, *U, *inv;  // llh_prepare results: [B][R-1][L][16], [B][2R-2][L][16], [B][L]
     const int32_t *Dn, *Un;
     const int32_t* qnode;       // [B][nb][4] A, B, C, D: node id of a subtree vector (tip or D), or -(p + 1) for U[p]
     const double* qlen;         // [B][nb][5] central, A, B, C, D at the tree's (clamped) lengths
@@ -61,7 +61,7 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh_nni(const NniArgs a) {
     if (tid < LLH_MODEL) mdl[tid] = a.model[(size_t)b * LLH_MODEL + tid];
     if (tid < 5) tq[tid] = a.qlen[(size_t)bi * 5 + tid];
     __syncthreads();
-    const double pinv = mdl[44], wk = (1.0 - pinv) * 0.25;
+    const double pinv = mdl[MDL_PINV], wk = (1.0 - pinv) * 0.25;
     for (int e = 0; e < 5; ++e) pmat1(Pm + 64 * e, mdl, tq[e]);
     // the two sides of the central branch: X = (edge 1, x2), Y = (edge 2, y2); alternative 1 is AC|BD, alternative 2 AD|BC
     const int x2 = alt ? 4 : 3, y2 = alt ? 3 : 4;
@@ -79,22 +79,14 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh_nni(const NniArgs a) {
         pm_apply(Pm + 64 * f, y, x);
         return n + mul_scaled(out, x);
     };
-    // log L of the alternative at the current lengths, at the central branch with the formula of k_llh's root; writes the sites
+    // log L of the alternative at the current lengths, at the central branch; writes the sites
     auto evaluate = [&]() {
         double acc = 0.0, dummy = 0.0;
         for (int s = tid; s < L; s += LLH_THREADS) {
             double X[16], Y[16], p1[16];
             const int n = half(1, x2, s, X) + half(2, y2, s, Y);
             pm_apply(Pm, X, p1);
-            double l = 0.0;
-#pragma unroll
-            for (int k = 0; k < 4; ++k)
-#pragma unroll
-                for (int c = 0; c < 4; ++c) l = fma(mdl[36 + c] * p1[k * 4 + c], Y[k * 4 + c], l);
-            double st;
-            if (n == 0) st = log(wk * l + pinv * invt[s]);
-            else if (pinv * invt[s] == 0.0) st = log(wk * l) - n * SCALE_LN;
-            else st = log(ldexp(wk * l, -SCALE_EXP * n) + pinv * invt[s]);
+            const double st = site_loglik(mdl, p1, Y, n, wk, pinv, invt[s]);
             site[s] = st;
             acc += wts[s] * st;
         }
@@ -193,39 +185,43 @@ __global__ void __launch_bounds__(RELL_THREADS) k_rell(const int32_t* __restrict
     if (s0 >= fmax(s1, s2)) atomicAdd(lbp + bi, 1);
 }
 
-static inline size_t up256(size_t v) { return (v + 255) & ~(size_t)255; }
-
-struct SupLayout { size_t S, Sn, site, site0, qnode, qlen, model, llh, len, cum, cnt, sh, lbp, total; };
-static SupLayout sup_layout(int B, int R, int L, int n_rell) {
+struct SupBuffers {
+    double* S; int32_t* Sn;             // each CTA's sumtable
+    double *site, *site0;               // per-pattern log-likelihoods (when the caller passes no site_dev) and l0
+    int32_t* qnode; double *qlen, *model, *llh, *len;
+    uint32_t* cum; int32_t *cnt, *sh, *lbp;
+    size_t total;
+};
+static SupBuffers sup_layout(char* base, int B, int R, int L, int n_rell) {
     const size_t nb = R > 3 ? (size_t)(R - 3) : 0, items = (size_t)B * nb * 2;
     const size_t chunk = n_rell < RELL_CHUNK ? (size_t)(n_rell > 0 ? n_rell : 1) : RELL_CHUNK;
-    SupLayout l;
-    l.S = up256(items * L * 16 * 8); l.Sn = up256(items * L * 4);
-    l.site = up256((size_t)B * nb * 3 * L * 8); l.site0 = up256((size_t)B * L * 8);
-    l.qnode = up256((size_t)B * nb * 4 * 4); l.qlen = up256((size_t)B * nb * 5 * 8); l.model = up256((size_t)B * LLH_MODEL * 8);
-    l.llh = up256(items * 8); l.len = up256(items * 5 * 8);
-    l.cum = up256((size_t)B * (L + 1) * 4); l.cnt = up256((size_t)B * L * chunk * 4);
-    l.sh = up256((size_t)B * nb * 4); l.lbp = up256((size_t)B * nb * 4);
-    l.total = l.S + l.Sn + l.site + l.site0 + l.qnode + l.qlen + l.model + l.llh + l.len + l.cum + l.cnt + l.sh + l.lbp + 256;
-    return l;
+    WsCarver c(base);
+    SupBuffers w;
+    w.S = c.take<double>(items * L * 16); w.Sn = c.take<int32_t>(items * L);
+    w.site = c.take<double>((size_t)B * nb * 3 * L); w.site0 = c.take<double>((size_t)B * L);
+    w.qnode = c.take<int32_t>((size_t)B * nb * 4); w.qlen = c.take<double>((size_t)B * nb * 5); w.model = c.take<double>((size_t)B * LLH_MODEL);
+    w.llh = c.take<double>(items); w.len = c.take<double>(items * 5);
+    w.cum = c.take<uint32_t>((size_t)B * (L + 1)); w.cnt = c.take<int32_t>((size_t)B * L * chunk);
+    w.sh = c.take<int32_t>((size_t)B * nb); w.lbp = c.take<int32_t>((size_t)B * nb);
+    w.total = c.off + 256;
+    return w;
 }
 
 }  // namespace
 
-size_t llh_support_ws_bytes(int B, int R, int L, int n_rell) { return llh_ws_bytes(B, R, L) + sup_layout(B, R, L, n_rell).total; }
+size_t llh_support_ws_bytes(int B, int R, int L, int n_rell) { return llh_ws_bytes(B, R, L) + sup_layout(nullptr, B, R, L, n_rell).total; }
 
-int run_llh_support(const uint8_t* tips, const double* weights, const int32_t* children_h, const double* brlen_h, const double* model_h, int B, int R,
-                    int L, uint64_t seed, int64_t rep0, int n_rell, int32_t* branch_node_h, double* llh_h, double* nni_brlen_h, int32_t* sh_h,
-                    int32_t* lbp_h, double* site_dev, void* ws, size_t ws_bytes, cudaStream_t st) {
-    const int nb = R - 3;
+int run_llh_support(const LlhTrees& in, uint64_t seed, int64_t rep0, int n_rell, int32_t* branch_node_h, double* llh_h, double* nni_brlen_h,
+                    int32_t* sh_h, int32_t* lbp_h, double* site_dev, void* ws, size_t ws_bytes, cudaStream_t st) {
+    const int B = in.B, R = in.R, L = in.L, nb = R - 3;
+    const int32_t* children_h = in.children;
     const size_t base = llh_ws_bytes(B, R, L);
-    const SupLayout lay = sup_layout(B, R, L, n_rell);
-    if (ws_bytes < base + lay.total) return set_error(NNJ_ERR_WORKSPACE, "llh_branch_support: workspace too small (nnj_llh_support_workspace_bytes)");
+    if (ws_bytes < base + sup_layout(nullptr, B, R, L, n_rell).total) return set_error(NNJ_ERR_WORKSPACE, "llh_branch_support: workspace too small (nnj_llh_support_workspace_bytes)");
     // ---- host checks: trees, integral weights (the RELL draws pick sites, and a pattern of weight w is w sites)
     for (int b = 0; b < B; ++b)
         if (llh_check_tree(children_h + (size_t)b * (R - 1) * 2, R)) return set_error(NNJ_ERR_INVALID, "llh_branch_support: children is not a binary tree in join order");
     std::vector<double> w((size_t)B * L);
-    cudaError_t e = cudaMemcpyAsync(w.data(), weights, w.size() * 8, cudaMemcpyDeviceToHost, st);
+    cudaError_t e = cudaMemcpyAsync(w.data(), in.weights, w.size() * 8, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
     std::vector<uint32_t> cum((size_t)B * (L + 1));
@@ -252,7 +248,7 @@ int run_llh_support(const uint8_t* tips, const double* weights, const int32_t* c
         std::vector<int> parent(2 * R - 1, -1);
         for (int k = 0; k < R - 1; ++k) { parent[ch[2 * k]] = R + k; parent[ch[2 * k + 1]] = R + k; }
         std::vector<double> t(2 * R - 2);
-        for (int v = 0; v < 2 * R - 2; ++v) t[v] = clampd(brlen_h[(size_t)b * (2 * R - 2) + v], BRLEN_MIN, BRLEN_MAX);
+        for (int v = 0; v < 2 * R - 2; ++v) t[v] = clampd(in.brlen[(size_t)b * (2 * R - 2) + v], BRLEN_MIN, BRLEN_MAX);
         const int root = 2 * R - 2, c1 = ch[2 * (R - 2)], c2 = ch[2 * (R - 2) + 1];
         t[c1] = t[c2] = clampd(t[c1] + t[c2], BRLEN_MIN, BRLEN_MAX);
         int i = 0;
@@ -273,39 +269,24 @@ int run_llh_support(const uint8_t* tips, const double* weights, const int32_t* c
         }
         if (i != nb) return set_error(NNJ_ERR_INVALID, "llh_branch_support: internal error (branch count)");
     }
-    char* p = reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(ws) + base + 255) & ~(uintptr_t)255);
-    NniArgs a;
-    double* S = reinterpret_cast<double*>(p); p += lay.S;
-    int32_t* Sn = reinterpret_cast<int32_t*>(p); p += lay.Sn;
-    double* site_ws = reinterpret_cast<double*>(p); p += lay.site;
-    double* site0 = reinterpret_cast<double*>(p); p += lay.site0;
-    int32_t* d_qnode = reinterpret_cast<int32_t*>(p); p += lay.qnode;
-    double* d_qlen = reinterpret_cast<double*>(p); p += lay.qlen;
-    double* d_model = reinterpret_cast<double*>(p); p += lay.model;
-    double* d_llh = reinterpret_cast<double*>(p); p += lay.llh;
-    double* d_len = reinterpret_cast<double*>(p); p += lay.len;
-    uint32_t* d_cum = reinterpret_cast<uint32_t*>(p); p += lay.cum;
-    int32_t* d_cnt = reinterpret_cast<int32_t*>(p); p += lay.cnt;
-    int32_t* d_sh = reinterpret_cast<int32_t*>(p); p += lay.sh;
-    int32_t* d_lbp = reinterpret_cast<int32_t*>(p);
-    // ---- 1. subtree vectors, the U pass and l0 (k_llh mode 3)
-    std::vector<double> l0_tree((size_t)B * 2);
-    LlhState stt;
-    int rc = run_llh(tips, weights, children_h, const_cast<double*>(brlen_h), const_cast<double*>(model_h), B, R, L, 3, 1, 0.0, 0.0, 0, 0, l0_tree.data(),
-                     ws, base, st, site0, &stt);
-    if (rc) return rc;
+    const SupBuffers sw = sup_layout(ws_align(static_cast<char*>(ws) + base), B, R, L, n_rell);
+    // ---- 1. subtree vectors, the U pass and l0
+    std::vector<double> l0_tree(B);
+    const LlhPrepared pre = llh_prepare(in, sw.site0, l0_tree.data(), ws, base, st);
+    if (pre.rc) return pre.rc;
     // ---- 2. the NNI quartets
-    e = cudaMemcpyAsync(d_qnode, qnode.data(), qnode.size() * 4, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_qlen, qlen.data(), qlen.size() * 8, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_model, model_h, (size_t)B * LLH_MODEL * 8, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_cum, cum.data(), cum.size() * 4, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaMemsetAsync(d_sh, 0, (size_t)B * nb * 4, st);
-    if (e == cudaSuccess) e = cudaMemsetAsync(d_lbp, 0, (size_t)B * nb * 4, st);
+    e = cudaMemcpyAsync(sw.qnode, qnode.data(), qnode.size() * 4, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(sw.qlen, qlen.data(), qlen.size() * 8, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(sw.model, in.model, (size_t)B * LLH_MODEL * 8, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(sw.cum, cum.data(), cum.size() * 4, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(sw.sh, 0, (size_t)B * nb * 4, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(sw.lbp, 0, (size_t)B * nb * 4, st);
     if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
-    a.tips = tips; a.weights = weights; a.model = d_model;
-    a.D = stt.D; a.U = stt.U; a.inv = stt.inv; a.Dn = stt.Dn; a.Un = stt.Un;
-    a.qnode = d_qnode; a.qlen = d_qlen; a.S = S; a.Sn = Sn; a.site0 = site0; a.site = site_dev ? site_dev : site_ws;
-    a.llh = d_llh; a.len = d_len; a.R = R; a.L = L; a.nb = nb;
+    NniArgs a;
+    a.tips = in.tips; a.weights = in.weights; a.model = sw.model;
+    a.D = pre.D; a.U = pre.U; a.inv = pre.inv; a.Dn = pre.Dn; a.Un = pre.Un;
+    a.qnode = sw.qnode; a.qlen = sw.qlen; a.S = sw.S; a.Sn = sw.Sn; a.site0 = sw.site0; a.site = site_dev ? site_dev : sw.site;
+    a.llh = sw.llh; a.len = sw.len; a.R = R; a.L = L; a.nb = nb;
     prof_begin(KC_LLH, st);
     k_llh_nni<<<B * nb * 2, LLH_THREADS, 0, st>>>(a);
     ++g_launches; prof_end(st);
@@ -314,29 +295,29 @@ int run_llh_support(const uint8_t* tips, const double* weights, const int32_t* c
     // ---- 3. RELL, in chunks of replicates
     for (int r0 = 0; r0 < n_rell; r0 += RELL_CHUNK) {
         const int nr = n_rell - r0 < RELL_CHUNK ? n_rell - r0 : RELL_CHUNK;
-        e = cudaMemsetAsync(d_cnt, 0, (size_t)B * L * nr * 4, st);
+        e = cudaMemsetAsync(sw.cnt, 0, (size_t)B * L * nr * 4, st);
         if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
         const dim3 grid((nmax + RELL_THREADS - 1) / RELL_THREADS, B * nr < 65535 ? B * nr : 65535);
         prof_begin(KC_LLH, st);
-        k_rell_counts<<<grid, RELL_THREADS, 0, st>>>(d_cum, B, L, seed, rep0 + r0, nr, d_cnt);
+        k_rell_counts<<<grid, RELL_THREADS, 0, st>>>(sw.cum, B, L, seed, rep0 + r0, nr, sw.cnt);
         ++g_launches; prof_end(st);
         const size_t threads = (size_t)B * nb * nr;
         prof_begin(KC_LLH, st);
-        k_rell<<<(unsigned)((threads + RELL_THREADS - 1) / RELL_THREADS), RELL_THREADS, 0, st>>>(d_cnt, weights, a.site, B, nb, L, nr, d_sh, d_lbp);
+        k_rell<<<(unsigned)((threads + RELL_THREADS - 1) / RELL_THREADS), RELL_THREADS, 0, st>>>(sw.cnt, in.weights, a.site, B, nb, L, nr, sw.sh, sw.lbp);
         ++g_launches; prof_end(st);
         e = cudaGetLastError();
         if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
     }
     // ---- results
     std::vector<double> l12((size_t)B * nb * 2);
-    e = cudaMemcpyAsync(l12.data(), d_llh, l12.size() * 8, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(nni_brlen_h, d_len, (size_t)B * nb * 10 * 8, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(sh_h, d_sh, (size_t)B * nb * 4, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(lbp_h, d_lbp, (size_t)B * nb * 4, cudaMemcpyDeviceToHost, st);
+    e = cudaMemcpyAsync(l12.data(), sw.llh, l12.size() * 8, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(nni_brlen_h, sw.len, (size_t)B * nb * 10 * 8, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(sh_h, sw.sh, (size_t)B * nb * 4, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(lbp_h, sw.lbp, (size_t)B * nb * 4, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
     for (size_t bi = 0; bi < (size_t)B * nb; ++bi) {
-        llh_h[bi * 3] = l0_tree[2 * (bi / nb) + 1];
+        llh_h[bi * 3] = l0_tree[bi / nb];
         llh_h[bi * 3 + 1] = l12[bi * 2];
         llh_h[bi * 3 + 2] = l12[bi * 2 + 1];
     }

@@ -1048,8 +1048,6 @@ __global__ void k_reindex_copy(const float* __restrict__ in, const float* __rest
 }
 
 // ------------------------------------------------------------------ host side
-static inline size_t aup(size_t v) { return (v + 255) / 256 * 256; }
-
 struct NjBuffers {
     float *Y, *K, *kap, *alpha_part, *alpha, *score_part, *new_scores, *logits[2], *newx;
     int32_t *slot[2], *free_slot, *new_slot, *pair_i, *pair_j;
@@ -1083,37 +1081,35 @@ static NjBuffers nj_layout(char* base, int B, int S, int R, int C, bool X_in_ws,
     nb.RP = (S + 3) & ~3;     // >= S: tensor-core alpha partials are indexed by physical slot
     nb.P0 = R * (R - 1) / 2;
     nb.pair_stride = nb.P0 > R ? nb.P0 : R;
-    size_t off = 0;
-    auto take = [&](size_t bytes) { char* p = base ? base + off : nullptr; off += aup(bytes); return p; };
-    const size_t pool = (size_t)B * S * C * D * sizeof(float);
-    nb.X = X_in_ws ? (float*)take(pool) : nullptr;
-    nb.Y = (float*)take(pool);
-    nb.K = (float*)take(pool);
-    nb.kap = (float*)take((size_t)B * S * nb.nCT * sizeof(float));
-    nb.alpha_part = (float*)take((size_t)B * PAIR_CHUNK * nb.nAP * nb.RP * sizeof(float));
-    nb.alpha = (float*)take((size_t)B * PAIR_CHUNK * nb.RP * sizeof(float));
-    nb.score_part = (float*)take((size_t)B * PAIR_CHUNK * nb.nSB * sizeof(float));
-    nb.new_scores = (float*)take((size_t)B * nb.pair_stride * sizeof(float));
-    nb.logits[0] = (float*)take((size_t)B * nb.P0 * sizeof(float));
-    nb.logits[1] = (float*)take((size_t)B * nb.P0 * sizeof(float));
-    nb.newx = need_newx ? (float*)take((size_t)B * C * D * sizeof(float)) : nullptr;
-    nb.slot[0] = (int32_t*)take((size_t)B * S * sizeof(int32_t));
-    nb.slot[1] = (int32_t*)take((size_t)B * S * sizeof(int32_t));
-    nb.free_slot = (int32_t*)take((size_t)B * sizeof(int32_t));
-    nb.new_slot = (int32_t*)take((size_t)B * sizeof(int32_t));
-    nb.pair_i = (int32_t*)take((size_t)B * nb.pair_stride * sizeof(int32_t));
-    nb.pair_j = (int32_t*)take((size_t)B * nb.pair_stride * sizeof(int32_t));
+    WsCarver c(base);
+    const size_t pool = (size_t)B * S * C * D;
+    nb.X = X_in_ws ? c.take<float>(pool) : nullptr;
+    nb.Y = c.take<float>(pool);
+    nb.K = c.take<float>(pool);
+    nb.kap = c.take<float>((size_t)B * S * nb.nCT);
+    nb.alpha_part = c.take<float>((size_t)B * PAIR_CHUNK * nb.nAP * nb.RP);
+    nb.alpha = c.take<float>((size_t)B * PAIR_CHUNK * nb.RP);
+    nb.score_part = c.take<float>((size_t)B * PAIR_CHUNK * nb.nSB);
+    nb.new_scores = c.take<float>((size_t)B * nb.pair_stride);
+    nb.logits[0] = c.take<float>((size_t)B * nb.P0);
+    nb.logits[1] = c.take<float>((size_t)B * nb.P0);
+    nb.newx = need_newx ? c.take<float>((size_t)B * C * D) : nullptr;
+    nb.slot[0] = c.take<int32_t>((size_t)B * S);
+    nb.slot[1] = c.take<int32_t>((size_t)B * S);
+    nb.free_slot = c.take<int32_t>(B);
+    nb.new_slot = c.take<int32_t>(B);
+    nb.pair_i = c.take<int32_t>((size_t)B * nb.pair_stride);
+    nb.pair_j = c.take<int32_t>((size_t)B * nb.pair_stride);
     nb.tc = tc; nb.big = big; nb.pc = big ? BIG_PAIRS : TC_PAIRS;
-    if (tc) {
-        const size_t xp = (size_t)B * nb.pc * C * D * 4, np = (size_t)B * C * S * D * 2;
-        nb.xf = (float*)take(xp); nb.nodes_h = take(2 * np); nb.nodes_l = take(2 * np); nb.kp_h = take(np); nb.kp_l = take(np);
-        if (big) { nb.xh = take(xp / 2); nb.xl = take(xp / 2); }
+    if (tc) {                 // bf16 planes as 16-bit words
+        const size_t xp = (size_t)B * nb.pc * C * D, np = (size_t)B * C * S * D;
+        nb.xf = c.take<float>(xp); nb.nodes_h = c.take<uint16_t>(2 * np); nb.nodes_l = c.take<uint16_t>(2 * np); nb.kp_h = c.take<uint16_t>(np);
+        nb.kp_l = c.take<uint16_t>(np);
+        if (big) { nb.xh = c.take<uint16_t>(xp); nb.xl = c.take<uint16_t>(xp); }
     }
-    nb.total = off + 256;
+    nb.total = c.off + 256;
     return nb;
 }
-
-static inline char* ws_align(void* ws) { return reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(ws) + 255) / 256 * 256); }
 
 static size_t smem_score(int Rp) { return (2 * 4096 + 2 * TILE_ROWS * LDA + 128 + 64 + ((Rp + 3) & ~3) + (size_t)Rp * 32) * sizeof(float); }
 static size_t smem_merge(int Rp) { return (2 * TILE_ROWS * LDA + 4096 + 128 + 2 * ((Rp + 3) & ~3) + 8) * sizeof(float); }

@@ -155,14 +155,21 @@ __global__ void __launch_bounds__(RL_THREADS) k_rank_final(const double* __restr
     if (tid == 0) { out[0] = (float)(s_loss[0] / T); out[1] = (float)(s_prec[0] / s_cnt[0]); }
 }
 
-inline size_t up256(size_t v) { return (v + 255) & ~(size_t)255; }
+struct RankLossBuffers { int32_t* set_count; double* part; int32_t* widest; size_t total; };
+RankLossBuffers rank_loss_layout(char* base, int B, int R) {
+    const size_t T = (size_t)R - 2;
+    WsCarver c(base);
+    RankLossBuffers w;
+    w.set_count = c.take<int32_t>((size_t)B * T);
+    w.part = c.take<double>((size_t)B * T * 3);
+    w.widest = c.take<int32_t>(T);
+    w.total = c.off + 256;
+    return w;
+}
 
 }  // namespace
 
-size_t rank_loss_ws_bytes(int B, int R) {
-    const size_t T = (size_t)R - 2;
-    return up256((size_t)B * T * sizeof(int32_t)) + up256((size_t)B * T * 3 * sizeof(double)) + up256(T * sizeof(int32_t)) + 256;
-}
+size_t rank_loss_ws_bytes(int B, int R) { return rank_loss_layout(nullptr, B, R).total; }
 
 int run_rank_loss(const float* logits_trace, const uint8_t* in_set, int B, int R, float margin, double ratio, float* out, void* ws, size_t ws_bytes,
                   cudaStream_t st) {
@@ -171,10 +178,9 @@ int run_rank_loss(const float* logits_trace, const uint8_t* in_set, int B, int R
     if (!(ratio > 0.0) || !(ratio <= 1.0)) return set_error(NNJ_ERR_INVALID, "rank_loss: ratio must be in (0, 1]");
     if (ws_bytes < rank_loss_ws_bytes(B, R)) return set_error(NNJ_ERR_WORKSPACE, "rank_loss: workspace too small (nnj_rank_loss_workspace_bytes)");
     const int T = R - 2;
-    char* base = reinterpret_cast<char*>(((uintptr_t)ws + 255) & ~(uintptr_t)255);
-    int32_t* set_count = reinterpret_cast<int32_t*>(base);
-    double* part = reinterpret_cast<double*>(base + up256((size_t)B * T * sizeof(int32_t)));
-    int32_t* widest = reinterpret_cast<int32_t*>(reinterpret_cast<char*>(part) + up256((size_t)B * T * 3 * sizeof(double)));
+    const RankLossBuffers w = rank_loss_layout(ws_align(ws), B, R);
+    int32_t *set_count = w.set_count, *widest = w.widest;
+    double* part = w.part;
     {
         cudaError_t e = cudaMemsetAsync(widest, 0, (size_t)T * sizeof(int32_t), st);
         if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);

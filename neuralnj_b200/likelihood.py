@@ -38,6 +38,9 @@ BRLEN_MIN, BRLEN_MAX = 1e-6, 100.0     # every length is clamped to this range, 
 PLACEHOLDER = 0.12345                  # environment.py:287 prints missing lengths like this; treated as "no length"
 RATE_LO, RATE_HI, ALPHA_LO, ALPHA_HI, PINV_HI = 1e-3, 1e3, 0.02, 100.0, 0.99
 _GOLD = 0.3819660112501051
+# the packed model the kernels read, [B, LLH_MODEL] doubles: its slots as in nnj_llh.cuh (MDL_*)
+LLH_MODEL = 64
+MDL_LAM, MDL_U, MDL_UINV, MDL_FREQ, MDL_RATE, MDL_PINV, MDL_ALPHA, MDL_FLAGS, MDL_GTR = 0, 4, 20, 36, 40, 44, 45, 46, 48
 _IUPAC = {"A": 1, "C": 2, "G": 4, "T": 8, "U": 8, "R": 5, "Y": 10, "S": 6, "W": 9, "K": 12, "M": 3, "B": 14, "D": 13, "H": 11, "V": 7}
 
 
@@ -105,7 +108,7 @@ class SubstModel:
         return p
 
     def pack(self) -> np.ndarray:
-        """[B, 64] doubles for the kernels: eigenvalues 4 | U 16 | U^-1 16 | freqs 4 | class rates 4 | p_inv | alpha | flags | pad | 6 rates | pad 10."""
+        """[B, LLH_MODEL] doubles for the kernels: eigenvalues, U, U^-1, freqs, class rates, p_inv, alpha, flags, the 6 GTR rates (MDL_*)."""
         B, pi = self.B, self.freqs
         r = np.zeros((B, 4, 4))
         for k, (a, b) in enumerate(itertools.combinations(range(4), 2)):
@@ -131,13 +134,16 @@ class SubstModel:
                     _lib.check(L.nnj_gamma_rates(a, 4, buf), "nnj_gamma_rates")
                     cache[a] = np.array(buf[:])
                 cat[b] = cache[a]
-        flags = np.full((B, 1), float((1 if self.gtr else 0) | (2 if self.gamma else 0) | (4 if self.inv else 0)))
-        return np.ascontiguousarray(np.concatenate([lam, U.reshape(B, 16), Ui.reshape(B, 16), pi, cat, self.pinv[:, None], self.alpha[:, None], flags,
-                                                    np.zeros((B, 1)), self.rates, np.zeros((B, 10))], axis=1))
+        out = np.zeros((B, LLH_MODEL))
+        out[:, MDL_LAM:MDL_LAM + 4], out[:, MDL_U:MDL_U + 16], out[:, MDL_UINV:MDL_UINV + 16] = lam, U.reshape(B, 16), Ui.reshape(B, 16)
+        out[:, MDL_FREQ:MDL_FREQ + 4], out[:, MDL_RATE:MDL_RATE + 4] = pi, cat
+        out[:, MDL_PINV], out[:, MDL_ALPHA], out[:, MDL_GTR:MDL_GTR + 6] = self.pinv, self.alpha, self.rates
+        out[:, MDL_FLAGS] = float((1 if self.gtr else 0) | (2 if self.gamma else 0) | (4 if self.inv else 0))
+        return out
 
     def unpack(self, packed: np.ndarray) -> None:
         """Take the parameters the kernel optimised (nnj_llh_optimize_all) back into this object."""
-        self.pinv, self.alpha, self.rates = packed[:, 44].copy(), packed[:, 45].copy(), packed[:, 48:54].copy()
+        self.pinv, self.alpha, self.rates = packed[:, MDL_PINV].copy(), packed[:, MDL_ALPHA].copy(), packed[:, MDL_GTR:MDL_GTR + 6].copy()
 
 
 # ------------------------------------------------------------------ trees
@@ -314,38 +320,42 @@ class TreeLikelihood:
         if self.R < 3:
             raise ValueError("need at least 3 taxa")
         self.weights = np.ones(self.masks.shape[:-2] + (self.L,)) if weights is None else np.ascontiguousarray(weights, dtype=np.float64)
-        self._dev = {}
+        self._staged_B, self._staged_tw = None, None      # the device tips and weights of the last tree count
         self._ws = None
 
     def _staged(self, B: int):
-        key = B
-        if key not in self._dev:
+        if self._staged_B != B:
             m = torch.from_numpy(self.masks)
             w = torch.from_numpy(self.weights)
             if self.shared:
                 m, w = m.unsqueeze(0).expand(B, -1, -1), w.unsqueeze(0).expand(B, -1)
             elif m.shape[0] != B:
                 raise ValueError(f"{m.shape[0]} alignments but {B} trees")
-            self._dev = {key: (m.contiguous().to(self.device), w.contiguous().to(self.device))}
-        return self._dev[key]
+            self._staged_B, self._staged_tw = B, (m.contiguous().to(self.device), w.contiguous().to(self.device))
+        return self._staged_tw
 
-    def _workspace(self, B: int):
-        need = int(_lib.lib().nnj_llh_workspace_bytes(B, self.R, self.L))
+    def _workspace(self, need: int, what: str):
+        """The grow-only device workspace, at least `need` bytes (what the library's `what` returned; < 0: a shape it refuses)."""
         if need < 0:
-            raise _lib.NnjError("nnj_llh_workspace_bytes: bad shape")
+            raise _lib.NnjError(f"{what}: bad shape")
         if self._ws is None or self._ws.numel() < need:
             self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
         return self._ws
 
-    def _call(self, mode: str, children, brlen, model: SubstModel, max_passes=32, eps=1e-3, lh_eps=1.0, max_rounds=10):
-        """One C-ABI call over all B trees: mode "eval" (nnj_llh_eval), "brlen" (nnj_llh_optimize_brlen) or "all" (nnj_llh_optimize_all)."""
+    def _trees(self, children, brlen, model: SubstModel):
+        """-> children int32 [B, R-1, 2], a copy of brlen float64 [B, 2R-2], B; one model row per tree."""
         children = np.ascontiguousarray(children, dtype=np.int32)
         B = children.shape[0]
         brlen = np.ascontiguousarray(brlen, dtype=np.float64).copy()
         if children.shape != (B, self.R - 1, 2) or brlen.shape != (B, 2 * self.R - 2) or model.B != B:
             raise ValueError("children must be [B, R-1, 2], brlen [B, 2R-2], one model row per tree")
+        return children, brlen, B
+
+    def _call(self, mode: str, children, brlen, model: SubstModel, max_passes=32, eps=1e-3, lh_eps=1.0, max_rounds=10):
+        """One C-ABI call over all B trees: mode "eval" (nnj_llh_eval), "brlen" (nnj_llh_optimize_brlen) or "all" (nnj_llh_optimize_all)."""
+        children, brlen, B = self._trees(children, brlen, model)
         tips, w = self._staged(B)
-        ws = self._workspace(B)
+        ws = self._workspace(int(_lib.lib().nnj_llh_workspace_bytes(B, self.R, self.L)), "nnj_llh_workspace_bytes")
         packed = model.pack()
         L = _lib.lib()
         after, before = np.zeros(B), np.zeros(B)
@@ -385,22 +395,14 @@ class TreeLikelihood:
         model, which should be optimised already (optimize_all).  -> dict of numpy arrays: branch_node [B, R-3], llh [B, R-3, 3]
         (L0, L1, L2), nni_brlen [B, R-3, 2, 5], sh_count and lbp_count [B, R-3] over replicates rep0 .. rep0+n_rell-1, and with
         site_llh=True the per-pattern log-likelihoods [B, R-3, 3, L] as a device tensor."""
-        children = np.ascontiguousarray(children, dtype=np.int32)
-        B, R, L = children.shape[0], self.R, self.L
-        brlen = np.ascontiguousarray(brlen, dtype=np.float64)
-        if children.shape != (B, R - 1, 2) or brlen.shape != (B, 2 * R - 2) or model.B != B:
-            raise ValueError("children must be [B, R-1, 2], brlen [B, 2R-2], one model row per tree")
+        children, brlen, B = self._trees(children, brlen, model)
+        R, L = self.R, self.L
         if not 0 <= int(seed) < 2 ** 64 or int(rep0) < 0 or int(n_rell) < 0:
             raise ValueError("need 0 <= seed < 2^64, rep0 >= 0, n_rell >= 0")
         nb = max(R - 3, 0)
         tips, w = self._staged(B)
         lib = _lib.lib()
-        need = int(lib.nnj_llh_support_workspace_bytes(B, R, L, int(n_rell)))
-        if need < 0:
-            raise _lib.NnjError("nnj_llh_support_workspace_bytes: bad shape")
-        if self._ws is None or self._ws.numel() < need:
-            self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
-        ws = self._ws
+        ws = self._workspace(int(lib.nnj_llh_support_workspace_bytes(B, R, L, int(n_rell))), "nnj_llh_support_workspace_bytes")
         packed = model.pack()
         out = dict(branch_node=np.zeros((B, nb), dtype=np.int32), llh=np.zeros((B, nb, 3)), nni_brlen=np.zeros((B, nb, 2, 5)),
                    sh_count=np.zeros((B, nb), dtype=np.int32), lbp_count=np.zeros((B, nb), dtype=np.int32))

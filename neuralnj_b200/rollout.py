@@ -26,7 +26,7 @@ from .config import empty_config
 from .environment import PhyInferEnv
 from .model import PhyloATTN
 from .phydata import load_pi_instance
-from .support import _support
+from .support import _support, likelihood_support
 from .treeutil import normalized_rf, rf_distance
 
 EXPLORE_TEMPERTURE = lambda step: 1.0   # finetune_rl_search.py:39
@@ -203,18 +203,16 @@ def Argmax_inference(test_file_path, write_dir, write_file_name=None, branch_opt
     written = []
 
     def write_support(file, msa, tree):
+        runs = []                     # (labelled trees it writes, the support computation)
         if alrt > 0:
-            from .support import likelihood_support
-            res = likelihood_support(msa, policy, tree=tree, n_rell=alrt, seed=alrt_seed)
-            for kind in ("alrt", "abayes"):
+            runs.append((("alrt", "abayes"), lambda: likelihood_support(msa, policy, tree=tree, n_rell=alrt, seed=alrt_seed)))
+        if bootstrap > 0:             # no replicate sharding: the file is this rank's
+            runs.append((("fbp", "tbe"), lambda: _support(msa, policy, bootstrap, bootstrap_seed, tree, None)))
+        for kinds, run in runs:
+            res = run()
+            for kind in kinds:
                 with open(os.path.join(write_dir, f"{file[:-4]}.{kind}.tre"), "w") as f:
                     f.write(res["newick_" + kind])
-        if bootstrap <= 0:
-            return
-        res = _support(msa, policy, bootstrap, bootstrap_seed, tree, None)     # no replicate sharding: the file is this rank's
-        for kind in ("fbp", "tbe"):
-            with open(os.path.join(write_dir, f"{file[:-4]}.{kind}.tre"), "w") as f:
-                f.write(res["newick_" + kind])
 
     if files_per_call <= 1:
         for file in files:

@@ -112,16 +112,21 @@ def internal_clades(newick: str, keys) -> List[Tuple[int, frozenset]]:
     return out
 
 
+def light_side(clade: frozenset, keys) -> frozenset:
+    """The side of the split a clade defines that names a split: the smaller one, on a tie the one whose sorted taxon names come first."""
+    rest = frozenset(range(len(keys))) - clade
+    return min(clade, rest, key=lambda t: (len(t), sorted(keys[i] for i in t)))
+
+
 def reference_splits(newick: str, keys):
     """Non-trivial splits of `newick`: (light sides as leaf-index frozensets in order of first appearance, split index of each
     labelled node as (offset, split))."""
     R = len(keys)
-    everything = frozenset(range(R))
     splits, where, labelled = [], {}, []
     for pos, clade in internal_clades(newick, keys):
         if not 2 <= len(clade) <= R - 2:
             continue
-        light = min(clade, everything - clade, key=lambda t: (len(t), sorted(keys[i] for i in t)))
+        light = light_side(clade, keys)
         if light not in where:                   # the two root children of a rooted binary tree are one split
             where[light] = len(splits)
             splits.append(light)
@@ -173,15 +178,36 @@ def bootstrap_support(msa, policy_network, n_replicates: int, seed: int = 0, tre
     return _support(msa, policy_network, n_replicates, seed, tree, _process_group())
 
 
-def _support(msa, policy_network, n_replicates: int, seed: int, tree: Optional[str], group) -> dict:
-    if int(n_replicates) < 1:
-        raise ValueError("n_replicates must be >= 1")
+def _count_and_seed(n: int, what: str, seed: int) -> Tuple[int, int]:
+    if int(n) < 1:
+        raise ValueError(f"{what} must be >= 1")
     if not 0 <= int(seed) < 2 ** 64:
         raise ValueError("seed must be in [0, 2^64)")
-    N, seed = int(n_replicates), int(seed)
+    return int(n), int(seed)
+
+
+def _one_alignment(msa, caller: str) -> dict:
+    """A path (.phy / .fasta / .aln) or a `load_pi_instance` batch -> the batch, which must hold one alignment."""
     batch = load_pi_instance(os.fspath(msa)) if isinstance(msa, (str, os.PathLike)) else msa
     if batch["data"].shape[0] != 1:
-        raise ValueError("bootstrap_support takes one alignment")
+        raise ValueError(f"{caller} takes one alignment")
+    return batch
+
+
+def _argmax_tree(policy_network, batch: dict, data: torch.Tensor, mask: torch.Tensor) -> str:
+    """Unrooted Newick of the Argmax rollout of one alignment (data int8 [R, L, 4] and the padding mask [L] on the network's device),
+    as `Argmax_inference` writes it."""
+    with torch.no_grad():
+        merges, _, _ = policy_network.rollout_fused(data[None], mask[None])
+    env = PhyInferEnv(empty_config(), data.device)
+    env.init_states(batch["seqs"], batch["seq_keys"], batch["data"])
+    env.replay_merges(merges)
+    return env.states[0].subtrees[0].utree_op_str
+
+
+def _support(msa, policy_network, n_replicates: int, seed: int, tree: Optional[str], group) -> dict:
+    N, seed = _count_and_seed(n_replicates, "n_replicates", seed)
+    batch = _one_alignment(msa, "bootstrap_support")
     R, L = batch["data"].shape[1:3]
     if R > MAX_TAXA:
         raise ValueError(f"bootstrap_support: {R} taxa, at most {MAX_TAXA} are supported: every replicate is an Argmax rollout, and the "
@@ -195,12 +221,7 @@ def _support(msa, policy_network, n_replicates: int, seed: int, tree: Optional[s
     data = batch["data"][0].to(device=device, dtype=torch.int8).contiguous()
     mask = padded.to(device)
     if tree is None:
-        with torch.no_grad():
-            merges, _, _ = policy_network.rollout_fused(data[None], mask[None])
-        env = PhyInferEnv(empty_config(), device)
-        env.init_states(batch["seqs"], batch["seq_keys"], batch["data"])
-        env.replay_merges(merges)
-        tree = env.states[0].subtrees[0].utree_op_str
+        tree = _argmax_tree(policy_network, batch, data, mask)
     splits, labelled = reference_splits(tree, keys)
     S = len(splits)
     splits_dev = split_bitsets(splits, R).to(device)
@@ -253,14 +274,8 @@ def likelihood_support(msa, policy_network=None, tree: Optional[str] = None, n_r
     where an NNI has the higher likelihood, delta < 0), `newick_alrt` (SH-aLRT, %.1f) and `newick_abayes` (%.3f), `n_rell`, `seed`."""
     from . import likelihood as LH
     from .treeutil import treestr_to_tuples
-    if int(n_rell) < 1:
-        raise ValueError("n_rell must be >= 1")
-    if not 0 <= int(seed) < 2 ** 64:
-        raise ValueError("seed must be in [0, 2^64)")
-    N, seed = int(n_rell), int(seed)
-    batch = load_pi_instance(os.fspath(msa)) if isinstance(msa, (str, os.PathLike)) else msa
-    if batch["data"].shape[0] != 1:
-        raise ValueError("likelihood_support takes one alignment")
+    N, seed = _count_and_seed(n_rell, "n_rell", seed)
+    batch = _one_alignment(msa, "likelihood_support")
     R = batch["data"].shape[1]
     if R > 4096:
         raise ValueError(f"likelihood_support: {R} taxa, the tree likelihood supports at most 4096")
@@ -271,12 +286,7 @@ def likelihood_support(msa, policy_network=None, tree: Optional[str] = None, n_r
             raise ValueError("likelihood_support: tree=None needs a policy_network to build the Argmax tree")
         device = next(policy_network.parameters()).device
         data = batch["data"][0].to(device=device, dtype=torch.int8).contiguous()
-        with torch.no_grad():
-            merges, _, _ = policy_network.rollout_fused(data[None], torch.from_numpy(~real).to(device)[None])
-        env = PhyInferEnv(empty_config(), device)
-        env.init_states(batch["seqs"], batch["seq_keys"], batch["data"])
-        env.replay_merges(merges)
-        tree = env.states[0].subtrees[0].utree_op_str
+        tree = _argmax_tree(policy_network, batch, data, torch.from_numpy(~real).to(device))
     else:
         device = next(policy_network.parameters()).device if policy_network is not None else torch.device("cuda")
     masks = LH.onehot_to_masks(batch["data"][0])[:, real]
@@ -291,15 +301,16 @@ def likelihood_support(msa, policy_network=None, tree: Optional[str] = None, n_r
     splits, labelled = reference_splits(out_tree, keys)
     S = len(splits)
     where = {sp: k for k, sp in enumerate(splits)}
-    everything = frozenset(range(R))
     order = np.zeros(S, dtype=np.int64)
     nodes = res["branch_node"][0]
     if len(nodes) != S:
         raise NnjError(f"likelihood_support: {len(nodes)} internal branches but {S} splits in the tree")
-    for i, v in enumerate(nodes.tolist()):
-        clade = frozenset(_leaves_below(children, int(v)))
-        light = min(clade, everything - clade, key=lambda x: (len(x), sorted(keys[j] for j in x)))
-        order[where[light]] = i
+    branch = {v: i for i, v in enumerate(nodes.tolist())}
+    below = [frozenset([i]) for i in range(R)] + [None] * (R - 1)      # leaves below each node; a child's set goes once joined
+    for k, (a, b) in enumerate(children.tolist()):
+        below[R + k], below[a], below[b] = below[a] | below[b], None, None
+        if R + k in branch:
+            order[where[light_side(below[R + k], keys)]] = branch[R + k]
     llh3 = res["llh"][0][order]
     delta = llh3[:, 0] - np.maximum(llh3[:, 1], llh3[:, 2])
     with np.errstate(over="ignore"):
@@ -311,14 +322,3 @@ def likelihood_support(msa, policy_network=None, tree: Optional[str] = None, n_r
                 newick_alrt=label_newick(out_tree, labelled, [f"{x:.1f}" for x in sh]),
                 newick_abayes=label_newick(out_tree, labelled, [f"{x:.3f}" for x in abayes]), n_rell=N, seed=seed)
 
-
-def _leaves_below(children, v: int) -> List[int]:
-    R = len(children) + 1
-    out, stack = [], [v]
-    while stack:
-        x = stack.pop()
-        if x < R:
-            out.append(x)
-        else:
-            stack.extend(int(c) for c in children[x - R])
-    return out

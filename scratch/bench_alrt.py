@@ -5,7 +5,7 @@ in the same run.
 
 Shapes: 50 taxa x 1024 patterns at B = 1 and B = 64, 200 x 4096 at B = 1; N = 1000 RELL replicates; simulated data, random trees,
 GTR+I+G with fixed parameters.  Per shape: the whole call (CUDA events, after one warm-up call of the same shape), its three stages
-from torch.profiler kernel times in a separate profiled call (prepare = k_llh mode 3, NNI = k_llh_nni, RELL = k_rell_counts + k_rell),
+from torch.profiler kernel times in a separate profiled call (prepare = llh_prepare's k_llh launch, NNI = k_llh_nni, RELL = k_rell_counts + k_rell),
 and beside them optimize_all and optimize_branches of the same trees.  Also the numpy oracle (oracle/alrt_oracle.py) on one
 50-taxon tree, on the host CPU."""
 import argparse
