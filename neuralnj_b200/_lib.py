@@ -10,7 +10,7 @@ import sys
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libnnj.so")
-SOURCES = ["nnj_api.cu", "nnj_encoder.cu", "nnj_encoder_tc.cu", "nnj_njloop.cu", "nnj_tc.cu", "nnj_score_tc.cu", "nnj_alpha_tc.cu", "nnj_score_big.cu", "nnj_llh.cu", "nnj_score_small.cu", "nnj_alpha_small.cu", "nnj_rankloss.cu", "nnj_support.cu", "nnj_llh_nni.cu"]
+SOURCES = ["nnj_api.cu", "nnj_encoder.cu", "nnj_encoder_tc.cu", "nnj_njloop.cu", "nnj_tc.cu", "nnj_score_tc.cu", "nnj_score_inc.cu", "nnj_alpha_tc.cu", "nnj_score_big.cu", "nnj_llh.cu", "nnj_score_small.cu", "nnj_alpha_small.cu", "nnj_rankloss.cu", "nnj_support.cu", "nnj_llh_nni.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared", "-cudart", "static"]
 

@@ -185,7 +185,7 @@ struct PairChunk {
 int launch_alpha_v3(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st);        // nnj_alpha_tc.cu
 int launch_alpha_small(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st);     // nnj_alpha_small.cu
 int launch_score_tc(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st);        // nnj_score_tc.cu
-int launch_score_inc(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st);       // nnj_score_tc.cu
+int launch_score_inc(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st);       // nnj_score_inc.cu
 int launch_score_small(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st);     // nnj_score_small.cu
 int launch_score_big(const Model* m, const PairChunk& c, int* n_part, cudaStream_t st);       // nnj_score_big.cu
 int launch_blend_planes(const Model* m, const PairChunk& c, cudaStream_t st);                 // nnj_score_big.cu: x planes, fp32 and bf16

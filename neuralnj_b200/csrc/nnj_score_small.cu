@@ -5,7 +5,7 @@
 //     x'           = x + sigmoid(g + b_g) (x_glob - x)                  gate
 //     s            = x' W_s^T                                           GEMM 2, K = 64
 //     score[p]    += w2 . GELU(s + b_s) + b2 over unmasked sites
-// k_score_inc puts pairs on TMEM lanes: a work item costs the same ~2 950 clocks whether a tree has 32 live pairs or 2
+// The round-2 k_score_inc put pairs on TMEM lanes: a work item cost the same ~2 950 clocks whether a tree has 32 live pairs or 2
 // (profiles/r02_ncu_launches: 715 us per launch of 128 trees at n = 2, 770 us at n = 32), because a tcgen05 tile is 128 rows and
 // every epilogue instruction is a full warp.  With 16 rows the natural tile is the 16 x 8 x 16 register-fragment instruction
 // (mma.sync, 8 clocks per sub-partition, scratch/hmma_bench.cu): one warp owns one site at a time, the alpha operand of the tree

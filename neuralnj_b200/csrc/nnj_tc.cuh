@@ -303,6 +303,9 @@ __device__ __forceinline__ void tmem_ld8_nw(uint32_t taddr, uint32_t (&v)[8]) {
                  : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
                  : "r"(taddr));
 }
+__device__ __forceinline__ void tmem_ld4_nw(uint32_t taddr, uint32_t (&v)[4]) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]) : "r"(taddr));
+}
 __device__ __forceinline__ void tmem_st4(uint32_t taddr, uint32_t v0, uint32_t v1, uint32_t v2, uint32_t v3) {
     asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1,%2,%3,%4};" ::"r"(taddr), "r"(v0), "r"(v1), "r"(v2), "r"(v3) : "memory");
 }
