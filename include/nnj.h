@@ -197,6 +197,29 @@ int nnj_llh_branch_support(const uint8_t* tips_dev, const double* weights_dev, c
                            const double* model_host, int B, int R, int L, uint64_t seed, int64_t rep0, int n_rell,
                            int32_t* branch_node_host, double* llh_host, double* nni_brlen_host, int32_t* sh_count_host,
                            int32_t* lbp_count_host, double* site_llh_dev, void* ws_dev, int64_t ws_bytes, void* stream);
+/* Tree topology test over K candidate trees of one alignment (IQ-TREE -z trees -zb n_boot -au, CONSEL; DESIGN.md 13).  Each tree is
+ * scored at its own lengths and model (fit them first, e.g. with nnj_llh_optimize_all): l_k[p] is its per-pattern log-likelihood and
+ * L_k = sum_p w[p] l_k[p] (pattern order, a multiply then an add); k* is the largest L_k, the lowest index on a tie.  Scales
+ * s = 0..9, r_s = (5 + s) / 10, draw n_s = floor(r_s n + 0.5) sites per replicate (n = sum of the weights); draw i of replicate j
+ * is the site u = (x0 * n) >> 32, x0 = word 0 of Philox4x32-10 with counter (i, j & 0xffffffff, j >> 32, s + 1) and key
+ * (seed & 0xffffffff, seed >> 32); pattern p takes the sites cum[p] <= u < cum[p+1].  T_s[j][k] = sum_p c_{s,j}[p] l_k[p] in pattern
+ * order, a multiply then an add.  2 <= K <= 1024, 4 <= R <= 4096, 1 <= n_boot <= 10^6 (others: NNJ_ERR_INVALID).
+ *   tips_dev       uint8  [R,L]      the one alignment's state masks, shared by every tree
+ *   weights_dev    double [L]        pattern weights: non-negative integers, 0 < n < 2^31
+ *   children_host  int32  [K,R-1,2]  the trees in join order; brlen_host double [K,2R-2], model_host double [K,64] as nnj_llh_eval
+ *   llh_host       double [K]        L_k
+ *   win_host       int32  [10,K]     win[s][k]: replicates of scale s whose largest T_s[j][.] is tree k's (every tied tree counts)
+ *   kh_host        int32  [K]        replicates with a_{j,k*} - a_{j,k} >= L_k* - L_k, a_{j,k} = T_5[j][k] - m_k, m_k = (sum_j T_5[j][k]) / n_boot
+ *   sh_host        int32  [K]        replicates with max_k' a_{j,k'} - a_{j,k} >= L_k* - L_k
+ *   elw_host       double [K]        (sum_j q_{j,k}) / n_boot, q_{j,k} = e_k / sum_k' e_k' (k order), e_k = exp(T_5[j][k] - max_k' T_5[j][k'])
+ *   site_llh_dev   double [K,L]      l_k[p] (device; may be NULL)
+ * The sums over j run in replicate order.  Bad weights, an invalid tree: NNJ_ERR_INVALID; a workspace smaller than
+ * nnj_llh_topotest_workspace_bytes(K, R, L, n_boot): NNJ_ERR_WORKSPACE.  Synchronises `stream`. */
+int64_t nnj_llh_topotest_workspace_bytes(int K, int R, int L, int n_boot);
+int nnj_llh_topology_test(const uint8_t* tips_dev, const double* weights_dev, const int32_t* children_host, const double* brlen_host,
+                          const double* model_host, int K, int R, int L, uint64_t seed, int n_boot,
+                          double* llh_host, int32_t* win_host, int32_t* kh_host, int32_t* sh_host, double* elw_host,
+                          double* site_llh_dev, void* ws_dev, int64_t ws_bytes, void* stream);
 /* Mean rates of the ncat equal-probability classes of Gamma(alpha, alpha) (Yang 1994): rates_host double [ncat]. */
 int nnj_gamma_rates(double alpha, int ncat, double* rates_host);
 

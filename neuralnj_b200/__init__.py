@@ -14,9 +14,10 @@ from .rollout import (Agmax_one_instance, Argmax_inference, RL_Search, Search_in
 from .treeutil import rf_distance, treestr_to_tuples   # noqa: F401
 from .likelihood import compute_llh, optimize_brlen          # noqa: F401
 from .supervise import balanced_elu_loss, supervise_rollout   # noqa: F401
-from .support import bootstrap_support, likelihood_support                       # noqa: F401
+from .support import bootstrap_support, likelihood_support, topology_test        # noqa: F401
 
 __all__ = ["PhyloATTN", "PhyInferEnv", "PhyloTree", "reinforce_rollout", "Agmax_one_instance", "Argmax_inference",
            "RL_Search", "Search_inference", "load_pi_instance", "empty_config", "inference_config", "CfgNode",
            "rf_distance", "treestr_to_tuples", "format_rtree", "build", "lib", "NnjError", "optimize_brlen", "compute_llh",
-           "supervise_rollout", "balanced_elu_loss", "bootstrap_support", "likelihood_support"]
+           "supervise_rollout", "balanced_elu_loss", "bootstrap_support", "likelihood_support",
+           "topology_test"]

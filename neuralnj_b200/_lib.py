@@ -10,7 +10,7 @@ import sys
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libnnj.so")
-SOURCES = ["nnj_api.cu", "nnj_encoder.cu", "nnj_encoder_tc.cu", "nnj_njloop.cu", "nnj_tc.cu", "nnj_score_tc.cu", "nnj_score_inc.cu", "nnj_alpha_tc.cu", "nnj_score_big.cu", "nnj_llh.cu", "nnj_score_small.cu", "nnj_alpha_small.cu", "nnj_rankloss.cu", "nnj_support.cu", "nnj_llh_nni.cu"]
+SOURCES = ["nnj_api.cu", "nnj_encoder.cu", "nnj_encoder_tc.cu", "nnj_njloop.cu", "nnj_tc.cu", "nnj_score_tc.cu", "nnj_score_inc.cu", "nnj_alpha_tc.cu", "nnj_score_big.cu", "nnj_llh.cu", "nnj_score_small.cu", "nnj_alpha_small.cu", "nnj_rankloss.cu", "nnj_support.cu", "nnj_llh_nni.cu", "nnj_llh_topo.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared", "-cudart", "static"]
 
@@ -19,7 +19,7 @@ EXPORTS = ["nnj_last_error", "nnj_abi_version", "nnj_model_create", "nnj_model_d
            "nnj_merge", "nnj_rollout", "nnj_rollout_from_state", "nnj_rollout_host", "nnj_launch_count",
            "nnj_profile_enable", "nnj_profile_classes", "nnj_profile_name", "nnj_profile_read", "nnj_gemm_split_bf16", "nnj_tc_selftest",
            "nnj_llh_workspace_bytes", "nnj_llh_eval", "nnj_llh_optimize_brlen", "nnj_llh_optimize_all", "nnj_gamma_rates",
-           "nnj_llh_support_workspace_bytes", "nnj_llh_branch_support",
+           "nnj_llh_support_workspace_bytes", "nnj_llh_branch_support", "nnj_llh_topotest_workspace_bytes", "nnj_llh_topology_test",
            "nnj_rank_loss_workspace_bytes", "nnj_rank_loss",
            "nnj_bootstrap_columns", "nnj_split_distances"]
 
@@ -185,6 +185,10 @@ def lib() -> C.CDLL:
     L.nnj_llh_support_workspace_bytes.restype = i64
     L.nnj_llh_branch_support.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, C.c_uint64, i64, i32, vp, vp, vp, vp, vp, vp, vp, i64, vp]
     L.nnj_llh_branch_support.restype = i32
+    L.nnj_llh_topotest_workspace_bytes.argtypes = [i32, i32, i32, i32]
+    L.nnj_llh_topotest_workspace_bytes.restype = i64
+    L.nnj_llh_topology_test.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, C.c_uint64, i32, vp, vp, vp, vp, vp, vp, vp, i64, vp]
+    L.nnj_llh_topology_test.restype = i32
     L.nnj_gamma_rates.argtypes = [C.c_double, i32, dp]
     L.nnj_gamma_rates.restype = i32
     L.nnj_rank_loss_workspace_bytes.argtypes = [i32, i32]

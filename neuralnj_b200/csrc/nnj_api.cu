@@ -455,6 +455,21 @@ int nnj_llh_branch_support(const uint8_t* tips, const double* weights, const int
                            (cudaStream_t)stream);
 }
 
+static bool topo_shape_ok(int K, int R, int L, int n_boot) { return K >= 2 && K <= 1024 && R >= 4 && R <= 4096 && L >= 1 && n_boot >= 1 && n_boot <= 1000000; }
+
+int64_t nnj_llh_topotest_workspace_bytes(int K, int R, int L, int n_boot) {
+    return topo_shape_ok(K, R, L, n_boot) ? (int64_t)llh_topo_ws_bytes(K, R, L, n_boot) : -1;
+}
+
+int nnj_llh_topology_test(const uint8_t* tips, const double* weights, const int32_t* children_h, const double* brlen_h, const double* model_h, int K, int R,
+                          int L, uint64_t seed, int n_boot, double* llh_h, int32_t* win_h, int32_t* kh_h, int32_t* sh_h, double* elw_h, double* site_llh_dev,
+                          void* ws, int64_t ws_bytes, void* stream) {
+    CHECK_ARGS(tips && weights && children_h && brlen_h && model_h && llh_h && win_h && kh_h && sh_h && elw_h && ws && topo_shape_ok(K, R, L, n_boot),
+               "llh_topology_test: bad arguments (2 <= K <= 1024, 4 <= R <= 4096, 1 <= n_boot <= 10^6)");
+    return run_llh_topo(tips, weights, children_h, brlen_h, model_h, K, R, L, seed, n_boot, llh_h, win_h, kh_h, sh_h, elw_h, site_llh_dev, ws,
+                        (size_t)ws_bytes, (cudaStream_t)stream);
+}
+
 int nnj_gamma_rates(double alpha, int ncat, double* rates_h) {
     CHECK_ARGS(rates_h, "gamma_rates: bad arguments");
     return gamma_rates(alpha, ncat, rates_h);

@@ -251,6 +251,11 @@ LlhPrepared llh_prepare(const LlhTrees& in, double* site_dev, double* llh_h, voi
 size_t llh_support_ws_bytes(int B, int R, int L, int n_rell);
 int run_llh_support(const LlhTrees& in, uint64_t seed, int64_t rep0, int n_rell, int32_t* branch_node_h, double* llh_h, double* nni_brlen_h,
                     int32_t* sh_h, int32_t* lbp_h, double* site_dev, void* ws, size_t ws_bytes, cudaStream_t st);
+// tree topology test over K trees of one alignment (nnj_llh_topo.cu): tips [R][L] and weights [L] on the device, the trees on the host
+size_t llh_topo_ws_bytes(int K, int R, int L, int n_boot);
+int run_llh_topo(const uint8_t* tips, const double* weights, const int32_t* children_h, const double* brlen_h, const double* model_h, int K, int R,
+                 int L, uint64_t seed, int n_boot, double* llh_h, int32_t* win_h, int32_t* kh_h, int32_t* sh_h, double* elw_h, double* site_dev,
+                 void* ws, size_t ws_bytes, cudaStream_t st);
 int gamma_rates(double alpha, int ncat, double* out);
 
 // pre-training loss over a teacher-forced rollout's logits trace (nnj_rankloss.cu)

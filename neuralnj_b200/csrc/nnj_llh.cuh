@@ -1,8 +1,10 @@
-// nnj_llh.cuh — device helpers of the tree likelihood shared by k_llh (nnj_llh.cu) and the NNI quartet kernel (nnj_llh_nni.cu).
+// nnj_llh.cuh — device helpers of the tree likelihood shared by k_llh (nnj_llh.cu), the NNI quartet kernel (nnj_llh_nni.cu) and the
+// RELL draws of branch support and the topology test (nnj_llh_nni.cu, nnj_llh_topo.cu).
 // Everything is fp64; CLVs are [4 rate classes][4 states] per (node, pattern), scaled by 2^256 as described in nnj_llh.cu.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "nnj_common.cuh"
 
 namespace nnj {
 
@@ -184,6 +186,31 @@ __device__ __forceinline__ double newton_brlen(const double* St, const int32_t* 
         if (done) break;
     }
     return tv;
+}
+
+// RELL replicate counts, shared by branch support (nnj_llh_nni.cu) and the topology test (nnj_llh_topo.cu).  cum [B][L+1] holds each
+// tree's cumulative pattern weights, n_b = cum[L] its site count.  Replicate rep0 + r makes `draws` draws (0: n_b of its tree); draw i
+// is the site u = (x0 * n_b) >> 32, x0 = word 0 of Philox4x32-10 with counter (i, r lo, r hi, w3) and key (seed lo, seed hi), and
+// cnt[b][p][r] += 1 for the pattern p with cum[p] <= u < cum[p + 1].  Grid: x over draws, y over (tree, replicate).
+constexpr int RELL_THREADS = 256;
+static __global__ void __launch_bounds__(RELL_THREADS) k_rell_counts(const uint32_t* __restrict__ cum, int B, int L, uint64_t seed, int64_t rep0, int nr,
+                                                                     uint32_t draws, uint32_t w3, int32_t* __restrict__ cnt) {
+    const uint32_t i = blockIdx.x * RELL_THREADS + threadIdx.x;
+    for (int y = blockIdx.y; y < B * nr; y += gridDim.y) {
+        const int b = y / nr, rl = y - b * nr;
+        const uint32_t* cb = cum + (size_t)b * (L + 1);
+        const uint32_t n = cb[L];
+        if (i >= (draws ? draws : n)) continue;
+        const uint64_t r = (uint64_t)rep0 + (uint64_t)rl;
+        const uint32_t x0 = philox_x0(i, (uint32_t)r, (uint32_t)(r >> 32), w3, (uint32_t)seed, (uint32_t)(seed >> 32));
+        const uint32_t u = (uint32_t)(((uint64_t)x0 * (uint64_t)n) >> 32);
+        int lo = 0, hi = L;                                   // cb[lo] <= u < cb[hi]
+        while (hi - lo > 1) {
+            const int mid = (lo + hi) >> 1;
+            if (__ldg(cb + mid) <= u) lo = mid; else hi = mid;
+        }
+        atomicAdd(cnt + ((size_t)b * L + lo) * nr + rl, 1);
+    }
 }
 
 }  // namespace nnj

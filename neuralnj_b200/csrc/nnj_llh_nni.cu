@@ -23,7 +23,6 @@ constexpr int NNI_MAX_ROUNDS = 8;
 constexpr double NNI_EPS = 1e-3;
 constexpr double SH_TOL = 0.05;
 constexpr int RELL_CHUNK = 256;          // replicates per pass of the two RELL kernels (the counts c[b][p][r] live in the workspace)
-constexpr int RELL_THREADS = 256;
 
 struct NniArgs {
     const uint8_t* tips;        // [B][R][L]
@@ -135,27 +134,6 @@ __global__ void __launch_bounds__(LLH_THREADS) k_llh_nni(const NniArgs a) {
     if (alt == 0) {
         double* s0 = a.site + (size_t)bi * 3 * L;
         for (int s = tid; s < L; s += LLH_THREADS) s0[s] = a.site0[(size_t)b * L + s];
-    }
-}
-
-// cnt[b][p][r] += 1 for every draw i < n_b of replicate rep0 + r: pattern p with cum[p] <= u < cum[p + 1], u = (x0 * n_b) >> 32
-__global__ void __launch_bounds__(RELL_THREADS) k_rell_counts(const uint32_t* __restrict__ cum, int B, int L, uint64_t seed, int64_t rep0, int nr,
-                                                              int32_t* __restrict__ cnt) {
-    const uint32_t i = blockIdx.x * RELL_THREADS + threadIdx.x;
-    for (int y = blockIdx.y; y < B * nr; y += gridDim.y) {
-        const int b = y / nr, rl = y - b * nr;
-        const uint32_t* cb = cum + (size_t)b * (L + 1);
-        const uint32_t n = cb[L];
-        if (i >= n) continue;
-        const uint64_t r = (uint64_t)rep0 + (uint64_t)rl;
-        const uint32_t x0 = philox_x0(i, (uint32_t)r, (uint32_t)(r >> 32), 0u, (uint32_t)seed, (uint32_t)(seed >> 32));
-        const uint32_t u = (uint32_t)(((uint64_t)x0 * (uint64_t)n) >> 32);
-        int lo = 0, hi = L;                                   // cb[lo] <= u < cb[hi]
-        while (hi - lo > 1) {
-            const int mid = (lo + hi) >> 1;
-            if (__ldg(cb + mid) <= u) lo = mid; else hi = mid;
-        }
-        atomicAdd(cnt + ((size_t)b * L + lo) * nr + rl, 1);
     }
 }
 
@@ -299,7 +277,7 @@ int run_llh_support(const LlhTrees& in, uint64_t seed, int64_t rep0, int n_rell,
         if (e != cudaSuccess) return set_cuda_error(e, __FILE__, __LINE__);
         const dim3 grid((nmax + RELL_THREADS - 1) / RELL_THREADS, B * nr < 65535 ? B * nr : 65535);
         prof_begin(KC_LLH, st);
-        k_rell_counts<<<grid, RELL_THREADS, 0, st>>>(sw.cum, B, L, seed, rep0 + r0, nr, sw.cnt);
+        k_rell_counts<<<grid, RELL_THREADS, 0, st>>>(sw.cum, B, L, seed, rep0 + r0, nr, 0u, 0u, sw.cnt);
         ++g_launches; prof_end(st);
         const size_t threads = (size_t)B * nb * nr;
         prof_begin(KC_LLH, st);

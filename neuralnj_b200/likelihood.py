@@ -419,6 +419,41 @@ class TreeLikelihood:
             out["site_llh"] = site if site is not None else torch.empty((B, 0, 3, L), dtype=torch.float64, device=self.device)
         return out
 
+    def topology_test(self, children, brlen, model: SubstModel, n_boot: int, seed: int, site_llh: bool = False) -> dict:
+        """Tree topology test over the K trees (nnj_llh_topology_test, DESIGN.md 13) at the given lengths and models, which should be
+        optimised already (optimize_all).  Needs the shared-alignment form (masks [R, L]).  -> dict of numpy arrays: llh [K] (L_k),
+        win [10, K] (winner counts per scale), kh, sh [K] (KH / SH counts) and elw [K], over n_boot replicates per scale drawn with
+        `seed`; with site_llh=True the per-pattern log-likelihoods [K, L] as a device tensor."""
+        if not self.shared:
+            raise ValueError("topology_test compares trees of one alignment: construct TreeLikelihood with masks [R, L]")
+        children, brlen, K = self._trees(children, brlen, model)
+        R, L = self.R, self.L
+        if K < 2:
+            raise ValueError("topology_test needs at least two trees")
+        if R > 4096:
+            raise ValueError(f"topology_test: {R} taxa, the tree likelihood supports at most 4096")
+        if not 0 <= int(seed) < 2 ** 64 or not 1 <= int(n_boot) <= 10 ** 6:
+            raise ValueError("need 0 <= seed < 2^64 and 1 <= n_boot <= 10^6")
+        tips = torch.from_numpy(self.masks).to(self.device)
+        w = torch.from_numpy(self.weights).to(self.device)
+        lib = _lib.lib()
+        ws = self._workspace(int(lib.nnj_llh_topotest_workspace_bytes(K, R, L, int(n_boot))), "nnj_llh_topotest_workspace_bytes")
+        packed = model.pack()
+        out = dict(llh=np.zeros(K), win=np.zeros((10, K), dtype=np.int32), kh=np.zeros(K, dtype=np.int32), sh=np.zeros(K, dtype=np.int32),
+                   elw=np.zeros(K))
+        site = torch.empty((K, L), dtype=torch.float64, device=self.device) if site_llh else None
+        vp = C.c_void_p
+        ptr = [out[k].ctypes.data_as(vp) for k in ("llh", "win", "kh", "sh", "elw")]
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream(self.device).cuda_stream
+            rc = lib.nnj_llh_topology_test(vp(tips.data_ptr()), vp(w.data_ptr()), children.ctypes.data_as(vp), brlen.ctypes.data_as(vp),
+                                           packed.ctypes.data_as(vp), K, R, L, C.c_uint64(int(seed)), int(n_boot), *ptr,
+                                           vp(site.data_ptr() if site is not None else 0), vp(ws.data_ptr()), ws.numel(), vp(stream))
+        _lib.check(rc, "nnj_llh_topology_test")
+        if site_llh:
+            out["site_llh"] = site
+        return out
+
 
 # ------------------------------------------------------------------ raxmlpy-compatible entry points
 def _prepare(tree_str: str, msa: dict, model: str):

@@ -246,7 +246,7 @@ def Argmax_inference(test_file_path, write_dir, write_file_name=None, branch_opt
 
 
 def RL_Search(cfgs, MSA_file, policy_network, env, c_best_tree_file=None, raw_tree_file=None, scorer=None, stop_step=None,
-              generator: Optional[torch.Generator] = None):
+              generator: Optional[torch.Generator] = None, topotest_top: int = 20):
     """NeuralNJ-MC: sampled rollouts, keep the best-scoring tree (finetune_rl_search.py:338-427).
 
     One encoder pass is shared by every sampled rollout (the reference re-encodes the same MSA each time, :112), the
@@ -255,6 +255,9 @@ def RL_Search(cfgs, MSA_file, policy_network, env, c_best_tree_file=None, raw_tr
     environment.py:365-379) - here on the GPU (`neuralnj_b200.likelihood.score_topologies`), all new topologies of an
     episode in one call.  `scorer` overrides it: a callable `scorer(newick, seq_keys, seqs) -> float`, or "logp" to rank by
     the policy's own trajectory log-probability (no likelihood at all).
+
+    Beside the reference's keys the result holds `candidates` (not a reference key): the up to `topotest_top` distinct topologies
+    with the highest scores as (score, Newick) pairs, best first, ties in the order first seen - the input of a tree topology test.
     """
     from . import likelihood as LH
     from .environment import EVOLUTION_MODEL
@@ -305,23 +308,43 @@ def RL_Search(cfgs, MSA_file, policy_network, env, c_best_tree_file=None, raw_tr
             if step_cur >= stop:
                 break
     rel_rf = normalized_rf(raw_tree_str, best_tree) if raw_tree_str else None
+    values = list(seen.values())                                          # in the order first seen
+    order = sorted(range(len(values)), key=lambda i: (-values[i][0], i))
     return dict(the_best_tree=best_tree, the_best_score=best_score, raw_tree_score=None, c_best_tree_score=None,
-                time_when_best_score_max=t_best, relative_rf_distance=rel_rf, step_cur=step_cur, distinct_topologies=len(seen))
+                time_when_best_score_max=t_best, relative_rf_distance=rel_rf, step_cur=step_cur, distinct_topologies=len(seen),
+                candidates=[values[i] for i in order[:max(int(topotest_top), 0)]])
 
 
-def Search_inference(test_file_path, write_dir, write_file_name=None, cfgs=None, device=None, scorer=None, stop_step=None, precision=None):
+def Search_inference(test_file_path, write_dir, write_file_name=None, cfgs=None, device=None, scorer=None, stop_step=None, precision=None,
+                     policy_network=None, topotest=0, topotest_top=20, topotest_seed=0):
+    """One `.tre` per `.phy` of a directory: the best tree of RL_Search (finetune_rl_search.py:512-541).
+
+    `topotest=N` (not a reference argument) also writes, for an alignment with at least two distinct candidate topologies,
+    `<name>.trees` (the up to `topotest_top` best-scoring candidates, one Newick per line, best first) and `<name>.topotest.txt`
+    (IQ-TREE's tree test table of those trees from N RELL replicates per scale drawn with `topotest_seed`,
+    `neuralnj_b200.support.topology_test`).  The `.tre` is the same with and without it."""
+    from .environment import EVOLUTION_MODEL
+    from .support import topology_test
     c = _cfg(cfgs)
     device = device or torch.device("cuda")
     env = PhyInferEnv(c, device)
-    policy = _load_policy(c, device, precision)
+    policy = policy_network if policy_network is not None else _load_policy(c, device, precision)
     os.makedirs(write_dir, exist_ok=True)
     written = []
     for file in sorted(f for f in os.listdir(test_file_path) if f.endswith(".phy")):
-        res = RL_Search(c, os.path.join(test_file_path, file), policy, env, scorer=scorer, stop_step=stop_step)
+        path = os.path.join(test_file_path, file)
+        res = RL_Search(c, path, policy, env, scorer=scorer, stop_step=stop_step, topotest_top=topotest_top)
         dst = os.path.join(write_dir, file[:-4] + ".tre")
         with open(dst, "w") as f:
             f.write(res["the_best_tree"])
         written.append(dst)
+        if topotest > 0 and len(res["candidates"]) >= 2:
+            trees = [newick for _, newick in res["candidates"]]
+            with open(os.path.join(write_dir, file[:-4] + ".trees"), "w") as f:
+                f.write("".join(t + "\n" for t in trees))
+            tt = topology_test(path, trees, n_boot=topotest, seed=topotest_seed, model=EVOLUTION_MODEL, device=device)
+            with open(os.path.join(write_dir, file[:-4] + ".topotest.txt"), "w") as f:
+                f.write(tt["table"])
         print(f"finish NerualNJ-MC for {file}")
     return written
 
@@ -346,11 +369,20 @@ def main(argv=None):
     ap.add_argument("--alrt", type=int, default=0,
                     help="Argmax: also write <name>.alrt.tre / <name>.abayes.tre with SH-aLRT from N RELL replicates and aBayes (not a reference flag)")
     ap.add_argument("--alrt_seed", type=int, default=0, help="seed of the RELL replicates (not a reference flag)")
+    ap.add_argument("--topotest", type=int, default=0,
+                    help="Search: also write <name>.trees / <name>.topotest.txt, a tree topology test (KH, SH, ELW, AU) of the best candidates "
+                         "from N RELL replicates per scale (not a reference flag)")
+    ap.add_argument("--topotest_top", type=int, default=20, help="Search: candidates the topology test compares, at least 2 (not a reference flag)")
+    ap.add_argument("--topotest_seed", type=int, default=0, help="seed of the topology test's replicates (not a reference flag)")
     args = ap.parse_args(argv)
     if args.bootstrap and args.infer_opt != "Argmax":
         raise SystemExit("--bootstrap applies to --infer_opt Argmax")
     if args.alrt and args.infer_opt != "Argmax":
         raise SystemExit("--alrt applies to --infer_opt Argmax")
+    if args.topotest and args.infer_opt != "Search":
+        raise SystemExit("--topotest applies to --infer_opt Search (pass the Argmax tree and its alternatives to support.topology_test)")
+    if args.topotest_top < 2:
+        raise SystemExit("--topotest_top must be at least 2: a topology test compares trees")
     PRECISION = args.precision
     cfgs = empty_config()
     if args.config_path:
@@ -362,7 +394,8 @@ def main(argv=None):
         return Argmax_inference(cfgs.instance_path, write_dir, None, branch_optimize=args.branch_optimize, files_per_call=args.files_per_call,
                                 bootstrap=args.bootstrap, bootstrap_seed=args.bootstrap_seed, alrt=args.alrt, alrt_seed=args.alrt_seed)
     if args.infer_opt == "Search":
-        return Search_inference(cfgs.instance_path, write_dir, None)
+        return Search_inference(cfgs.instance_path, write_dir, None, topotest=args.topotest, topotest_top=args.topotest_top,
+                                topotest_seed=args.topotest_seed)
     raise SystemExit(f'--infer_opt {args.infer_opt}: "Finetune" (NeuralNJ-RL) trains the policy and is outside this path')
 
 

@@ -322,3 +322,90 @@ def likelihood_support(msa, policy_network=None, tree: Optional[str] = None, n_r
                 newick_alrt=label_newick(out_tree, labelled, [f"{x:.1f}" for x in sh]),
                 newick_abayes=label_newick(out_tree, labelled, [f"{x:.3f}" for x in abayes]), n_rell=N, seed=seed)
 
+
+# ---------------------------------------------------------------------------------------------------------- tree topology tests
+
+TOPO_SCALES = 10       # multiscale bootstrap: r_s = (5 + s) / 10, s = 0..9; scale 5 (r = 1) is the RELL bootstrap of bp, KH, SH and ELW
+
+
+def scale_draws(n: int) -> List[int]:
+    """Sites drawn per replicate at each scale: n_s = floor(r_s n + 0.5), r_s = (5 + s) / 10 (the rule of nnj_llh_topology_test)."""
+    return [int(np.floor((5 + s) / 10 * n + 0.5)) for s in range(TOPO_SCALES)]
+
+
+def au_pvalue(win_s, n_s, n: int, N: int) -> float:
+    """Approximately unbiased p-value of one tree (Shimodaira 2002, first-order fit as in CONSEL): win_s [10] replicates of each scale
+    the tree wins, n_s [10] sites drawn at each scale, n the site count, N replicates per scale.  Over the scales with 0 < win_s < N,
+    z_s = Phi^-1(1 - bp_s) is fitted as v sqrt(r_s) + c / sqrt(r_s), r_s = n_s / n, by least squares weighted with
+    N phi(z_s)^2 / (bp_s (1 - bp_s)); p-AU = 1 - Phi(v - c).  With fewer than two such scales: bp at r = 1."""
+    from statistics import NormalDist
+    nd = NormalDist()
+    win_s = np.asarray(win_s, dtype=np.float64)
+    use = [s for s in range(len(win_s)) if 0 < win_s[s] < N]
+    if len(use) < 2:
+        return float(win_s[5] / N)
+    bp = win_s[use] / N
+    r = np.asarray(n_s, dtype=np.float64)[use] / n
+    z = np.array([nd.inv_cdf(1.0 - b) for b in bp])
+    sw = np.sqrt(N * np.array([nd.pdf(x) for x in z]) ** 2 / (bp * (1.0 - bp)))
+    (v, c), *_ = np.linalg.lstsq(np.stack([np.sqrt(r), 1.0 / np.sqrt(r)], 1) * sw[:, None], z * sw, rcond=None)
+    return 1.0 - nd.cdf(v - c)
+
+
+def _mark(p: float) -> str:
+    return "+" if p >= 0.05 else "-"
+
+
+def topology_table(llh, delta, bp, p_kh, p_sh, elw, p_au) -> str:
+    """IQ-TREE's tree test table: one row per tree in input order; + / - after a value marks value >= / < 0.05."""
+    head = f"{'Tree':>4} {'logL':>14} {'deltaL':>10} {'bp-RELL':>9} {'p-KH':>8} {'p-SH':>8} {'c-ELW':>9} {'p-AU':>9}"
+    rows = [head, "-" * len(head)]
+    for k in range(len(llh)):
+        rows.append(f"{k + 1:>4} {llh[k]:>14.4f} {delta[k]:>10.4f} {bp[k]:>7.4f} {_mark(bp[k])} {p_kh[k]:>6.4f} {_mark(p_kh[k])} "
+                    f"{p_sh[k]:>6.4f} {_mark(p_sh[k])} {elw[k]:>7.4f} {_mark(elw[k])} {p_au[k]:>7.4f} {_mark(p_au[k])}")
+    return "\n".join(rows) + "\n"
+
+
+def topology_test(msa, trees: List[str], n_boot: int = 10000, seed: int = 0, model: str = "GTR+I+G", device=None) -> dict:
+    """Tree topology test (DESIGN.md 13) of candidate trees of one alignment - what IQ-TREE reports with `-z trees -zb 10000 -au`:
+    bp-RELL, p-KH, p-SH, c-ELW and p-AU of every tree, which trees the data reject at the 5% level and which they cannot.
+
+    `msa` is a path or a `load_pi_instance` batch of one alignment, `trees` two or more Newick strings on its taxa (up to 4096).  Each
+    tree's branch lengths (starting from the given ones) and model parameters are optimised (`TreeLikelihood.optimize_all`), then
+    n_boot RELL replicates at each of 10 scales are drawn with `seed` and scored against every tree on the device
+    (`TreeLikelihood.topology_test`); the AU fit runs on the host (`au_pvalue`).
+
+    Returns, per tree in input order: `tree` (unrooted Newick with the fitted lengths), `llh`, `delta` (largest llh - llh), `bp`,
+    `p_kh`, `p_sh`, `elw`, `p_au` and `win` [K, 10] (replicates each scale's winner); and `table` (IQ-TREE's columns), `n_boot`, `seed`."""
+    from . import likelihood as LH
+    from .treeutil import treestr_to_tuples
+    N, seed = _count_and_seed(n_boot, "n_boot", seed)
+    if N > 10 ** 6:
+        raise ValueError("n_boot must be <= 10^6")
+    if len(trees) < 2:
+        raise ValueError("topology_test compares at least two trees")
+    batch = _one_alignment(msa, "topology_test")
+    R = batch["data"].shape[1]
+    if R > 4096:
+        raise ValueError(f"topology_test: {R} taxa, the tree likelihood supports at most 4096")
+    keys = [str(k) for k in batch["seq_keys"][0]]
+    real = (batch["seq_weights"][0] != 0).cpu().numpy()
+    masks = LH.onehot_to_masks(batch["data"][0])[:, real]
+    pats, w = LH.compress_patterns(masks)
+    arrays = [LH.tree_arrays_from_tuples(treestr_to_tuples(t), keys) for t in trees]
+    ch = np.stack([a[0] for a in arrays])
+    K = len(trees)
+    eng = LH.TreeLikelihood(pats, w, device=device)
+    sm = LH.SubstModel(model, LH.empirical_freqs(masks), K)
+    t, _, _ = eng.optimize_all(ch, np.stack([a[1] for a in arrays]), sm)
+    res = eng.topology_test(ch, t, sm, N, seed)
+    n = int(w.sum())
+    n_s = scale_draws(n)
+    llh = res["llh"]
+    delta = llh.max() - llh
+    bp, p_kh, p_sh, elw = res["win"][5] / N, res["kh"] / N, res["sh"] / N, res["elw"]
+    p_au = np.array([au_pvalue(res["win"][:, k], n_s, n, N) for k in range(K)])
+    return dict(tree=[LH.tuples_to_newick(LH.tuples_with_lengths(ch[k], t[k], keys, unrooted=True)) for k in range(K)], llh=llh, delta=delta,
+                bp=bp, p_kh=p_kh, p_sh=p_sh, elw=elw, p_au=p_au, win=res["win"].T.copy(),
+                table=topology_table(llh, delta, bp, p_kh, p_sh, elw, p_au), n_boot=N, seed=seed)
+
